@@ -16,6 +16,8 @@ against the library's default all-FP64 DMMA path, which is measured in the same 
 CUDA events liblmm records on its own compute stream around all device work of the call.
 `e2e`: the same call with pinned HOST buffers, H2D/D2H inside the timed region, wall clock between
 device-synchronised points.  Prints ONE JSON line on rank 0.
+`--dump-outputs DIR`: rank 0 writes what the last device-resident timed step returned as DIR/*.npy (see `dump_outputs`); the
+inputs depend on the arguments only, so two builds run with the same arguments can be compared file for file.
 """
 import argparse
 import json
@@ -259,6 +261,40 @@ def ncu_traffic_ozaki():
         return None
 
 
+DUMP_SAMPLES = 1 << 20
+
+
+def seeded_sample(a, k, seed):
+    """`a` itself if it has at most k entries, else k of its entries at positions drawn from a fixed seed."""
+    if a.size <= k:
+        return a
+    return np.ravel(a)[np.random.default_rng(seed).choice(a.size, size=k, replace=False)]
+
+
+def dump_outputs(path, post, lp, latents, N):
+    """What a caller of the timed path receives from one step, as float64 .npy files (at most 48 MB in all):
+    logpdf.npy   -- (1,) the log marginal likelihood;
+    alpha.npy    -- the posterior weights alpha_i = (K_i + noise_i I)^-1 delta_i, one row per latent in `latents` (at most 2^21
+                    values: a fixed, seeded sample of a larger array);
+    delta.npy    -- the projected observations delta_i the posterior holds, sampled the same way;
+    L_sample.npy -- (2, k) entries of the lower Cholesky factors of the first and of the last latent in `latents`, at the same
+                    2^20 seeded lower-triangle positions in both (a factor has N^2 entries)."""
+    os.makedirs(path, exist_ok=True)
+    lat = post.f.fs
+    np.save(os.path.join(path, "logpdf.npy"), np.array([lp], dtype=np.float64))
+    vec = np.array([lat[i]._export()[1:] for i in latents])  # (latents, 2, N): alpha, delta
+    np.save(os.path.join(path, "alpha.npy"), seeded_sample(vec[:, 0], 2 * DUMP_SAMPLES, 1))
+    np.save(os.path.join(path, "delta.npy"), seeded_sample(vec[:, 1], 2 * DUMP_SAMPLES, 2))
+    rng = np.random.default_rng(3)
+    k = min(DUMP_SAMPLES, N * (N + 1) // 2)
+    r, c = rng.integers(0, N, k), rng.integers(0, N, k)
+    rows, cols = np.maximum(r, c), np.minimum(r, c)
+    L_sample = np.empty((2, k))
+    for j, i in enumerate((latents[0], latents[-1])):
+        L_sample[j] = lat[i].C[rows, cols]
+    np.save(os.path.join(path, "L_sample.npy"), L_sample)
+
+
 def multi_gpu_extras(lmm, ctx, dist, torch, world, rank):
     """Driver-visible records of the two other multi-GPU paths of the north star, run by every rank AFTER the timed region
     (they are collective) and attached to rank 0's JSON line; neither touches `value`.
@@ -342,7 +378,13 @@ def main():
     ap.add_argument("--ozaki-bits", type=int, default=8, help="bits per digit plane: 7 = radix 128 (8 planes = 55 bits), 8 = radix 256 (7 planes = 54 bits)")
     ap.add_argument("--no-dmma", action="store_true", help="skip the untimed kernel-timing pass and the DMMA comparison (for runs under ncu)")
     ap.add_argument("--streams", type=int, default=0, help="latent groups on separate CUDA streams (0 = library default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/*.npy (float64, seeded samples of "
+                                                          "large arrays) for output-for-output comparison of two builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 implementation")
     p, m, N = args.p, args.m, args.N
     cfg = {"p": p, "m": m, "N": N,
            "config": {"workload": ("BASELINE config 4" if (p, m, N) == (64, 64, 16384) else "reduced shape (NOT the headline config)") + f": OILMM p={p} m={m} N={N} SEKernel (per-latent lengthscales), sigma2=0.1, "
@@ -394,10 +436,13 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def step(fx, yy):
+    def step(fx, yy, keep=None):
         post, lp = lmm.posterior(fx, yy, with_logpdf=True)
         tm = ctx.last_timings().copy()
-        post.f.fs[0]._owner.free()
+        if keep is not None:  # handed to the caller, which frees it
+            keep.append(post)
+        else:
+            post.f.fs[0]._owner.free()
         return lp, tm
 
     for _ in range(args.warmup):
@@ -409,14 +454,20 @@ def main():
         sampler.start()
     l0, h0, d0 = ctx.counters()
     ev_ms, chol_ms, kmat_ms, solve_ms, proj_ms = 0.0, 0.0, 0.0, 0.0, 0.0
+    kept = []  # the last step's posterior when its outputs are dumped
     t0 = time.perf_counter()
-    for _ in range(args.steps):
-        lp, tm = step(fx_dev, yd)
+    for k in range(args.steps):
+        lp, tm = step(fx_dev, yd, kept if args.dump_outputs and k == args.steps - 1 else None)
         ev_ms += tm[0]; kmat_ms += tm[1]; chol_ms += tm[2]; solve_ms += tm[3]; proj_ms += tm[4]
     barrier()
     wall_ms = (time.perf_counter() - t0) * 1e3
     clocks = sampler.stop() if rank == 0 else None
     l1, h1, d1 = ctx.counters()
+    if kept:
+        if rank == 0:
+            dump_outputs(args.dump_outputs, kept[0], lp, range(*lmm.dist.shard_range(m, world, rank)), N)
+        kept[0].f.fs[0]._owner.free()
+        barrier()
     # ---- timed: end to end from pinned host buffers (public API call, H2D + D2H inside)
     step(fx_host, yh_np)
     barrier()
