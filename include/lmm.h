@@ -230,6 +230,26 @@ int lmm_imogp_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* fs, int m, const doub
                           double* grad_latents, double* grad_ard, double* grad_sigma2, double* grad_y,
                           int* info_latent);
 
+/* The same rrules for every latent the value path accepts (KernelSum / KernelProduct of up to LMM_MAX_TERMS terms,
+ * PeriodicKernel, RationalQuadraticKernel), with the gradient w.r.t. the hyper-parameters of each term.  grad_terms
+ * (required) receives m x LMM_MAX_TERMS x LMM_GRAD_TERM_STRIDE doubles: term t of latent i starts at
+ * (i*LMM_MAX_TERMS + t)*LMM_GRAD_TERM_STRIDE and holds d/d variance, d/d inv_lengthscale, d/d param (α / r) and
+ * d/d ard[0..LMM_MAX_ARD); term 0 is the descriptor's own fields, terms 1.. are `extra[]`.  Slots of absent terms, the
+ * `param` slot of kinds without a shape parameter and the ARD slots of terms without an ARDTransform (or k >= D) are 0.
+ * grad_latents[:, 0:2] and grad_ard hold term 0's values (for single-kernel latents exactly what lmm_*_logpdf_grad
+ * returns), grad_latents[:, 2] the mean gradient; every other output is that of lmm_*_logpdf_grad.  With a communicator
+ * grad_terms is summed over the ranks like grad_ard. */
+#define LMM_GRAD_TERM_STRIDE (3 + LMM_MAX_ARD)
+int lmm_oilmm_logpdf_grad_terms(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N,
+                                int D, const double* U, const double* S, int p, double sigma2,
+                                const double* y, int out_dim, double* out_logpdf, double* grad_latents,
+                                double* grad_ard, double* grad_sigma2, double* grad_y, double* grad_U,
+                                double* grad_S, double* grad_terms, int* info_latent);
+int lmm_imogp_logpdf_grad_terms(lmm_ctx* ctx, const lmm_gp_desc* fs, int m, const double* x, int N, int D,
+                                double sigma2, const double* y, int out_dim, double* out_logpdf,
+                                double* grad_latents, double* grad_ard, double* grad_sigma2, double* grad_y,
+                                double* grad_terms, int* info_latent);
+
 /* ---- posterior handle: the OILMM/ILMM/IndependentMOGP whose latents are PosteriorGPs -------- */
 /* mean_and_var(post(x*, σ²))  src/oilmm.jl:57-76 on PosteriorGP latents (AbstractGPs posterior
  * mean/var); for an IndependentMOGP posterior: src/independent_mogp.jl:50-57; ILMM: src/ilmm.jl:122-129. */
@@ -345,6 +365,12 @@ int lmm_ilmm_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const 
                          const double* H, int p, double sigma2, const double* y, int out_dim,
                          double* out_logpdf, double* grad_latents, double* grad_ard, double* grad_sigma2,
                          double* grad_y, double* grad_H, int* info);
+/* The same for every latent the value path accepts, with per-term gradients in grad_terms (layout of
+ * lmm_oilmm_logpdf_grad_terms above). */
+int lmm_ilmm_logpdf_grad_terms(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D,
+                               const double* H, int p, double sigma2, const double* y, int out_dim,
+                               double* out_logpdf, double* grad_latents, double* grad_ard, double* grad_sigma2,
+                               double* grad_y, double* grad_H, double* grad_terms, int* info);
 
 /* Heterotopic / missing-data ILMM (SURVEY.md §8f-4; unsupported in the reference, examples/oilmm_and_ilmm.ipynb:112).
  * Entries of y (host memory) that are NaN are unobserved; exact inference on the observed entries of the dense model

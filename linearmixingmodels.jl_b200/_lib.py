@@ -13,6 +13,8 @@ LIB_PATH = os.path.join(_HERE, "liblmm.so")
 
 LMM_OK = 0
 LMM_E_ARG, LMM_E_OUT_DIM, LMM_E_UNSUPPORTED, LMM_E_CUDA, LMM_E_NCCL, LMM_E_NOT_ORTHOGONAL, LMM_E_OOM = -1, -2, -3, -4, -5, -6, -7
+LMM_MAX_TERMS, LMM_MAX_ARD = 4, 8
+LMM_GRAD_TERM_STRIDE = 3 + LMM_MAX_ARD  # per term: d/d variance, d/d inv_lengthscale, d/d param, d/d ard[0..8)
 
 
 class LibraryNotBuilt(ImportError):
@@ -81,6 +83,9 @@ SIGNATURES = {
     "lmm_oilmm_logpdf_sweep": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, C.c_int, _vp, C.c_int, _vp, _ip]),
     "lmm_oilmm_logpdf_grad": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _dp, _vp, _vp, _vp, _ip]),
     "lmm_imogp_logpdf_grad": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _dp, _vp, _ip]),
+    # per-term gradients of composite / periodic / rational-quadratic latents: grad_terms (m x 4 x 11) before the info pointer
+    "lmm_oilmm_logpdf_grad_terms": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _dp, _vp, _vp, _vp, _vp, _ip]),
+    "lmm_imogp_logpdf_grad_terms": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _dp, _vp, _vp, _ip]),
     "lmm_post_mean_and_var": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp]),
     "lmm_post_latent_mean_and_var": (C.c_int, [_vp, C.c_int, _vp, C.c_int, C.c_double, _vp, _vp]),
     "lmm_post_mean_and_cov": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp]),
@@ -105,6 +110,7 @@ SIGNATURES = {
     "lmm_ilmm_prior_mean_and_var": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, C.c_int, C.c_double, C.c_int, _vp, _vp]),
     "lmm_ilmm_rand": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, C.c_int, C.c_double, C.c_int, _vp, _vp, _vp, _ip]),
     "lmm_ilmm_logpdf_grad": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, C.c_int, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _dp, _vp, _vp, _ip]),
+    "lmm_ilmm_logpdf_grad_terms": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, C.c_int, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _dp, _vp, _vp, _vp, _ip]),
     "lmm_ilmm_masked_posterior": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, C.c_int, C.c_double, _vp, C.c_int, C.POINTER(_vp), _dp, _ip, _ip]),
     "lmm_oilmm_masked_posterior": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, C.c_int, C.POINTER(_vp), _dp, _ip, _ip]),
     "lmm_potrf_batched": (C.c_int, [_vp, _vp, C.c_int, C.c_int, _vp, _vp, _vp]),

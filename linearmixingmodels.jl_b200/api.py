@@ -1021,12 +1021,31 @@ def _rand_one(rng, fx: FiniteGP) -> np.ndarray:
     raise TypeError(f"rand not defined for FiniteGP of {type(f).__name__}")
 
 
-def logpdf_and_gradient(fx: FiniteGP, y, with_grad_y: bool = False):
+def _terms_grads(fs, gt: np.ndarray, D: int) -> list:
+    """grad_terms (m x LMM_MAX_TERMS x LMM_GRAD_TERM_STRIDE) -> per latent, one dict per term in Kernel.all_terms() order."""
+    out = []
+    for i, g in enumerate(fs):
+        k = (g.prior if isinstance(g, PosteriorGP) else g).kernel
+        rows = gt.reshape(len(fs), _lib.LMM_MAX_TERMS, _lib.LMM_GRAD_TERM_STRIDE)[i]
+        out.append([{"variance": float(r[0]), "inv_lengthscale": float(r[1]), "param": float(r[2]), "ard": r[3:3 + D].copy()}
+                    for r in rows[:len(k.all_terms())]])
+    return out
+
+
+def logpdf_and_gradient(fx: FiniteGP, y, with_grad_y: bool = False, kernel_terms: bool = False):
     """Value and gradient of `logpdf(fx, y)` for an OILMM, general ILMM or IndependentMOGP prior -- the pullback
     a ChainRulesCore `rrule` around the ccall returns (test/oilmm.jl:31-32, test/ilmm.jl:31 `gradient(logpdf, fx, y)`).
     A general ILMM returns "H" (p, m) instead of "U"/"S".
     Returns (logpdf, grads) with grads = {"variance": (m,), "inv_lengthscale": (m,), "mean_const": (m,),
-    "sigma2": float[, "y": (p*N,)][, "U": (p, m), "S": (m,) for an OILMM]}."""
+    "sigma2": float[, "y": (p*N,)][, "U": (p, m), "S": (m,) for an OILMM]}.
+
+    Composite (KernelSum / KernelProduct), PeriodicKernel and RationalQuadraticKernel latents need `kernel_terms=True`
+    (without it a composite latent raises ValueError).  It adds grads["terms"]: per latent, a list in `Kernel.all_terms()`
+    order of {"variance", "inv_lengthscale", "param" (α / r; 0 for kinds without one), "ard" (D,)} -- the gradient w.r.t.
+    each term's own hyper-parameters; "variance" / "inv_lengthscale" / "ard" then hold term 0's.  A transform shared by all
+    terms is a function of them: for `(k1 + k2) ∘ ScaleTransform(s)` each term carries s_t = s·c_t, so
+    d/ds = Σ_t (s_t / s)·terms[t]["inv_lengthscale"].  A posterior FiniteGP has no kernel gradient (only σ² and y*):
+    `kernel_terms=True` on one raises ValueError."""
     f = fx.f
     ctx = _ctx_of(fx)
     _require_by_outputs(fx)
@@ -1037,6 +1056,8 @@ def logpdf_and_gradient(fx: FiniteGP, y, with_grad_y: bool = False):
     gy = np.zeros(N * fx.x.out_dim) if with_grad_y else None
     owner = _post_owner(fx)
     if owner is not None:
+        if kernel_terms:
+            raise ValueError("kernel_terms: the posterior-predictive logpdf gradient covers σ² and y* only")
         # logpdf(post(x*, σ²), y*): gradient w.r.t. σ² and y* (test/oilmm.jl:32 `gradient(logpdf, po, y_test)`)
         if isinstance(f, ILMM) and f.H.shape[0] != fx.x.out_dim:
             raise RuntimeError("out dim of x != out dim of f.")
@@ -1053,14 +1074,26 @@ def logpdf_and_gradient(fx: FiniteGP, y, with_grad_y: bool = False):
         gU = np.zeros(H.shape, order="F")
         gS = np.zeros(m)
         ga = np.zeros((m, D))
-        rc = ctx.lib.lmm_oilmm_logpdf_grad(ctx.handle, _descs(lat.fs), m, ptr(pts), N, D, ptr(H.U), ptr(H.S), H.shape[0], fx.sigma2, ptr(yv),
-                                           fx.x.out_dim, C.byref(out), ptr(gl), ptr(ga), C.byref(gs2), ptr(gy), ptr(gU), ptr(gS), C.byref(il))
+        fs = lat.fs
+        args = (ctx.handle, _descs(fs), m, ptr(pts), N, D, ptr(H.U), ptr(H.S), H.shape[0], fx.sigma2, ptr(yv), fx.x.out_dim, C.byref(out),
+                ptr(gl), ptr(ga), C.byref(gs2), ptr(gy), ptr(gU), ptr(gS))
+        if kernel_terms:
+            gt = np.zeros(m * _lib.LMM_MAX_TERMS * _lib.LMM_GRAD_TERM_STRIDE)
+            rc = ctx.lib.lmm_oilmm_logpdf_grad_terms(*args, ptr(gt), C.byref(il))
+        else:
+            rc = ctx.lib.lmm_oilmm_logpdf_grad(*args, C.byref(il))
     elif isinstance(f, IndependentMOGP):
         m = len(f.fs)
         gl = np.zeros((m, 3))
         ga = np.zeros((m, D))
-        rc = ctx.lib.lmm_imogp_logpdf_grad(ctx.handle, _descs(f.fs), m, ptr(pts), N, D, fx.sigma2, ptr(yv), fx.x.out_dim, C.byref(out),
-                                           ptr(gl), ptr(ga), C.byref(gs2), ptr(gy), C.byref(il))
+        fs = f.fs
+        args = (ctx.handle, _descs(fs), m, ptr(pts), N, D, fx.sigma2, ptr(yv), fx.x.out_dim, C.byref(out), ptr(gl), ptr(ga), C.byref(gs2),
+                ptr(gy))
+        if kernel_terms:
+            gt = np.zeros(m * _lib.LMM_MAX_TERMS * _lib.LMM_GRAD_TERM_STRIDE)
+            rc = ctx.lib.lmm_imogp_logpdf_grad_terms(*args, ptr(gt), C.byref(il))
+        else:
+            rc = ctx.lib.lmm_imogp_logpdf_grad(*args, C.byref(il))
     elif isinstance(f, ILMM) and isinstance(f.f, IndependentMOGP):  # general mixing matrix, src/ilmm.jl:150-163
         lat = f.f
         m = len(lat.fs)
@@ -1068,11 +1101,18 @@ def logpdf_and_gradient(fx: FiniteGP, y, with_grad_y: bool = False):
         gl = np.zeros((m, 3))
         gH = np.zeros(Hm.shape, order="F")
         ga = np.zeros((m, D))
-        rc = ctx.lib.lmm_ilmm_logpdf_grad(ctx.handle, _descs(lat.fs), m, ptr(pts), N, D, ptr(Hm), Hm.shape[0], fx.sigma2, ptr(yv),
-                                          fx.x.out_dim, C.byref(out), ptr(gl), ptr(ga), C.byref(gs2), ptr(gy), ptr(gH), C.byref(il))
+        args = (ctx.handle, _descs(lat.fs), m, ptr(pts), N, D, ptr(Hm), Hm.shape[0], fx.sigma2, ptr(yv), fx.x.out_dim, C.byref(out), ptr(gl),
+                ptr(ga), C.byref(gs2), ptr(gy), ptr(gH))
+        if kernel_terms:
+            gt = np.zeros(m * _lib.LMM_MAX_TERMS * _lib.LMM_GRAD_TERM_STRIDE)
+            rc = ctx.lib.lmm_ilmm_logpdf_grad_terms(*args, ptr(gt), C.byref(il))
+        else:
+            rc = ctx.lib.lmm_ilmm_logpdf_grad(*args, C.byref(il))
         ctx.check(rc, il.value)
         grads = {"variance": gl[:, 0].copy(), "inv_lengthscale": gl[:, 1].copy(), "mean_const": gl[:, 2].copy(), "sigma2": gs2.value,
                  "H": np.ascontiguousarray(gH), "ard": ga}
+        if kernel_terms:
+            grads["terms"] = _terms_grads(lat.fs, gt, D)
         if with_grad_y:
             grads["y"] = gy
         return out.value, grads
@@ -1081,6 +1121,8 @@ def logpdf_and_gradient(fx: FiniteGP, y, with_grad_y: bool = False):
     ctx.check(rc, il.value)
     grads = {"variance": gl[:, 0].copy(), "inv_lengthscale": gl[:, 1].copy(), "mean_const": gl[:, 2].copy(), "sigma2": gs2.value,
              "ard": ga}  # (m, D): d/d ARDTransform multipliers, zeros for latents without one
+    if kernel_terms:
+        grads["terms"] = _terms_grads(fs, gt, D)
     if with_grad_y:
         grads["y"] = gy
     if isinstance(f, ILMM):

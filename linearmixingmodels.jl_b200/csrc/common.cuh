@@ -174,21 +174,10 @@ __device__ __forceinline__ double sqdist(const double* a, const double* b, int D
   return d2;
 }
 
-// One term of a kernel on RAW (unscaled) points a, b (D coordinates each): the term's own input scaling, its own pairwise
-// distance (Distances.jl form or direct differences; the PeriodicKernel's Sinus metric always works on differences), κ,
-// variance.  This is what KernelFunctions evaluates per component of a KernelSum / KernelProduct.
-__device__ __forceinline__ double term_value(int kind, int ard_dim, double variance, double inv_ls, double param, const double* ard,
-                                             const double* a, const double* b, int D, int form, bool same_point) {
-  if (same_point) return variance;  // d = 0 exactly on the diagonal (Distances.jl), κ(0) = 1 for every supported kernel
-  if (kind == 5) {  // PeriodicKernel(r): Sinus(r) metric = Σ (sinpi(a_k - b_k) / r)², κ = exp(-d/2)
-    double d = 0.0;
-    for (int k = 0; k < D; ++k) {
-      const double sc = ard_dim ? inv_ls * ard[k] : inv_ls;
-      const double sn = sinpi(sc * a[k] - sc * b[k]) / param;
-      d = fma(sn, sn, d);
-    }
-    return variance * exp_nonpos(-0.5 * d);
-  }
+// Squared distance of one (Sq)Euclidean term on RAW points a, b: the term's own input scaling, then the Distances.jl form
+// (form 0) or direct differences (form 1).  Shared by the value path (term_value) and the per-term gradient (grad.cu).
+__device__ __forceinline__ double term_sqdist(int ard_dim, double inv_ls, const double* ard, const double* a, const double* b, int D,
+                                              int form) {
   double d2;
   if (form == 0) {
     double sa = 0.0, sb = 0.0, dot = 0.0;
@@ -209,7 +198,25 @@ __device__ __forceinline__ double term_value(int kind, int ard_dim, double varia
       d2 = fma(df, df, d2);
     }
   }
-  return kappa_eval(kind, variance, d2, param);
+  return d2;
+}
+
+// One term of a kernel on RAW (unscaled) points a, b (D coordinates each): the term's own input scaling, its own pairwise
+// distance (Distances.jl form or direct differences; the PeriodicKernel's Sinus metric always works on differences), κ,
+// variance.  This is what KernelFunctions evaluates per component of a KernelSum / KernelProduct.
+__device__ __forceinline__ double term_value(int kind, int ard_dim, double variance, double inv_ls, double param, const double* ard,
+                                             const double* a, const double* b, int D, int form, bool same_point) {
+  if (same_point) return variance;  // d = 0 exactly on the diagonal (Distances.jl), κ(0) = 1 for every supported kernel
+  if (kind == 5) {  // PeriodicKernel(r): Sinus(r) metric = Σ (sinpi(a_k - b_k) / r)², κ = exp(-d/2)
+    double d = 0.0;
+    for (int k = 0; k < D; ++k) {
+      const double sc = ard_dim ? inv_ls * ard[k] : inv_ls;
+      const double sn = sinpi(sc * a[k] - sc * b[k]) / param;
+      d = fma(sn, sn, d);
+    }
+    return variance * exp_nonpos(-0.5 * d);
+  }
+  return kappa_eval(kind, variance, term_sqdist(ard_dim, inv_ls, ard, a, b, D, form), param);
 }
 // Value of a (possibly composite) latent kernel on raw points; gp points at global memory.
 __device__ __forceinline__ double kernel_value_raw(const LatentParams* gp, const double* a, const double* b, int D, int form, bool same_point) {

@@ -422,6 +422,217 @@ cudaError_t launch_kgrad_ard(cudaStream_t st, const double* mat_base, size_t mat
   return cudaGetLastError();
 }
 
+// ---- per-term gradient: every hyper-parameter of every term of a (possibly composite) latent --------------------------
+// Term t of a latent is the LatentParams' own fields (t = 0) or extra[t - 1].  For each term the kernel accumulates
+// <G, ∂K/∂θ> for θ = variance, inv_lengthscale s, param (α / r) and ard[k], over the lower triangle with off-diagonal
+// entries counted twice (as kgrad_kernel).  Points are staged RAW: every term applies its own scaling, as kernel_value_raw.
+
+// Per unit variance: κ, ∂κ/∂s, ∂κ/∂param and the ARD factor wa with ∂κ/∂ard_k = wa · ard_factor(k) / ard_k.
+// (Sq)Euclidean kinds: the d² of the value path (term_sqdist), ∂κ/∂s of kappa_and_ds, wa = (∂κ/∂s) s / d² (kgrad_ard_kernel).
+// PeriodicKernel(r), q = Σ_k sin²(π u_k) / r², κ = e^{-q/2}: ∂κ/∂s = wa Σ_k u_k sin(2π u_k) / s, ∂κ/∂r = κ q / r,
+// wa = -κ π / (2 r²).
+__device__ __forceinline__ void term_grad(const TermParams& q, const double* a, const double* b, int D, int form, double& kap,
+                                          double& ds, double& dp, double& wa) {
+  if (q.kind == 5) {
+    double qs = 0.0, us = 0.0;
+    for (int k = 0; k < D; ++k) {
+      const double sc = q.ard_dim ? q.inv_ls * q.ard[k] : q.inv_ls;
+      const double u = sc * a[k] - sc * b[k];
+      const double sn = sinpi(u) / q.param;
+      qs = fma(sn, sn, qs);
+      us = fma(u, sinpi(2.0 * u), us);
+    }
+    kap = exp_nonpos(-0.5 * qs);
+    wa = -kap * 1.5707963267948966 / (q.param * q.param);
+    ds = wa * us / q.inv_ls;
+    dp = kap * qs / q.param;
+    return;
+  }
+  const double d2 = term_sqdist(q.ard_dim, q.inv_ls, q.ard, a, b, D, form);
+  kappa_and_ds(q.kind, d2, 1.0 / q.inv_ls, kap, ds, q.param);
+  wa = d2 > 0.0 ? ds * q.inv_ls / d2 : 0.0;
+  dp = 0.0;
+  if (q.kind == 4) {  // RationalQuadraticKernel: ∂κ/∂α = κ (d² / (2α base) - log(base)), base = 1 + d²/(2α)
+    const double base = 1.0 + d2 / (2.0 * q.param);
+    dp = kap * (d2 / (2.0 * q.param * base) - log(base));
+  }
+}
+// u_k² ((Sq)Euclidean kinds) or u_k sin(2π u_k) (PeriodicKernel), u_k = s ard_k (a_k - b_k)
+__device__ __forceinline__ double ard_factor(const TermParams& q, const double* a, const double* b, int k) {
+  const double sc = q.inv_ls * q.ard[k];
+  const double u = sc * a[k] - sc * b[k];
+  return q.kind == 5 ? u * sinpi(2.0 * u) : u * u;
+}
+
+constexpr int GRAD_TERM_STRIDE = 3 + MAX_ARD;            // == LMM_GRAD_TERM_STRIDE
+constexpr int GRAD_TERM_SLOTS = MAX_TERMS * GRAD_TERM_STRIDE;
+
+// One lower-triangle chunk of one latent with NT terms; ARD: some term has an ARDTransform.  The per-thread sums are
+// reduced across each warp by shuffles and written to wsum[slot][warp] (fixed order, no atomics).
+template <int NT, bool ARD>
+__device__ __forceinline__ void kgrad_terms_body(const TermParams* tp, bool product, const double* __restrict__ base, int off,
+                                                 const double* xa, const double* xb, const double* aa, const double* ab, int I, int J,
+                                                 int N, int D, int form, double (*wsum)[8]) {
+  const int t = threadIdx.x;
+  double acc[NT][3], aca[ARD ? NT : 1][MAX_ARD];
+#pragma unroll
+  for (int u = 0; u < NT; ++u) {
+    acc[u][0] = acc[u][1] = acc[u][2] = 0.0;
+#pragma unroll
+    for (int k = 0; k < MAX_ARD; ++k) aca[ARD ? u : 0][k] = 0.0;
+  }
+  for (int e = t; e < TT; e += 256) {
+    const int c = ((e >> 9) << 2) + (e & 3), r = (e >> 2) & 127;
+    const int gr = I * TILE + r, gc = J * TILE + c;
+    if (gr >= N || gc >= N || gc > gr) continue;
+    const double G = 0.5 * (aa[r] * ab[c] + sym_get(base, off + gr, off + gc));
+    const double* pa = xa + (size_t)r * D;
+    const double* pb = xb + (size_t)c * D;
+    double kap[NT], ds[NT], dp[NT], wa[NT];
+    double w2;
+    if (gr == gc) {  // κ(0) = 1: only the variances have a derivative on the diagonal
+#pragma unroll
+      for (int u = 0; u < NT; ++u) { kap[u] = 1.0; ds[u] = dp[u] = wa[u] = 0.0; }
+      w2 = G;
+    } else {
+#pragma unroll
+      for (int u = 0; u < NT; ++u) term_grad(tp[u], pa, pb, D, form, kap[u], ds[u], dp[u], wa[u]);
+      w2 = 2.0 * G;
+    }
+    // weight of term u: 2G for a sum; 2G Π_{v≠u} k_v for a product, from prefix / suffix products (a term far from its
+    // own centre underflows to exactly 0, so K / k_u is no option)
+    double suf[NT + 1];
+    suf[NT] = 1.0;
+    if (product) {
+#pragma unroll
+      for (int u = NT - 1; u >= 0; --u) suf[u] = suf[u + 1] * (tp[u].variance * kap[u]);
+    }
+    double pre = 1.0;
+#pragma unroll
+    for (int u = 0; u < NT; ++u) {
+      const double w = product ? w2 * pre * suf[u + 1] : w2;
+      if (product) pre *= tp[u].variance * kap[u];
+      acc[u][0] = fma(w, kap[u], acc[u][0]);
+      acc[u][1] = fma(w, ds[u], acc[u][1]);
+      acc[u][2] = fma(w, dp[u], acc[u][2]);
+      if (ARD && tp[u].ard_dim && wa[u] != 0.0) {
+        const double wk = w * wa[u];
+#pragma unroll
+        for (int k = 0; k < MAX_ARD; ++k)
+          if (k < D) aca[ARD ? u : 0][k] = fma(wk, ard_factor(tp[u], pa, pb, k), aca[ARD ? u : 0][k]);
+      }
+    }
+  }
+  const int lane = t & 31, warp = t >> 5;
+#pragma unroll
+  for (int u = 0; u < NT; ++u) {
+#pragma unroll
+    for (int j = 0; j < (ARD ? GRAD_TERM_STRIDE : 3); ++j) {
+      double v = j < 3 ? acc[u][j] : aca[ARD ? u : 0][j - 3];
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+      if (lane == 0) wsum[u * GRAD_TERM_STRIDE + j][warp] = v;
+    }
+  }
+}
+
+// grid (chunks of the lower triangle, latents), storage as kgrad_ard_kernel.  partial[(lat*nchunks + chunk)*GRAD_TERM_SLOTS
+// + t*GRAD_TERM_STRIDE + {0, 1, 2, 3 + k}] = <G, ∂K/∂{variance_t, s_t, param_t, ard_t[k]}> of the chunk; unused slots 0.
+// NTMAX / ARDANY bound the terms and ARD use of the batch, so a batch of small kernels gets the registers it needs only.
+template <int NTMAX, bool ARDANY>
+__global__ void __launch_bounds__(256, (NTMAX <= 2 && !ARDANY) ? 2 : 1) kgrad_terms_kernel(const double* __restrict__ mat_base, size_t mat_batch_stride, int off_per_lat,
+                                                          const double* __restrict__ x, int N, int D,
+                                                          const LatentParams* __restrict__ params, const double* __restrict__ alpha,
+                                                          size_t alpha_stride, int form, double* __restrict__ partial) {
+  extern __shared__ __align__(16) double sm[];
+  double* xa = sm;  // raw points
+  double* xb = xa + TILE * D;
+  double* aa = xb + TILE * D;
+  double* ab = aa + TILE;
+  __shared__ TermParams tp[MAX_TERMS];
+  __shared__ double wsum[GRAD_TERM_SLOTS][8];
+  const int lat = blockIdx.y, tl = blockIdx.x, t = threadIdx.x;
+  const LatentParams* lp = params + lat;
+  int I = (int)((sqrt(8.0 * (double)tl + 1.0) - 1.0) * 0.5);
+  while ((size_t)(I + 1) * (I + 2) / 2 <= (size_t)tl) ++I;
+  while ((size_t)I * (I + 1) / 2 > (size_t)tl) --I;
+  const int J = tl - (int)((size_t)I * (I + 1) / 2);
+  const double* al = alpha + (size_t)lat * alpha_stride;
+  if (t == 0) {
+    tp[0].kind = lp->kind; tp[0].ard_dim = lp->ard_dim; tp[0].variance = lp->variance; tp[0].inv_ls = lp->inv_ls; tp[0].param = lp->param;
+    for (int k = 0; k < MAX_ARD; ++k) tp[0].ard[k] = lp->ard[k];
+  } else if (t < MAX_TERMS) {
+    tp[t] = lp->extra[t - 1];
+  }
+  for (int i = t; i < TILE * D; i += 256) {
+    const int ra = I * TILE + i / D, rb = J * TILE + i / D;
+    xa[i] = ra < N ? x[(size_t)ra * D + i % D] : 0.0;
+    xb[i] = rb < N ? x[(size_t)rb * D + i % D] : 0.0;
+  }
+  if (t < TILE) {
+    aa[t] = (I * TILE + t < N) ? al[I * TILE + t] : 0.0;
+    ab[t] = (J * TILE + t < N) ? al[J * TILE + t] : 0.0;
+  }
+  __syncthreads();
+  const int nterms = lp->nterms;
+  const bool product = lp->compose == 2;
+  bool ard = false;
+  for (int u = 0; u < nterms; ++u) ard |= tp[u].ard_dim > 0;
+  const double* base = mat_base + (size_t)lat * mat_batch_stride;
+  const int off = lat * off_per_lat;
+#define LMM_TERMS_CASE(n, a)                                                                           \
+  if constexpr (n <= NTMAX && (ARDANY || !a))                                                          \
+    if (nterms == n && ard == a) kgrad_terms_body<n, a>(tp, product, base, off, xa, xb, aa, ab, I, J, N, D, form, wsum);
+  LMM_TERMS_CASE(1, false) LMM_TERMS_CASE(1, true) LMM_TERMS_CASE(2, false) LMM_TERMS_CASE(2, true)
+  LMM_TERMS_CASE(3, false) LMM_TERMS_CASE(3, true) LMM_TERMS_CASE(4, false) LMM_TERMS_CASE(4, true)
+#undef LMM_TERMS_CASE
+  __syncthreads();
+  if (t < GRAD_TERM_SLOTS) {
+    const int u = t / GRAD_TERM_STRIDE, j = t % GRAD_TERM_STRIDE;
+    double s = 0.0;
+    if (u < nterms && (j < 3 || (ard && tp[u].ard_dim && j - 3 < D))) {
+      for (int w = 0; w < 8; ++w) s += wsum[t][w];
+      if (j >= 1) s *= tp[u].variance;  // ∂K/∂θ carries the term's variance (∂K/∂variance does not)
+      if (j >= 3) s /= tp[u].ard[j - 3];
+    }
+    partial[((size_t)lat * gridDim.x + tl) * GRAD_TERM_SLOTS + t] = s;
+  }
+}
+// out[lat*GRAD_TERM_SLOTS + slot] = Σ chunks (fixed order)
+__global__ void __launch_bounds__(256) kgrad_terms_finish_kernel(const double* __restrict__ partial, int nchunks, double* __restrict__ out) {
+  __shared__ double red[256];
+  const int lat = blockIdx.x, slot = blockIdx.y, t = threadIdx.x;
+  double s = 0.0;
+  for (int i = t; i < nchunks; i += 256) s += partial[((size_t)lat * nchunks + i) * GRAD_TERM_SLOTS + slot];
+  red[t] = s;
+  __syncthreads();
+  for (int w = 128; w > 0; w >>= 1) {
+    if (t < w) red[t] += red[t + w];
+    __syncthreads();
+  }
+  if (t == 0) out[(size_t)lat * GRAD_TERM_SLOTS + slot] = red[0];
+}
+cudaError_t launch_kgrad_terms(cudaStream_t st, const double* mat_base, size_t mat_batch_stride, int off_per_lat, const double* x, int N,
+                               int D, const LatentParams* params, int nlat, int max_terms, bool any_ard, const double* alpha, size_t alpha_stride,
+                               int form, double* partial, double* out) {
+  const size_t smem = (size_t)(2 * TILE * D + 2 * TILE) * sizeof(double);
+  const int ntn = (N + TILE - 1) / TILE;
+  const int nchunks = (int)sym_tiles(ntn);
+  dim3 grid((unsigned)nchunks, (unsigned)nlat);
+  auto kern = any_ard ? (max_terms <= 1 ? kgrad_terms_kernel<1, true> : max_terms == 2 ? kgrad_terms_kernel<2, true>
+                                          : max_terms == 3 ? kgrad_terms_kernel<3, true> : kgrad_terms_kernel<4, true>)
+                      : (max_terms <= 1 ? kgrad_terms_kernel<1, false> : max_terms == 2 ? kgrad_terms_kernel<2, false>
+                                          : max_terms == 3 ? kgrad_terms_kernel<3, false> : kgrad_terms_kernel<4, false>);
+  if (smem + 4096 > 48 * 1024) {  // static shared memory counts against the default limit too
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+  }
+  kern<<<grid, 256, smem, st>>>(mat_base, mat_batch_stride, off_per_lat, x, N, D, params, alpha, alpha_stride, form, partial);
+  dim3 g2((unsigned)nlat, (unsigned)GRAD_TERM_SLOTS);
+  kgrad_terms_finish_kernel<<<g2, 256, 0, st>>>(partial, nchunks, out);
+  return cudaGetLastError();
+}
+
 // v[i] = a[i] * sa - b[i]
 __global__ void scale_sub_kernel(double* __restrict__ v, const double* __restrict__ a, double sa, const double* __restrict__ b, size_t n) {
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;

@@ -1,5 +1,7 @@
 // rrule of logpdf (OILMM, IndependentMOGP, general ILMM), sequential conditioning of per-latent posteriors, prior
 // cross-covariance of an IndependentMOGP.
+#include <algorithm>
+
 #include "host_internal.h"
 
 // ------------------------------------------------------------------------------------------------
@@ -156,7 +158,38 @@ struct GradOut {
   double* grad_S = nullptr;  // m (OILMM only, nullable)
   const double* Yhost_or_dev = nullptr;
   double* grad_ard = nullptr;  // m x D row-major: d/d ARD multiplier (zeros for latents without an ARDTransform; nullable)
+  double* grad_terms = nullptr;  // m x LMM_MAX_TERMS x LMM_GRAD_TERM_STRIDE: per-term gradients (nullable)
 };
+
+constexpr int TERM_SLOTS = LMM_MAX_TERMS * LMM_GRAD_TERM_STRIDE;  // grad_terms doubles per latent
+
+// Launch bounds of the per-term contraction for latents [lo, hi): the most terms, and whether any term has an ARDTransform.
+void terms_shape(const lmm_gp_desc* latents, int lo, int hi, int& max_terms, bool& any_ard) {
+  max_terms = 1;
+  any_ard = false;
+  for (int i = lo; i < hi; ++i) {
+    max_terms = std::max(max_terms, 1 + latents[i].n_extra);
+    any_ard |= latents[i].ard != nullptr;
+    for (int t = 0; t < latents[i].n_extra; ++t) any_ard |= latents[i].extra[t].ard != nullptr;
+  }
+}
+
+// grad_terms -> outputs: the whole per-term block, and term 0's values in place of the single-kernel contraction's
+// grad_latents[:, 0:2] / grad_ard rows for composite latents (single-kernel latents keep kgrad / kgrad_ard's values).
+void scatter_terms(const lmm_gp_desc* latents, int m, int D, const std::vector<double>& ht, double* grad_terms, double* grad_latents,
+                   double* grad_ard) {
+  std::copy(ht.begin(), ht.end(), grad_terms);
+  for (int i = 0; i < m; ++i) {
+    if (!desc_is_composite(latents[i])) continue;
+    const double* g = ht.data() + (size_t)i * TERM_SLOTS;
+    if (grad_latents) {
+      grad_latents[(size_t)i * 3 + 0] = g[0];
+      grad_latents[(size_t)i * 3 + 1] = g[1];
+    }
+    if (grad_ard)
+      for (int k = 0; k < D && k < MAX_ARD; ++k) grad_ard[(size_t)i * D + k] = latents[i].ard ? g[3 + k] : 0.0;
+  }
+}
 
 int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m, const double* x, int N, int D, int p, double sigma2,
                      const double* y, const Projection& pr, const double* Shost, GradOut out) {
@@ -231,6 +264,14 @@ int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m,
     CU(b_gard.alloc(ctx, (size_t)m * MAX_ARD * sizeof(double)));
     CU(cudaMemsetAsync(b_gard.p, 0, (size_t)m * MAX_ARD * sizeof(double), st));
   }
+  DevBuf b_tpart, b_gterms;
+  int max_terms = 1;
+  bool terms_ard = false;
+  if (out.grad_terms) {
+    terms_shape(latents, lo, hi, max_terms, terms_ard);
+    CU(b_gterms.alloc(ctx, (size_t)m * TERM_SLOTS * sizeof(double)));
+    CU(cudaMemsetAsync(b_gterms.p, 0, (size_t)m * TERM_SLOTS * sizeof(double), st));
+  }
   std::vector<int> hinfo(nl, 0);
   std::vector<double> hg4((size_t)nl * 4, 0.0);
   if (mloc > 0) {
@@ -250,6 +291,7 @@ int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m,
     CU(b_gpart.alloc(ctx, (size_t)chunk * ntl * 3 * sizeof(double)));
     CU(b_g4.alloc(ctx, (size_t)mloc * 4 * sizeof(double)));
     if (want_ard) CU(b_apart.alloc(ctx, (size_t)chunk * ntl * MAX_ARD * sizeof(double)));
+    if (out.grad_terms) CU(b_tpart.alloc(ctx, (size_t)chunk * ntl * TERM_SLOTS * sizeof(double)));
     CU(cudaMemsetAsync(b_logdet.p, 0, (size_t)mloc * sizeof(double), st));
     CU(cudaMemsetAsync(b_info.p, 0, (size_t)mloc * sizeof(int), st));
     for (int c0 = 0; c0 < mloc; c0 += chunk) {
@@ -285,6 +327,11 @@ int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m,
                             b_apart.as<double>(), b_gard.as<double>() + (size_t)(lo + c0) * MAX_ARD));
         ctx->launches += 2;
       }
+      if (out.grad_terms) {
+        CU(launch_kgrad_terms(st, L.base, L.batch_stride, 0, b_x.as<double>(), N, D, dp, nb, max_terms, terms_ard, alpha, npad,
+                              ctx->distance_form, b_tpart.as<double>(), b_gterms.as<double>() + (size_t)(lo + c0) * TERM_SLOTS));
+        ctx->launches += 2;
+      }
     }
     std::vector<double> hquad(mloc, 0.0);
     CU(copy_out(ctx, hinfo.data(), b_info.p, (size_t)mloc * sizeof(int)));
@@ -317,6 +364,16 @@ int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m,
     CU(cudaStreamSynchronize(st));
     for (int i = 0; i < m; ++i)
       for (int k = 0; k < D && k < MAX_ARD; ++k) out.grad_ard[(size_t)i * D + k] = latents[i].ard ? hgard[(size_t)i * MAX_ARD + k] : 0.0;
+  }
+  std::vector<double> hterms;
+  if (out.grad_terms) {
+    if (multi) {
+      int r = nccl_api().AllReduce(b_gterms.p, b_gterms.p, (size_t)m * TERM_SLOTS, NCCL_DOUBLE, NCCL_SUM, ctx->comm, st);
+      if (r != 0) return ctx->fail(LMM_E_NCCL, "ncclAllReduce failed");
+    }
+    hterms.resize((size_t)m * TERM_SLOTS);
+    CU(copy_out(ctx, hterms.data(), b_gterms.p, hterms.size() * sizeof(double)));
+    CU(cudaStreamSynchronize(st));
   }
   // d/dy: -sum_i T[i,:]' α_i  (- R/σ² from the regulariser on rank 0)
   if (out.grad_y) {
@@ -402,6 +459,7 @@ int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m,
       out.grad_latents[(size_t)i * 3 + 1] = hv[(size_t)2 * m + i];
       out.grad_latents[(size_t)i * 3 + 2] = hv[(size_t)3 * m + i];
     }
+  if (out.grad_terms) scatter_terms(latents, m, D, hterms, out.grad_terms, out.grad_latents, out.grad_ard);
   if (out.grad_sigma2) {
     double s = dreg;
     for (int i = 0; i < m; ++i) s += hv[(size_t)4 * m + i] * (orth ? 1.0 / Shost[i] : 1.0);  // ν_i = σ²/S_i (OILMM) or σ²
@@ -424,17 +482,24 @@ int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m,
 
 }  // namespace lmm_host
 
-extern "C" int lmm_oilmm_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D, const double* U,
-                                     const double* S, int p, double sigma2, const double* y, int out_dim, double* out_logpdf,
-                                     double* grad_latents, double* grad_ard, double* grad_sigma2, double* grad_y, double* grad_U,
-                                     double* grad_S, int* info_latent) {
+namespace lmm_host {
+// The single-kernel entry points (grad_terms == NULL) reject composite / periodic latents: their grad_latents has no
+// place for the further terms' hyper-parameters.  The _terms entry points accept every latent the value path accepts.
+int reject_composite(lmm_ctx* ctx, const lmm_gp_desc* latents, int m) {
+  for (int i = 0; i < m; ++i)
+    if (desc_is_composite(latents[i]))
+      return ctx->fail(LMM_E_UNSUPPORTED, "the logpdf gradient is built for single (Sq)Euclidean base kernels; composite / periodic latents: value only");
+  return LMM_OK;
+}
+
+int oilmm_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D, const double* U, const double* S, int p,
+                      double sigma2, const double* y, int out_dim, double* out_logpdf, double* grad_latents, double* grad_ard,
+                      double* grad_sigma2, double* grad_y, double* grad_U, double* grad_S, double* grad_terms, int* info_latent) {
   if (!ctx) return LMM_E_ARG;
   std::lock_guard<std::mutex> lk(ctx->mu);
   int rc = check_common(ctx, latents, m, x, N, D, p, out_dim);
   if (rc) return rc;
-  for (int i = 0; i < m; ++i)
-    if (desc_is_composite(latents[i]))
-      return ctx->fail(LMM_E_UNSUPPORTED, "the logpdf gradient is built for single (Sq)Euclidean base kernels; composite / periodic latents: value only");
+  if (!grad_terms && (rc = reject_composite(ctx, latents, m))) return rc;
   if (!U || !S || !y) return ctx->fail(LMM_E_ARG, "null pointer");
   if (m > p) return ctx->fail(LMM_E_ARG, "more latents than outputs");
   Projection pr;
@@ -444,19 +509,18 @@ extern "C" int lmm_oilmm_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, i
   out.grad_U = grad_U;
   out.grad_S = grad_S;
   out.grad_ard = grad_ard;
+  out.grad_terms = grad_terms;
   return latents_grad_run(ctx, true, latents, m, x, N, D, p, sigma2, y, pr, S, out);
 }
 
-extern "C" int lmm_imogp_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* fs, int m, const double* x, int N, int D, double sigma2,
-                                     const double* y, int out_dim, double* out_logpdf, double* grad_latents, double* grad_ard,
-                                     double* grad_sigma2, double* grad_y, int* info_latent) {
+int imogp_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* fs, int m, const double* x, int N, int D, double sigma2, const double* y, int out_dim,
+                      double* out_logpdf, double* grad_latents, double* grad_ard, double* grad_sigma2, double* grad_y, double* grad_terms,
+                      int* info_latent) {
   if (!ctx) return LMM_E_ARG;
   std::lock_guard<std::mutex> lk(ctx->mu);
   int rc = check_common(ctx, fs, m, x, N, D, m, out_dim);
   if (rc) return rc;
-  for (int i = 0; i < m; ++i)
-    if (desc_is_composite(fs[i]))
-      return ctx->fail(LMM_E_UNSUPPORTED, "the logpdf gradient is built for single (Sq)Euclidean base kernels; composite / periodic latents: value only");
+  if (!grad_terms && (rc = reject_composite(ctx, fs, m))) return rc;
   if (!y) return ctx->fail(LMM_E_ARG, "null pointer");
   if (!(sigma2 > 0.0)) return ctx->fail(LMM_E_ARG, "noise variance must be positive");
   Projection pr;
@@ -466,7 +530,39 @@ extern "C" int lmm_imogp_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* fs, int m,
   pr.has_reg = false;
   GradOut out{out_logpdf, grad_latents, grad_sigma2, grad_y, info_latent};
   out.grad_ard = grad_ard;
+  out.grad_terms = grad_terms;
   return latents_grad_run(ctx, false, fs, m, x, N, D, m, sigma2, y, pr, nullptr, out);
+}
+}  // namespace lmm_host
+
+extern "C" int lmm_oilmm_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D, const double* U,
+                                     const double* S, int p, double sigma2, const double* y, int out_dim, double* out_logpdf,
+                                     double* grad_latents, double* grad_ard, double* grad_sigma2, double* grad_y, double* grad_U,
+                                     double* grad_S, int* info_latent) {
+  return oilmm_logpdf_grad(ctx, latents, m, x, N, D, U, S, p, sigma2, y, out_dim, out_logpdf, grad_latents, grad_ard, grad_sigma2, grad_y,
+                           grad_U, grad_S, nullptr, info_latent);
+}
+extern "C" int lmm_oilmm_logpdf_grad_terms(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D, const double* U,
+                                           const double* S, int p, double sigma2, const double* y, int out_dim, double* out_logpdf,
+                                           double* grad_latents, double* grad_ard, double* grad_sigma2, double* grad_y, double* grad_U,
+                                           double* grad_S, double* grad_terms, int* info_latent) {
+  if (ctx && !grad_terms) return ctx->fail(LMM_E_ARG, "null grad_terms");
+  return oilmm_logpdf_grad(ctx, latents, m, x, N, D, U, S, p, sigma2, y, out_dim, out_logpdf, grad_latents, grad_ard, grad_sigma2, grad_y,
+                           grad_U, grad_S, grad_terms, info_latent);
+}
+
+extern "C" int lmm_imogp_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* fs, int m, const double* x, int N, int D, double sigma2,
+                                     const double* y, int out_dim, double* out_logpdf, double* grad_latents, double* grad_ard,
+                                     double* grad_sigma2, double* grad_y, int* info_latent) {
+  return imogp_logpdf_grad(ctx, fs, m, x, N, D, sigma2, y, out_dim, out_logpdf, grad_latents, grad_ard, grad_sigma2, grad_y, nullptr,
+                           info_latent);
+}
+extern "C" int lmm_imogp_logpdf_grad_terms(lmm_ctx* ctx, const lmm_gp_desc* fs, int m, const double* x, int N, int D, double sigma2,
+                                           const double* y, int out_dim, double* out_logpdf, double* grad_latents, double* grad_ard,
+                                           double* grad_sigma2, double* grad_y, double* grad_terms, int* info_latent) {
+  if (ctx && !grad_terms) return ctx->fail(LMM_E_ARG, "null grad_terms");
+  return imogp_logpdf_grad(ctx, fs, m, x, N, D, sigma2, y, out_dim, out_logpdf, grad_latents, grad_ard, grad_sigma2, grad_y, grad_terms,
+                           info_latent);
 }
 // ------------------------------------------------------------------------------------------------
 // cov(f::IndependentMOGP, x, y): dense block-diagonal cross-covariance of the PRIOR process between
@@ -511,16 +607,15 @@ extern "C" int lmm_imogp_cross_cov(lmm_ctx* ctx, const lmm_gp_desc* fs, int m, c
 //   and ΣT = σ² T T' is m x m / m x p host arithmetic.
 // ------------------------------------------------------------------------------------------------
 
-extern "C" int lmm_ilmm_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D, const double* H,
-                                    int p, double sigma2, const double* y, int out_dim, double* out_logpdf, double* grad_latents,
-                                    double* grad_ard, double* grad_sigma2, double* grad_y, double* grad_H, int* info) {
+namespace lmm_host {
+int ilmm_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D, const double* H, int p, double sigma2,
+                     const double* y, int out_dim, double* out_logpdf, double* grad_latents, double* grad_ard, double* grad_sigma2,
+                     double* grad_y, double* grad_H, double* grad_terms, int* info) {
   if (!ctx) return LMM_E_ARG;
   std::lock_guard<std::mutex> lk(ctx->mu);
   int rc = check_common(ctx, latents, m, x, N, D, p, out_dim);
   if (rc) return rc;
-  for (int i = 0; i < m; ++i)
-    if (desc_is_composite(latents[i]))
-      return ctx->fail(LMM_E_UNSUPPORTED, "the logpdf gradient is built for single (Sq)Euclidean base kernels; composite / periodic latents: value only");
+  if (!grad_terms && (rc = reject_composite(ctx, latents, m))) return rc;
   if (!H || !y) return ctx->fail(LMM_E_ARG, "null pointer");
   CU(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
@@ -638,6 +733,20 @@ extern "C" int lmm_ilmm_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, in
     hgard.resize((size_t)m * MAX_ARD);
     CU(copy_out(ctx, hgard.data(), b_gard.p, hgard.size() * sizeof(double)));
   }
+  DevBuf b_tpart, b_gterms;
+  std::vector<double> hterms;
+  if (grad_terms) {
+    int max_terms;
+    bool terms_ard;
+    terms_shape(latents, 0, m, max_terms, terms_ard);
+    CU(b_tpart.alloc(ctx, (size_t)m * nchunks * TERM_SLOTS * sizeof(double)));
+    CU(b_gterms.alloc(ctx, (size_t)m * TERM_SLOTS * sizeof(double)));
+    CU(launch_kgrad_terms(st, L.base, 0, N, b_x.as<double>(), N, D, b_params.as<LatentParams>(), m, max_terms, terms_ard, b_alpha.as<double>(),
+                          (size_t)N, ctx->distance_form, b_tpart.as<double>(), b_gterms.as<double>()));
+    ctx->launches += 2;
+    hterms.resize((size_t)m * TERM_SLOTS);
+    CU(copy_out(ctx, hterms.data(), b_gterms.p, hterms.size() * sizeof(double)));
+  }
   // V = H'R/σ² - A ;  dT(direct) = V Y' ;  dH(direct) = R Z'/σ² ;  dy = T'V - R/σ²
   CU(b_HtR.alloc(ctx, (size_t)m * N * sizeof(double)));
   CU(launch_project(st, b_R.as<double>(), N, p, b_Ht.as<double>(), m, 0, m, b_zero.as<double>(), b_HtR.as<double>(), (size_t)N, nullptr,
@@ -695,9 +804,25 @@ extern "C" int lmm_ilmm_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, in
       grad_latents[(size_t)a * 3 + 1] = g3[(size_t)a * 3 + 1];
       grad_latents[(size_t)a * 3 + 2] = g3[(size_t)a * 3 + 2];
     }
+  if (grad_terms) scatter_terms(latents, m, D, hterms, grad_terms, grad_latents, grad_ard);
   if (grad_sigma2 || grad_H) {
     rc = ilmm_grad_chain(ctx, gp, Hh, p, m, N, sigma2, hres, B, bT, bH, grad_sigma2, grad_H);
     if (rc != LMM_OK) return rc;
   }
   return LMM_OK;
+}
+}  // namespace lmm_host
+
+extern "C" int lmm_ilmm_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D, const double* H,
+                                    int p, double sigma2, const double* y, int out_dim, double* out_logpdf, double* grad_latents,
+                                    double* grad_ard, double* grad_sigma2, double* grad_y, double* grad_H, int* info) {
+  return ilmm_logpdf_grad(ctx, latents, m, x, N, D, H, p, sigma2, y, out_dim, out_logpdf, grad_latents, grad_ard, grad_sigma2, grad_y, grad_H,
+                          nullptr, info);
+}
+extern "C" int lmm_ilmm_logpdf_grad_terms(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D, const double* H,
+                                          int p, double sigma2, const double* y, int out_dim, double* out_logpdf, double* grad_latents,
+                                          double* grad_ard, double* grad_sigma2, double* grad_y, double* grad_H, double* grad_terms, int* info) {
+  if (ctx && !grad_terms) return ctx->fail(LMM_E_ARG, "null grad_terms");
+  return ilmm_logpdf_grad(ctx, latents, m, x, N, D, H, p, sigma2, y, out_dim, out_logpdf, grad_latents, grad_ard, grad_sigma2, grad_y, grad_H,
+                          grad_terms, info);
 }

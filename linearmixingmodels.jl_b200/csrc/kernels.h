@@ -177,6 +177,14 @@ cudaError_t launch_block_trace(cudaStream_t st, TiledSym negCinv, const double* 
 cudaError_t launch_kgrad_ard(cudaStream_t st, const double* mat_base, size_t mat_batch_stride, int off_per_lat, const double* x, int N, int D,
                              const LatentParams* params, int nlat, const double* alpha, size_t alpha_stride, int form, double* partial,
                              double* out);
+// gradient w.r.t. every hyper-parameter of every term of a (possibly composite) latent, storage as launch_kgrad_ard; x holds
+// RAW points.  out[lat*44 + t*11 + {0, 1, 2, 3 + k}] = d/d {variance, inv_lengthscale, param, ard[k]} of term t (the
+// LMM_GRAD_TERM_STRIDE layout of lmm.h), zeros where a term, shape parameter or ARD slot is absent.
+// partial: nlat * sym_tiles(ceil(N/128)) * 44 doubles of scratch.  D <= 8 when a term has an ARDTransform.  max_terms /
+// any_ard: the most terms of a latent of the batch, and whether a term of any latent has an ARDTransform.
+cudaError_t launch_kgrad_terms(cudaStream_t st, const double* mat_base, size_t mat_batch_stride, int off_per_lat, const double* x, int N,
+                               int D, const LatentParams* params, int nlat, int max_terms, bool any_ard, const double* alpha,
+                               size_t alpha_stride, int form, double* partial, double* out);
 cudaError_t launch_scale_sub(cudaStream_t st, double* v, const double* a, double sa, const double* b, size_t n);
 }  // namespace lmm
 

@@ -305,10 +305,12 @@ function AbstractGPs.rand(rng::AbstractRNG, fx::FiniteGP{<:PosteriorOILMM})
 end
 
 # --- rrule for logpdf (keeps `Zygote.gradient(logpdf, fx, y)` working: test/oilmm.jl:31-32) ---------
-# The ccall is opaque to AD, so the pullback comes from `lmm_oilmm_logpdf_grad` (batched potri +
-# fused kernel-gradient reduction).  Tangents are returned for y, σ² and, per latent, the kernel
-# variance / inverse lengthscale / constant mean; mapping them back onto the nested kernel structs
-# (ScaledKernel.σ², ScaleTransform.s, ConstMean.c) is mechanical and omitted here.
+# The ccall is opaque to AD, so the pullback comes from `lmm_oilmm_logpdf_grad_terms` (batched potri +
+# fused kernel-gradient reductions), which accepts every latent kernel the value path does (KernelSum /
+# KernelProduct, PeriodicKernel, RationalQuadraticKernel).  Tangents are returned for y, σ² and, per latent,
+# the hyper-parameters of every kernel term (gt) and the constant mean; mapping them back onto the nested
+# kernel structs (ScaledKernel.σ², ScaleTransform.s, PeriodicKernel.r, ConstMean.c) is mechanical and omitted here.
+const GRAD_TERM_DOUBLES = 4 * 11   # LMM_MAX_TERMS * LMM_GRAD_TERM_STRIDE doubles of grad_terms per latent
 using ChainRulesCore
 function ChainRulesCore.rrule(::typeof(AbstractGPs.logpdf), fx::FiniteGP{<:OILMM{<:IndependentMOGP{<:Vector{<:GP}}}},
                               y::AbstractVector{<:Real})
@@ -319,11 +321,12 @@ function ChainRulesCore.rrule(::typeof(AbstractGPs.logpdf), fx::FiniteGP{<:OILMM
     gl = Matrix{Float64}(undef, 3, m)            # column i = (d/dvariance, d/dinv_lengthscale, d/dmean) of latent i
     gy = Vector{Float64}(undef, length(y))
     gU = Matrix{Float64}(undef, size(H, 1), m); gS = Vector{Float64}(undef, m)   # tangents of H.U and H.S.diag
-    check(GC.@preserve keep ccall((:lmm_oilmm_logpdf_grad, liblmm), Cint,
+    gt = Matrix{Float64}(undef, GRAD_TERM_DOUBLES, m)   # column i: latent i's terms, 11 slots each (variance, s, param, ard[1:8])
+    check(GC.@preserve keep ccall((:lmm_oilmm_logpdf_grad_terms, liblmm), Cint,
         (Ptr{Cvoid}, Ptr{GpDesc}, Cint, Ptr{Float64}, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Cint, Float64, Ptr{Float64}, Cint,
-         Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Cint}),
+         Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Cint}),
         ctx(), descs, m, X, length(x), D, Matrix{Float64}(H.U), Vector{Float64}(diag(H.S)), size(H, 1), Float64(σ²),
-        Vector{Float64}(y), fx.x.out_dim, out, gl, C_NULL #= grad_ard (m x D, row-major): pass a Matrix{Float64}(undef, D, m) to receive d/d ARD multipliers =#, gs2, gy, gU, gS, il))
+        Vector{Float64}(y), fx.x.out_dim, out, gl, C_NULL #= grad_ard (m x D, row-major): pass a Matrix{Float64}(undef, D, m) to receive d/d ARD multipliers =#, gs2, gy, gU, gS, gt, il))
     function logpdf_pullback(Δ)
         Σy_tangent = Tangent{typeof(fx.Σy)}(; diag = Tangent{typeof(fx.Σy.diag)}(; value = Δ * gs2[]))
         return NoTangent(), Tangent{typeof(fx)}(; Σy = Σy_tangent), Δ .* gy
@@ -339,10 +342,11 @@ function ChainRulesCore.rrule(::typeof(AbstractGPs.logpdf), fx::FiniteGP{<:ILMM{
     descs, keep = gpdescs(fs.fs); m = length(descs)
     out = Ref{Float64}(0.0); gs2 = Ref{Float64}(0.0); info = Ref{Cint}(0)
     gl = Matrix{Float64}(undef, 3, m); gy = Vector{Float64}(undef, length(y)); gH = similar(H)
-    check(GC.@preserve keep ccall((:lmm_ilmm_logpdf_grad, liblmm), Cint,
+    gt = Matrix{Float64}(undef, GRAD_TERM_DOUBLES, m)
+    check(GC.@preserve keep ccall((:lmm_ilmm_logpdf_grad_terms, liblmm), Cint,
         (Ptr{Cvoid}, Ptr{GpDesc}, Cint, Ptr{Float64}, Cint, Cint, Ptr{Float64}, Cint, Float64, Ptr{Float64}, Cint,
-         Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Cint}),
-        ctx(), descs, m, X, length(x), D, H, size(H, 1), Float64(σ²), Vector{Float64}(y), fx.x.out_dim, out, gl, C_NULL, gs2, gy, gH, info))
+         Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Cint}),
+        ctx(), descs, m, X, length(x), D, H, size(H, 1), Float64(σ²), Vector{Float64}(y), fx.x.out_dim, out, gl, C_NULL, gs2, gy, gH, gt, info))
     function logpdf_pullback(Δ)
         Σy_tangent = Tangent{typeof(fx.Σy)}(; diag = Tangent{typeof(fx.Σy.diag)}(; value = Δ * gs2[]))
         f_tangent = Tangent{typeof(fx.f)}(; H = Δ .* gH)
