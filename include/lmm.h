@@ -390,6 +390,22 @@ int lmm_ilmm_masked_posterior(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, c
 int lmm_oilmm_masked_posterior(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D,
                                const double* U, const double* S, int p, double sigma2, const double* y, int out_dim,
                                lmm_post** out_post, double* out_logpdf, int* n_observed_inputs, int* info_latent);
+/* rrule of the missing-data logpdf of the dense model (lmm_ilmm_masked_posterior's value).  NaN entries of y are
+ * unobserved; grad_y is 0 there.  grad_terms nullable: NULL rejects composite / periodic latents, as lmm_*_logpdf_grad.
+ * Outputs as lmm_ilmm_logpdf_grad_terms: grad_latents m x 3 (term 0's variance and inv_lengthscale, mean_const), grad_ard
+ * m x D, grad_H p x m column-major, grad_y p*N by outputs; all nullable.  Workspace ≈ 12 n_observed² bytes (the factor and
+ * the square X of its potri); with a communicator every rank computes the whole, replicated result. */
+int lmm_ilmm_masked_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D,
+                                const double* H, int p, double sigma2, const double* y, int out_dim, double* out_logpdf,
+                                double* grad_latents, double* grad_ard, double* grad_sigma2, double* grad_y, double* grad_H,
+                                double* grad_terms, int* n_observed, int* info);
+/* Per-input mask (whole inputs missing): the OILMM gradient (lmm_oilmm_logpdf_grad[_terms]) on the observed inputs; grad_y
+ * scattered back to p*N with 0 at missing inputs.  A mask that is not per-input returns LMM_E_UNSUPPORTED. */
+int lmm_oilmm_masked_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D,
+                                 const double* U, const double* S, int p, double sigma2, const double* y, int out_dim,
+                                 double* out_logpdf, double* grad_latents, double* grad_ard, double* grad_sigma2,
+                                 double* grad_y, double* grad_U, double* grad_S, double* grad_terms,
+                                 int* n_observed_inputs, int* info_latent);
 
 /* ---- batched blocked Cholesky primitive: the `cholesky(Symmetric(C))` / dpotrf call site ---- */
 /* A: batch matrices, each N x N column-major (lower triangle read).  L_out (nullable): same

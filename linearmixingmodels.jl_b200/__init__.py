@@ -20,6 +20,7 @@ from .api import (  # noqa: F401
     load_posterior,
     posterior_missing,
     logpdf_missing,
+    logpdf_missing_and_gradient,
 )
 from . import _lib, api, dist  # noqa: F401
 

@@ -113,6 +113,9 @@ SIGNATURES = {
     "lmm_ilmm_logpdf_grad_terms": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, C.c_int, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _dp, _vp, _vp, _vp, _ip]),
     "lmm_ilmm_masked_posterior": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, C.c_int, C.c_double, _vp, C.c_int, C.POINTER(_vp), _dp, _ip, _ip]),
     "lmm_oilmm_masked_posterior": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, C.c_int, C.POINTER(_vp), _dp, _ip, _ip]),
+    # missing-data logpdf gradient: dense model (grad_terms nullable, n_observed, info) and per-input-mask OILMM
+    "lmm_ilmm_masked_logpdf_grad": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, C.c_int, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _dp, _vp, _vp, _vp, _ip, _ip]),
+    "lmm_oilmm_masked_logpdf_grad": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _dp, _vp, _vp, _vp, _vp, _ip, _ip]),
     "lmm_potrf_batched": (C.c_int, [_vp, _vp, C.c_int, C.c_int, _vp, _vp, _vp]),
     "lmm_mvn_logpdf_rand": (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _dp, _vp, _vp, _ip]),
     "lmm_potrf_bench": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int, C.c_double, C.c_int, _vp, _dp, _dp]),

@@ -1266,3 +1266,58 @@ def logpdf_missing(fx: FiniteGP, y) -> float:
                                            C.byref(out), None, C.byref(info))
     ctx.check(rc)
     return out.value
+
+
+def logpdf_missing_and_gradient(fx: FiniteGP, y, with_grad_y: bool = False, kernel_terms: bool = False):
+    """Value and gradient of `logpdf_missing(fx, y)`: entries of `y` that are NaN are unobserved.  Routes as
+    `logpdf_missing` does.  An OILMM (`Orthogonal` H) with a per-input mask is the OILMM gradient on the observed inputs and
+    returns "U" / "S" as `logpdf_and_gradient` does.  Any other model or mask runs the dense model on the observed entries
+    and returns "H" (p, m), d/dH of C_ab = Σ_l H[j_a,l] H[j_b,l] k_l + σ²[a = b].  With an `Orthogonal` H it also returns
+    "U" = gH·diag(√S) and "S"[l] = Σ_j gH[j,l] U[j,l] / (2√S_l), the chain rule of H = U√S.  That is the Euclidean
+    gradient of the dense-model expression: it agrees with the OILMM path's "U" in the tangent space of orthogonal U
+    (after projecting G -> G - U sym(U'G)), not off it.
+    "variance" / "inv_lengthscale" / "mean_const" / "sigma2" / "ard" / "terms" mean what they mean in
+    `logpdf_and_gradient` (composite latents need `kernel_terms=True`); "y" (p*N,) is 0 at every NaN entry.  A posterior
+    FiniteGP raises TypeError."""
+    lat, H, s2, _ = unpack(fx)
+    if not isinstance(lat, IndependentMOGP) or any(isinstance(g, PosteriorGP) for g in lat.fs):
+        raise TypeError("logpdf_missing_and_gradient needs an ILMM / OILMM over prior latents")
+    ctx = default_context()
+    pts = _points(fx.x.x)
+    N, D = int(pts.shape[0]), int(pts.shape[1])
+    Hm = as_f64(np.asarray(H), "F")
+    p, m = Hm.shape
+    yv = np.ascontiguousarray(np.asarray(y, dtype=np.float64).reshape(-1))
+    if yv.shape[0] != N * p:
+        raise ValueError("length of y does not match the inputs")
+    out, gs2, nobs, info = C.c_double(), C.c_double(), C.c_int(0), C.c_int(-1)
+    gl = np.zeros((m, 3))
+    ga = np.zeros((m, D))
+    gy = np.zeros(N * p) if with_grad_y else None
+    gt = np.zeros(m * _lib.LMM_MAX_TERMS * _lib.LMM_GRAD_TERM_STRIDE) if kernel_terms else None
+    if isinstance(H, Orthogonal) and _nan_mask_is_per_input(yv, p, N):
+        gU = np.zeros(H.shape, order="F")
+        gS = np.zeros(m)
+        rc = ctx.lib.lmm_oilmm_masked_logpdf_grad(ctx.handle, _descs(lat.fs), m, ptr(pts), N, D, ptr(H.U), ptr(H.S), p, s2, ptr(yv),
+                                                  fx.x.out_dim, C.byref(out), ptr(gl), ptr(ga), C.byref(gs2), ptr(gy), ptr(gU), ptr(gS),
+                                                  ptr(gt), C.byref(nobs), C.byref(info))
+        ctx.check(rc, info.value)
+        grads = {"U": np.ascontiguousarray(gU), "S": gS}
+    else:
+        gH = np.zeros((p, m), order="F")
+        rc = ctx.lib.lmm_ilmm_masked_logpdf_grad(ctx.handle, _descs(lat.fs), m, ptr(pts), N, D, ptr(Hm), p, s2, ptr(yv), fx.x.out_dim,
+                                                 C.byref(out), ptr(gl), ptr(ga), C.byref(gs2), ptr(gy), ptr(gH), ptr(gt), C.byref(nobs),
+                                                 C.byref(info))
+        ctx.check(rc)
+        grads = {"H": np.ascontiguousarray(gH)}
+        if isinstance(H, Orthogonal):
+            rs = np.sqrt(np.asarray(H.S, dtype=np.float64))
+            grads["U"] = grads["H"] * rs[None, :]
+            grads["S"] = np.sum(grads["H"] * np.asarray(H.U), axis=0) / (2.0 * rs)
+    grads.update({"variance": gl[:, 0].copy(), "inv_lengthscale": gl[:, 1].copy(), "mean_const": gl[:, 2].copy(), "sigma2": gs2.value,
+                  "ard": ga})
+    if kernel_terms:
+        grads["terms"] = _terms_grads(lat.fs, gt, D)
+    if with_grad_y:
+        grads["y"] = gy
+    return out.value, grads

@@ -633,6 +633,293 @@ cudaError_t launch_kgrad_terms(cudaStream_t st, const double* mat_base, size_t m
   return cudaGetLastError();
 }
 
+// ---- missing-data (heterotopic) dense model: contraction over the observed-entry matrix ----------------------------------
+// Rows and columns a of the (nobs x nobs) matrix are the observed entries obs[a] = j_a*N + i_a (output j_a at input i_a),
+// C_ab = Σ_l H[j_a,l] H[j_b,l] k_l(x_{i_a}, x_{i_b}) + σ² [a = b].  Per latent l and term t the hyper-parameter gradient is
+// Σ_ab G_ab H[j_a,l] H[j_b,l] ∂k_l/∂θ_t; d/dH needs the row sums v_l(a) = Σ_b G_ab H[j_b,l] k_l(a,b).  Every entry pair
+// couples every latent, so one CTA per lower tile reads its block of -C⁻¹ ONCE -- a 32-row strip at a time, into
+// registers -- and loops over all latents and terms on it.  The kernel diagonal is decided by point identity
+// (i_a == i_b: κ = 1, no derivative but d/d variance, as kernel_pair in the value path); the factor 2 of the off-diagonal
+// lower triangle by entry identity (a != b).
+constexpr int MSTRIP = 32;  // rows of a strip: 16 elements per thread
+
+// One latent on one strip.  Thread t = (warp w, lane) holds rows 8gi + lane/4 (gi < 4) and columns 16w + 4h + lane%4 (h < 4)
+// of the strip; sg[4gi + h][t] is G there (0 outside the lower triangle and past nobs: padding rows hold the identity).  The
+// row sums Σ_h G H[j_b,l] k_l are reduced over the 4 lanes of a row and written to rowred[w][row]; the column sums
+// Σ_gi G H[j_a,l] k_l (entry-diagonal elements excluded: they count once, in the row sums) are left in scs[h][t]; the per-slot
+// sums are warp-reduced into wsum[slot][warp] as in kgrad_terms_body.  The 16 elements are a loop, not unrolled: one copy of
+// the term derivatives per instantiation.
+template <int NT, bool ARD>
+__device__ __forceinline__ void kgrad_masked_body(const TermParams* tp, bool product, double (*sg)[256], const double* xa, const double* xb,
+                                                  const int* pta, const int* ptb, const int* ja, const int* jb,
+                                                  const double* __restrict__ Hl, int D, int form, int rbase, int cbase, bool diag_tile,
+                                                  double (*rowred)[MSTRIP], double (*scs)[256], double (*wsum)[8]) {
+  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  double acc[NT][3], aca[ARD ? NT : 1][MAX_ARD];
+#pragma unroll
+  for (int u = 0; u < NT; ++u) {
+    acc[u][0] = acc[u][1] = acc[u][2] = 0.0;
+#pragma unroll
+    for (int k = 0; k < MAX_ARD; ++k) aca[ARD ? u : 0][k] = 0.0;
+  }
+#pragma unroll
+  for (int h = 0; h < 4; ++h) scs[h][t] = 0.0;
+  double rsum = 0.0, hr = 0.0;
+#pragma unroll 1
+  for (int e = 0; e < 16; ++e) {
+    const int gi = e >> 2, h = e & 3;
+    const int r = rbase + 8 * gi, c = cbase + 4 * h;
+    if (h == 0) hr = Hl[ja[r]];
+    const double G = sg[e][t];
+    if (G != 0.0) {  // every contribution carries G: outside the triangle, padding, or an exact zero
+      const bool same_entry = diag_tile && r == c;
+      const double* pa = xa + (size_t)r * D;
+      const double* pb = xb + (size_t)c * D;
+      double kap[NT], ds[NT], dp[NT], wa[NT];
+      if (pta[r] == ptb[c]) {  // same input point: κ(0) = 1, only the variances have a derivative
+#pragma unroll
+        for (int u = 0; u < NT; ++u) { kap[u] = 1.0; ds[u] = dp[u] = wa[u] = 0.0; }
+      } else {
+#pragma unroll
+        for (int u = 0; u < NT; ++u) term_grad(tp[u], pa, pb, D, form, kap[u], ds[u], dp[u], wa[u]);
+      }
+      const double hc = Hl[jb[c]];
+      const double w2 = (same_entry ? G : 2.0 * G) * (hr * hc);
+      double suf[NT + 1];
+      suf[NT] = 1.0;
+      double kval = 0.0;  // k_l(a, b) of the whole latent kernel
+      if (product) {
+#pragma unroll
+        for (int u = NT - 1; u >= 0; --u) suf[u] = suf[u + 1] * (tp[u].variance * kap[u]);
+        kval = suf[0];
+      } else {
+#pragma unroll
+        for (int u = 0; u < NT; ++u) kval = fma(tp[u].variance, kap[u], kval);
+      }
+      double pre = 1.0;
+#pragma unroll
+      for (int u = 0; u < NT; ++u) {
+        const double w = product ? w2 * pre * suf[u + 1] : w2;
+        if (product) pre *= tp[u].variance * kap[u];
+        acc[u][0] = fma(w, kap[u], acc[u][0]);
+        acc[u][1] = fma(w, ds[u], acc[u][1]);
+        acc[u][2] = fma(w, dp[u], acc[u][2]);
+        if (ARD && tp[u].ard_dim && wa[u] != 0.0) {
+          const double wk = w * wa[u];
+#pragma unroll
+          for (int k = 0; k < MAX_ARD; ++k)
+            if (k < D) aca[ARD ? u : 0][k] = fma(wk, ard_factor(tp[u], pa, pb, k), aca[ARD ? u : 0][k]);
+        }
+      }
+      rsum = fma(G * hc, kval, rsum);
+      if (!same_entry) scs[h][t] = fma(G * hr, kval, scs[h][t]);
+    }
+    if (h == 3) {  // row 8gi + lane/4 done on this thread: the 4 lanes sharing it hold the warp's 16 columns
+      rsum += __shfl_xor_sync(0xffffffffu, rsum, 1);
+      rsum += __shfl_xor_sync(0xffffffffu, rsum, 2);
+      if ((lane & 3) == 0) rowred[warp][8 * gi + (lane >> 2)] = rsum;
+      rsum = 0.0;
+    }
+  }
+#pragma unroll
+  for (int u = 0; u < NT; ++u) {
+#pragma unroll
+    for (int j = 0; j < (ARD ? GRAD_TERM_STRIDE : 3); ++j) {
+      double v = j < 3 ? acc[u][j] : aca[ARD ? u : 0][j - 3];
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+      if (lane == 0) wsum[u * GRAD_TERM_STRIDE + j][warp] = v;
+    }
+  }
+}
+
+// grid (lower tiles of the nobs x nobs matrix).  Per latent l and tile tl (all in fixed order, no atomics):
+//   tpart[(l*ntl + tl)*GRAD_TERM_SLOTS + slot]  per-term slots as kgrad_terms_kernel (summed over the tile's 4 strips),
+//   rowpart[(l*ntl + tl)*TILE + r]  Σ_c G_rc H[j_c,l] k_l(r,c) over the tile's lower-triangle columns,
+//   colpart[(l*ntl + tl)*TILE + c]  Σ_r G_rc H[j_r,l] k_l(r,c) over its rows, the entry diagonal excluded.
+// NTMAX / ARDANY bound the terms and ARD use of all latents (register budget as kgrad_terms_kernel).
+template <int NTMAX, bool ARDANY>
+__global__ void __launch_bounds__(256, (NTMAX <= 2 && !ARDANY) ? 2 : 1) kgrad_masked_kernel(TiledSym negCinv, const int* __restrict__ obs, int nobs,
+                                                                                          const double* __restrict__ x, int N, int D,
+                                                                                          const LatentParams* __restrict__ params, int m, int p,
+                                                                                          const double* __restrict__ Hm, const double* __restrict__ alpha,
+                                                                                          int form, double* __restrict__ tpart,
+                                                                                          double* __restrict__ rowpart, double* __restrict__ colpart) {
+  extern __shared__ __align__(16) double sm[];
+  double* xa = sm;  // raw points of the tile's row entries
+  double* xb = xa + TILE * D;
+  double* aa = xb + TILE * D;
+  double* ab = aa + TILE;
+  double(*sg)[256] = reinterpret_cast<double(*)[256]>(ab + TILE);  // the strip's G, one column per thread
+  double(*scs)[256] = sg + 16;                                      // the thread's column sums
+  __shared__ int pta[TILE], ptb[TILE], ja[TILE], jb[TILE];  // input point and output of the row / column entries
+  __shared__ TermParams tp[MAX_TERMS];
+  __shared__ double wsum[GRAD_TERM_SLOTS][8];
+  __shared__ double rowred[8][MSTRIP];
+  const int tl = blockIdx.x, ntl = gridDim.x, t = threadIdx.x, w = t >> 5, lane = t & 31;
+  int I = (int)((sqrt(8.0 * (double)tl + 1.0) - 1.0) * 0.5);
+  while ((size_t)(I + 1) * (I + 2) / 2 <= (size_t)tl) ++I;
+  while ((size_t)I * (I + 1) / 2 > (size_t)tl) --I;
+  const int J = tl - (int)((size_t)I * (I + 1) / 2);
+  const bool diag_tile = I == J;
+  if (t < TILE) {
+    const int gr = I * TILE + t, gc = J * TILE + t;
+    const int oa = gr < nobs ? obs[gr] : 0, ob = gc < nobs ? obs[gc] : 0;
+    ja[t] = oa / N; pta[t] = oa % N;
+    jb[t] = ob / N; ptb[t] = ob % N;
+    aa[t] = gr < nobs ? alpha[gr] : 0.0;
+    ab[t] = gc < nobs ? alpha[gc] : 0.0;
+  }
+  __syncthreads();
+  for (int i = t; i < TILE * D; i += 256) {
+    const int r = i / D, k = i % D;
+    xa[i] = x[(size_t)pta[r] * D + k];
+    xb[i] = x[(size_t)ptb[r] * D + k];
+  }
+  const double* tile = negCinv.tile(0, I, J);
+  const int cbase = 16 * w + (lane & 3);
+  for (int s = 0; s < TILE / MSTRIP; ++s) {
+    const int rbase = MSTRIP * s + (lane >> 2);
+    // the strip's 32 x 128 block of -C⁻¹, read once for all latents (only thread t reads sg[.][t] back)
+#pragma unroll
+    for (int gi = 0; gi < 4; ++gi)
+#pragma unroll
+      for (int h = 0; h < 4; ++h) {
+        const int r = rbase + 8 * gi, c = cbase + 4 * h;
+        const double nc = tile[(4 * w + h) * 512 + (4 * s + gi) * 32 + lane];  // = tile_elem(r, c): 256 B per warp
+        const bool in = I * TILE + r < nobs && J * TILE + c < nobs && (!diag_tile || c <= r);
+        sg[4 * gi + h][t] = in ? 0.5 * (aa[r] * ab[c] + nc) : 0.0;
+      }
+    for (int l = 0; l < m; ++l) {
+      const LatentParams* lp = params + l;
+      if (t == 0) {
+        tp[0].kind = lp->kind; tp[0].ard_dim = lp->ard_dim; tp[0].variance = lp->variance; tp[0].inv_ls = lp->inv_ls; tp[0].param = lp->param;
+        for (int k = 0; k < MAX_ARD; ++k) tp[0].ard[k] = lp->ard[k];
+      } else if (t < MAX_TERMS) {
+        tp[t] = lp->extra[t - 1];
+      }
+      __syncthreads();  // also orders the staged points (first pass) and the previous latent's reads of wsum / rowred
+      const int nterms = lp->nterms;
+      const bool product = lp->compose == 2;
+      bool ard = false;
+      for (int u = 0; u < nterms; ++u) ard |= tp[u].ard_dim > 0;
+      const double* Hl = Hm + (size_t)l * p;
+#define LMM_MASKED_CASE(n, a)                                                                                                  \
+  if constexpr (n <= NTMAX && (ARDANY || !a))                                                                                \
+    if (nterms == n && ard == a)                                                                                             \
+      kgrad_masked_body<n, a>(tp, product, sg, xa, xb, pta, ptb, ja, jb, Hl, D, form, rbase, cbase, diag_tile, rowred, scs, wsum);
+      LMM_MASKED_CASE(1, false) LMM_MASKED_CASE(1, true) LMM_MASKED_CASE(2, false) LMM_MASKED_CASE(2, true)
+      LMM_MASKED_CASE(3, false) LMM_MASKED_CASE(3, true) LMM_MASKED_CASE(4, false) LMM_MASKED_CASE(4, true)
+#undef LMM_MASKED_CASE
+      // columns: the 8 lanes sharing lane % 4 hold one column's 32 rows of the strip; the column belongs to this warp only
+      double cv = 0.0;
+#pragma unroll
+      for (int h = 0; h < 4; ++h) {
+        double v = scs[h][t];
+        v += __shfl_xor_sync(0xffffffffu, v, 4);
+        v += __shfl_xor_sync(0xffffffffu, v, 8);
+        v += __shfl_xor_sync(0xffffffffu, v, 16);
+        if ((lane >> 2) == h) cv = v;
+      }
+      __syncthreads();
+      const size_t lt = (size_t)l * ntl + tl;
+      if (lane < 16) {
+        double* dst = colpart + lt * TILE + cbase + 4 * (lane >> 2);
+        *dst = s == 0 ? cv : *dst + cv;  // the same thread adds the strips in order
+      }
+      if (t < MSTRIP) {
+        double v = 0.0;
+        for (int k = 0; k < 8; ++k) v += rowred[k][t];
+        rowpart[lt * TILE + MSTRIP * s + t] = v;
+      }
+      if (t < GRAD_TERM_SLOTS) {
+        const int u = t / GRAD_TERM_STRIDE, j = t % GRAD_TERM_STRIDE;
+        double v = 0.0;
+        if (u < nterms && (j < 3 || (ard && tp[u].ard_dim && j - 3 < D))) {
+          for (int k = 0; k < 8; ++k) v += wsum[t][k];
+          if (j >= 1) v *= tp[u].variance;  // ∂K/∂θ carries the term's variance (∂K/∂variance does not)
+          if (j >= 3) v /= tp[u].ard[j - 3];
+        }
+        double* dst = tpart + lt * GRAD_TERM_SLOTS + t;
+        *dst = s == 0 ? v : *dst + v;
+      }
+      __syncthreads();
+    }
+  }
+}
+
+// v[l*nobs + a] = Σ_{J <= A} rowpart[(A,J)] + Σ_{I >= A} colpart[(I,A)] (A = a / 128), in that order: grid (ceil(nobs/256), m)
+__global__ void __launch_bounds__(256) kgrad_masked_rows_kernel(const double* __restrict__ rowpart, const double* __restrict__ colpart, int nobs,
+                                                                int nt, double* __restrict__ v) {
+  const int a = blockIdx.x * 256 + threadIdx.x, l = blockIdx.y;
+  if (a >= nobs) return;
+  const size_t ntl = sym_tiles(nt);
+  const int A = a / TILE, r = a % TILE;
+  const double* rp = rowpart + (size_t)l * ntl * TILE;
+  const double* cp = colpart + (size_t)l * ntl * TILE;
+  double s = 0.0;
+  for (int J = 0; J <= A; ++J) s += rp[sym_tile_index(A, J) * TILE + r];
+  for (int I = A; I < nt; ++I) s += cp[sym_tile_index(I, A) * TILE + r];
+  v[(size_t)l * nobs + a] = s;
+}
+
+// gH[l*p + j] = 2 Σ_{a in [seg[j], seg[j+1])} v[l*nobs + a] (obs is sorted by outputs); grid (p, m).  An output with no
+// observed entry gets exactly 0.
+__global__ void __launch_bounds__(256) kgrad_masked_outputs_kernel(const double* __restrict__ v, const int* __restrict__ seg, int nobs, int p,
+                                                                   double* __restrict__ gH) {
+  __shared__ double red[256];
+  const int j = blockIdx.x, l = blockIdx.y, t = threadIdx.x;
+  double s = 0.0;
+  for (int a = seg[j] + t; a < seg[j + 1]; a += 256) s += v[(size_t)l * nobs + a];
+  red[t] = s;
+  __syncthreads();
+  for (int w = 128; w > 0; w >>= 1) {
+    if (t < w) red[t] += red[t + w];
+    __syncthreads();
+  }
+  if (t == 0) gH[(size_t)l * p + j] = 2.0 * red[0];
+}
+
+// out[0] = Σ_a (-C⁻¹)_aa over the nobs observed entries (fixed order, one block)
+__global__ void __launch_bounds__(256) sym_diag_sum_kernel(TiledSym M, int n, double* __restrict__ out) {
+  __shared__ double red[256];
+  const int t = threadIdx.x;
+  double s = 0.0;
+  for (int a = t; a < n; a += 256) s += M.tile(0, a / TILE, a / TILE)[tile_elem(a % TILE, a % TILE)];
+  red[t] = s;
+  __syncthreads();
+  for (int w = 128; w > 0; w >>= 1) {
+    if (t < w) red[t] += red[t + w];
+    __syncthreads();
+  }
+  if (t == 0) out[0] = red[0];
+}
+
+cudaError_t launch_kgrad_masked(cudaStream_t st, TiledSym negCinv, const int* obs, int nobs, const double* x, int N, int D, const LatentParams* params,
+                                int m, int p, const double* Hm, const double* alpha, int max_terms, bool any_ard, int form, const int* seg,
+                                double* tpart, double* rowpart, double* colpart, double* v, double* out_terms, double* out_H, double* out_diag) {
+  const size_t smem = (size_t)(2 * TILE * D + 2 * TILE + 20 * 256) * sizeof(double);
+  const int nt = negCinv.nt;
+  const int ntl = (int)sym_tiles(nt);
+  auto kern = any_ard ? (max_terms <= 1 ? kgrad_masked_kernel<1, true> : max_terms == 2 ? kgrad_masked_kernel<2, true>
+                                          : max_terms == 3 ? kgrad_masked_kernel<3, true> : kgrad_masked_kernel<4, true>)
+                      : (max_terms <= 1 ? kgrad_masked_kernel<1, false> : max_terms == 2 ? kgrad_masked_kernel<2, false>
+                                          : max_terms == 3 ? kgrad_masked_kernel<3, false> : kgrad_masked_kernel<4, false>);
+  if (smem + 8192 > 48 * 1024) {  // static shared memory counts against the default limit too
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+  }
+  kern<<<(unsigned)ntl, 256, smem, st>>>(negCinv, obs, nobs, x, N, D, params, m, p, Hm, alpha, form, tpart, rowpart, colpart);
+  dim3 g2((unsigned)m, (unsigned)GRAD_TERM_SLOTS);
+  kgrad_terms_finish_kernel<<<g2, 256, 0, st>>>(tpart, ntl, out_terms);
+  dim3 g3((unsigned)((nobs + 255) / 256), (unsigned)m);
+  kgrad_masked_rows_kernel<<<g3, 256, 0, st>>>(rowpart, colpart, nobs, nt, v);
+  dim3 g4((unsigned)p, (unsigned)m);
+  kgrad_masked_outputs_kernel<<<g4, 256, 0, st>>>(v, seg, nobs, p, out_H);
+  sym_diag_sum_kernel<<<1, 256, 0, st>>>(negCinv, nobs, out_diag);
+  return cudaGetLastError();
+}
+
 // v[i] = a[i] * sa - b[i]
 __global__ void scale_sub_kernel(double* __restrict__ v, const double* __restrict__ a, double sa, const double* __restrict__ b, size_t n) {
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;

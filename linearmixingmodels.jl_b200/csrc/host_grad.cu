@@ -608,6 +608,19 @@ extern "C" int lmm_imogp_cross_cov(lmm_ctx* ctx, const lmm_gp_desc* fs, int m, c
 // ------------------------------------------------------------------------------------------------
 
 namespace lmm_host {
+// Joint potri of one factor (batch 1): X = L^{-T} by the triangular-aware TRSM sweep on an identity, then -C^{-1} = -X X'
+// by a triangular-aware SYRK into L's own tiles.  X: L.nt x L.nt tiles of scratch.
+cudaError_t joint_neg_inverse(lmm_ctx* ctx, cudaStream_t st, TiledSym L, const double* W, size_t wstride, TiledRect X) {
+  cudaError_t e;
+  if ((e = launch_rect_identity(st, X, 1)) != cudaSuccess) return e;
+  if ((e = trsm_right_lt_upper(ctx, st, X, L, W, wstride, 1)) != cudaSuccess) return e;
+  if ((e = cudaMemsetAsync(L.base, 0, sym_tiles(L.nt) * TT * sizeof(double), st)) != cudaSuccess) return e;
+  GemmArgs g{};
+  g.A = operand(X); g.B = operand(X); g.C = operand(L);
+  g.i0 = 0; g.j0 = 0; g.k0 = 0; g.k1 = L.nt; g.sym = 1; g.k_from_row = 1;
+  return launch_gemm(st, GEMM_UPDATE, g, L.nt, L.nt, 1);
+}
+
 int ilmm_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D, const double* H, int p, double sigma2,
                      const double* y, int out_dim, double* out_logpdf, double* grad_latents, double* grad_ard, double* grad_sigma2,
                      double* grad_y, double* grad_H, double* grad_terms, int* info) {
@@ -698,18 +711,9 @@ int ilmm_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const doub
   CU(cudaMemcpyAsync(b_r.p, b_z.p, bpad * sizeof(double), cudaMemcpyDeviceToDevice, st));
   CU(launch_bwd_solve(st, L, b_W.as<double>(), wstride, b_r.as<double>(), b_alpha.as<double>(), bpad, 1, &ctx->launches));
   ++ctx->launches;
-  // joint potri: X = L^{-T} (triangular-aware TRSM sweep on an identity), -C^{-1} = -X X' into L's tiles
   CU(b_X.alloc(ctx, (size_t)bnt * bnt * TT * sizeof(double)));
   TiledRect X{b_X.as<double>(), bnt, bnt, (size_t)bnt * bnt * TT};
-  CU(launch_rect_identity(st, X, 1));
-  CU(trsm_right_lt_upper(ctx, st, X, L, b_W.as<double>(), wstride, 1));
-  CU(cudaMemsetAsync(b_L.p, 0, sym_tiles(bnt) * TT * sizeof(double), st));
-  {
-    GemmArgs g{};
-    g.A = operand(X); g.B = operand(X); g.C = operand(L);
-    g.i0 = 0; g.j0 = 0; g.k0 = 0; g.k1 = bnt; g.sym = 1; g.k_from_row = 1;
-    CU(launch_gemm(st, GEMM_UPDATE, g, bnt, bnt, 1));
-  }
+  CU(joint_neg_inverse(ctx, st, L, b_W.as<double>(), wstride, X));
   const int nchunks = (int)sym_tiles(ntiles(N));
   CU(b_gpart.alloc(ctx, (size_t)m * nchunks * 2 * sizeof(double)));
   CU(b_g3.alloc(ctx, (size_t)m * 3 * sizeof(double)));
@@ -825,4 +829,203 @@ extern "C" int lmm_ilmm_logpdf_grad_terms(lmm_ctx* ctx, const lmm_gp_desc* laten
   if (ctx && !grad_terms) return ctx->fail(LMM_E_ARG, "null grad_terms");
   return ilmm_logpdf_grad(ctx, latents, m, x, N, D, H, p, sigma2, y, out_dim, out_logpdf, grad_latents, grad_ard, grad_sigma2, grad_y, grad_H,
                           grad_terms, info);
+}
+// ------------------------------------------------------------------------------------------------
+// rrule of the missing-data logpdf of the dense model (the value of lmm_ilmm_masked_posterior).  Over the observed entries
+// a = (j_a, i_a):  C_ab = Σ_l H[j_a,l] H[j_b,l] k_l(x_{i_a}, x_{i_b}) + σ² [a = b],  δ_a = y_a - Σ_l H[j_a,l] m_l,
+// α = C^{-1}δ,  G = (αα' - C^{-1})/2:
+//   d/dθ_{l,t} = Σ_ab G_ab H[j_a,l] H[j_b,l] ∂k_l/∂θ_t            (kgrad_masked_kernel, with the potri's -C^{-1})
+//   d/dH[j,l]  = 2 Σ_{a: j_a = j} Σ_b G_ab H[j_b,l] k_l(a,b) + m_l Σ_{a: j_a = j} α_a
+//   d/dm_l     = Σ_a α_a H[j_a,l],   d/dσ² = tr G = (α'α - tr C^{-1})/2,   d/dy_a = -α_a (0 at NaN entries)
+// Workspace: the packed factor and the potri's square X (≈ 12 nobs² bytes); X is freed before the contraction's partials.
+// ------------------------------------------------------------------------------------------------
+namespace lmm_host {
+int ilmm_masked_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D, const double* H, int p,
+                            double sigma2, const double* y, int out_dim, double* out_logpdf, double* grad_latents, double* grad_ard,
+                            double* grad_sigma2, double* grad_y, double* grad_H, double* grad_terms, int* n_observed, int* info) {
+  if (!ctx) return LMM_E_ARG;
+  std::lock_guard<std::mutex> lk(ctx->mu);
+  int rc = check_common(ctx, latents, m, x, N, D, p, out_dim);
+  if (rc) return rc;
+  if (!grad_terms && (rc = reject_composite(ctx, latents, m))) return rc;
+  if (!H || !y) return ctx->fail(LMM_E_ARG, "null pointer");
+  if (!(sigma2 > 0.0)) return ctx->fail(LMM_E_ARG, "noise variance must be positive");
+  if (is_device_ptr(y) || is_device_ptr(H)) return ctx->fail(LMM_E_UNSUPPORTED, "the missing-data path takes host y and H (the mask is read on the host)");
+  CU(cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  for (double& t : ctx->timings) t = 0.0;
+  std::vector<int> obs;
+  std::vector<double> delta;
+  masked_observations(latents, m, H, p, N, y, obs, delta);
+  const int nobs = (int)obs.size();
+  if (n_observed) *n_observed = nobs;
+  if (nobs == 0) return ctx->fail(LMM_E_ARG, "every observation is missing");
+  if (nobs > (1 << 20)) return ctx->fail(LMM_E_UNSUPPORTED, "joint dimension too large");
+  const int bnt = ntiles(nobs), ntl = (int)sym_tiles(bnt);
+  const size_t bpad = (size_t)bnt * TILE, wstride = (size_t)bnt * TT;
+  std::vector<int> seg(p + 1, 0);  // the entries of output j are [seg[j], seg[j+1]) (obs is sorted by outputs)
+  for (int o : obs) ++seg[o / N + 1];
+  for (int j = 0; j < p; ++j) seg[j + 1] += seg[j];
+  CU(cudaEventRecord(ctx->ev[0], st));
+  DevBuf b_x, b_params, b_H, b_obs, b_seg, b_delta, b_L, b_W, b_X, b_logdet, b_info, b_quad, b_r, b_z, b_alpha, b_tpart, b_rpart, b_cpart,
+      b_v, b_gterms, b_gH, b_diag;
+  CU(b_x.alloc(ctx, (size_t)N * D * sizeof(double)));
+  CU(copy_in(ctx, b_x.as<double>(), x, (size_t)N * D));
+  std::vector<double> noise0(m, 0.0);
+  if ((rc = upload_params(ctx, b_params, latents, noise0.data(), 0, m, D))) return rc;
+  CU(b_H.alloc(ctx, (size_t)p * m * sizeof(double)));
+  CU(copy_in(ctx, b_H.as<double>(), H, (size_t)p * m));
+  CU(b_obs.alloc(ctx, (size_t)nobs * sizeof(int)));
+  CU(b_seg.alloc(ctx, (size_t)(p + 1) * sizeof(int)));
+  ctx->h2d += (int64_t)((size_t)(nobs + p + 1) * sizeof(int));
+  CU(cudaMemcpyAsync(b_obs.p, obs.data(), (size_t)nobs * sizeof(int), cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(b_seg.p, seg.data(), (size_t)(p + 1) * sizeof(int), cudaMemcpyHostToDevice, st));
+  CU(b_delta.alloc(ctx, bpad * sizeof(double)));
+  CU(cudaMemsetAsync(b_delta.p, 0, bpad * sizeof(double), st));
+  CU(copy_in(ctx, b_delta.as<double>(), delta.data(), (size_t)nobs));
+  // factor, logdet, α (as lmm_ilmm_masked_posterior)
+  CU(b_L.alloc(ctx, sym_tiles(bnt) * TT * sizeof(double)));
+  CU(b_W.alloc(ctx, (size_t)bnt * TT * sizeof(double)));
+  CU(b_logdet.alloc(ctx, sizeof(double)));
+  CU(b_info.alloc(ctx, sizeof(int)));
+  CU(b_quad.alloc(ctx, sizeof(double)));
+  CU(cudaMemsetAsync(b_logdet.p, 0, sizeof(double), st));
+  CU(cudaMemsetAsync(b_info.p, 0, sizeof(int), st));
+  TiledSym L{b_L.as<double>(), bnt, sym_tiles(bnt) * TT};
+  CU(launch_assemble_masked(st, L, b_obs.as<int>(), nobs, b_x.as<double>(), N, D, b_params.as<LatentParams>(), m, p, b_H.as<double>(), sigma2,
+                            ctx->distance_form));
+  ++ctx->launches;
+  {
+    PartitionScope scope(ctx);
+    CU(chol_factor(ctx, L, b_W.as<double>(), wstride, 1, b_logdet.as<double>(), b_info.as<int>()));
+  }
+  CU(b_r.alloc(ctx, bpad * sizeof(double)));
+  CU(b_z.alloc(ctx, bpad * sizeof(double)));
+  CU(b_alpha.alloc(ctx, bpad * sizeof(double)));
+  CU(cudaMemcpyAsync(b_r.p, b_delta.p, bpad * sizeof(double), cudaMemcpyDeviceToDevice, st));
+  CU(launch_fwd_solve(st, L, b_W.as<double>(), wstride, b_r.as<double>(), b_z.as<double>(), bpad, 1, &ctx->launches));
+  CU(launch_sumsq(st, b_z.as<double>(), bpad, (int)bpad, 1, b_quad.as<double>()));
+  CU(cudaMemcpyAsync(b_r.p, b_z.p, bpad * sizeof(double), cudaMemcpyDeviceToDevice, st));
+  CU(launch_bwd_solve(st, L, b_W.as<double>(), wstride, b_r.as<double>(), b_alpha.as<double>(), bpad, 1, &ctx->launches));
+  ++ctx->launches;
+  // potri into the factor's tiles, then the contraction (X is released first: the partials reuse its memory)
+  CU(b_X.alloc(ctx, (size_t)bnt * bnt * TT * sizeof(double)));
+  TiledRect X{b_X.as<double>(), bnt, bnt, (size_t)bnt * bnt * TT};
+  CU(joint_neg_inverse(ctx, st, L, b_W.as<double>(), wstride, X));
+  b_X.release();
+  b_W.release();
+  int max_terms;
+  bool terms_ard;
+  terms_shape(latents, 0, m, max_terms, terms_ard);
+  CU(b_tpart.alloc(ctx, (size_t)m * ntl * TERM_SLOTS * sizeof(double)));
+  CU(b_rpart.alloc(ctx, (size_t)m * ntl * TILE * sizeof(double)));
+  CU(b_cpart.alloc(ctx, (size_t)m * ntl * TILE * sizeof(double)));
+  CU(b_v.alloc(ctx, (size_t)m * nobs * sizeof(double)));
+  CU(b_gterms.alloc(ctx, (size_t)m * TERM_SLOTS * sizeof(double)));
+  CU(b_gH.alloc(ctx, (size_t)p * m * sizeof(double)));
+  CU(b_diag.alloc(ctx, sizeof(double)));
+  CU(launch_kgrad_masked(st, L, b_obs.as<int>(), nobs, b_x.as<double>(), N, D, b_params.as<LatentParams>(), m, p, b_H.as<double>(),
+                         b_alpha.as<double>(), max_terms, terms_ard, ctx->distance_form, b_seg.as<int>(), b_tpart.as<double>(),
+                         b_rpart.as<double>(), b_cpart.as<double>(), b_v.as<double>(), b_gterms.as<double>(), b_gH.as<double>(),
+                         b_diag.as<double>()));
+  ctx->launches += 5;
+  double hlogdet = 0.0, hquad = 0.0, hdiag = 0.0;
+  int hinfo = 0;
+  std::vector<double> ha(nobs), hterms((size_t)m * TERM_SLOTS), hgH((size_t)p * m);
+  CU(copy_out(ctx, &hlogdet, b_logdet.p, sizeof(double)));
+  CU(copy_out(ctx, &hquad, b_quad.p, sizeof(double)));
+  CU(copy_out(ctx, &hinfo, b_info.p, sizeof(int)));
+  CU(copy_out(ctx, &hdiag, b_diag.p, sizeof(double)));
+  CU(copy_out(ctx, ha.data(), b_alpha.p, (size_t)nobs * sizeof(double)));
+  CU(copy_out(ctx, hterms.data(), b_gterms.p, hterms.size() * sizeof(double)));
+  CU(copy_out(ctx, hgH.data(), b_gH.p, hgH.size() * sizeof(double)));
+  CU(cudaEventRecord(ctx->ev[1], st));
+  CU(cudaStreamSynchronize(st));
+  {
+    float ms = 0;
+    cudaEventElapsedTime(&ms, ctx->ev[0], ctx->ev[1]);
+    ctx->timings[0] = ms;
+  }
+  if (hinfo > 0) {
+    if (info) *info = hinfo > nobs ? nobs : hinfo;
+    ctx->err = "PosDefException: the covariance of the observed entries is not positive definite";
+    return hinfo > nobs ? nobs : hinfo;
+  }
+  if (info) *info = 0;
+  if (out_logpdf) *out_logpdf = -((double)nobs * LOG2PI + hlogdet + hquad) / 2.0;
+  std::vector<double> asum(p, 0.0);  // Σ_{a: j_a = j} α_a
+  double aa = 0.0;
+  for (int j = 0; j < p; ++j)
+    for (int a = seg[j]; a < seg[j + 1]; ++a) asum[j] += ha[a];
+  for (int a = 0; a < nobs; ++a) aa += ha[a] * ha[a];
+  if (grad_latents)
+    for (int l = 0; l < m; ++l) {
+      double gm = 0.0;
+      for (int j = 0; j < p; ++j) gm += H[(size_t)l * p + j] * asum[j];
+      grad_latents[(size_t)l * 3 + 0] = hterms[(size_t)l * TERM_SLOTS + 0];
+      grad_latents[(size_t)l * 3 + 1] = hterms[(size_t)l * TERM_SLOTS + 1];
+      grad_latents[(size_t)l * 3 + 2] = gm;
+    }
+  if (grad_ard)
+    for (int l = 0; l < m; ++l)
+      for (int k = 0; k < D; ++k)
+        grad_ard[(size_t)l * D + k] = (latents[l].ard && k < MAX_ARD) ? hterms[(size_t)l * TERM_SLOTS + 3 + k] : 0.0;
+  if (grad_terms) std::copy(hterms.begin(), hterms.end(), grad_terms);
+  if (grad_sigma2) *grad_sigma2 = 0.5 * (aa + hdiag);
+  if (grad_y) {
+    std::fill(grad_y, grad_y + (size_t)p * N, 0.0);
+    for (int a = 0; a < nobs; ++a) grad_y[obs[a]] = -ha[a];
+  }
+  if (grad_H)
+    for (int l = 0; l < m; ++l)
+      for (int j = 0; j < p; ++j) grad_H[(size_t)l * p + j] = hgH[(size_t)l * p + j] + latents[l].mean_const * asum[j];
+  return LMM_OK;
+}
+}  // namespace lmm_host
+
+extern "C" int lmm_ilmm_masked_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D, const double* H,
+                                           int p, double sigma2, const double* y, int out_dim, double* out_logpdf, double* grad_latents,
+                                           double* grad_ard, double* grad_sigma2, double* grad_y, double* grad_H, double* grad_terms,
+                                           int* n_observed, int* info) {
+  return ilmm_masked_logpdf_grad(ctx, latents, m, x, N, D, H, p, sigma2, y, out_dim, out_logpdf, grad_latents, grad_ard, grad_sigma2, grad_y,
+                                 grad_H, grad_terms, n_observed, info);
+}
+
+// Per-input mask: the OILMM gradient on the observed inputs (gather, call, scatter); grad_y is 0 at the missing inputs.
+extern "C" int lmm_oilmm_masked_logpdf_grad(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D, const double* U,
+                                            const double* S, int p, double sigma2, const double* y, int out_dim, double* out_logpdf,
+                                            double* grad_latents, double* grad_ard, double* grad_sigma2, double* grad_y, double* grad_U,
+                                            double* grad_S, double* grad_terms, int* n_observed_inputs, int* info_latent) {
+  if (!ctx) return LMM_E_ARG;
+  {
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    int rc = check_common(ctx, latents, m, x, N, D, p, out_dim);
+    if (rc) return rc;
+    if (!U || !S || !y) return ctx->fail(LMM_E_ARG, "null pointer");
+    if (is_device_ptr(y) || is_device_ptr(x)) return ctx->fail(LMM_E_UNSUPPORTED, "the missing-data path takes host x and y (the mask is read on the host)");
+  }
+  std::vector<int> keep;
+  if (!per_input_mask(y, p, N, keep)) {
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    return ctx->fail(LMM_E_UNSUPPORTED, "the mask is not per-input (some outputs observed, some missing at one input): use lmm_ilmm_masked_logpdf_grad");
+  }
+  const int No = (int)keep.size();
+  if (n_observed_inputs) *n_observed_inputs = No;
+  if (No == 0) {
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    return ctx->fail(LMM_E_ARG, "every observation is missing");
+  }
+  std::vector<double> xo((size_t)No * D), yo((size_t)p * No), gyo(grad_y ? (size_t)p * No : 0);
+  for (int k = 0; k < No; ++k) {
+    for (int d = 0; d < D; ++d) xo[(size_t)k * D + d] = x[(size_t)keep[k] * D + d];
+    for (int j = 0; j < p; ++j) yo[(size_t)j * No + k] = y[(size_t)j * N + keep[k]];
+  }
+  const int rc = oilmm_logpdf_grad(ctx, latents, m, xo.data(), No, D, U, S, p, sigma2, yo.data(), out_dim, out_logpdf, grad_latents, grad_ard,
+                                   grad_sigma2, grad_y ? gyo.data() : nullptr, grad_U, grad_S, grad_terms, info_latent);
+  if (rc == LMM_OK && grad_y) {
+    std::fill(grad_y, grad_y + (size_t)p * N, 0.0);
+    for (int k = 0; k < No; ++k)
+      for (int j = 0; j < p; ++j) grad_y[(size_t)j * N + keep[k]] = gyo[(size_t)j * No + k];
+  }
+  return rc;
 }

@@ -940,6 +940,35 @@ extern "C" int lmm_imogp_posterior_noise(lmm_ctx* ctx, const lmm_gp_desc* fs, in
 // the ground truth of the ILMM, test/ilmm.jl:5): one factor of the (n_obs x n_obs) covariance, assembled straight into the
 // factor tiles from the index list of observed entries.  With nothing missing it equals the ILMM's dense form.
 // ------------------------------------------------------------------------------------------------
+namespace lmm_host {
+// Observed entries of a by-outputs y (host, NaN = missing): obs[a] = j*N + i ascending, δ_a = y_a - (H m)_j.
+void masked_observations(const lmm_gp_desc* latents, int m, const double* H, int p, int N, const double* y, std::vector<int>& obs,
+                         std::vector<double>& delta) {
+  std::vector<double> hm(p, 0.0);
+  for (int j = 0; j < p; ++j)
+    for (int a = 0; a < m; ++a) hm[j] += H[(size_t)a * p + j] * latents[a].mean_const;
+  for (int j = 0; j < p; ++j)
+    for (int i = 0; i < N; ++i) {
+      const double v = y[(size_t)j * N + i];
+      if (v == v) {  // not NaN
+        obs.push_back(j * N + i);
+        delta.push_back(v - hm[j]);
+      }
+    }
+}
+// Inputs at which every output is observed, for a PER-INPUT mask (at each input all p outputs observed or all NaN).
+// Returns false if the mask is not per-input.
+bool per_input_mask(const double* y, int p, int N, std::vector<int>& keep) {
+  for (int i = 0; i < N; ++i) {
+    int nan = 0;
+    for (int j = 0; j < p; ++j) nan += (y[(size_t)j * N + i] != y[(size_t)j * N + i]) ? 1 : 0;
+    if (nan == 0) keep.push_back(i);
+    else if (nan != p) return false;
+  }
+  return true;
+}
+}  // namespace lmm_host
+
 extern "C" int lmm_ilmm_masked_posterior(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D, const double* H,
                                          int p, double sigma2, const double* y, int out_dim, lmm_post** out_post, double* out_logpdf,
                                          int* n_observed, int* info) {
@@ -957,17 +986,7 @@ extern "C" int lmm_ilmm_masked_posterior(lmm_ctx* ctx, const lmm_gp_desc* latent
   // observed entries and centred observations (host: a scan of p*N doubles)
   std::vector<int> obs;
   std::vector<double> delta;
-  std::vector<double> hm(p, 0.0);
-  for (int j = 0; j < p; ++j)
-    for (int a = 0; a < m; ++a) hm[j] += H[(size_t)a * p + j] * latents[a].mean_const;
-  for (int j = 0; j < p; ++j)
-    for (int i = 0; i < N; ++i) {
-      const double v = y[(size_t)j * N + i];
-      if (v == v) {  // not NaN
-        obs.push_back(j * N + i);
-        delta.push_back(v - hm[j]);
-      }
-    }
+  masked_observations(latents, m, H, p, N, y, obs, delta);
   const int nobs = (int)obs.size();
   if (n_observed) *n_observed = nobs;
   if (nobs == 0) return ctx->fail(LMM_E_ARG, "every observation is missing");
@@ -1229,14 +1248,9 @@ extern "C" int lmm_oilmm_masked_posterior(lmm_ctx* ctx, const lmm_gp_desc* laten
     if (is_device_ptr(y) || is_device_ptr(x)) return ctx->fail(LMM_E_UNSUPPORTED, "the missing-data path takes host x and y (the mask is read on the host)");
   }
   std::vector<int> keep;
-  for (int i = 0; i < N; ++i) {
-    int nan = 0;
-    for (int j = 0; j < p; ++j) nan += (y[(size_t)j * N + i] != y[(size_t)j * N + i]) ? 1 : 0;
-    if (nan == 0) keep.push_back(i);
-    else if (nan != p) {
-      std::lock_guard<std::mutex> lk(ctx->mu);
-      return ctx->fail(LMM_E_UNSUPPORTED, "the mask is not per-input (some outputs observed, some missing at one input): use lmm_ilmm_masked_posterior");
-    }
+  if (!per_input_mask(y, p, N, keep)) {
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    return ctx->fail(LMM_E_UNSUPPORTED, "the mask is not per-input (some outputs observed, some missing at one input): use lmm_ilmm_masked_posterior");
   }
   const int No = (int)keep.size();
   if (n_observed_inputs) *n_observed_inputs = No;

@@ -338,6 +338,9 @@ size_t rowcyclic_dist_workspace_tiles(int nrows, int G, int ob);
 int rowcyclic_dist_block(const lmm_ctx* ctx, int nc);
 cudaError_t trsm_right_lt(lmm_ctx* ctx, TiledRect X, TiledSym L, const double* W, size_t wstride, int batch, const LatentParams* xbound = nullptr);
 cudaError_t trsm_right_lt_upper(lmm_ctx* ctx, cudaStream_t st, TiledRect X, TiledSym L, const double* W, size_t wstride, int batch);
+void masked_observations(const lmm_gp_desc* latents, int m, const double* H, int p, int N, const double* y, std::vector<int>& obs,
+                         std::vector<double>& delta);
+bool per_input_mask(const double* y, int p, int N, std::vector<int>& keep);
 
 }  // namespace lmm_host
 namespace lmm_host {

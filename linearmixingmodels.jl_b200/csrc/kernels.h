@@ -185,6 +185,14 @@ cudaError_t launch_kgrad_ard(cudaStream_t st, const double* mat_base, size_t mat
 cudaError_t launch_kgrad_terms(cudaStream_t st, const double* mat_base, size_t mat_batch_stride, int off_per_lat, const double* x, int N,
                                int D, const LatentParams* params, int nlat, int max_terms, bool any_ard, const double* alpha,
                                size_t alpha_stride, int form, double* partial, double* out);
+// Missing-data dense model: contraction of G = (αα' - C^{-1})/2 over the (nobs x nobs) observed-entry matrix (negCinv = -C^{-1},
+// batch 1; obs sorted by outputs, seg[j] = first entry of output j, seg[p] = nobs; x [N][D] raw points, Hm p x m col-major).
+// out_terms[l*44 + ...] as launch_kgrad_terms with the weight H[j_a,l] H[j_b,l]; out_H[l*p + j] = 2 Σ_{a: j_a = j} Σ_b G_ab
+// H[j_b,l] k_l(a,b); out_diag[0] = tr(-C^{-1}).  Scratch (ntl = sym_tiles(negCinv.nt)): tpart m*ntl*44, rowpart and colpart
+// m*ntl*128 each, v m*nobs doubles.
+cudaError_t launch_kgrad_masked(cudaStream_t st, TiledSym negCinv, const int* obs, int nobs, const double* x, int N, int D, const LatentParams* params,
+                                int m, int p, const double* Hm, const double* alpha, int max_terms, bool any_ard, int form, const int* seg,
+                                double* tpart, double* rowpart, double* colpart, double* v, double* out_terms, double* out_H, double* out_diag);
 cudaError_t launch_scale_sub(cudaStream_t st, double* v, const double* a, double sa, const double* b, size_t n);
 }  // namespace lmm
 

@@ -527,6 +527,86 @@ function posterior_missing(fx::FiniteGP{<:OILMM{<:IndependentMOGP{<:Vector{<:GP}
     return ILMM(IndependentMOGP([DeviceLatentPosterior(owner, i - 1, f) for (i, f) in enumerate(fs.fs)]), H), lp[], Int(nobs[])
 end
 
+# logpdf of the observed (non-NaN) entries of y: the value of posterior_missing without keeping the factor
+function logpdf_missing(fx::FiniteGP{<:ILMM{<:IndependentMOGP{<:Vector{<:GP}}}}, y::AbstractVector{<:Real})
+    fs, H, σ², x = unpack(fx)
+    X, D = points(x)
+    descs, keep = gpdescs(fs.fs)
+    Hm = Matrix{Float64}(collect(H))
+    lp = Ref{Float64}(0.0); nobs = Ref{Cint}(0); info = Ref{Cint}(0)
+    check(GC.@preserve keep ccall((:lmm_ilmm_masked_posterior, liblmm), Cint,
+        (Ptr{Cvoid}, Ptr{GpDesc}, Cint, Ptr{Float64}, Cint, Cint, Ptr{Float64}, Cint, Float64, Ptr{Float64}, Cint,
+         Ptr{Ptr{Cvoid}}, Ptr{Float64}, Ptr{Cint}, Ptr{Cint}),
+        ctx(), descs, length(descs), X, length(x), D, Hm, size(Hm, 1), Float64(σ²), Vector{Float64}(y), fx.x.out_dim, C_NULL, lp, nobs, info))
+    return lp[]
+end
+function logpdf_missing(fx::FiniteGP{<:OILMM{<:IndependentMOGP{<:Vector{<:GP}}}}, y::AbstractVector{<:Real})
+    fs, H, σ², x = unpack(fx)
+    X, D = points(x)
+    descs, keep = gpdescs(fs.fs)
+    lp = Ref{Float64}(0.0); nobs = Ref{Cint}(0); il = Ref{Cint}(-1)
+    rc = GC.@preserve keep ccall((:lmm_oilmm_masked_posterior, liblmm), Cint,
+        (Ptr{Cvoid}, Ptr{GpDesc}, Cint, Ptr{Float64}, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Cint, Float64, Ptr{Float64}, Cint,
+         Ptr{Ptr{Cvoid}}, Ptr{Float64}, Ptr{Cint}, Ptr{Cint}),
+        ctx(), descs, length(descs), X, length(x), D, Matrix{Float64}(H.U), Vector{Float64}(diag(H.S)), size(H, 1), Float64(σ²),
+        Vector{Float64}(y), fx.x.out_dim, C_NULL, lp, nobs, il)
+    if rc == -3   # the mask is not per-input: the dense model on H = U sqrt(S)
+        return invoke(logpdf_missing, Tuple{FiniteGP{<:ILMM{<:IndependentMOGP{<:Vector{<:GP}}}},AbstractVector{<:Real}}, fx, y)
+    end
+    check(rc)
+    return lp[]
+end
+
+# rrules of logpdf_missing, modelled on the two logpdf rrules above.  NaN entries of y get a zero tangent.
+function ChainRulesCore.rrule(::typeof(logpdf_missing), fx::FiniteGP{<:ILMM{<:IndependentMOGP{<:Vector{<:GP}},<:Matrix{Float64}}},
+                              y::AbstractVector{<:Real})
+    fs, H, σ², x = unpack(fx)
+    X, D = points(x)
+    descs, keep = gpdescs(fs.fs); m = length(descs)
+    out = Ref{Float64}(0.0); gs2 = Ref{Float64}(0.0); nobs = Ref{Cint}(0); info = Ref{Cint}(0)
+    gl = Matrix{Float64}(undef, 3, m); gy = Vector{Float64}(undef, length(y)); gH = similar(H)
+    gt = Matrix{Float64}(undef, GRAD_TERM_DOUBLES, m)
+    check(GC.@preserve keep ccall((:lmm_ilmm_masked_logpdf_grad, liblmm), Cint,
+        (Ptr{Cvoid}, Ptr{GpDesc}, Cint, Ptr{Float64}, Cint, Cint, Ptr{Float64}, Cint, Float64, Ptr{Float64}, Cint,
+         Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Cint}, Ptr{Cint}),
+        ctx(), descs, m, X, length(x), D, H, size(H, 1), Float64(σ²), Vector{Float64}(y), fx.x.out_dim, out, gl, C_NULL, gs2, gy, gH, gt,
+        nobs, info))
+    function logpdf_missing_pullback(Δ)
+        Σy_tangent = Tangent{typeof(fx.Σy)}(; diag = Tangent{typeof(fx.Σy.diag)}(; value = Δ * gs2[]))
+        f_tangent = Tangent{typeof(fx.f)}(; H = Δ .* gH)
+        return NoTangent(), Tangent{typeof(fx)}(; f = f_tangent, Σy = Σy_tangent), Δ .* gy
+    end
+    return out[], logpdf_missing_pullback
+end
+function ChainRulesCore.rrule(::typeof(logpdf_missing), fx::FiniteGP{<:OILMM{<:IndependentMOGP{<:Vector{<:GP}}}}, y::AbstractVector{<:Real})
+    fs, H, σ², x = unpack(fx)
+    X, D = points(x)
+    descs, keep = gpdescs(fs.fs); m = length(descs)
+    out = Ref{Float64}(0.0); gs2 = Ref{Float64}(0.0); nobs = Ref{Cint}(0); il = Ref{Cint}(-1)
+    gl = Matrix{Float64}(undef, 3, m); gy = Vector{Float64}(undef, length(y))
+    gU = Matrix{Float64}(undef, size(H, 1), m); gS = Vector{Float64}(undef, m)
+    gt = Matrix{Float64}(undef, GRAD_TERM_DOUBLES, m)
+    rc = GC.@preserve keep ccall((:lmm_oilmm_masked_logpdf_grad, liblmm), Cint,
+        (Ptr{Cvoid}, Ptr{GpDesc}, Cint, Ptr{Float64}, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Cint, Float64, Ptr{Float64}, Cint,
+         Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Cint}, Ptr{Cint}),
+        ctx(), descs, m, X, length(x), D, Matrix{Float64}(H.U), Vector{Float64}(diag(H.S)), size(H, 1), Float64(σ²),
+        Vector{Float64}(y), fx.x.out_dim, out, gl, C_NULL, gs2, gy, gU, gS, gt, nobs, il)
+    if rc == -3   # the mask is not per-input: the dense model on H = U sqrt(S), whose gradient is w.r.t. H
+        Hm = Matrix{Float64}(collect(H)); gH = similar(Hm); info = Ref{Cint}(0)
+        rc = GC.@preserve keep ccall((:lmm_ilmm_masked_logpdf_grad, liblmm), Cint,
+            (Ptr{Cvoid}, Ptr{GpDesc}, Cint, Ptr{Float64}, Cint, Cint, Ptr{Float64}, Cint, Float64, Ptr{Float64}, Cint,
+             Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Cint}, Ptr{Cint}),
+            ctx(), descs, m, X, length(x), D, Hm, size(Hm, 1), Float64(σ²), Vector{Float64}(y), fx.x.out_dim, out, gl, C_NULL, gs2, gy, gH, gt,
+            nobs, info)
+    end
+    check(rc)
+    function logpdf_missing_pullback(Δ)
+        Σy_tangent = Tangent{typeof(fx.Σy)}(; diag = Tangent{typeof(fx.Σy.diag)}(; value = Δ * gs2[]))
+        return NoTangent(), Tangent{typeof(fx)}(; Σy = Σy_tangent), Δ .* gy
+    end
+    return out[], logpdf_missing_pullback
+end
+
 # --- one latent of a posterior on its own: mean_and_var(get_latent_gp(post).fs[i](x*, σ²)), the call src/oilmm.jl:61 makes ---
 function AbstractGPs.mean_and_var(fx::FiniteGP{<:DeviceLatentPosterior})
     X, _ = points(fx.x)
