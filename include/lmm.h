@@ -286,6 +286,22 @@ int lmm_post_logpdf(lmm_post* post, const double* xs, int Ns, double sigma2, con
  * own data (α, C, x) and kernel hyper-parameters are held fixed.  All outputs nullable. */
 int lmm_post_logpdf_grad(lmm_post* post, const double* xs, int Ns, double sigma2, const double* ys,
                          double* out_logpdf, double* grad_sigma2, double* grad_y, int* info_latent);
+/* The same logpdf differentiated through the conditioning as well: logpdf(posterior(f(x, σ²), y)(x*, σ*²), y*) w.r.t.
+ * the latents' hyper-parameters and means, the training σ² and y, σ*², y*, and (OILMM) U and S -- held-out / forecast
+ * likelihood and the conditional likelihood of new data given old.  Per-latent posteriors only (OILMM, IndependentMOGP,
+ * also the OILMM handles of lmm_oilmm_masked_posterior, whose y_train is the p x n_observed_inputs block); joint and
+ * sequentially conditioned handles return LMM_E_UNSUPPORTED.  y_train (required) is the p*N data the handle was
+ * conditioned on: T y_train - m must reproduce the handle's δ to 1e-12 (norm-relative), else LMM_E_ARG.
+ * out_logpdf, grad_sigma2 (σ*²) and grad_y (y*, p*Ns) are what lmm_post_logpdf_grad returns, bit for bit.  grad_latents
+ * (m x 3: term 0's variance and inv_lengthscale, mean_const), grad_ard (m x D) and grad_terms (m x LMM_MAX_TERMS x
+ * LMM_GRAD_TERM_STRIDE) use the layouts of lmm_oilmm_logpdf_grad_terms; grad_train_sigma2 is d/dσ², grad_train_y p*N by
+ * outputs; grad_U (p x m column-major) and grad_S (m) are the Euclidean gradient, as lmm_oilmm_logpdf_grad returns them,
+ * and must be NULL for an IndependentMOGP handle (LMM_E_ARG).  Every output is nullable.  The handle is not changed. */
+int lmm_post_logpdf_grad_full(lmm_post* post, const double* xs, int Ns, double sigma2, const double* ys,
+                              const double* y_train, double* out_logpdf, double* grad_sigma2, double* grad_y,
+                              double* grad_latents, double* grad_ard, double* grad_terms,
+                              double* grad_train_sigma2, double* grad_train_y, double* grad_U, double* grad_S,
+                              int* info_latent);
 /* rand(rng, post(x*, σ²))  src/oilmm.jl:40-54 with PosteriorGP latents. */
 int lmm_post_rand(lmm_post* post, const double* xs, int Ns, double sigma2, const double* z_latent,
                   const double* z_noise, double* out, int* info_latent);

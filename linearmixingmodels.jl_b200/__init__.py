@@ -13,6 +13,7 @@ from .api import (  # noqa: F401
     logpdf_terms,
     logpdf_sweep,
     logpdf_and_gradient,
+    predictive_logpdf_and_gradient,
     potrf_batched,
     set_default_context,
     set_ilmm_form,

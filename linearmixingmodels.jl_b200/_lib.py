@@ -93,6 +93,8 @@ SIGNATURES = {
     "lmm_post_condition": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, C.POINTER(_vp), _ip]),
     "lmm_post_logpdf": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _dp, _ip]),
     "lmm_post_logpdf_grad": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _dp, _dp, _vp, _ip]),
+    # through the conditioning: y_train, value, σ*², y*, latents, ard, terms, training σ², training y, U, S, info
+    "lmm_post_logpdf_grad_full": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp, _dp, _dp, _vp, _vp, _vp, _vp, _dp, _vp, _vp, _vp, _ip]),
     "lmm_post_rand": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp, _vp, _ip]),
     "lmm_post_export": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp]),
     "lmm_post_info": (C.c_int, [_vp, _ip, _ip, _ip, _ip, _ip, C.POINTER(C.c_int64)]),

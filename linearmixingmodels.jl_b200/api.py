@@ -1044,8 +1044,9 @@ def logpdf_and_gradient(fx: FiniteGP, y, with_grad_y: bool = False, kernel_terms
     order of {"variance", "inv_lengthscale", "param" (α / r; 0 for kinds without one), "ard" (D,)} -- the gradient w.r.t.
     each term's own hyper-parameters; "variance" / "inv_lengthscale" / "ard" then hold term 0's.  A transform shared by all
     terms is a function of them: for `(k1 + k2) ∘ ScaleTransform(s)` each term carries s_t = s·c_t, so
-    d/ds = Σ_t (s_t / s)·terms[t]["inv_lengthscale"].  A posterior FiniteGP has no kernel gradient (only σ² and y*):
-    `kernel_terms=True` on one raises ValueError."""
+    d/ds = Σ_t (s_t / s)·terms[t]["inv_lengthscale"].  On a posterior FiniteGP this gives σ² and y* only, with the
+    posterior's data and hyper-parameters held fixed, and `kernel_terms=True` raises ValueError: the gradient through the
+    conditioning is `predictive_logpdf_and_gradient`."""
     f = fx.f
     ctx = _ctx_of(fx)
     _require_by_outputs(fx)
@@ -1126,6 +1127,60 @@ def logpdf_and_gradient(fx: FiniteGP, y, with_grad_y: bool = False, kernel_terms
     if with_grad_y:
         grads["y"] = gy
     if isinstance(f, ILMM):
+        grads["U"], grads["S"] = np.ascontiguousarray(gU), gS
+    return out.value, grads
+
+
+def predictive_logpdf_and_gradient(fx_post: FiniteGP, y, y_train, with_grad_y: bool = False):
+    """Value and gradient of the posterior-predictive logpdf `logpdf(posterior(f(x, σ²), y_train)(x*, σ*²), y)`
+    differentiated through the conditioning: the held-out / forecast likelihood, or the likelihood of new data given old,
+    as a function of everything the posterior was built from.  `fx_post` is `post(x*, σ*²)` for a posterior of an OILMM
+    or an IndependentMOGP (a masked OILMM posterior counts as an OILMM over its observed inputs); `y_train` is the data
+    it was conditioned on (p*N by outputs; checked against the posterior).  Joint posteriors (general ILMM, dense Σy,
+    missing data through the dense model) and posteriors conditioned a second time raise ValueError.
+
+    Returns (logpdf, grads) with grads = {
+      "sigma2": d/dσ*² (float)[, "y": d/dy* (p*Ns,)] -- exactly what `logpdf_and_gradient` returns on the posterior,
+      "terms": per latent, per term in `Kernel.all_terms()` order, {"variance", "inv_lengthscale", "param", "ard" (D,)},
+      "variance", "inv_lengthscale", "ard" (m, D): term 0's, "mean_const" (m,),
+      "train": {"sigma2": d/dσ², "y": d/dy_train (p*N,)},
+      "U" (p, m), "S" (m,) for an OILMM: the Euclidean gradient, as `logpdf_and_gradient` returns it}.
+    Hyper-parameters enter the training and the test side through the same kernel, so each entry is the total derivative.
+    A transform shared by all terms is a function of them: for `(k1 + k2) ∘ ScaleTransform(s)` each term carries
+    s_t = s·c_t, so d/ds = Σ_t (s_t / s)·terms[t]["inv_lengthscale"]."""
+    f = fx_post.f
+    ctx = _ctx_of(fx_post)
+    _require_by_outputs(fx_post)
+    owner = _post_owner(fx_post)
+    if owner is None:
+        raise TypeError("predictive_logpdf_and_gradient needs a posterior FiniteGP, post(x*, σ²)")
+    lat = f.f if isinstance(f, ILMM) else f
+    if isinstance(f, ILMM) and f.H.shape[0] != fx_post.x.out_dim:
+        raise RuntimeError("out dim of x != out dim of f.")
+    pts = _points(fx_post.x.x)
+    Ns, D = int(pts.shape[0]), int(pts.shape[1])
+    p = fx_post.x.out_dim
+    yv = _yvec(y, Ns * p)
+    ytr = _yvec(y_train, owner.N * p)
+    fs = lat.fs if isinstance(lat, IndependentMOGP) else lat.prior.fs if isinstance(lat, _JointPosterior) else []
+    m = len(fs)
+    orth = isinstance(f, ILMM) and isinstance(f.H, Orthogonal)
+    out, gs2, gts2, il = C.c_double(), C.c_double(), C.c_double(), C.c_int(-1)
+    gy = np.zeros(Ns * p) if with_grad_y else None
+    gl = np.zeros((m, 3))
+    ga = np.zeros((m, D))
+    gt = np.zeros(m * _lib.LMM_MAX_TERMS * _lib.LMM_GRAD_TERM_STRIDE)
+    gty = np.zeros(owner.N * p)
+    gU = np.zeros((p, m), order="F") if orth else None
+    gS = np.zeros(m) if orth else None
+    rc = ctx.lib.lmm_post_logpdf_grad_full(owner.handle, ptr(pts), Ns, fx_post.sigma2, ptr(yv), ptr(ytr), C.byref(out), C.byref(gs2),
+                                           ptr(gy), ptr(gl), ptr(ga), ptr(gt), C.byref(gts2), ptr(gty), ptr(gU), ptr(gS), C.byref(il))
+    ctx.check(rc, il.value)
+    grads = {"sigma2": gs2.value, "terms": _terms_grads(fs, gt, D), "variance": gl[:, 0].copy(), "inv_lengthscale": gl[:, 1].copy(),
+             "ard": ga, "mean_const": gl[:, 2].copy(), "train": {"sigma2": gts2.value, "y": gty}}
+    if with_grad_y:
+        grads["y"] = gy
+    if orth:
         grads["U"], grads["S"] = np.ascontiguousarray(gU), gS
     return out.value, grads
 

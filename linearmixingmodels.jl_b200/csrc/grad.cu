@@ -467,6 +467,52 @@ __device__ __forceinline__ double ard_factor(const TermParams& q, const double* 
 constexpr int GRAD_TERM_STRIDE = 3 + MAX_ARD;            // == LMM_GRAD_TERM_STRIDE
 constexpr int GRAD_TERM_SLOTS = MAX_TERMS * GRAD_TERM_STRIDE;
 
+// Adds w2 ∂K/∂θ at one element to the per-term sums acc (variance, s, param) and aca (ARD).  kap / ds / dp / wa are the
+// terms' per-unit-variance values of term_grad.  Weight of term u: w2 for a sum; w2 Π_{v≠u} k_v for a product, from prefix /
+// suffix products (a term far from its own centre underflows to exactly 0, so K / k_u is no option).
+template <int NT, bool ARD>
+__device__ __forceinline__ void accumulate_terms(const TermParams* tp, bool product, double w2, const double* kap, const double* ds,
+                                                 const double* dp, const double* wa, const double* pa, const double* pb, int D,
+                                                 double (*acc)[3], double (*aca)[MAX_ARD]) {
+  double suf[NT + 1];
+  suf[NT] = 1.0;
+  if (product) {
+#pragma unroll
+    for (int u = NT - 1; u >= 0; --u) suf[u] = suf[u + 1] * (tp[u].variance * kap[u]);
+  }
+  double pre = 1.0;
+#pragma unroll
+  for (int u = 0; u < NT; ++u) {
+    const double w = product ? w2 * pre * suf[u + 1] : w2;
+    if (product) pre *= tp[u].variance * kap[u];
+    acc[u][0] = fma(w, kap[u], acc[u][0]);
+    acc[u][1] = fma(w, ds[u], acc[u][1]);
+    acc[u][2] = fma(w, dp[u], acc[u][2]);
+    if (ARD && tp[u].ard_dim && wa[u] != 0.0) {
+      const double wk = w * wa[u];
+#pragma unroll
+      for (int k = 0; k < MAX_ARD; ++k)
+        if (k < D) aca[ARD ? u : 0][k] = fma(wk, ard_factor(tp[u], pa, pb, k), aca[ARD ? u : 0][k]);
+    }
+  }
+}
+
+// Per-thread term sums -> wsum[slot][warp] by warp shuffles (fixed order, no atomics).
+template <int NT, bool ARD>
+__device__ __forceinline__ void warp_term_sums(double (*acc)[3], double (*aca)[MAX_ARD], double (*wsum)[8]) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int u = 0; u < NT; ++u) {
+#pragma unroll
+    for (int j = 0; j < (ARD ? GRAD_TERM_STRIDE : 3); ++j) {
+      double v = j < 3 ? acc[u][j] : aca[ARD ? u : 0][j - 3];
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+      if (lane == 0) wsum[u * GRAD_TERM_STRIDE + j][warp] = v;
+    }
+  }
+}
+
 // One lower-triangle chunk of one latent with NT terms; ARD: some term has an ARDTransform.  The per-thread sums are
 // reduced across each warp by shuffles and written to wsum[slot][warp] (fixed order, no atomics).
 template <int NT, bool ARD>
@@ -499,41 +545,33 @@ __device__ __forceinline__ void kgrad_terms_body(const TermParams* tp, bool prod
       for (int u = 0; u < NT; ++u) term_grad(tp[u], pa, pb, D, form, kap[u], ds[u], dp[u], wa[u]);
       w2 = 2.0 * G;
     }
-    // weight of term u: 2G for a sum; 2G Π_{v≠u} k_v for a product, from prefix / suffix products (a term far from its
-    // own centre underflows to exactly 0, so K / k_u is no option)
-    double suf[NT + 1];
-    suf[NT] = 1.0;
-    if (product) {
-#pragma unroll
-      for (int u = NT - 1; u >= 0; --u) suf[u] = suf[u + 1] * (tp[u].variance * kap[u]);
-    }
-    double pre = 1.0;
-#pragma unroll
-    for (int u = 0; u < NT; ++u) {
-      const double w = product ? w2 * pre * suf[u + 1] : w2;
-      if (product) pre *= tp[u].variance * kap[u];
-      acc[u][0] = fma(w, kap[u], acc[u][0]);
-      acc[u][1] = fma(w, ds[u], acc[u][1]);
-      acc[u][2] = fma(w, dp[u], acc[u][2]);
-      if (ARD && tp[u].ard_dim && wa[u] != 0.0) {
-        const double wk = w * wa[u];
-#pragma unroll
-        for (int k = 0; k < MAX_ARD; ++k)
-          if (k < D) aca[ARD ? u : 0][k] = fma(wk, ard_factor(tp[u], pa, pb, k), aca[ARD ? u : 0][k]);
-      }
-    }
+    accumulate_terms<NT, ARD>(tp, product, w2, kap, ds, dp, wa, pa, pb, D, acc, aca);
   }
-  const int lane = t & 31, warp = t >> 5;
-#pragma unroll
-  for (int u = 0; u < NT; ++u) {
-#pragma unroll
-    for (int j = 0; j < (ARD ? GRAD_TERM_STRIDE : 3); ++j) {
-      double v = j < 3 ? acc[u][j] : aca[ARD ? u : 0][j - 3];
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
-      if (lane == 0) wsum[u * GRAD_TERM_STRIDE + j][warp] = v;
-    }
+  warp_term_sums<NT, ARD>(acc, aca, wsum);
+}
+
+// Term 0 (the LatentParams' own fields) and the extra terms of a latent -> tp[0 .. MAX_TERMS) (threads 0 .. MAX_TERMS-1).
+__device__ __forceinline__ void stage_terms(const LatentParams* lp, TermParams* tp) {
+  const int t = threadIdx.x;
+  if (t == 0) {
+    tp[0].kind = lp->kind; tp[0].ard_dim = lp->ard_dim; tp[0].variance = lp->variance; tp[0].inv_ls = lp->inv_ls; tp[0].param = lp->param;
+    for (int k = 0; k < MAX_ARD; ++k) tp[0].ard[k] = lp->ard[k];
+  } else if (t < MAX_TERMS) {
+    tp[t] = lp->extra[t - 1];
   }
+}
+
+// Threads t < GRAD_TERM_SLOTS: the CTA's sum of slot t (fixed order over the warps), scaled as a gradient: ∂K/∂θ carries the
+// term's variance (∂K/∂variance does not) and ∂/∂ard_k the 1 / ard_k of ard_factor.  Absent slots are 0.
+__device__ __forceinline__ double cta_slot_sum(const TermParams* tp, int nterms, bool ard, int D, double (*wsum)[8]) {
+  const int t = threadIdx.x, u = t / GRAD_TERM_STRIDE, j = t % GRAD_TERM_STRIDE;
+  double s = 0.0;
+  if (u < nterms && (j < 3 || (ard && tp[u].ard_dim && j - 3 < D))) {
+    for (int w = 0; w < 8; ++w) s += wsum[t][w];
+    if (j >= 1) s *= tp[u].variance;
+    if (j >= 3) s /= tp[u].ard[j - 3];
+  }
+  return s;
 }
 
 // grid (chunks of the lower triangle, latents), storage as kgrad_ard_kernel.  partial[(lat*nchunks + chunk)*GRAD_TERM_SLOTS
@@ -558,12 +596,7 @@ __global__ void __launch_bounds__(256, (NTMAX <= 2 && !ARDANY) ? 2 : 1) kgrad_te
   while ((size_t)I * (I + 1) / 2 > (size_t)tl) --I;
   const int J = tl - (int)((size_t)I * (I + 1) / 2);
   const double* al = alpha + (size_t)lat * alpha_stride;
-  if (t == 0) {
-    tp[0].kind = lp->kind; tp[0].ard_dim = lp->ard_dim; tp[0].variance = lp->variance; tp[0].inv_ls = lp->inv_ls; tp[0].param = lp->param;
-    for (int k = 0; k < MAX_ARD; ++k) tp[0].ard[k] = lp->ard[k];
-  } else if (t < MAX_TERMS) {
-    tp[t] = lp->extra[t - 1];
-  }
+  stage_terms(lp, tp);
   for (int i = t; i < TILE * D; i += 256) {
     const int ra = I * TILE + i / D, rb = J * TILE + i / D;
     xa[i] = ra < N ? x[(size_t)ra * D + i % D] : 0.0;
@@ -587,16 +620,7 @@ __global__ void __launch_bounds__(256, (NTMAX <= 2 && !ARDANY) ? 2 : 1) kgrad_te
   LMM_TERMS_CASE(3, false) LMM_TERMS_CASE(3, true) LMM_TERMS_CASE(4, false) LMM_TERMS_CASE(4, true)
 #undef LMM_TERMS_CASE
   __syncthreads();
-  if (t < GRAD_TERM_SLOTS) {
-    const int u = t / GRAD_TERM_STRIDE, j = t % GRAD_TERM_STRIDE;
-    double s = 0.0;
-    if (u < nterms && (j < 3 || (ard && tp[u].ard_dim && j - 3 < D))) {
-      for (int w = 0; w < 8; ++w) s += wsum[t][w];
-      if (j >= 1) s *= tp[u].variance;  // ∂K/∂θ carries the term's variance (∂K/∂variance does not)
-      if (j >= 3) s /= tp[u].ard[j - 3];
-    }
-    partial[((size_t)lat * gridDim.x + tl) * GRAD_TERM_SLOTS + t] = s;
-  }
+  if (t < GRAD_TERM_SLOTS) partial[((size_t)lat * gridDim.x + tl) * GRAD_TERM_SLOTS + t] = cta_slot_sum(tp, nterms, ard, D, wsum);
 }
 // out[lat*GRAD_TERM_SLOTS + slot] = Σ chunks (fixed order)
 __global__ void __launch_bounds__(256) kgrad_terms_finish_kernel(const double* __restrict__ partial, int nchunks, double* __restrict__ out) {
@@ -630,6 +654,121 @@ cudaError_t launch_kgrad_terms(cudaStream_t st, const double* mat_base, size_t m
   kern<<<grid, 256, smem, st>>>(mat_base, mat_batch_stride, off_per_lat, x, N, D, params, alpha, alpha_stride, form, partial);
   dim3 g2((unsigned)nlat, (unsigned)GRAD_TERM_SLOTS);
   kgrad_terms_finish_kernel<<<g2, 256, 0, st>>>(partial, nchunks, out);
+  return cudaGetLastError();
+}
+
+// ---- posterior-predictive gradient: the rectangular cross block K(x, x*) ----------------------------------------------
+// The posterior-predictive logpdf depends on K(x, x*) through the predictive mean and covariance; its derivative w.r.t.
+// that block is Gc = G + u v' (N x N*, rows: training points, columns: test points).  Every element counts once: the block
+// has no diagonal, so point identity plays no role (two equal points have d = 0 like any other pair).
+template <int NT, bool ARD>
+__device__ __forceinline__ void kgrad_cross_body(const TermParams* tp, bool product, const double* __restrict__ tile, const double* xa,
+                                                 const double* xb, const double* ua, const double* vb, int R, int J, int Na, int Nb, int D,
+                                                 int form, double (*wsum)[8]) {
+  double acc[NT][3], aca[ARD ? NT : 1][MAX_ARD];
+#pragma unroll
+  for (int u = 0; u < NT; ++u) {
+    acc[u][0] = acc[u][1] = acc[u][2] = 0.0;
+#pragma unroll
+    for (int k = 0; k < MAX_ARD; ++k) aca[ARD ? u : 0][k] = 0.0;
+  }
+  for (int e = threadIdx.x; e < TT; e += 256) {
+    const int c = ((e >> 9) << 2) + (e & 3), r = (e >> 2) & 127;  // tile_rc: coalesced reads of the tile
+    if (R * TILE + r >= Na || J * TILE + c >= Nb) continue;
+    const double w = tile[e] + ua[r] * vb[c];
+    const double* pa = xa + (size_t)r * D;
+    const double* pb = xb + (size_t)c * D;
+    double kap[NT], ds[NT], dp[NT], wa[NT];
+#pragma unroll
+    for (int u = 0; u < NT; ++u) term_grad(tp[u], pa, pb, D, form, kap[u], ds[u], dp[u], wa[u]);
+    accumulate_terms<NT, ARD>(tp, product, w, kap, ds, dp, wa, pa, pb, D, acc, aca);
+  }
+  warp_term_sums<NT, ARD>(acc, aca, wsum);
+}
+
+// grid (tiles of G, latents).  partial[(lat*ntiles + tile)*GRAD_TERM_SLOTS + slot] as kgrad_terms_kernel; points RAW
+// ([Na][D] rows, [Nb][D] columns).  NTMAX / ARDANY as kgrad_terms_kernel.
+template <int NTMAX, bool ARDANY>
+__global__ void __launch_bounds__(256, (NTMAX <= 2 && !ARDANY) ? 2 : 1) kgrad_cross_terms_kernel(TiledRect G, const double* __restrict__ xa_raw, int Na,
+                                                                                               const double* __restrict__ xb_raw, int Nb, int D,
+                                                                                               const LatentParams* __restrict__ params,
+                                                                                               const double* __restrict__ u, size_t u_stride,
+                                                                                               const double* __restrict__ v, size_t v_stride, int form,
+                                                                                               double* __restrict__ partial) {
+  extern __shared__ __align__(16) double sm[];
+  double* xa = sm;
+  double* xb = xa + TILE * D;
+  double* ua = xb + TILE * D;
+  double* vb = ua + TILE;
+  __shared__ TermParams tp[MAX_TERMS];
+  __shared__ double wsum[GRAD_TERM_SLOTS][8];
+  const int lat = blockIdx.y, tl = blockIdx.x, t = threadIdx.x;
+  const int R = tl / G.ntc, J = tl % G.ntc;
+  const LatentParams* lp = params + lat;
+  stage_terms(lp, tp);
+  for (int i = t; i < TILE * D; i += 256) {
+    const int ra = R * TILE + i / D, rb = J * TILE + i / D;
+    xa[i] = ra < Na ? xa_raw[(size_t)ra * D + i % D] : 0.0;
+    xb[i] = rb < Nb ? xb_raw[(size_t)rb * D + i % D] : 0.0;
+  }
+  if (t < TILE) {
+    ua[t] = R * TILE + t < Na ? u[(size_t)lat * u_stride + R * TILE + t] : 0.0;
+    vb[t] = J * TILE + t < Nb ? v[(size_t)lat * v_stride + J * TILE + t] : 0.0;
+  }
+  __syncthreads();
+  const int nterms = lp->nterms;
+  const bool product = lp->compose == 2;
+  bool ard = false;
+  for (int q = 0; q < nterms; ++q) ard |= tp[q].ard_dim > 0;
+  const double* tile = G.tile(lat, R, J);
+#define LMM_CROSS_CASE(n, a)                                                                           \
+  if constexpr (n <= NTMAX && (ARDANY || !a))                                                          \
+    if (nterms == n && ard == a) kgrad_cross_body<n, a>(tp, product, tile, xa, xb, ua, vb, R, J, Na, Nb, D, form, wsum);
+  LMM_CROSS_CASE(1, false) LMM_CROSS_CASE(1, true) LMM_CROSS_CASE(2, false) LMM_CROSS_CASE(2, true)
+  LMM_CROSS_CASE(3, false) LMM_CROSS_CASE(3, true) LMM_CROSS_CASE(4, false) LMM_CROSS_CASE(4, true)
+#undef LMM_CROSS_CASE
+  __syncthreads();
+  if (t < GRAD_TERM_SLOTS) partial[((size_t)lat * gridDim.x + tl) * GRAD_TERM_SLOTS + t] = cta_slot_sum(tp, nterms, ard, D, wsum);
+}
+
+cudaError_t launch_kgrad_cross_terms(cudaStream_t st, TiledRect G, const double* xa, int Na, const double* xb, int Nb, int D,
+                                     const LatentParams* params, int nlat, int max_terms, bool any_ard, const double* u, size_t u_stride,
+                                     const double* v, size_t v_stride, int form, double* partial, double* out) {
+  const size_t smem = (size_t)(2 * TILE * D + 2 * TILE) * sizeof(double);
+  const int ntiles_ = G.ntr * G.ntc;
+  dim3 grid((unsigned)ntiles_, (unsigned)nlat);
+  auto kern = any_ard ? (max_terms <= 1 ? kgrad_cross_terms_kernel<1, true> : max_terms == 2 ? kgrad_cross_terms_kernel<2, true>
+                                          : max_terms == 3 ? kgrad_cross_terms_kernel<3, true> : kgrad_cross_terms_kernel<4, true>)
+                      : (max_terms <= 1 ? kgrad_cross_terms_kernel<1, false> : max_terms == 2 ? kgrad_cross_terms_kernel<2, false>
+                                          : max_terms == 3 ? kgrad_cross_terms_kernel<3, false> : kgrad_cross_terms_kernel<4, false>);
+  if (smem + 4096 > 48 * 1024) {  // static shared memory counts against the default limit too
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+  }
+  kern<<<grid, 256, smem, st>>>(G, xa, Na, xb, Nb, D, params, u, u_stride, v, v_stride, form, partial);
+  dim3 g2((unsigned)nlat, (unsigned)GRAD_TERM_SLOTS);
+  kgrad_terms_finish_kernel<<<g2, 256, 0, st>>>(partial, ntiles_, out);
+  return cudaGetLastError();
+}
+
+// M(r, c) += s v_r v_c on the stored (lower) tiles of a batch of packed-lower matrices; grid (tiles, batch).
+__global__ void __launch_bounds__(256) sym_rank1_kernel(TiledSym M, const double* __restrict__ v, size_t v_stride, double s) {
+  const int b = blockIdx.y, tl = blockIdx.x;
+  int I = (int)((sqrt(8.0 * (double)tl + 1.0) - 1.0) * 0.5);
+  while ((size_t)(I + 1) * (I + 2) / 2 <= (size_t)tl) ++I;
+  while ((size_t)I * (I + 1) / 2 > (size_t)tl) --I;
+  const int J = tl - (int)((size_t)I * (I + 1) / 2);
+  double* tile = M.tile(b, I, J);
+  const double* vb = v + (size_t)b * v_stride;
+  for (int e = threadIdx.x; e < TT; e += 256) {
+    int r, c;
+    tile_rc(e, r, c);
+    tile[e] = fma(s * vb[I * TILE + r], vb[J * TILE + c], tile[e]);
+  }
+}
+cudaError_t launch_sym_rank1(cudaStream_t st, TiledSym M, int batch, const double* v, size_t v_stride, double s) {
+  dim3 grid((unsigned)sym_tiles(M.nt), (unsigned)batch);
+  sym_rank1_kernel<<<grid, 256, 0, st>>>(M, v, v_stride, s);
   return cudaGetLastError();
 }
 

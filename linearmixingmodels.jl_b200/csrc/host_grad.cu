@@ -161,8 +161,6 @@ struct GradOut {
   double* grad_terms = nullptr;  // m x LMM_MAX_TERMS x LMM_GRAD_TERM_STRIDE: per-term gradients (nullable)
 };
 
-constexpr int TERM_SLOTS = LMM_MAX_TERMS * LMM_GRAD_TERM_STRIDE;  // grad_terms doubles per latent
-
 // Launch bounds of the per-term contraction for latents [lo, hi): the most terms, and whether any term has an ARDTransform.
 void terms_shape(const lmm_gp_desc* latents, int lo, int hi, int& max_terms, bool& any_ard) {
   max_terms = 1;

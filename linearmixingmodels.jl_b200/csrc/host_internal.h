@@ -342,6 +342,19 @@ void masked_observations(const lmm_gp_desc* latents, int m, const double* H, int
                          std::vector<double>& delta);
 bool per_input_mask(const double* y, int p, int N, std::vector<int>& keep);
 
+constexpr int TERM_SLOTS = LMM_MAX_TERMS * LMM_GRAD_TERM_STRIDE;  // grad_terms doubles per latent
+void terms_shape(const lmm_gp_desc* latents, int lo, int hi, int& max_terms, bool& any_ard);
+// What post_logpdf_impl leaves behind for the gradient through the conditioning (host_post_grad.cu): the predictive factors
+// and inputs (P), β_i = Σ*_i⁻¹(ỹ*_i - μ_i) of the resident latents [nloc][P.nspad], and the rank-summed gradient pieces
+// hg = [β_i'β_i (m) | tr(Σ*_i⁻¹) (m) | |R*|² (1)].
+struct PredictiveKeep {
+  Predictive P;
+  DevBuf beta;
+  std::vector<double> hg;
+};
+int post_logpdf_impl(lmm_post* post, const double* xs, int Ns, double sigma2, const double* ys, double* out_logpdf, double* grad_sigma2,
+                     double* grad_y, int* info_latent, PredictiveKeep* keep = nullptr);
+
 }  // namespace lmm_host
 namespace lmm_host {
 int masked_post_mean_and_var(lmm_post* post, const double* xs, int Ns, double sigma2, double* mean, double* var);

@@ -319,8 +319,9 @@ namespace lmm_host {
 // logpdf(post(x*, σ²), y*) and, optionally, its gradient w.r.t. σ² and y* (the posterior's own data
 // α, C, x and the kernel hyper-parameters are held fixed):
 //   d/dy* = -T' α* - R/σ²,   d/dν_i = (α*_i'α*_i - tr(C*_i^{-1}))/2 with ν_i = σ²/S_i (OILMM) or σ².
+// keep (nullable): hands the predictive factors, β and the gradient pieces to the caller (requires grad_sigma2).
 int post_logpdf_impl(lmm_post* post, const double* xs, int Ns, double sigma2, const double* ys, double* out_logpdf, double* grad_sigma2,
-                     double* grad_y, int* info_latent) {
+                     double* grad_y, int* info_latent, PredictiveKeep* keep) {
   lmm_ctx* ctx = post->ctx;
   CU(cudaSetDevice(ctx->device));
   if (post->kind == POST_MASKED) return ctx->fail(LMM_E_UNSUPPORTED, "a missing-data posterior offers mean_and_var only");
@@ -340,7 +341,8 @@ int post_logpdf_impl(lmm_post* post, const double* xs, int Ns, double sigma2, co
     pr.noise.assign(m, sigma2);
     pr.has_reg = false;
   }
-  Predictive P;
+  Predictive P_own;
+  Predictive& P = keep ? keep->P : P_own;
   if ((rc = build_predictive(post, xs, Ns, pr.noise, P, info_latent))) return rc;
   // project y*: δ*_i = (T Y*)_i  (means handled below: predictive mean ML already includes m_i)
   DevBuf b_y, b_T, b_Pm, b_Q, b_zero, b_ty, b_part, b_resid, b_terms, b_r, b_z, b_quad;
@@ -370,7 +372,8 @@ int post_logpdf_impl(lmm_post* post, const double* xs, int Ns, double sigma2, co
   CU(b_resid.alloc(ctx, sizeof(double)));
   CU(b_terms.alloc(ctx, (size_t)(m + 1) * sizeof(double)));
   CU(cudaMemsetAsync(b_terms.p, 0, (size_t)(m + 1) * sizeof(double), st));
-  DevBuf b_R, b_alpha, b_X, b_tr, b_gy, b_gvec;
+  DevBuf b_R, b_alpha_own, b_X, b_tr, b_gy, b_gvec;
+  DevBuf& b_alpha = keep ? keep->beta : b_alpha_own;
   const bool want_R = do_reg && want_grad;
   if (want_R) CU(b_R.alloc(ctx, (size_t)p * Ns * sizeof(double)));
   CU(cudaMemsetAsync(b_resid.p, 0, sizeof(double), st));
@@ -476,6 +479,7 @@ int post_logpdf_impl(lmm_post* post, const double* xs, int Ns, double sigma2, co
   CU(copy_out(ctx, ht.data(), b_terms.p, (size_t)(m + 1) * sizeof(double)));
   if (want_grad) CU(copy_out(ctx, hg.data(), b_gvec.p, ngv * sizeof(double)));
   CU(cudaStreamSynchronize(st));
+  if (keep) keep->hg = hg;
   double s = 0.0;
   for (int i = 0; i < m; ++i) s += ht[i];
   if (out_logpdf) *out_logpdf = s + ht[m];

@@ -185,6 +185,14 @@ cudaError_t launch_kgrad_ard(cudaStream_t st, const double* mat_base, size_t mat
 cudaError_t launch_kgrad_terms(cudaStream_t st, const double* mat_base, size_t mat_batch_stride, int off_per_lat, const double* x, int N,
                                int D, const LatentParams* params, int nlat, int max_terms, bool any_ard, const double* alpha,
                                size_t alpha_stride, int form, double* partial, double* out);
+// Posterior-predictive gradient, rectangular cross block: contraction of Gc = G + u v' (G: N x N* TiledRect per latent, rows the
+// training points xa, columns the test points xb, both RAW [n][D]; u [nlat][u_stride], v [nlat][v_stride]) with ∂k(xa_r, xb_c)/∂θ
+// for every term, every element once.  out[lat*44 + ...] as launch_kgrad_terms; partial: nlat * G.ntr * G.ntc * 44 doubles.
+cudaError_t launch_kgrad_cross_terms(cudaStream_t st, TiledRect G, const double* xa, int Na, const double* xb, int Nb, int D,
+                                     const LatentParams* params, int nlat, int max_terms, bool any_ard, const double* u, size_t u_stride,
+                                     const double* v, size_t v_stride, int form, double* partial, double* out);
+// M += s v v' on the stored tiles of a batch of packed-lower matrices (v [batch][v_stride], zero past the matrix size)
+cudaError_t launch_sym_rank1(cudaStream_t st, TiledSym M, int batch, const double* v, size_t v_stride, double s);
 // Missing-data dense model: contraction of G = (αα' - C^{-1})/2 over the (nobs x nobs) observed-entry matrix (negCinv = -C^{-1},
 // batch 1; obs sorted by outputs, seg[j] = first entry of output j, seg[p] = nobs; x [N][D] raw points, Hm p x m col-major).
 // out_terms[l*44 + ...] as launch_kgrad_terms with the weight H[j_a,l] H[j_b,l]; out_H[l*p + j] = 2 Σ_{a: j_a = j} Σ_b G_ab

@@ -134,10 +134,14 @@ points(x::ColVecs) = (Matrix{Float64}(x.X), size(x.X, 1))              # D x N c
 points(x::RowVecs) = (Matrix{Float64}(permutedims(x.X)), size(x.X, 2))
 
 # --- device-resident posterior -----------------------------------------------------------------
+# y / σ²: the training data and noise the handle was conditioned on (empty / NaN when unknown, e.g. a loaded handle); the
+# gradient through the conditioning (lmm_post_logpdf_grad_full) needs them.
 mutable struct DevicePosterior
     handle::Ptr{Cvoid}
-    function DevicePosterior(h)
-        p = new(h)
+    y::Vector{Float64}
+    σ²::Float64
+    function DevicePosterior(h, y::Vector{Float64} = Float64[], σ²::Float64 = NaN)
+        p = new(h, y, σ²)
         finalizer(q -> ccall((:lmm_post_free, liblmm), Cint, (Ptr{Cvoid},), q.handle), p)
         return p
     end
@@ -176,7 +180,7 @@ function AbstractGPs.posterior(fx::FiniteGP{<:OILMM{<:IndependentMOGP{<:Vector{<
          Ptr{Float64}, Cint, Ptr{Ptr{Cvoid}}, Ptr{Float64}, Ptr{Float64}, Ptr{Cint}),
         ctx(), descs, length(descs), X, length(x), D, U, S, size(U, 1), Float64(σ²), yv, fx.x.out_dim, h, C_NULL, C_NULL, il)
     check(rc)
-    owner = DevicePosterior(h[])
+    owner = DevicePosterior(h[], yv, Float64(σ²))
     latents = [DeviceLatentPosterior(owner, i - 1, f) for (i, f) in enumerate(fs.fs)]
     return ILMM(IndependentMOGP(latents), H)          # an OILMM whose latents are (device) posteriors
 end
@@ -355,20 +359,68 @@ function ChainRulesCore.rrule(::typeof(AbstractGPs.logpdf), fx::FiniteGP{<:ILMM{
     return out[], logpdf_pullback
 end
 
-# --- rrule for logpdf(post(x*, σ²), y*) (test/oilmm.jl:32 `gradient(logpdf, po, y_test)`): tangents for σ² and y* ---
+# --- rrule for logpdf(post(x*, σ²), y*) (test/oilmm.jl:32 `gradient(logpdf, po, y_test)`) -----------------------------
+# Through the conditioning (lmm_post_logpdf_grad_full): besides the Σy and y* tangents, the posterior's latents get a tangent
+# on their `prior` (per-term hyper-parameters gt as in the prior rrule, mapping onto the kernel structs omitted as there; the
+# constant means), H gets U / S, and the owner gets (σ², y) of the training data -- the rrule of `posterior` below maps those
+# back onto the prior FiniteGP and the training y.  A handle that does not know its training data (a loaded one) gives the
+# σ² and y* tangents only (lmm_post_logpdf_grad).
 function ChainRulesCore.rrule(::typeof(AbstractGPs.logpdf), fx::FiniteGP{<:PosteriorOILMM}, y::AbstractVector{<:Real})
     fs, H, σ², x = unpack(fx)
-    X, _ = points(x)
+    X, D = points(x)
+    owner = fs.fs[1].owner
     out = Ref{Float64}(0.0); gs2 = Ref{Float64}(0.0); il = Ref{Cint}(-1)
     gy = Vector{Float64}(undef, length(y))
-    check(ccall((:lmm_post_logpdf_grad, liblmm), Cint,
-        (Ptr{Cvoid}, Ptr{Float64}, Cint, Float64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Cint}),
-        fs.fs[1].owner.handle, X, length(x), Float64(σ²), Vector{Float64}(y), out, gs2, gy, il))
-    function logpdf_pullback(Δ)
-        Σy_tangent = Tangent{typeof(fx.Σy)}(; diag = Tangent{typeof(fx.Σy.diag)}(; value = Δ * gs2[]))
-        return NoTangent(), Tangent{typeof(fx)}(; Σy = Σy_tangent), Δ .* gy
+    if isempty(owner.y)
+        check(ccall((:lmm_post_logpdf_grad, liblmm), Cint,
+            (Ptr{Cvoid}, Ptr{Float64}, Cint, Float64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Cint}),
+            owner.handle, X, length(x), Float64(σ²), Vector{Float64}(y), out, gs2, gy, il))
+        function logpdf_pullback(Δ)
+            Σy_tangent = Tangent{typeof(fx.Σy)}(; diag = Tangent{typeof(fx.Σy.diag)}(; value = Δ * gs2[]))
+            return NoTangent(), Tangent{typeof(fx)}(; Σy = Σy_tangent), Δ .* gy
+        end
+        return out[], logpdf_pullback
     end
-    return out[], logpdf_pullback
+    m = length(fs.fs); p = size(H, 1)
+    gl = Matrix{Float64}(undef, 3, m); gt = Matrix{Float64}(undef, GRAD_TERM_DOUBLES, m)
+    gts2 = Ref{Float64}(0.0); gyt = Vector{Float64}(undef, length(owner.y))
+    gU = Matrix{Float64}(undef, p, m); gS = Vector{Float64}(undef, m)
+    check(ccall((:lmm_post_logpdf_grad_full, liblmm), Cint,
+        (Ptr{Cvoid}, Ptr{Float64}, Cint, Float64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+         Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Cint}),
+        owner.handle, X, length(x), Float64(σ²), Vector{Float64}(y), owner.y, out, gs2, gy, gl, C_NULL, gt, gts2, gyt, gU, gS, il))
+    function logpdf_full_pullback(Δ)
+        Σy_tangent = Tangent{typeof(fx.Σy)}(; diag = Tangent{typeof(fx.Σy.diag)}(; value = Δ * gs2[]))
+        owner_tangent = Tangent{DevicePosterior}(; y = Δ .* gyt, σ² = Δ * gts2[])
+        lat_tangents = [Tangent{typeof(f)}(; owner = owner_tangent, prior = Tangent{typeof(f.prior)}(; mean = Tangent{typeof(f.prior.mean)}(; c = Δ * gl[3, i])))
+                        for (i, f) in enumerate(fs.fs)]
+        f_tangent = Tangent{typeof(fx.f)}(; f = Tangent{typeof(fs)}(; fs = lat_tangents),
+                                          H = Tangent{typeof(H)}(; U = Δ .* gU, S = Tangent{typeof(H.S)}(; diag = Δ .* gS)))
+        return NoTangent(), Tangent{typeof(fx)}(; f = f_tangent, Σy = Σy_tangent), Δ .* gy
+    end
+    return out[], logpdf_full_pullback
+end
+
+# --- rrule for posterior(fx::FiniteGP{<:OILMM}, y): maps the posterior's tangent back onto fx and y ---------------------
+# The latents' `prior` tangents become the prior's latents, H stays H, and the owner's stored (σ², y) become Σy and y.
+function ChainRulesCore.rrule(::typeof(AbstractGPs.posterior), fx::FiniteGP{<:OILMM{<:IndependentMOGP{<:Vector{<:GP}}}},
+                              y::AbstractVector{<:Real})
+    post = AbstractGPs.posterior(fx, y)
+    function posterior_pullback(Δpost)
+        Δ = unthunk(Δpost)
+        Δ isa AbstractZero && return NoTangent(), NoTangent(), NoTangent()
+        lat = Δ.f isa AbstractZero ? nothing : Δ.f.fs
+        prior_fs = lat === nothing ? NoTangent() : [t isa AbstractZero ? NoTangent() : t.prior for t in lat]
+        owner = lat === nothing ? nothing : findfirst(t -> !(t isa AbstractZero) && !(t.owner isa AbstractZero), lat)
+        ow = owner === nothing ? nothing : lat[owner].owner
+        f_tangent = Tangent{typeof(fx.f)}(; f = Tangent{typeof(fx.f.f)}(; fs = prior_fs), H = Δ.H)
+        if ow === nothing
+            return NoTangent(), Tangent{typeof(fx)}(; f = f_tangent), NoTangent()
+        end
+        Σy_tangent = Tangent{typeof(fx.Σy)}(; diag = Tangent{typeof(fx.Σy.diag)}(; value = ow.σ²))
+        return NoTangent(), Tangent{typeof(fx)}(; f = f_tangent, Σy = Σy_tangent), ow.y
+    end
+    return post, posterior_pullback
 end
 
 # --- IndependentMOGP with Σy = Diagonal(v) or a dense Σy (AbstractGPs generic FiniteGP path,
