@@ -24,6 +24,17 @@ __device__ __forceinline__ void dmma884d(double& d0, double& d1, double a, doubl
   asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1},{%2},{%3},{%0,%1};" : "+d"(d0), "+d"(d1) : "d"(a), "d"(b));
 }
 
+// First k-tile of the UPDATE of tile (I, J) of latent b: k0, or I (k_from_row: A(I,k) = 0 for k < I), or the later of the two
+// rows' envelopes -- every product skipped below it has an all-zero operand, so the sums are those of the full range.
+__device__ __forceinline__ int gemm_first_k(const GemmArgs& g, int I, int J, int b) {
+  int kb = (g.k_from_row && I > g.k0) ? I : g.k0;
+  if (g.env) {
+    const int* e = g.env + (size_t)b * g.env_stride;
+    kb = max(kb, max(e[I], e[J]));
+  }
+  return kb;
+}
+
 // Which column blocks a warp owns, and for how many k4-steps each is non-zero.
 template <int MODE>
 __device__ __forceinline__ void direct_blocks(int warp, int ktiles, int& nb0, int& nb1, int& lim0, int& nsteps) {
@@ -128,7 +139,8 @@ __global__ void __launch_bounds__(256) gemm_direct2_kernel(GemmArgs g) {
   const int I = g.i0 + blockIdx.y * (g.row_step > 0 ? g.row_step : 1), b = blockIdx.z;
   if (g.sym && I < J) return;
   if (g.upper && I > J) return;
-  const int kb = (g.k_from_row && I > g.k0) ? I : g.k0;
+  if (MODE == GEMM_TRSM && g.env && g.env[(size_t)b * g.env_stride + I] > J) return;  // a zero tile stays zero
+  const int kb = gemm_first_k(g, I, J, b);
   if (MODE == GEMM_UPDATE && kb >= g.k1) return;
   double* Ctile = g.C.tile(b, I, J);
   const int warp = threadIdx.x >> 5;

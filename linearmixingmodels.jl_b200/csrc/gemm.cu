@@ -79,7 +79,8 @@ __global__ void __launch_bounds__(256, 1) gemm_tile_kernel_v2(GemmArgs g) {
   const int J = g.j0 + blockIdx.x, I = g.i0 + blockIdx.y * (g.row_step > 0 ? g.row_step : 1), b = blockIdx.z;
   if (g.sym && I < J) return;
   if (g.upper && I > J) return;
-  const int kb = (g.k_from_row && I > g.k0) ? I : g.k0;  // first k-tile of this CTA
+  if (MODE == GEMM_TRSM && g.env && g.env[(size_t)b * g.env_stride + I] > J) return;  // a zero tile stays zero
+  const int kb = gemm_first_k(g, I, J, b);  // first k-tile of this CTA
   if (MODE == GEMM_UPDATE && kb >= g.k1) return;
 
   double* Ctile = g.C.tile(b, I, J);
@@ -232,7 +233,7 @@ static bool g_pdl = true;   // programmatic dependent launch along the panel cha
 void set_pdl(int v) { g_pdl = v != 0; }
 bool pdl_enabled() { return g_pdl; }
 
-cudaError_t launch_gemm(cudaStream_t st, int mode, const GemmArgs& a, int ncols, int nrows, int batch) {
+cudaError_t launch_gemm(cudaStream_t st, int mode, const GemmArgs& a, int ncols, int nrows, int batch, long long select_tiles) {
   if (ncols <= 0 || nrows <= 0 || batch <= 0) return cudaSuccess;
   static bool configured_dev[64] = {false};  // function attributes are per device
   int dev = 0;
@@ -245,7 +246,7 @@ cudaError_t launch_gemm(cudaStream_t st, int mode, const GemmArgs& a, int ncols,
     if (e != cudaSuccess) return e;
     configured = true;
   }
-  if ((long long)ncols * nrows * batch <= g_gemm_small) {
+  if ((select_tiles > 0 ? select_tiles : (long long)ncols * nrows * batch) <= g_gemm_small) {
     dim3 gs((unsigned)ncols * DIRECT_SPLIT, (unsigned)nrows, (unsigned)batch);
     if (mode == GEMM_UPDATE) return launch_pdl(g_pdl, gemm_direct2_kernel<GEMM_UPDATE>, gs, dim3(256), 0, st, a);
     return launch_pdl(g_pdl, gemm_direct2_kernel<GEMM_TRSM>, gs, dim3(256), 0, st, a);

@@ -41,9 +41,27 @@ struct OzWs {
   int S, min_k, bits;  // digit planes, smallest K (k-tiles) the int8 update takes, bits per digit (7: radix 128, 8: radix 256)
 };
 
+// Tile envelope (env_h: host copy, [batch][nt]; L(I,k) = 0 for k < env[b][I]): the last tile row >= r0 that some latent of the
+// batch has inside its envelope for the columns < lim (env[b][I] < lim); r0 - 1 when there is none.  Grids end there; the rows
+// up to it that a latent does not need return at the top of the kernel.
+static int env_last_row(const int* env_h, int nt, int batch, int r0, int lim) {
+  int last = r0 - 1;
+  for (int b = 0; b < batch; ++b)
+    for (int I = nt - 1; I > last; --I)
+      if (env_h[(size_t)b * nt + I] < lim) {
+        last = I;
+        break;
+      }
+  return last;
+}
+
 cudaError_t chol_factor_stream(lmm_ctx* ctx, cudaStream_t st, TiledSym L, double* W, size_t wstride, int batch, double* logdet,
-                               int* info, int jstart = 0, int* counters = nullptr, const OzWs* oz = nullptr) {
+                               int* info, int jstart = 0, int* counters = nullptr, const OzWs* oz = nullptr, const int* env_d = nullptr,
+                               const int* env_h = nullptr) {
   const int nt = L.nt;
+  if (jstart != 0 || !env_h) env_d = env_h = nullptr;
+  // tile rows of a launch whose first row is r0: all of them, or up to the last one inside some latent's envelope (see above)
+  auto rows = [&](int r0, int lim) { return (env_h ? env_last_row(env_h, nt, batch, r0, lim) + 1 : nt) - r0; };
   int ob = ctx->outer_block;
   if (oz && (jstart != 0 || nt <= ob || nt < oz->min_k + 1)) oz = nullptr;  // no wide update this scheme would take
   if (oz) {
@@ -62,38 +80,61 @@ cudaError_t chol_factor_stream(lmm_ctx* ctx, cudaStream_t st, TiledSym L, double
   g.W = W;
   g.w_batch_stride = wstride;
   g.sym = 1;
+  g.env = env_d;
+  g.env_stride = nt;
   cudaError_t e;
   bool factored_ahead = false;  // diagonal tile jj was factored by the previous column's fused chain launch
   for (int s0 = 0; s0 < nt; s0 += ob) {
     const int s1 = (s0 + ob < nt) ? s0 + ob : nt;
     if (s0 > 0) {
       const int r0 = s0 > jstart ? s0 : jstart;  // first tile row that still has to be computed
+      const int nr = rows(r0, s0);  // tile (I, J) has products with two nonzero operands iff env[I] < s0 and env[J] < s0
       g.i0 = r0; g.j0 = s0; g.k0 = 0; g.k1 = s0;
+      e = cudaSuccess;
       // exact int32 accumulation: (pairs per accumulator <= S) * K * (largest digit)^2 < 2^31
       if (oz && s0 >= oz->min_k && (long long)s0 * TILE * oz->S * (oz->bits == 8 ? 16384 : 4096) < (1ll << 31)) {
-        cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-        if (ctx->ozaki_time && cudaEventCreate(&ev0) == cudaSuccess && cudaEventCreate(&ev1) == cudaSuccess) cudaEventRecord(ev0, st);
-        e = launch_ozaki_update(st, L, oz->slices, oz->slice_stride, oz->scale, oz->scale_stride, r0, nt - r0, s0, s1 - s0, s0, batch, oz->S, oz->bits);
-        if (ev0 && ev1) {
-          cudaEventRecord(ev1, st);
-          ctx->oz_events.push_back(ev0);
-          ctx->oz_events.push_back(ev1);
-          double tp = 0.0;  // 128^3 tile products of this launch: tiles (I, J), I >= J, times s0 k-tiles
-          for (int J = s0; J < s1; ++J) tp += (double)(nt - (J > r0 ? J : r0)) * s0;
-          ctx->oz_tile_products += tp * batch;
+        if (nr > 0) {
+          cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+          if (ctx->ozaki_time && cudaEventCreate(&ev0) == cudaSuccess && cudaEventCreate(&ev1) == cudaSuccess) cudaEventRecord(ev0, st);
+          e = launch_ozaki_update(st, L, oz->slices, oz->slice_stride, oz->scale, oz->scale_stride, r0, nr, s0, s1 - s0, s0, batch, oz->S, oz->bits,
+                                  env_d);
+          if (ev0 && ev1) {
+            cudaEventRecord(ev1, st);
+            ctx->oz_events.push_back(ev0);
+            ctx->oz_events.push_back(ev1);
+            // 128^3 tile products this launch runs: tiles (I, J), I >= J, times their k-tiles (s0, or from the later envelope on)
+            double tp = 0.0;
+            for (int J = s0; J < s1; ++J)
+              for (int I = J > r0 ? J : r0; I < r0 + nr; ++I) {
+                if (!env_h) {
+                  tp += (double)s0 * batch;
+                  continue;
+                }
+                for (int b = 0; b < batch; ++b) {
+                  const int* eb = env_h + (size_t)b * nt;
+                  const int kb = eb[I] > eb[J] ? eb[I] : eb[J];
+                  if (kb < s0) tp += (double)(s0 - kb);
+                }
+              }
+            ctx->oz_tile_products += tp;
+          }
         }
-      } else
-        e = launch_gemm(st, GEMM_UPDATE, g, s1 - s0, nt - r0, batch);
+      } else if (nr > 0) {
+        e = launch_gemm(st, GEMM_UPDATE, g, s1 - s0, nr, batch, (long long)(s1 - s0) * (nt - r0) * batch);
+      }
       if (e != cudaSuccess) return e;
-      ++ctx->launches;
-      ctx->timings[6] += 1;
+      if (nr > 0) {
+        ++ctx->launches;
+        ctx->timings[6] += 1;
+      }
     }
     for (int jj = s0; jj < s1; ++jj) {
       const int r0 = jj > jstart ? jj : jstart;
       if (!factored_ahead) {
-        if (jj > s0) {
+        const int nr = jj > s0 ? rows(r0, jj) : 0;
+        if (nr > 0) {
           g.i0 = r0; g.j0 = jj; g.k0 = s0; g.k1 = jj;
-          if ((e = launch_gemm(st, GEMM_UPDATE, g, 1, nt - r0, batch)) != cudaSuccess) return e;
+          if ((e = launch_gemm(st, GEMM_UPDATE, g, 1, nr, batch, (long long)(nt - r0) * batch)) != cudaSuccess) return e;
           ++ctx->launches;
           ctx->timings[6] += 1;
         }
@@ -112,13 +153,16 @@ cudaError_t chol_factor_stream(lmm_ctx* ctx, cudaStream_t st, TiledSym L, double
         factored_ahead = true;
         continue;
       }
+      const int nr = rows(t0, jj + 1);
+      if (nr <= 0) continue;
       g.i0 = t0; g.j0 = jj;
-      if ((e = launch_gemm(st, GEMM_TRSM, g, 1, nt - t0, batch)) != cudaSuccess) return e;
+      if ((e = launch_gemm(st, GEMM_TRSM, g, 1, nr, batch, (long long)(nt - t0) * batch)) != cudaSuccess) return e;
       ++ctx->launches;
     }
-    if (oz && s1 < nt) {  // the block column is final: digit planes of its tiles below the block, for the later wide updates
-      if ((e = launch_ozaki_slice(st, L, oz->scale, oz->scale_stride, oz->slices, oz->slice_stride, s1, nt - s1, s0, s1 - s0, batch, oz->S, oz->bits)) !=
-          cudaSuccess)
+    const int ns = oz && s1 < nt ? rows(s1, s1) : 0;
+    if (ns > 0) {  // the block column is final: digit planes of its tiles below the block, for the later wide updates
+      if ((e = launch_ozaki_slice(st, L, oz->scale, oz->scale_stride, oz->slices, oz->slice_stride, s1, ns, s0, s1 - s0, batch, oz->S, oz->bits,
+                                  env_d)) != cudaSuccess)
         return e;
       ++ctx->launches;
     }
@@ -530,8 +574,11 @@ cudaError_t chol_factor_rowcyclic_dist(lmm_ctx* ctx, TiledSym Lown, int nrows, i
 
 // Fork the batch into latent groups on separate streams (joined back into ctx->stream).  jstart > 0: extend a factor whose
 // tile rows < jstart are final (see chol_factor_stream).
-cudaError_t chol_factor(lmm_ctx* ctx, TiledSym L, double* W, size_t wstride, int batch, double* logdet, int* info, int jstart) {
+cudaError_t chol_factor(lmm_ctx* ctx, TiledSym L, double* W, size_t wstride, int batch, double* logdet, int* info, int jstart,
+                        const int* env_d, const int* env_h) {
   const int G = ctx->ngroups < batch ? ctx->ngroups : batch;
+  if (!env_d || !env_h) env_d = env_h = nullptr;
+  auto env_at = [&](const int* e, int b0) { return e ? e + (size_t)b0 * L.nt : nullptr; };
   if (jstart == 0) {  // the look-ahead / partitioned schedules factor from scratch only
     if (ctx->partition_ilmm && ctx->partition_now && batch == 1 && ctx->comm && ctx->nranks > 1 && L.nt >= 2 * ctx->nranks && nccl_api().AllGather)
       return chol_factor_rowcyclic(ctx, L, W, wstride, logdet, info);
@@ -553,7 +600,9 @@ cudaError_t chol_factor(lmm_ctx* ctx, TiledSym L, double* W, size_t wstride, int
         for (int c0 = 0; c0 < batch; c0 += fit) {
           const int cb = batch - c0 < fit ? batch - c0 : fit;
           TiledSym Lc{L.base + (size_t)c0 * L.batch_stride, L.nt, L.batch_stride};
-          if ((e = chol_factor(ctx, Lc, W + (size_t)c0 * wstride, wstride, cb, logdet + c0, info + c0, 0)) != cudaSuccess) return e;
+          if ((e = chol_factor(ctx, Lc, W + (size_t)c0 * wstride, wstride, cb, logdet + c0, info + c0, 0, env_at(env_d, c0), env_at(env_h, c0))) !=
+              cudaSuccess)
+            return e;
         }
         return cudaSuccess;
       }
@@ -571,7 +620,8 @@ cudaError_t chol_factor(lmm_ctx* ctx, TiledSym L, double* W, size_t wstride, int
   int* counters = nullptr;
   const bool chain_all = ctx->chain_fused && (long long)(L.nt - 1) * batch <= CHAIN_MAX_TILES && L.nt > 1;
   if (ctx->chain_fused && L.nt > 1 && (e = chain_counters(ctx, ctx->stream, L.nt, batch, &counters)) != cudaSuccess) return e;
-  if (G <= 1 || L.nt <= 1 || chain_all) return chol_factor_stream(ctx, ctx->stream, L, W, wstride, batch, logdet, info, jstart, counters, oz);
+  if (G <= 1 || L.nt <= 1 || chain_all)
+    return chol_factor_stream(ctx, ctx->stream, L, W, wstride, batch, logdet, info, jstart, counters, oz, env_d, env_h);
   if ((e = cudaEventRecord(ctx->ev_fork, ctx->stream)) != cudaSuccess) return e;
   for (int gi = 0; gi < G; ++gi) {
     const int b0 = (int)((int64_t)batch * gi / G), b1 = (int)((int64_t)batch * (gi + 1) / G);
@@ -580,7 +630,8 @@ cudaError_t chol_factor(lmm_ctx* ctx, TiledSym L, double* W, size_t wstride, int
     TiledSym Lg{L.base + (size_t)b0 * L.batch_stride, L.nt, L.batch_stride};
     OzWs oztmp{};
     if ((e = chol_factor_stream(ctx, st, Lg, W + (size_t)b0 * wstride, wstride, b1 - b0, logdet + b0, info + b0, jstart,
-                                counters ? counters + (size_t)b0 * chain_counter_ints(L.nt) : nullptr, oz_at(b0, oztmp))) != cudaSuccess)
+                                counters ? counters + (size_t)b0 * chain_counter_ints(L.nt) : nullptr, oz_at(b0, oztmp), env_at(env_d, b0),
+                                env_at(env_h, b0))) != cudaSuccess)
       return e;
     if ((e = cudaEventRecord(ctx->ev_join[gi], st)) != cudaSuccess) return e;
     if ((e = cudaStreamWaitEvent(ctx->stream, ctx->ev_join[gi], 0)) != cudaSuccess) return e;

@@ -331,7 +331,11 @@ int ilmm_post_mean_and_var(lmm_post* post, const double* xs, int Ns, double sigm
 int ilmm_post_rand(lmm_post* post, const double* xs, int Ns, double sigma2, const double* z_latent, const double* z_noise, double* out, int* info);
 int ilmm_post_logpdf(lmm_post* post, const double* xs, int Ns, double sigma2, const double* ys, double* out_logpdf, double* grad_sigma2, double* grad_y, int* info);
 int ilmm_post_condition(lmm_post* post, const double* xs, int Ns, double sigma2, const double* ys, lmm_post** out_post, int* info);
-cudaError_t chol_factor(lmm_ctx* ctx, TiledSym L, double* W, size_t wstride, int batch, double* logdet, int* info, int jstart = 0);
+// env_d / env_h (both or neither; jstart = 0): the tile envelope of the batch (launch_kmat_sym) on the device and a host copy of it.
+// The batched left-looking schedule then skips every tile product, TRSM and slice that has an all-zero operand -- the factor is
+// bit-identical to the dense schedule's -- and sizes its grids from the host copy.  The other schedules ignore it.
+cudaError_t chol_factor(lmm_ctx* ctx, TiledSym L, double* W, size_t wstride, int batch, double* logdet, int* info, int jstart = 0,
+                        const int* env_d = nullptr, const int* env_h = nullptr);
 cudaError_t chol_factor_rowcyclic_dist(lmm_ctx* ctx, TiledSym Lown, int nrows, int nc, double* W, size_t wstride, double* logdet, int* info,
                                        double* zvec);
 size_t rowcyclic_dist_workspace_tiles(int nrows, int G, int ob);

@@ -84,7 +84,7 @@ int latents_run(lmm_ctx* ctx, int kind, const lmm_gp_desc* latents, int m, const
   const size_t per_lat = factor_bytes_per_latent(nt);
   int chunk = mloc;
   if (!keep && mloc > 0) CU(mem_fit(ctx, per_lat + 6 * npad * sizeof(double), mloc, &chunk));
-  DevBuf b_L, b_W, b_alpha, b_r, b_z, b_logdet, b_quad, b_info, b_nv;
+  DevBuf b_L, b_W, b_alpha, b_r, b_z, b_logdet, b_quad, b_info, b_nv, b_env;
   if (noise_vec) {
     const int nl = mloc > 0 ? mloc : 1;
     CU(b_nv.alloc(ctx, (size_t)nl * npad * sizeof(double)));
@@ -97,8 +97,12 @@ int latents_run(lmm_ctx* ctx, int kind, const lmm_gp_desc* latents, int m, const
     }
   }
   std::vector<int> hinfo(mloc > 0 ? mloc : 1, 0);
+  // tile envelope of each chunk's kernel matrices: far-apart points give exact zeros that the factorisation and the solves skip
+  std::vector<int> henv;
   float ms_kmat = 0, ms_chol = 0, ms_solve = 0;
   if (mloc > 0) {
+    henv.resize((size_t)chunk * nt);
+    CU(b_env.alloc(ctx, henv.size() * sizeof(int)));
     CU(b_L.alloc(ctx, (size_t)chunk * sym_tiles(nt) * TT * sizeof(double)));
     CU(b_W.alloc(ctx, (size_t)chunk * nt * TT * sizeof(double)));
     CU(b_r.alloc(ctx, (size_t)chunk * npad * sizeof(double)));
@@ -117,19 +121,22 @@ int latents_run(lmm_ctx* ctx, int kind, const lmm_gp_desc* latents, int m, const
       const LatentParams* dp = b_params.as<LatentParams>() + c0;
       double* delta = b_ty.as<double>() + (size_t)c0 * npad;
       CU(cudaEventRecord(ctx->ev[2], st));
+      const int* env = b_env.as<int>();
       CU(launch_kmat_sym(st, L, nb, b_x.as<double>(), N, D, dp, ctx->distance_form,
-                         noise_vec ? b_nv.as<double>() + (size_t)c0 * npad : nullptr, npad));
+                         noise_vec ? b_nv.as<double>() + (size_t)c0 * npad : nullptr, npad, 0, b_env.as<int>()));
       ++ctx->launches;
       CU(cudaEventRecord(ctx->ev[3], st));
-      CU(chol_factor(ctx, L, W, wstride, nb, b_logdet.as<double>() + c0, b_info.as<int>() + c0));
+      CU(copy_out(ctx, henv.data(), env, (size_t)nb * nt * sizeof(int)));  // sizes the factorisation's grids
+      CU(cudaStreamSynchronize(st));
+      CU(chol_factor(ctx, L, W, wstride, nb, b_logdet.as<double>() + c0, b_info.as<int>() + c0, 0, env, henv.data()));
       CU(cudaEventRecord(ctx->ev[4], st));
       CU(cudaMemcpyAsync(b_r.p, delta, (size_t)nb * npad * sizeof(double), cudaMemcpyDeviceToDevice, st));
-      CU(launch_fwd_solve(st, L, W, wstride, b_r.as<double>(), b_z.as<double>(), npad, nb, &ctx->launches));
+      CU(launch_fwd_solve(st, L, W, wstride, b_r.as<double>(), b_z.as<double>(), npad, nb, &ctx->launches, env));
       CU(launch_sumsq(st, b_z.as<double>(), npad, (int)npad, nb, b_quad.as<double>() + c0));
       ++ctx->launches;
       if (keep) {
         CU(cudaMemcpyAsync(b_r.p, b_z.p, (size_t)nb * npad * sizeof(double), cudaMemcpyDeviceToDevice, st));
-        CU(launch_bwd_solve(st, L, W, wstride, b_r.as<double>(), b_alpha.as<double>() + (size_t)c0 * npad, npad, nb, &ctx->launches));
+        CU(launch_bwd_solve(st, L, W, wstride, b_r.as<double>(), b_alpha.as<double>() + (size_t)c0 * npad, npad, nb, &ctx->launches, env));
       }
       CU(launch_lml_terms(st, b_terms.as<double>(), lo + c0, nb, b_logdet.as<double>() + c0, b_quad.as<double>() + c0, N, LOG2PI));
       ++ctx->launches;

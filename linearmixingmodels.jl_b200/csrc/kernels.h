@@ -8,8 +8,11 @@ namespace lmm {
 // ---- kmat.cu
 // noise_vec (nullable): per-point diagonal noise [batch][noise_stride] overriding params[b].noise
 // row0: only the tile rows I >= row0 are built (the rows above belong to a factor that is being extended)
+// env (nullable, [batch][nt] ints, row0 = 0): the tile envelope -- env[b][I] = first tile column of tile row I with an entry != 0.
+// The Cholesky factor keeps it (L(I,k) = 0 for k < env[b][I]), so the factorisation and the solves may skip those tiles.
 cudaError_t launch_kmat_sym(cudaStream_t st, TiledSym out, int batch, const double* xpad, int N, int D,
-                            const LatentParams* params, int form, const double* noise_vec = nullptr, size_t noise_stride = 0, int row0 = 0);
+                            const LatentParams* params, int form, const double* noise_vec = nullptr, size_t noise_stride = 0, int row0 = 0,
+                            int* env = nullptr);
 cudaError_t launch_kmat_cross(cudaStream_t st, TiledRect out, int batch, const double* xa_pad, int Na, const double* xb_pad,
                               int Nb, int D, const LatentParams* params, int form);
 
@@ -49,9 +52,13 @@ struct GemmArgs {
   int k_from_row;         // UPDATE: k range starts at max(k0, I) (A(I,k) = 0 for k < I)
   int row_step;           // tile row I = i0 + blockIdx.y * row_step (0 or 1: consecutive rows; G: the rows one rank of a
                           // row-cyclic partition owns)
+  const int* env;         // nullable: tile envelope [batch][env_stride] of a packed-lower factor (launch_kmat_sym).  UPDATE: the k range
+  int env_stride;         // starts at max(k0, env[b][I], env[b][J]); TRSM: tiles with env[b][I] > J are zero and are skipped
 };
 enum { GEMM_UPDATE = 0, GEMM_TRSM = 1 };
-cudaError_t launch_gemm(cudaStream_t st, int mode, const GemmArgs& a, int ncols, int nrows, int batch);
+// select_tiles > 0: choose between the direct and the TMA-pipelined kernel as for a grid of that many tiles (the two sum in different
+// orders; a grid trimmed to the envelope keeps the kernel, and so the bits, of the full grid)
+cudaError_t launch_gemm(cudaStream_t st, int mode, const GemmArgs& a, int ncols, int nrows, int batch, long long select_tiles = 0);
 void set_gemm_small_threshold(int tiles);  // grids of <= tiles tiles use the latency-optimised direct kernel (default 74; 0 = off)
 void set_pdl(int v);       // 1: programmatic dependent launch along the batch-1 panel chain (default 1)
 bool pdl_enabled();
@@ -69,10 +76,11 @@ cudaError_t launch_chain_column(cudaStream_t st, TiledSym L, double* W, size_t w
 
 // ---- solve.cu
 // forward: z = L^{-1} r; backward: a = L^{-T} r.  rvec[batch][nt*128] is consumed (destroyed).
+// env (nullable, [batch][nt]): tile envelope of the factor (launch_kmat_sym); the persistent sweeps skip the tiles outside it.
 cudaError_t launch_fwd_solve(cudaStream_t st, TiledSym L, const double* W, size_t w_batch_stride, double* rvec, double* zvec,
-                             size_t vec_stride, int batch, int64_t* launches);
+                             size_t vec_stride, int batch, int64_t* launches, const int* env = nullptr);
 cudaError_t launch_bwd_solve(cudaStream_t st, TiledSym L, const double* W, size_t w_batch_stride, double* rvec, double* avec,
-                             size_t vec_stride, int batch, int64_t* launches);
+                             size_t vec_stride, int batch, int64_t* launches, const int* env = nullptr);
 void set_solve_impl(int v);  // 1: persistent sweep kernels, one launch per direction (default); 0: one launch per tile column
 // out[b] = sum_i v[b][i]^2 (fixed order)
 cudaError_t launch_sumsq(cudaStream_t st, const double* v, size_t stride, int n, int batch, double* out);
@@ -102,11 +110,15 @@ cudaError_t launch_rhs_row_extract(cudaStream_t st, TiledSym L, int I, int s0, i
 // scale[b][row] = 2^(E_row - 6) from the diagonal of the matrix about to be factored (2^E > sqrt(A_ii))
 cudaError_t launch_ozaki_scales(cudaStream_t st, TiledSym L, int batch, double* scale, size_t scale_batch_stride);
 // slice the finished tiles (I, k), I in [i0, i0 + nrows), k in [k0, k0 + ncols), into S int8 digit planes (S * 16 KB per tile)
+// env (nullable, [batch][L.nt]): tiles with k < env[b][I] are zero, are never read, and are not sliced
 cudaError_t launch_ozaki_slice(cudaStream_t st, TiledSym L, const double* scale, size_t scale_batch_stride, uint8_t* slices,
-                               size_t slice_batch_stride, int i0, int nrows, int k0, int ncols, int batch, int S, int bits);
-// C(I,J) -= sum_{k < k1} L(I,k) L(J,k)' for I in [i0, i0 + nrows), J in [j0, j0 + ncols), I >= J, from the sliced factor
+                               size_t slice_batch_stride, int i0, int nrows, int k0, int ncols, int batch, int S, int bits,
+                               const int* env = nullptr);
+// C(I,J) -= sum_{k < k1} L(I,k) L(J,k)' for I in [i0, i0 + nrows), J in [j0, j0 + ncols), I >= J, from the sliced factor;
+// env (nullable, [batch][L.nt]): the k range of tile (I, J) starts at max(env[b][I], env[b][J])
 cudaError_t launch_ozaki_update(cudaStream_t st, TiledSym L, const uint8_t* slices, size_t slice_batch_stride, const double* scale,
-                                size_t scale_batch_stride, int i0, int nrows, int j0, int ncols, int k1, int batch, int S, int bits);
+                                size_t scale_batch_stride, int i0, int nrows, int j0, int ncols, int k1, int batch, int S, int bits,
+                                const int* env = nullptr);
 // the prediction sweep X <- X L^{-T} on the same path: row scales of a FINISHED factor (row 2-norms) and of X (prior variance bound),
 // digit planes of rectangular tiles, wide update with the left operand from the sliced X
 cudaError_t launch_ozaki_factor_scales(cudaStream_t st, TiledSym L, int batch, double* scale, size_t scale_batch_stride);

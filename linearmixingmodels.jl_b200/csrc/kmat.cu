@@ -70,11 +70,12 @@ __device__ __forceinline__ void stage_points(double* xa, double* xb, double* sa,
 // distance and κ (KernelFunctions evaluates the components separately and adds / multiplies the matrices).  Kept out of line
 // so that the single-kernel tile body keeps its register allocation (it runs at 90 % of the HBM write bandwidth).
 template <bool SYM>
-__device__ __noinline__ void kmat_tile_composite(double* __restrict__ tile, const double* xa, const double* xb, int dd, int r0, int c0, int Na,
+__device__ __noinline__ bool kmat_tile_composite(double* __restrict__ tile, const double* xa, const double* xb, int dd, int r0, int c0, int Na,
                                                  int Nb, double noise, int form, const double* __restrict__ noise_vec, const LatentParams* gp) {
   const int t = threadIdx.x;
   const int r = (((2 * t) >> 5) & 15) * 8 + (((2 * t) >> 2) & 7);
   const int gr = r0 + r;
+  bool nz = false;
   __syncthreads();  // stage_points returned right after the bulk copies landed
   for (int it = 0; it < 32; ++it) {
     const int c = 4 * it + ((2 * t) & 3);
@@ -93,8 +94,10 @@ __device__ __noinline__ void kmat_tile_composite(double* __restrict__ tile, cons
       }
       vv[q] = val;
     }
+    nz |= (v.x != 0.0) | (v.y != 0.0);
     *reinterpret_cast<double2*>(tile + it * 512 + 2 * t) = v;
   }
+  return nz;
 }
 
 // One 128x128 tile of kernel values.  Thread t owns the fixed tile row r(t) and walks the columns
@@ -102,8 +105,9 @@ __device__ __noinline__ void kmat_tile_composite(double* __restrict__ tile, cons
 // column points are shared-memory broadcasts, and each iteration ends in one coalesced 16-byte
 // store at tile offset e = it*512 + 2*t (the k4-interleaved layout makes e linear in (it, t)).
 // SYM: diagonal entries get d² = 0 exactly and + noise; padding is the identity (SYM) or zero.
+// Returns whether this thread stored an entry that is not exactly 0 (NaN counts as nonzero).
 template <bool SYM, int DS>
-__device__ __forceinline__ void kmat_tile_body(double* __restrict__ tile, const double* xa, const double* xb, const double* sa,
+__device__ __forceinline__ bool kmat_tile_body(double* __restrict__ tile, const double* xa, const double* xb, const double* sa,
                                                const double* sb, int D, int r0, int c0, int Na, int Nb, const LatentParams& lp, int form,
                                                const double* __restrict__ noise_vec = nullptr, const LatentParams* gp = nullptr) {
   const int t = threadIdx.x;
@@ -111,12 +115,12 @@ __device__ __forceinline__ void kmat_tile_body(double* __restrict__ tile, const 
   const int gr = r0 + r;
   const int dd = DS > 0 ? DS : D;
   if (gp != nullptr && needs_raw_points(gp)) {  // composite (KernelSum / KernelProduct) or periodic latent: out-of-line slow path
-    kmat_tile_composite<SYM>(tile, xa, xb, dd, r0, c0, Na, Nb, lp.noise, form, noise_vec, gp);
-    return;
+    return kmat_tile_composite<SYM>(tile, xa, xb, dd, r0, c0, Na, Nb, lp.noise, form, noise_vec, gp);
   }
   const double* ar = xa + (size_t)r * dd;
   const double sar = sa[r];
   const double a0 = ar[0];
+  bool nz = false;
   // interior off-diagonal tiles (almost all of them): no bounds / diagonal predicates in the element loop
   if (DS == 1 && form == 0 && r0 + TILE <= Na && c0 + TILE <= Nb && !(SYM && r0 == c0)) {
     const int cb = (2 * t) & 3;
@@ -133,9 +137,10 @@ __device__ __forceinline__ void kmat_tile_body(double* __restrict__ tile, const 
       double2 v;
       v.x = kappa_eval(lp.kind, lp.variance, d0, lp.param);
       v.y = kappa_eval(lp.kind, lp.variance, d1, lp.param);
+      nz |= (v.x != 0.0) | (v.y != 0.0);
       *reinterpret_cast<double2*>(tile + it * 512 + 2 * t) = v;
     }
-    return;
+    return nz;
   }
   for (int it = 0; it < 32; ++it) {
     const int c = 4 * it + ((2 * t) & 3);
@@ -162,15 +167,21 @@ __device__ __forceinline__ void kmat_tile_body(double* __restrict__ tile, const 
       }
       vv[q] = val;
     }
+    nz |= (v.x != 0.0) | (v.y != 0.0);
     *reinterpret_cast<double2*>(tile + it * 512 + 2 * t) = v;
   }
+  return nz;
 }
 
 // grid: (lower tiles, batch).  Writes K_b + noise_b*I (identity on the padding) into L tiles.
+// env (nullable, [batch][nt], pre-filled with a value >= nt): env[b][I] = first tile column J of tile row I with an entry that is not
+// exactly 0 -- taken from the values written, so it holds for every kernel, noise vector and point order.  The diagonal tile always
+// counts.  atomicMin is order-independent: the result is deterministic.
 template <int DS>
-__global__ void __launch_bounds__(256) kmat_sym_kernel(TiledSym out, const double* __restrict__ xpad, int N, int D,
+// (256, 4): 4 CTAs per SM as without the envelope test, which would otherwise take the single-kernel body from 64 to 76 registers
+__global__ void __launch_bounds__(256, 4) kmat_sym_kernel(TiledSym out, const double* __restrict__ xpad, int N, int D,
                                                        const LatentParams* __restrict__ params, int form,
-                                                       const double* __restrict__ noise_vec, size_t noise_stride, int tile0) {
+                                                       const double* __restrict__ noise_vec, size_t noise_stride, int tile0, int* env) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double* xa = reinterpret_cast<double*>(smem_raw);
   double* xb = xa + TILE * D;
@@ -189,8 +200,9 @@ __global__ void __launch_bounds__(256) kmat_sym_kernel(TiledSym out, const doubl
   const LatentParams lp = params[b];
 
   stage_points(xa, xb, sa, sb, xpad + (size_t)I * TILE * D, xpad + (size_t)J * TILE * D, D, params + b, &bar);
-  kmat_tile_body<true, DS>(out.tile(b, I, J), xa, xb, sa, sb, D, I * TILE, J * TILE, N, N, lp, form,
-                           noise_vec ? noise_vec + (size_t)b * noise_stride : nullptr, params + b);
+  const bool nz = kmat_tile_body<true, DS>(out.tile(b, I, J), xa, xb, sa, sb, D, I * TILE, J * TILE, N, N, lp, form,
+                                           noise_vec ? noise_vec + (size_t)b * noise_stride : nullptr, params + b);
+  if (env && (__syncthreads_or(nz) || I == J) && threadIdx.x == 0) atomicMin(env + (size_t)b * out.nt + I, J);
 }
 
 // grid: (ntr*ntc, batch).  Rows = points of xa_pad (e.g. x*), cols = points of xb_pad (train x).
@@ -216,7 +228,7 @@ __global__ void __launch_bounds__(256) kmat_cross_kernel(TiledRect out, const do
 static size_t kmat_smem(int D) { return (size_t)(2 * TILE * D + 2 * TILE) * sizeof(double); }
 
 cudaError_t launch_kmat_sym(cudaStream_t st, TiledSym out, int batch, const double* xpad, int N, int D,
-                            const LatentParams* params, int form, const double* noise_vec, size_t noise_stride, int row0) {
+                            const LatentParams* params, int form, const double* noise_vec, size_t noise_stride, int row0, int* env) {
   size_t sm = kmat_smem(D);
   if (sm + 1024 > 48 * 1024) {  // static shared memory counts against the default limit too
     cudaError_t e = cudaFuncSetAttribute(kmat_sym_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
@@ -224,11 +236,15 @@ cudaError_t launch_kmat_sym(cudaStream_t st, TiledSym out, int batch, const doub
   }
   const int tile0 = (int)sym_tiles(row0);  // row-panel-major order: the tiles of rows >= row0 are the tail of the list
   if (row0 >= out.nt) return cudaSuccess;
+  if (env) {
+    cudaError_t e = cudaMemsetAsync(env, 0x7f, (size_t)batch * out.nt * sizeof(int), st);
+    if (e != cudaSuccess) return e;
+  }
   dim3 grid((unsigned)(sym_tiles(out.nt) - tile0), (unsigned)batch);
   if (D == 1)
-    kmat_sym_kernel<1><<<grid, 256, sm, st>>>(out, xpad, N, D, params, form, noise_vec, noise_stride, tile0);
+    kmat_sym_kernel<1><<<grid, 256, sm, st>>>(out, xpad, N, D, params, form, noise_vec, noise_stride, tile0, env);
   else
-    kmat_sym_kernel<0><<<grid, 256, sm, st>>>(out, xpad, N, D, params, form, noise_vec, noise_stride, tile0);
+    kmat_sym_kernel<0><<<grid, 256, sm, st>>>(out, xpad, N, D, params, form, noise_vec, noise_stride, tile0, env);
   return cudaGetLastError();
 }
 

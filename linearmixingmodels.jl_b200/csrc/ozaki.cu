@@ -222,6 +222,8 @@ struct OzakiArgs {
   int a_ntc;                  // tiles per row of X
   const double* a_scale;      // [batch][ntr * 128]
   size_t a_scale_stride;
+  const int* env;             // nullable (factor only): tile envelope [batch][env_stride]; tile (I,J) sums k in [max(env[I], env[J]), k1)
+  int env_stride;
 };
 
 template <int S, int BITS>
@@ -229,13 +231,21 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_update_kernel(OzakiArgs g
   extern __shared__ __align__(1024) uint8_t oz_smem_raw[];
   const int J = g.j0 + blockIdx.x, I = g.i0 + blockIdx.y, b = blockIdx.z;
   if (!g.a_slices && I < J) return;
+  // first k-tile: the products below it have an all-zero operand (outside the envelope).  Decided from blockIdx only, so the whole
+  // CTA leaves together -- before any barrier or tensor memory exists.
+  int kb = 0;
+  if (g.env) {
+    const int* e = g.env + (size_t)b * g.env_stride;
+    kb = max(e[I], e[J]);
+    if (kb >= g.k1) return;
+  }
   // 1024-aligned carve-up: stages, then barriers
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(oz_smem_raw) + 127) & ~(uintptr_t)127);
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + (size_t)OZ_RING_BYTES);
   // each pass has its own ring geometry and its own barriers: [pass][full 0..5 | empty 0..5]
   uint64_t* acc_full = bars + 24;              // MMAs of the current pass complete
   uint64_t* acc_empty = acc_full + 1;          // epilogue of pass A has drained TMEM
-  uint64_t* init_done = acc_empty + 1;         // [2]: the issuer of quarter 0 has issued it (the accumulators of the pass are initialised)
+  uint64_t* init_done = acc_empty + 1;         // [2]: the issuer of the first quarter (k-tile kb) has issued it (the accumulators of the pass are initialised)
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 3);
   double* colscale = reinterpret_cast<double*>(bars + 32);  // [128]
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -257,15 +267,15 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_update_kernel(OzakiArgs g
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem = *tmem_slot;
   const size_t tile_bytes = (size_t)S * 16384;
-  const int nq = g.k1 * 4;  // K quarters per pass
+  const int nq = (g.k1 - kb) * 4;  // K quarters per pass, counted from k-tile kb
   const int nsA = S < 4 ? S : 4;
 
   if (warp == 8) {
     // ===== producer: per K quarter one bulk copy of the needed slices of A(I,k) and one of B(J,k)
     if (lane == 0) {
       const uint8_t* Abase = g.a_slices ? g.a_slices + (size_t)b * g.a_batch_stride + (size_t)I * g.a_ntc * tile_bytes
-                                        : g.slices + (size_t)b * g.slice_batch_stride + sym_tile_index(I, 0) * tile_bytes;
-      const uint8_t* Bbase = g.slices + (size_t)b * g.slice_batch_stride + sym_tile_index(J, 0) * tile_bytes;
+                                        : g.slices + (size_t)b * g.slice_batch_stride + sym_tile_index(I, kb) * tile_bytes;
+      const uint8_t* Bbase = g.slices + (size_t)b * g.slice_batch_stride + sym_tile_index(J, kb) * tile_bytes;
       for (int pass = 0; pass < 2; ++pass) {
         const int ns = pass ? S : nsA;
         if (pass && S <= 4) break;
@@ -290,8 +300,8 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_update_kernel(OzakiArgs g
     // odd K quarters: the per-stage hand-shake of an issuer (wait for the stage, fence, commit: ~450 clk, measured with the MMAs
     // switched off) does not overlap with its own MMAs -- with one issuer the tensor pipe idled that long after every stage
     // (66 % of peak whatever the operand stream did); with two, one issues while the other shakes hands.  int32 accumulation
-    // commutes, so the interleaving of the two streams is irrelevant EXCEPT for quarter 0, whose MMAs initialise the accumulators:
-    // the odd issuer starts a pass only after the even one has issued quarter 0 (init_done).  Each issuer commits its own
+    // commutes, so the interleaving of the two streams is irrelevant EXCEPT for the first quarter (kq = 0: the first quarter of k-tile
+    // kb), whose MMAs initialise the accumulators: the odd issuer starts a pass only after the even one has issued it (init_done).  Each issuer commits its own
     // stages; acc_full completes when both have committed their last one.
     if (lane == 0) {
       const int who = warp - 9;
@@ -372,9 +382,10 @@ __global__ void __launch_bounds__(128) ozaki_scale_kernel(TiledSym L, double* __
 // out_ntc = 0: the factor (packed-lower tile order, tiles with k > I skipped); > 0: a rectangular matrix with out_ntc tiles per row
 __global__ void __launch_bounds__(256) ozaki_slice_kernel(TileOperand L, const double* __restrict__ scale, size_t scale_batch_stride,
                                                           uint8_t* __restrict__ slices, size_t slice_batch_stride, int i0, int k0, int S, int bits,
-                                                          int out_ntc) {
+                                                          int out_ntc, const int* __restrict__ env, int env_stride) {
   const int k = k0 + blockIdx.x, I = i0 + blockIdx.y, b = blockIdx.z;
   if (!out_ntc && k > I) return;
+  if (env && k < env[(size_t)b * env_stride + I]) return;  // outside the envelope: zero, and never read by the update
   const double* tile = L.tile(b, I, k);
   uint8_t* out = slices + (size_t)b * slice_batch_stride + (out_ntc ? (size_t)I * out_ntc + k : sym_tile_index(I, k)) * ((size_t)S * 16384);
   for (int it = threadIdx.x; it < 1024; it += 256) {
@@ -437,17 +448,17 @@ cudaError_t launch_ozaki_scales(cudaStream_t st, TiledSym L, int batch, double* 
   return cudaGetLastError();
 }
 cudaError_t launch_ozaki_slice(cudaStream_t st, TiledSym L, const double* scale, size_t scale_batch_stride, uint8_t* slices,
-                               size_t slice_batch_stride, int i0, int nrows, int k0, int ncols, int batch, int S, int bits) {
+                               size_t slice_batch_stride, int i0, int nrows, int k0, int ncols, int batch, int S, int bits, const int* env) {
   if (nrows <= 0 || ncols <= 0 || batch <= 0) return cudaSuccess;
   ozaki_slice_kernel<<<dim3((unsigned)ncols, (unsigned)nrows, (unsigned)batch), 256, 0, st>>>(operand(L), scale, scale_batch_stride, slices,
-                                                                                            slice_batch_stride, i0, k0, S, bits, 0);
+                                                                                            slice_batch_stride, i0, k0, S, bits, 0, env, L.nt);
   return cudaGetLastError();
 }
 cudaError_t launch_ozaki_slice_rect(cudaStream_t st, TiledRect X, const double* scale, size_t scale_batch_stride, uint8_t* slices,
                                     size_t slice_batch_stride, int k0, int ncols, int batch, int S, int bits) {
   if (X.ntr <= 0 || ncols <= 0 || batch <= 0) return cudaSuccess;
   ozaki_slice_kernel<<<dim3((unsigned)ncols, (unsigned)X.ntr, (unsigned)batch), 256, 0, st>>>(operand(X), scale, scale_batch_stride, slices,
-                                                                                             slice_batch_stride, 0, k0, S, bits, X.ntc);
+                                                                                             slice_batch_stride, 0, k0, S, bits, X.ntc, nullptr, 0);
   return cudaGetLastError();
 }
 
@@ -501,9 +512,10 @@ static cudaError_t oz_launch(cudaStream_t st, dim3 grid, const OzakiArgs& a) {
 cudaError_t oz_dispatch(cudaStream_t st, dim3 grid, const OzakiArgs& a, int S, int bits);
 
 cudaError_t launch_ozaki_update(cudaStream_t st, TiledSym L, const uint8_t* slices, size_t slice_batch_stride, const double* scale,
-                                size_t scale_batch_stride, int i0, int nrows, int j0, int ncols, int k1, int batch, int S, int bits) {
+                                size_t scale_batch_stride, int i0, int nrows, int j0, int ncols, int k1, int batch, int S, int bits,
+                                const int* env) {
   if (nrows <= 0 || ncols <= 0 || batch <= 0 || k1 <= 0) return cudaSuccess;
-  OzakiArgs a{slices, slice_batch_stride, scale, scale_batch_stride, operand(L), i0, j0, k1, S, nullptr, 0, 0, nullptr, 0};
+  OzakiArgs a{slices, slice_batch_stride, scale, scale_batch_stride, operand(L), i0, j0, k1, S, nullptr, 0, 0, nullptr, 0, env, L.nt};
   const dim3 grid((unsigned)ncols, (unsigned)nrows, (unsigned)batch);
   return oz_dispatch(st, grid, a, S, bits);
 }
@@ -513,7 +525,8 @@ cudaError_t launch_ozaki_update_rect(cudaStream_t st, TiledRect X, const uint8_t
                                      size_t xscale_stride, const uint8_t* lslices, size_t lslice_batch_stride, const double* lscale,
                                      size_t lscale_stride, int j0, int ncols, int k1, int batch, int S, int bits) {
   if (X.ntr <= 0 || ncols <= 0 || batch <= 0 || k1 <= 0) return cudaSuccess;
-  OzakiArgs a{lslices, lslice_batch_stride, lscale, lscale_stride, operand(X), 0, j0, k1, S, xslices, xslice_batch_stride, X.ntc, xscale, xscale_stride};
+  OzakiArgs a{lslices, lslice_batch_stride, lscale, lscale_stride, operand(X), 0, j0, k1, S, xslices, xslice_batch_stride, X.ntc, xscale, xscale_stride,
+              nullptr, 0};
   const dim3 grid((unsigned)ncols, (unsigned)X.ntr, (unsigned)batch);
   return oz_dispatch(st, grid, a, S, bits);
 }

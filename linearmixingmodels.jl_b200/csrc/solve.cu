@@ -117,6 +117,9 @@ __global__ void __launch_bounds__(256) bwd_step_kernel(TiledSym L, const double*
 // The tile loads do not depend on the flags: they are issued one 16-value chunk ahead (register double buffer) so a
 // CTA that is waiting for z_K already has the first part of tile (I, K) in flight.  Summation order is fixed (per
 // thread: K ascending; then lane / warp reduction trees) -> bit-reproducible run to run.
+// With the tile envelope (env[b][I]: L(I,K) = 0 for K < env[b][I]) row I starts at K = env[b][I] and column J visits only the rows
+// with env[b][I] <= J: the skipped terms are exact zeros, so the sums -- and the solutions -- are those of the full sweep, without
+// the loads of the zero tiles or the waits for the blocks they would multiply.  The envelope need not be monotone (unsorted x).
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ int ld_acquire_gpu(const int* p) {
   int v;
@@ -162,25 +165,26 @@ constexpr int SW_CH = 16;  // tile elements per thread per chunk (a 128x128 tile
 // grid nt*batch (linear index = I*batch + b), 256 threads.
 __global__ void __launch_bounds__(256, 3) fwd_sweep_kernel(TiledSym L, const double* __restrict__ W, size_t w_batch_stride,
                                                            const double* __restrict__ rhs, double* __restrict__ sol, size_t vec_stride,
-                                                           int* __restrict__ flags, int batch) {
+                                                           int* __restrict__ flags, int batch, const int* __restrict__ env) {
   __shared__ __align__(16) double xs[2][TILE];
   __shared__ double ys[TILE];
   const int I = blockIdx.x / batch, b = blockIdx.x % batch, t = threadIdx.x, lane = t & 31, warp = t >> 5;
   const int nt = L.nt;
-  const double* row = L.tile(b, I, 0);  // tiles (I, 0..I-1) are contiguous
+  const int K0 = env ? min(env[(size_t)b * nt + I], I) : 0;  // first tile column of the row that is not zero
+  const double* row = L.tile(b, I, K0);  // tiles (I, K0..I-1) are contiguous
   double* zb = sol + (size_t)b * vec_stride;
   int* fl = flags + (size_t)b * nt;
   double a0 = 0.0, a1 = 0.0;
   double buf[SW_CH];
-  if (I > 0) {
+  if (I > K0) {
 #pragma unroll
     for (int u = 0; u < SW_CH; ++u) buf[u] = row[u * 256 + t];
   }
-  for (int K = 0; K < I; ++K) {
+  for (int K = K0; K < I; ++K) {
     if (warp == 0) stage_ready_block(fl + K, zb + (size_t)K * TILE, xs[K & 1], lane);
     __syncthreads();
     const double* xk = xs[K & 1];
-    const double* tile = row + (size_t)K * TT;
+    const double* tile = row + (size_t)(K - K0) * TT;
 #pragma unroll
     for (int c = 0; c < 64 / SW_CH; ++c) {
       double nxt[SW_CH];
@@ -242,7 +246,7 @@ constexpr int SW_CHB = 8;  // the backward sweep carries 32 accumulators per thr
 // grid nt*batch (linear index = (nt-1-J)*batch + b), 256 threads.
 __global__ void __launch_bounds__(256, 2) bwd_sweep_kernel(TiledSym L, const double* __restrict__ W, size_t w_batch_stride,
                                                            const double* __restrict__ rhs, double* __restrict__ sol, size_t vec_stride,
-                                                           int* __restrict__ flags, int batch) {
+                                                           int* __restrict__ flags, int batch, const int* __restrict__ env) {
   __shared__ __align__(16) double xs[2][TILE];
   __shared__ double ys[TILE];
   __shared__ double part[8 * TILE];
@@ -251,26 +255,36 @@ __global__ void __launch_bounds__(256, 2) bwd_sweep_kernel(TiledSym L, const dou
   const int rlo = warp * 8 + ((t >> 2) & 7);
   double* ab = sol + (size_t)b * vec_stride;
   int* fl = flags + (size_t)b * nt;
+  const int* eb = env ? env + (size_t)b * nt : nullptr;
+  // the next row above I whose tile in column J is inside the envelope; J when there is none
+  auto next_row = [&](int r) {
+    --r;
+    if (eb)
+      while (r > J && __ldg(eb + r) > J) --r;
+    return r;
+  };
   double acc[32];
 #pragma unroll
   for (int j = 0; j < 32; ++j) acc[j] = 0.0;
   double buf[SW_CHB];
-  if (J < nt - 1) {
-    const double* tile = L.tile(b, nt - 1, J);
+  int I = next_row(nt);
+  if (I > J) {
+    const double* tile = L.tile(b, I, J);
 #pragma unroll
     for (int u = 0; u < SW_CHB; ++u) buf[u] = tile[u * 256 + t];
   }
   int par = 0;
-  for (int I = nt - 1; I > J; --I, par ^= 1) {
+  for (; I > J; par ^= 1) {
+    const int In = next_row(I);
     if (warp == 0) stage_ready_block(fl + I, ab + (size_t)I * TILE, xs[par], lane);
     __syncthreads();
     const double x0 = xs[par][rlo], x1 = xs[par][rlo + 64];
     const double* tile = L.tile(b, I, J);
-    const double* tnext = (I - 1 > J) ? L.tile(b, I - 1, J) : tile;
+    const double* tnext = (In > J) ? L.tile(b, In, J) : tile;
 #pragma unroll
     for (int c = 0; c < 64 / SW_CHB; ++c) {
       double nxt[SW_CHB];
-      const bool more = (c + 1 < 64 / SW_CHB) || (I - 1 > J);
+      const bool more = (c + 1 < 64 / SW_CHB) || (In > J);
       const double* np = (c + 1 < 64 / SW_CHB) ? tile + (c + 1) * SW_CHB * 256 + t : tnext + t;
       if (more) {
 #pragma unroll
@@ -287,6 +301,7 @@ __global__ void __launch_bounds__(256, 2) bwd_sweep_kernel(TiledSym L, const dou
         for (int u = 0; u < SW_CHB; ++u) buf[u] = nxt[u];
       }
     }
+    I = In;
   }
   gemv_t_reduce_store(acc, part, ys);
   // r_J = rhs_J - (column sums) ;  a_J = W_J^T r_J
@@ -309,12 +324,12 @@ static cudaError_t sweep_flags(cudaStream_t st, int n, int** out) {
 
 // rvec is the right-hand side; it is left untouched by the persistent sweeps (the stepwise kernels consume it).
 cudaError_t launch_fwd_solve(cudaStream_t st, TiledSym L, const double* W, size_t w_batch_stride, double* rvec, double* zvec,
-                             size_t vec_stride, int batch, int64_t* launches) {
+                             size_t vec_stride, int batch, int64_t* launches, const int* env) {
   if (g_solve_impl == 1) {
     int* flags = nullptr;
     cudaError_t e = sweep_flags(st, L.nt * batch, &flags);
     if (e != cudaSuccess) return e;
-    fwd_sweep_kernel<<<(unsigned)(L.nt * batch), 256, 0, st>>>(L, W, w_batch_stride, rvec, zvec, vec_stride, flags, batch);
+    fwd_sweep_kernel<<<(unsigned)(L.nt * batch), 256, 0, st>>>(L, W, w_batch_stride, rvec, zvec, vec_stride, flags, batch, env);
     if (launches) ++*launches;
     e = cudaGetLastError();
     cudaFreeAsync(flags, st);
@@ -329,12 +344,12 @@ cudaError_t launch_fwd_solve(cudaStream_t st, TiledSym L, const double* W, size_
 }
 
 cudaError_t launch_bwd_solve(cudaStream_t st, TiledSym L, const double* W, size_t w_batch_stride, double* rvec, double* avec,
-                             size_t vec_stride, int batch, int64_t* launches) {
+                             size_t vec_stride, int batch, int64_t* launches, const int* env) {
   if (g_solve_impl == 1) {
     int* flags = nullptr;
     cudaError_t e = sweep_flags(st, L.nt * batch, &flags);
     if (e != cudaSuccess) return e;
-    bwd_sweep_kernel<<<(unsigned)(L.nt * batch), 256, 0, st>>>(L, W, w_batch_stride, rvec, avec, vec_stride, flags, batch);
+    bwd_sweep_kernel<<<(unsigned)(L.nt * batch), 256, 0, st>>>(L, W, w_batch_stride, rvec, avec, vec_stride, flags, batch, env);
     if (launches) ++*launches;
     e = cudaGetLastError();
     cudaFreeAsync(flags, st);
