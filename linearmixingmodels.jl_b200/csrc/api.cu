@@ -195,6 +195,7 @@ extern "C" int lmm_ctx_destroy(lmm_ctx* ctx) {
   if (ctx->xbuf) cudaFree(ctx->xbuf);
   if (ctx->oz_slices) cudaFree(ctx->oz_slices);
   if (ctx->oz_scale) cudaFree(ctx->oz_scale);
+  if (ctx->oz_fp) cudaFree(ctx->oz_fp);
   if (ctx->oz_x) cudaFree(ctx->oz_x);
   for (auto& e : ctx->oz_events) cudaEventDestroy(e);  // "ozaki_time" events nobody read back
   cudaStreamDestroy(ctx->panel_stream);

@@ -38,6 +38,8 @@ struct OzWs {
   size_t slice_stride;  // bytes per latent
   double* scale;
   size_t scale_stride;  // doubles per latent
+  uint8_t* fp;          // first digit plane with a nonzero digit of each sliced tile (S: all zero), written by the slice kernel
+  size_t fp_stride;     // bytes per latent (sym_tiles)
   int S, min_k, bits;  // digit planes, smallest K (k-tiles) the int8 update takes, bits per digit (7: radix 128, 8: radix 256)
 };
 
@@ -97,12 +99,13 @@ cudaError_t chol_factor_stream(lmm_ctx* ctx, cudaStream_t st, TiledSym L, double
           cudaEvent_t ev0 = nullptr, ev1 = nullptr;
           if (ctx->ozaki_time && cudaEventCreate(&ev0) == cudaSuccess && cudaEventCreate(&ev1) == cudaSuccess) cudaEventRecord(ev0, st);
           e = launch_ozaki_update(st, L, oz->slices, oz->slice_stride, oz->scale, oz->scale_stride, r0, nr, s0, s1 - s0, s0, batch, oz->S, oz->bits,
-                                  env_d);
+                                  env_d, oz->fp, oz->fp_stride);
           if (ev0 && ev1) {
             cudaEventRecord(ev1, st);
             ctx->oz_events.push_back(ev0);
             ctx->oz_events.push_back(ev1);
-            // 128^3 tile products this launch runs: tiles (I, J), I >= J, times their k-tiles (s0, or from the later envelope on)
+            // 128^3 tile products in this launch's envelope: tiles (I, J), I >= J, times their k-tiles (s0, or from the later envelope
+            // on).  Nominal: the kernel skips the k-tiles whose digit products are all zero (first_plane), which no host count sees.
             double tp = 0.0;
             for (int J = s0; J < s1; ++J)
               for (int I = J > r0 ? J : r0; I < r0 + nr; ++I) {
@@ -162,7 +165,7 @@ cudaError_t chol_factor_stream(lmm_ctx* ctx, cudaStream_t st, TiledSym L, double
     const int ns = oz && s1 < nt ? rows(s1, s1) : 0;
     if (ns > 0) {  // the block column is final: digit planes of its tiles below the block, for the later wide updates
       if ((e = launch_ozaki_slice(st, L, oz->scale, oz->scale_stride, oz->slices, oz->slice_stride, s1, ns, s0, s1 - s0, batch, oz->S, oz->bits,
-                                  env_d)) != cudaSuccess)
+                                  env_d, oz->fp, oz->fp_stride)) != cudaSuccess)
         return e;
       ++ctx->launches;
     }
@@ -205,7 +208,19 @@ static int ozaki_workspace(lmm_ctx* ctx, int nt, int batch, OzWs& ws) {
     }
     ctx->oz_scale_bytes = have * per_scale * sizeof(double);
   }
-  ws = OzWs{(uint8_t*)ctx->oz_slices, per_slices, ctx->oz_scale, per_scale, ctx->ozaki, ctx->ozaki_min_k, ctx->ozaki_bits};
+  const size_t per_fp = sym_tiles(nt);
+  if (ctx->oz_fp_bytes < have * per_fp) {
+    cudaStreamSynchronize(ctx->stream);
+    if (ctx->oz_fp) cudaFree(ctx->oz_fp);
+    ctx->oz_fp = nullptr;
+    ctx->oz_fp_bytes = 0;
+    if (cudaMalloc(&ctx->oz_fp, have * per_fp) != cudaSuccess) {
+      cudaGetLastError();
+      return 0;
+    }
+    ctx->oz_fp_bytes = have * per_fp;
+  }
+  ws = OzWs{(uint8_t*)ctx->oz_slices, per_slices, ctx->oz_scale, per_scale, ctx->oz_fp, per_fp, ctx->ozaki, ctx->ozaki_min_k, ctx->ozaki_bits};
   return (int)have;
 }
 
@@ -613,6 +628,7 @@ cudaError_t chol_factor(lmm_ctx* ctx, TiledSym L, double* W, size_t wstride, int
     tmp = *oz;
     tmp.slices += (size_t)b0 * oz->slice_stride;
     tmp.scale += (size_t)b0 * oz->scale_stride;
+    tmp.fp += (size_t)b0 * oz->fp_stride;
     return &tmp;
   };
   // small grids (few latents x few tile rows, e.g. the reference's notebook shape: 20 latents, 5 tile columns): ONE stream,

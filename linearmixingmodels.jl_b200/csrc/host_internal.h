@@ -96,6 +96,8 @@ struct lmm_ctx {
   size_t oz_x_bytes = 0;
   double* oz_scale = nullptr;
   size_t oz_scale_bytes = 0;
+  uint8_t* oz_fp = nullptr;   // [latents in flight][sym_tiles]: first digit plane of each sliced factor tile with a nonzero digit (S: none)
+  size_t oz_fp_bytes = 0;
   void* xbuf = nullptr;  // exchange buffers of the row-cyclic schedule (send | all-gathered), grown on demand
   size_t xbuf_bytes = 0;
 

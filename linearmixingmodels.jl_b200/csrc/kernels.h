@@ -111,14 +111,17 @@ cudaError_t launch_rhs_row_extract(cudaStream_t st, TiledSym L, int I, int s0, i
 cudaError_t launch_ozaki_scales(cudaStream_t st, TiledSym L, int batch, double* scale, size_t scale_batch_stride);
 // slice the finished tiles (I, k), I in [i0, i0 + nrows), k in [k0, k0 + ncols), into S int8 digit planes (S * 16 KB per tile)
 // env (nullable, [batch][L.nt]): tiles with k < env[b][I] are zero, are never read, and are not sliced
+// first_plane (nullable, [batch][fp_stride], packed-lower tile order): per sliced tile the first plane with a nonzero digit, S when
+// every digit is zero (such a tile's planes are then not written)
 cudaError_t launch_ozaki_slice(cudaStream_t st, TiledSym L, const double* scale, size_t scale_batch_stride, uint8_t* slices,
                                size_t slice_batch_stride, int i0, int nrows, int k0, int ncols, int batch, int S, int bits,
-                               const int* env = nullptr);
+                               const int* env = nullptr, uint8_t* first_plane = nullptr, size_t fp_stride = 0);
 // C(I,J) -= sum_{k < k1} L(I,k) L(J,k)' for I in [i0, i0 + nrows), J in [j0, j0 + ncols), I >= J, from the sliced factor;
-// env (nullable, [batch][L.nt]): the k range of tile (I, J) starts at max(env[b][I], env[b][J])
+// env (nullable, [batch][L.nt]): the k range of tile (I, J) starts at max(env[b][I], env[b][J]);
+// first_plane (nullable, as written by launch_ozaki_slice): k-tiles whose digit products are all exactly zero are skipped
 cudaError_t launch_ozaki_update(cudaStream_t st, TiledSym L, const uint8_t* slices, size_t slice_batch_stride, const double* scale,
                                 size_t scale_batch_stride, int i0, int nrows, int j0, int ncols, int k1, int batch, int S, int bits,
-                                const int* env = nullptr);
+                                const int* env = nullptr, const uint8_t* first_plane = nullptr, size_t fp_stride = 0);
 // the prediction sweep X <- X L^{-T} on the same path: row scales of a FINISHED factor (row 2-norms) and of X (prior variance bound),
 // digit planes of rectangular tiles, wide update with the left operand from the sliced X
 cudaError_t launch_ozaki_factor_scales(cudaStream_t st, TiledSym L, int batch, double* scale, size_t scale_batch_stride);

@@ -33,6 +33,12 @@
 // HBM layout of the sliced tile (I,k) (S * 16 KB, at sym_tile_index(I,k) * S * 16384 bytes): [K quarter kq][plane t][4096 B], the
 // 4096 B being the canonical K-major no-swizzle UMMA operand of 128 rows x 32 K-bytes: [16-byte K chunk (2)][row (128)][16 B]
 // (core matrix = 8 rows x 16 B contiguous; LBO = 2048, SBO = 128) -- a bulk copy lands it in shared memory ready for the MMA.
+// Exact zeros skipped, bit for bit: (1) the tile envelope -- a CTA starts at k-tile max(env[I], env[J]), below which one operand
+// is 0.0 in FP64; (2) the digit planes -- entries far below their row scale round to zero digits on the fixed-point grid (SE factors at
+// about 9 lengthscales, against 37.6 for the FP64 envelope).  The slice kernel records per tile the first plane tp with a nonzero
+// digit (S: none, and then writes no planes); k-tile k adds exactly 0 to every accumulator d < tp(I,k) + tp(J,k), so pass A walks
+// only the k-tiles with tp(I,k) + tp(J,k) <= 3, pass B those with the sum <= S - 1, and a CTA with no pass-B member leaves before
+// its barriers, tensor memory or C tile exist.  For the headline SE workload this keeps about 5 % of the envelope's tile products.
 // Measurements, kernel generations, what was tried and dropped (CTA pairs, A operand from tensor memory): profiles/r02_ozaki.md.
 #include "common.cuh"
 #include "kernels.h"
@@ -46,7 +52,11 @@ constexpr int OZ_RING_BYTES = 224 * 1024;      // stage = the planes one pass ne
 __host__ __device__ constexpr int oz_stages(int planes) {
   return OZ_RING_BYTES / (2 * planes * OZ_QB) >= 6 ? 6 : (OZ_RING_BYTES / (2 * planes * OZ_QB) >= 4 ? 4 : OZ_RING_BYTES / (2 * planes * OZ_QB));
 }
-constexpr size_t OZ_SMEM = (size_t)OZ_RING_BYTES + 2048;  // + alignment slack, barriers, column scales (231 424 of the 232 448 B a CTA may have)
+constexpr size_t OZ_SMEM = (size_t)OZ_RING_BYTES + 2048;  // + alignment slack, barriers, column scales, k-tile masks (231 424 of the 232 448 B a CTA may have)
+// Words of one k-tile member mask (bit k - kb: k-tile k takes part in the pass).  The host's exact-int32 bound keeps K at most 682
+// k-tiles (6 planes of 7 bits); longer K ranges run without the digit-plane filter.  The masks and two quarter counts take the
+// last 200 B of the 2048 after the ring; the carve-up before them ends at 127 B alignment + 256 B barriers + 1024 B column scales.
+constexpr int OZ_KMASK_WORDS = 24;
 
 __device__ __forceinline__ uint32_t oz_s32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void oz_mb_init(uint64_t* bar, int count) {
@@ -224,6 +234,8 @@ struct OzakiArgs {
   size_t a_scale_stride;
   const int* env;             // nullable (factor only): tile envelope [batch][env_stride]; tile (I,J) sums k in [max(env[I], env[J]), k1)
   int env_stride;
+  const uint8_t* fp;          // nullable (factor only, k1 - kb <= 32 OZ_KMASK_WORDS): first nonzero digit plane per tile [batch][fp_stride]
+  size_t fp_stride;
 };
 
 template <int S, int BITS>
@@ -245,11 +257,45 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_update_kernel(OzakiArgs g
   // each pass has its own ring geometry and its own barriers: [pass][full 0..5 | empty 0..5]
   uint64_t* acc_full = bars + 24;              // MMAs of the current pass complete
   uint64_t* acc_empty = acc_full + 1;          // epilogue of pass A has drained TMEM
-  uint64_t* init_done = acc_empty + 1;         // [2]: the issuer of the first quarter (k-tile kb) has issued it (the accumulators of the pass are initialised)
+  uint64_t* init_done = acc_empty + 1;         // [2]: the issuer of the first quarter (first member k-tile) has issued it (the accumulators of the pass are initialised)
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 3);
   double* colscale = reinterpret_cast<double*>(bars + 32);  // [128]
+  // at the fixed end of the dynamic region (constant addresses: the epilogue, which holds its C tile in registers, has no register
+  // to spare for a pointer): K quarters per pass (4 per member, read where needed), member k-tiles of pass A / pass B
+  int* nquarters = reinterpret_cast<int*>(oz_smem_raw + OZ_SMEM - 8);
+  uint32_t* kmask = reinterpret_cast<uint32_t*>(oz_smem_raw + OZ_SMEM - 8 - 8 * OZ_KMASK_WORDS);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  constexpr int nsA = S < 4 ? S : 4;
+  // Member k-tiles of each pass.  Planes 0 .. tp - 1 of a tile whose first nonzero plane is tp are zero, so the product of k-tile k
+  // adds exactly 0 to every accumulator d < tp(I,k) + tp(J,k): pass A (d <= nsA - 1) needs tp(I,k) + tp(J,k) <= nsA - 1, pass B
+  // (d <= S - 1) the sum <= S - 1.  Without fp every k-tile of [kb, k1) is a member.
+  const int nk = g.k1 - kb;
+  int nmA = nk, nmB = nk;
+  if (g.fp) {
+    const uint8_t* fpb = g.fp + (size_t)b * g.fp_stride;
+    const uint8_t *tI = fpb + sym_tile_index(I, kb), *tJ = fpb + sym_tile_index(J, kb);
+    for (int w = warp; w * 32 < nk; w += OZ_THREADS / 32) {
+      const int k = w * 32 + lane;
+      const int sum = k < nk ? (int)tI[k] + (int)tJ[k] : 2 * S;
+      const uint32_t mA = __ballot_sync(0xffffffffu, sum <= nsA - 1), mB = __ballot_sync(0xffffffffu, sum <= S - 1);
+      if (lane == 0) {
+        kmask[w] = mA;
+        kmask[OZ_KMASK_WORDS + w] = mB;
+      }
+    }
+    __syncthreads();
+    nmA = nmB = 0;
+    for (int w = 0; w * 32 < nk; ++w) {
+      nmA += __popc(kmask[w]);
+      nmB += __popc(kmask[OZ_KMASK_WORDS + w]);
+    }
+    // every product of the tile adds exactly zero: the whole CTA leaves together, before any barrier or tensor memory exists, and
+    // C(I,J) is neither read nor written
+    if ((S > 4 ? nmB : nmA) == 0) return;
+  }
   if (tid == 0) {
+    nquarters[0] = 4 * nmA;  // a multiple of 4: both issuers get half of a pass
+    nquarters[1] = 4 * nmB;
     for (int s = 0; s < 24; ++s) oz_mb_init(&bars[s], 1);
     oz_mb_init(acc_full, 2);
     oz_mb_init(&init_done[0], 1);
@@ -267,8 +313,6 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_update_kernel(OzakiArgs g
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem = *tmem_slot;
   const size_t tile_bytes = (size_t)S * 16384;
-  const int nq = (g.k1 - kb) * 4;  // K quarters per pass, counted from k-tile kb
-  const int nsA = S < 4 ? S : 4;
 
   if (warp == 8) {
     // ===== producer: per K quarter one bulk copy of the needed slices of A(I,k) and one of B(J,k)
@@ -284,12 +328,25 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_update_kernel(OzakiArgs g
         uint64_t* full = bars + 12 * pass;
         uint64_t* empty = full + 6;
         if (pass) oz_mb_wait(acc_full, 0);  // every MMA of pass A has read its stage: the ring can change geometry
+        const int nq = nquarters[pass];
+        const uint32_t* mask = kmask + (pass ? OZ_KMASK_WORDS : 0);
+        int mw = 0, k = 0;  // member walk: word, k-tile offset from kb
+        uint32_t mbits = g.fp ? mask[0] : 0u;
         for (int kq = 0; kq < nq; ++kq) {
+          if ((kq & 3) == 0) {  // next member k-tile
+            if (g.fp) {
+              while (!mbits) mbits = mask[++mw];
+              k = 32 * mw + __ffs(mbits) - 1;
+              mbits &= mbits - 1;
+            } else {
+              k = kq >> 2;
+            }
+          }
           const int s = kq % nst;
           oz_mb_wait(&empty[s], ((kq / nst) & 1) ^ 1);
           uint8_t* st = smem + (size_t)s * (2 * half);
           oz_mb_expect_tx(&full[s], 2 * bytes);
-          const size_t off = (size_t)(kq >> 2) * tile_bytes + (size_t)(kq & 3) * S * OZ_QB;
+          const size_t off = (size_t)k * tile_bytes + (size_t)(kq & 3) * S * OZ_QB;
           oz_bulk_load(st, Abase + off, bytes, &full[s]);
           oz_bulk_load(st + half, Bbase + off, bytes, &full[s]);
         }
@@ -300,9 +357,10 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_update_kernel(OzakiArgs g
     // odd K quarters: the per-stage hand-shake of an issuer (wait for the stage, fence, commit: ~450 clk, measured with the MMAs
     // switched off) does not overlap with its own MMAs -- with one issuer the tensor pipe idled that long after every stage
     // (66 % of peak whatever the operand stream did); with two, one issues while the other shakes hands.  int32 accumulation
-    // commutes, so the interleaving of the two streams is irrelevant EXCEPT for the first quarter (kq = 0: the first quarter of k-tile
-    // kb), whose MMAs initialise the accumulators: the odd issuer starts a pass only after the even one has issued it (init_done).  Each issuer commits its own
-    // stages; acc_full completes when both have committed their last one.
+    // commutes, so the interleaving of the two streams is irrelevant EXCEPT for the first quarter (kq = 0: the first quarter of the
+    // first member k-tile), whose MMAs initialise the accumulators: the odd issuer starts a pass only after the even one has issued it (init_done).  Each issuer commits its own
+    // stages; acc_full completes when both have committed their last one.  A pass without members (pass A when every member of pass B
+    // has tp(I,k) + tp(J,k) >= 4) issues nothing: both issuers arrive on acc_full directly, and the odd one must not wait for init_done.
     if (lane == 0) {
       const int who = warp - 9;
       for (int pass = 0; pass < 2; ++pass) {
@@ -323,6 +381,11 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_update_kernel(OzakiArgs g
         if (pass) {
           oz_mb_wait(acc_empty, 0);
           asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        }
+        const int nq = nquarters[pass];
+        if (nq == 0) {
+          oz_mb_arrive(acc_full);
+          continue;
         }
         if (who == 1) oz_mb_wait(&init_done[pass], 0);
         for (int kq = who; kq < nq; kq += (dual ? 2 : 1)) {
@@ -351,7 +414,9 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_update_kernel(OzakiArgs g
       if (pass && S <= 4) break;
       oz_mb_wait_relaxed(acc_full, (uint32_t)pass);
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      oz_epi_both<S, BITS>(tmem, quad, ch, pass, rs, colscale, c);
+      // a pass without members left TMEM unwritten and would subtract exact zeros: skip it (c - 0 = c, -0.0 included).  Only pass A
+      // can be one: a CTA without members in pass B has left at the top.
+      if (pass || nquarters[0] > 0) oz_epi_both<S, BITS>(tmem, quad, ch, pass, rs, colscale, c);
       asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
       if (pass == 0) oz_mb_arrive(acc_empty);
     }
@@ -380,13 +445,41 @@ __global__ void __launch_bounds__(128) ozaki_scale_kernel(TiledSym L, double* __
 
 // ---- slice the finished tiles (I, k), I in [i0, i0 + gridDim.y), k in [k0, k0 + gridDim.x): 256 threads, thread = (row, 16 columns)
 // out_ntc = 0: the factor (packed-lower tile order, tiles with k > I skipped); > 0: a rectangular matrix with out_ntc tiles per row
+// fp (nullable, factor only): fp[b][sym_tile_index(I, k)] = the first plane with a nonzero digit, S when all digits are zero -- such a
+// tile's planes are not written (the update never reads them).  A digit of plane t is nonzero iff some entry survives the rounding
+// to the grid of plane t; all of an entry's digits are zero iff it rounds to 0 on the finest grid, R^(S-1) (both radices).
 __global__ void __launch_bounds__(256) ozaki_slice_kernel(TileOperand L, const double* __restrict__ scale, size_t scale_batch_stride,
                                                           uint8_t* __restrict__ slices, size_t slice_batch_stride, int i0, int k0, int S, int bits,
-                                                          int out_ntc, const int* __restrict__ env, int env_stride) {
+                                                          int out_ntc, const int* __restrict__ env, int env_stride, uint8_t* __restrict__ fp,
+                                                          size_t fp_stride) {
   const int k = k0 + blockIdx.x, I = i0 + blockIdx.y, b = blockIdx.z;
   if (!out_ntc && k > I) return;
   if (env && k < env[(size_t)b * env_stride + I]) return;  // outside the envelope: zero, and never read by the update
   const double* tile = L.tile(b, I, k);
+  __shared__ uint32_t nz_planes;  // bit t: plane t has a nonzero digit
+  if (fp) {
+    // all-zero tile?  X = round(y R^(S-1)) == 0 for every entry (the radix-256 rule below: X itself; radix 128: the round-to-nearest
+    // remainders of |y R^t| <= 1/2 are y R^(t+1), exact, so every digit is zero iff |y R^(S-1)| <= 1/2, i.e. rint gives 0)
+    const double fine = __longlong_as_double((long long)(1023 + (bits == 8 ? 8 : 7) * (S - 1)) << 52);  // R^(S-1), exact
+    bool any = false;
+    for (int it = threadIdx.x; it < 1024; it += 256) {
+      const int r = it & 127, c16 = it >> 7;
+      const double inv = 1.0 / scale[(size_t)b * scale_batch_stride + (size_t)I * TILE + r];
+#pragma unroll
+      for (int gq = 0; gq < 4; ++gq) {
+        const double2* p = reinterpret_cast<const double2*>(tile + (size_t)(4 * c16 + gq) * 512 + 4 * r);
+        const double2 a = p[0], c = p[1];
+        any |= (__double2ll_rn(a.x * inv * fine) | __double2ll_rn(a.y * inv * fine) | __double2ll_rn(c.x * inv * fine) |
+                __double2ll_rn(c.y * inv * fine)) != 0;
+      }
+    }
+    if (threadIdx.x == 0) nz_planes = 0;
+    if (!__syncthreads_or(any)) {
+      if (threadIdx.x == 0) fp[(size_t)b * fp_stride + sym_tile_index(I, k)] = (uint8_t)S;
+      return;
+    }
+  }
+  uint32_t nz = 0;  // this thread's planes with a nonzero digit
   uint8_t* out = slices + (size_t)b * slice_batch_stride + (out_ntc ? (size_t)I * out_ntc + k : sym_tile_index(I, k)) * ((size_t)S * 16384);
   for (int it = threadIdx.x; it < 1024; it += 256) {
     const int r = it & 127, c16 = it >> 7;  // 16 columns c16*16 .. +15 of row r
@@ -419,7 +512,10 @@ __global__ void __launch_bounds__(256) ozaki_slice_kernel(TileOperand L, const d
       }
 #pragma unroll
       for (int t = 0; t < 8; ++t)
-        if (t < S) *reinterpret_cast<uint4*>(dst + (size_t)t * OZ_QB) = make_uint4(w[t][0], w[t][1], w[t][2], w[t][3]);
+        if (t < S) {
+          *reinterpret_cast<uint4*>(dst + (size_t)t * OZ_QB) = make_uint4(w[t][0], w[t][1], w[t][2], w[t][3]);
+          if (w[t][0] | w[t][1] | w[t][2] | w[t][3]) nz |= 1u << t;
+        }
       continue;
     }
     for (int t = 0; t < S; ++t) {
@@ -439,7 +535,13 @@ __global__ void __launch_bounds__(256) ozaki_slice_kernel(TileOperand L, const d
         w[gq] = pk;
       }
       *reinterpret_cast<uint4*>(dst + (size_t)t * OZ_QB) = make_uint4(w[0], w[1], w[2], w[3]);
+      if (w[0] | w[1] | w[2] | w[3]) nz |= 1u << t;
     }
+  }
+  if (fp) {
+    if (nz) atomicOr(&nz_planes, nz);
+    __syncthreads();
+    if (threadIdx.x == 0) fp[(size_t)b * fp_stride + sym_tile_index(I, k)] = (uint8_t)(nz_planes ? __ffs(nz_planes) - 1 : S);
   }
 }
 
@@ -448,17 +550,20 @@ cudaError_t launch_ozaki_scales(cudaStream_t st, TiledSym L, int batch, double* 
   return cudaGetLastError();
 }
 cudaError_t launch_ozaki_slice(cudaStream_t st, TiledSym L, const double* scale, size_t scale_batch_stride, uint8_t* slices,
-                               size_t slice_batch_stride, int i0, int nrows, int k0, int ncols, int batch, int S, int bits, const int* env) {
+                               size_t slice_batch_stride, int i0, int nrows, int k0, int ncols, int batch, int S, int bits, const int* env,
+                               uint8_t* first_plane, size_t fp_stride) {
   if (nrows <= 0 || ncols <= 0 || batch <= 0) return cudaSuccess;
   ozaki_slice_kernel<<<dim3((unsigned)ncols, (unsigned)nrows, (unsigned)batch), 256, 0, st>>>(operand(L), scale, scale_batch_stride, slices,
-                                                                                            slice_batch_stride, i0, k0, S, bits, 0, env, L.nt);
+                                                                                            slice_batch_stride, i0, k0, S, bits, 0, env, L.nt,
+                                                                                            first_plane, fp_stride);
   return cudaGetLastError();
 }
 cudaError_t launch_ozaki_slice_rect(cudaStream_t st, TiledRect X, const double* scale, size_t scale_batch_stride, uint8_t* slices,
                                     size_t slice_batch_stride, int k0, int ncols, int batch, int S, int bits) {
   if (X.ntr <= 0 || ncols <= 0 || batch <= 0) return cudaSuccess;
   ozaki_slice_kernel<<<dim3((unsigned)ncols, (unsigned)X.ntr, (unsigned)batch), 256, 0, st>>>(operand(X), scale, scale_batch_stride, slices,
-                                                                                             slice_batch_stride, 0, k0, S, bits, X.ntc, nullptr, 0);
+                                                                                             slice_batch_stride, 0, k0, S, bits, X.ntc, nullptr, 0,
+                                                                                             nullptr, 0);
   return cudaGetLastError();
 }
 
@@ -513,9 +618,11 @@ cudaError_t oz_dispatch(cudaStream_t st, dim3 grid, const OzakiArgs& a, int S, i
 
 cudaError_t launch_ozaki_update(cudaStream_t st, TiledSym L, const uint8_t* slices, size_t slice_batch_stride, const double* scale,
                                 size_t scale_batch_stride, int i0, int nrows, int j0, int ncols, int k1, int batch, int S, int bits,
-                                const int* env) {
+                                const int* env, const uint8_t* first_plane, size_t fp_stride) {
   if (nrows <= 0 || ncols <= 0 || batch <= 0 || k1 <= 0) return cudaSuccess;
-  OzakiArgs a{slices, slice_batch_stride, scale, scale_batch_stride, operand(L), i0, j0, k1, S, nullptr, 0, 0, nullptr, 0, env, L.nt};
+  if (k1 > 32 * OZ_KMASK_WORDS) first_plane = nullptr;  // the member masks cover at most this many k-tiles
+  OzakiArgs a{slices, slice_batch_stride, scale, scale_batch_stride, operand(L), i0, j0, k1, S, nullptr, 0, 0, nullptr, 0, env, L.nt,
+              first_plane, fp_stride};
   const dim3 grid((unsigned)ncols, (unsigned)nrows, (unsigned)batch);
   return oz_dispatch(st, grid, a, S, bits);
 }
@@ -526,7 +633,7 @@ cudaError_t launch_ozaki_update_rect(cudaStream_t st, TiledRect X, const uint8_t
                                      size_t lscale_stride, int j0, int ncols, int k1, int batch, int S, int bits) {
   if (X.ntr <= 0 || ncols <= 0 || batch <= 0 || k1 <= 0) return cudaSuccess;
   OzakiArgs a{lslices, lslice_batch_stride, lscale, lscale_stride, operand(X), 0, j0, k1, S, xslices, xslice_batch_stride, X.ntc, xscale, xscale_stride,
-              nullptr, 0};
+              nullptr, 0, nullptr, 0};
   const dim3 grid((unsigned)ncols, (unsigned)X.ntr, (unsigned)batch);
   return oz_dispatch(st, grid, a, S, bits);
 }

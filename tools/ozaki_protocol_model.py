@@ -14,7 +14,14 @@ mbarrier semantics as in PTX: a barrier has a phase bit and a pending count; the
 `try_wait.parity p` succeeds once the phase with parity p has completed, i.e. as soon as the current phase bit differs from p.
 With an ODD number of stages the two-issuer variant fails exactly as the GPU did (the odd issuer's second quarter lives in the even
 issuer's first stage, and its parity wait passes before that stage has ever been filled); the kernel therefore uses two issuers only
-with an even stage count (`dual`) -- `explore(..., force_dual=True)` reproduces the failure.  Test infrastructure, CPU only."""
+with an even stage count (`dual`) -- `explore(..., force_dual=True)` reproduces the failure.
+
+Digit-plane filter: each pass walks its own MEMBER k-tiles (4 K quarters each; quarter kq is quarter kq % 4 of the kq // 4-th
+member), so `members_a` / `members_b` may be any increasing lists, with gaps, a single member, or -- pass A only -- none.  A pass
+without members issues nothing: both issuers arrive on acc_full directly (the odd one does not wait for init_done, which nobody would
+arrive on), and the epilogue skips its TMEM read (`skip`); converting accumulators no MMA of the pass has written is a violation.
+`empty_pass_fix=False` models the issuers without that rule (a plain init_done wait and commit), which deadlocks.  Test
+infrastructure, CPU only."""
 from collections import deque
 
 
@@ -22,12 +29,15 @@ class Violation(Exception):
     pass
 
 
-def build_threads(nq, nst_a, nst_b, force_dual=False):
-    """Programs as lists of (op, args): wait(bar, parity) | arrive(bar) | load(stage, pass, kq) | consume(stage, pass, kq, who) |
-    commit(bar, who) | epi(pass)."""
+def build_threads(members, nst_a, nst_b, force_dual=False, empty_pass_fix=True):
+    """Programs as lists of (op, args): wait(bar, parity) | arrive(bar) | load(stage, pass, tag) | consume(stage, pass, kq, tag, who) |
+    commit(bar, who) | epi(pass) | skip(pass).  tag = (member k-tile, quarter within it)."""
     P, E = [], []
     issuers = [[], []]
     for pas, nst in ((0, nst_a), (1, nst_b)):
+        mem = members[pas]
+        nq = 4 * len(mem)
+        tag = lambda kq, mem=mem: (mem[kq // 4], kq % 4)
         full = lambda s, p=pas: ("full", p, s)
         empty = lambda s, p=pas: ("empty", p, s)
         dual = force_dual or nst % 2 == 0
@@ -36,7 +46,7 @@ def build_threads(nq, nst_a, nst_b, force_dual=False):
         for kq in range(nq):
             s = kq % nst
             P.append(("wait", empty(s), ((kq // nst) & 1) ^ 1))
-            P.append(("load", s, pas, kq))
+            P.append(("load", s, pas, tag(kq)))
         for who in (0, 1):
             T = issuers[who]
             if who == 1 and not dual:
@@ -46,25 +56,32 @@ def build_threads(nq, nst_a, nst_b, force_dual=False):
                 continue
             if pas:
                 T.append(("wait", ("acc_empty",), 0))
+            if nq == 0 and empty_pass_fix:
+                T.append(("arrive", ("acc_full",)))
+                continue
             if who == 1:
                 T.append(("wait", ("init_done", pas), 0))
             for kq in range(who, nq, 2 if dual else 1):
                 s = kq % nst
                 T.append(("wait", full(s), (kq // nst) & 1))
-                T.append(("consume", s, pas, kq, who))
+                T.append(("consume", s, pas, kq, tag(kq), who))
                 T.append(("commit", empty(s), who, s, pas))
                 if kq == 0:
                     T.append(("arrive", ("init_done", pas)))
             T.append(("commit", ("acc_full",), who, None, pas))
         E.append(("wait", ("acc_full",), pas))
-        E.append(("epi", pas))
+        E.append(("epi", pas) if nq or not empty_pass_fix else ("skip", pas))
         if pas == 0:
             E.append(("arrive", ("acc_empty",)))
     return [P, issuers[0], issuers[1], E]
 
 
-def explore(nq=8, nst_a=6, nst_b=4, force_dual=False, max_states=2_000_000):
-    threads = build_threads(nq, nst_a, nst_b, force_dual)
+def explore(nq=8, nst_a=6, nst_b=4, force_dual=False, max_states=2_000_000, members_a=None, members_b=None, empty_pass_fix=True):
+    """nq: K quarters per pass when the member lists are not given (every k-tile 0 .. nq/4 - 1 is a member)."""
+    dense = list(range(nq // 4))
+    members = (dense if members_a is None else list(members_a), dense if members_b is None else list(members_b))
+    nqs = (4 * len(members[0]), 4 * len(members[1]))
+    threads = build_threads(members, nst_a, nst_b, force_dual, empty_pass_fix)
     counts = {("acc_full",): 2, ("acc_empty",): 1}
     bars0 = {}
     for T in threads:
@@ -124,7 +141,7 @@ def explore(nq=8, nst_a=6, nst_b=4, force_dual=False, max_states=2_000_000):
             elif ins[0] == "arrive":
                 succ.append((npcs, arrive(bars, bidx[ins[1]]), content, flight, busy, fifo, issued, executed, epis, uncommitted))
             elif ins[0] == "load":
-                _, s, pas, kq = ins
+                _, s, pas, kq = ins  # kq: the tag (member k-tile, quarter)
                 if busy[s]:
                     raise Violation(f"producer overwrites stage {s} (pass {pas}, quarter {kq}) while its MMAs have not executed")
                 if flight[s] is not None:
@@ -133,9 +150,9 @@ def explore(nq=8, nst_a=6, nst_b=4, force_dual=False, max_states=2_000_000):
                 fl[s] = (pas, kq, bidx[("full", pas, s)])
                 succ.append((npcs, bars, content, tuple(fl), busy, fifo, issued, executed, epis, uncommitted))
             elif ins[0] == "consume":
-                _, s, pas, kq, who = ins
-                if content[s] != (pas, kq) or flight[s] is not None:
-                    raise Violation(f"issuer {who} consumes stage {s} for pass {pas} quarter {kq} but it holds {content[s]} (in flight: {flight[s]})")
+                _, s, pas, kq, tg, who = ins
+                if content[s] != (pas, tg) or flight[s] is not None:
+                    raise Violation(f"issuer {who} consumes stage {s} for pass {pas} quarter {kq} {tg} but it holds {content[s]} (in flight: {flight[s]})")
                 if kq != 0 and issued[pas] == 0:
                     raise Violation(f"pass {pas}: quarter {kq} issued before quarter 0 (accumulators not initialised)")
                 if pas == 1 and epis < 1:
@@ -156,8 +173,12 @@ def explore(nq=8, nst_a=6, nst_b=4, force_dual=False, max_states=2_000_000):
                 succ.append((npcs, bars, content, flight, busy, tuple(ff), issued, executed, epis, tuple(un)))
             elif ins[0] == "epi":
                 pas = ins[1]
-                if executed[pas] != nq:
-                    raise Violation(f"epilogue of pass {pas} starts with {executed[pas]} of {nq} quarters executed")
+                if executed[pas] != nqs[pas]:
+                    raise Violation(f"epilogue of pass {pas} starts with {executed[pas]} of {nqs[pas]} quarters executed")
+                if issued[pas] == 0:
+                    raise Violation(f"epilogue of pass {pas} reads accumulators that no MMA has initialised")
+                succ.append((npcs, bars, content, flight, busy, fifo, issued, executed, epis + 1, uncommitted))
+            elif ins[0] == "skip":
                 succ.append((npcs, bars, content, flight, busy, fifo, issued, executed, epis + 1, uncommitted))
         # asynchronous agents: a copy lands; the oldest outstanding commit of an issuer fires (its MMAs have executed)
         for s in range(nstages):
@@ -205,3 +226,9 @@ if __name__ == "__main__":
         explore(8, 6, 3, force_dual=True)
     except Violation as v:
         print("two issuers on 3 stages:", v)
+    print("empty pass A, members 1, 4 in pass B:", explore(members_a=[], members_b=[1, 4]))
+    print("single member in both passes:", explore(members_a=[3], members_b=[3]))
+    try:
+        explore(members_a=[], members_b=[0, 2], empty_pass_fix=False)
+    except Violation as v:
+        print("empty pass A without its rule:", v)
