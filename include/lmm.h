@@ -106,6 +106,9 @@ const char* lmm_version(void);
  *   "streams"         latent groups factored concurrently on separate CUDA streams (default 4, 1..8)
  *   "lookahead"       schedule for batches <= 2: 1 = right-looking block schedule, the next block column on a high-priority
  *                     panel stream, the rest of the trailing update as one large GEMM on a second stream [default]; 0 = plain
+ *   "kmat_skip"       OILMM / IndependentMOGP logpdf and posterior: 1 = build only the kernel-matrix tiles that are not provably
+ *                     exact zeros (far-apart point tiles of the SE / Matern kernels) [default]; a kept posterior writes those
+ *                     zeros on its first read.  0 = build every tile.  The results are the same bits either way.
  *   "chain_fused"     1 = where the grids are small (batches <= 2, or few latents x few tile rows) the panel chain of a tile
  *                     column -- TRSM of the column, update of the next column(s), factorisation of the next diagonal tile --
  *                     is ONE launch whose CTAs hand tiles to each other through ready counters in global memory, the

@@ -232,6 +232,9 @@ extern "C" int lmm_ctx_set_option(lmm_ctx* ctx, const char* key, double value) {
   } else if (k == "lookahead") {
     if (value != 0.0 && value != 1.0) return ctx->fail(LMM_E_ARG, "lookahead must be 0 (plain) or 1 (right-looking block schedule on two streams)");
     ctx->lookahead = (int)value;
+  } else if (k == "kmat_skip") {
+    if (value != 0.0 && value != 1.0) return ctx->fail(LMM_E_ARG, "kmat_skip must be 0 (build every kernel-matrix tile) or 1");
+    ctx->kmat_skip = (int)value;
   } else if (k == "chain_fused") {
     if (value != 0.0 && value != 1.0 && value != 2.0) return ctx->fail(LMM_E_ARG, "chain_fused must be 0, 1 (where it pays off) or 2 (everywhere)");
     ctx->chain_fused = (int)value;

@@ -155,6 +155,19 @@ __device__ __forceinline__ double kappa_eval(int kind, double variance, double d
   }
   return variance * v;
 }
+// kappa_eval(kind, variance, d2) is exactly 0 for every d2 > kappa_zero_d2(kind) and finite variance: exp_nonpos flushes below
+// -708, and the Matern prefactors stay finite.  The thresholds carry a 2^-40 relative guard for the rounded sqrt and the rounded
+// products by sqrt(3) / sqrt(5) in front of the exp.  +inf for the kinds that never give an exact 0 (RationalQuadratic).
+__host__ __device__ __forceinline__ double kappa_zero_d2(int kind) {
+  const double g = 1.0 + 0x1p-40;
+  switch (kind) {
+    case 0: return 1416.0 * g;                                                          // SE: exp(-d²/2)
+    case 1: return (708.0 / 1.7320508075688772) * (708.0 / 1.7320508075688772) * g;  // Matern32: exp(-√3 d)
+    case 2: return (708.0 / 2.23606797749979) * (708.0 / 2.23606797749979) * g;      // Matern52: exp(-√5 d)
+    case 3: return 708.0 * 708.0 * g;                                                   // Matern12: exp(-d)
+    default: return __builtin_huge_val();
+  }
+}
 
 // Squared distance of scaled points.  form 0: Distances.jl pairwise (|a|²+|b|² - 2 a·b, clamped at
 // 0); form 1: direct differences.  a, b point at D scaled coordinates.

@@ -151,7 +151,7 @@ cudaError_t chol_factor_stream(lmm_ctx* ctx, cudaStream_t st, TiledSym L, double
       if (t0 >= nt) continue;
       // small grid, not at a block boundary, nothing above jstart involved: TRSM(jj) + update(jj+1) + potrf(jj+1) in one launch
       if (counters && ctx->chain_fused && jj + 1 < s1 && jj >= jstart && (long long)(nt - 1 - jj) * batch <= CHAIN_MAX_TILES) {
-        if ((e = launch_chain_column(st, L, W, wstride, jj, s0, jj + 2, 1, batch, logdet, info, counters)) != cudaSuccess) return e;
+        if ((e = launch_chain_column(st, L, W, wstride, jj, s0, jj + 2, 1, batch, logdet, info, counters, env_d)) != cudaSuccess) return e;
         ++ctx->launches;
         factored_ahead = true;
         continue;
@@ -589,19 +589,35 @@ cudaError_t chol_factor_rowcyclic_dist(lmm_ctx* ctx, TiledSym Lown, int nrows, i
 
 // Fork the batch into latent groups on separate streams (joined back into ctx->stream).  jstart > 0: extend a factor whose
 // tile rows < jstart are final (see chol_factor_stream).
+static bool use_rowcyclic(const lmm_ctx* ctx, int nt, int batch) {
+  return ctx->partition_ilmm && ctx->partition_now && batch == 1 && ctx->comm && ctx->nranks > 1 && nt >= 2 * ctx->nranks && nccl_api().AllGather;
+}
+static bool use_rightlooking(const lmm_ctx* ctx, int nt, int batch) {
+  // (with the integer-slice update on, a LARGE single factor is faster on the batched left-looking schedule: its wide updates run
+  // at 2-3x the DMMA rate, which outweighs the exposed panel chain -- "ozaki_single_nt" tile rows and up)
+  // (measured, 7 planes of 8 bits: N = 16384: 45.9 -> 33.1 ms, two factors 88.9 -> 44.4 ms; N = 8192: 7.1 -> 8.6 ms, two: 12.6 -> 8.7 ms)
+  const bool oz_single = ctx->ozaki && ctx->ozaki_single_nt > 0 && nt >= (batch == 1 ? ctx->ozaki_single_nt : ctx->ozaki_single_nt * 2 / 3);
+  return ctx->lookahead && batch <= 2 && nt >= 12 && !oz_single;
+}
+
+bool chol_takes_envelope(const lmm_ctx* ctx, int nt, int batch) { return !use_rowcyclic(ctx, nt, batch) && !use_rightlooking(ctx, nt, batch); }
+
 cudaError_t chol_factor(lmm_ctx* ctx, TiledSym L, double* W, size_t wstride, int batch, double* logdet, int* info, int jstart,
                         const int* env_d, const int* env_h) {
   const int G = ctx->ngroups < batch ? ctx->ngroups : batch;
   if (!env_d || !env_h) env_d = env_h = nullptr;
   auto env_at = [&](const int* e, int b0) { return e ? e + (size_t)b0 * L.nt : nullptr; };
   if (jstart == 0) {  // the look-ahead / partitioned schedules factor from scratch only
-    if (ctx->partition_ilmm && ctx->partition_now && batch == 1 && ctx->comm && ctx->nranks > 1 && L.nt >= 2 * ctx->nranks && nccl_api().AllGather)
-      return chol_factor_rowcyclic(ctx, L, W, wstride, logdet, info);
-    // (with the integer-slice update on, a LARGE single factor is faster on the batched left-looking schedule: its wide updates run
-    // at 2-3x the DMMA rate, which outweighs the exposed panel chain -- "ozaki_single_nt" tile rows and up)
-    // (measured, 7 planes of 8 bits: N = 16384: 45.9 -> 33.1 ms, two factors 88.9 -> 44.4 ms; N = 8192: 7.1 -> 8.6 ms, two: 12.6 -> 8.7 ms)
-    const bool oz_single = ctx->ozaki && ctx->ozaki_single_nt > 0 && L.nt >= (batch == 1 ? ctx->ozaki_single_nt : ctx->ozaki_single_nt * 2 / 3);
-    if (ctx->lookahead && batch <= 2 && L.nt >= 12 && !oz_single) return chol_factor_rightlooking(ctx, L, W, wstride, batch, logdet, info);
+    if (env_d && !chol_takes_envelope(ctx, L.nt, batch)) {
+      // they read every tile: write the zeros a kernel-matrix build inside the envelope left out (a chunk of the batch that the
+      // integer-slice workspace split off can land here)
+      cudaError_t ez = launch_kmat_zero(ctx->stream, L, batch, env_d);
+      if (ez != cudaSuccess) return ez;
+      ++ctx->launches;
+      env_d = env_h = nullptr;
+    }
+    if (use_rowcyclic(ctx, L.nt, batch)) return chol_factor_rowcyclic(ctx, L, W, wstride, logdet, info);
+    if (use_rightlooking(ctx, L.nt, batch)) return chol_factor_rightlooking(ctx, L, W, wstride, batch, logdet, info);
   }
   cudaError_t e;
   // optional integer-slice trailing update: workspace for as many latents as fit; a larger batch is factored in chunks

@@ -19,6 +19,7 @@ extern "C" int lmm_post_condition(lmm_post* post, const double* xs, int Ns, doub
   lmm_ctx* ctx = post->ctx;
   std::lock_guard<std::mutex> lk(ctx->mu);
   CU(cudaSetDevice(ctx->device));
+  if (int rcz = post_fill_zeros(post)) return rcz;  // the factor is read below
   if (post->kind == POST_MASKED) return ctx->fail(LMM_E_UNSUPPORTED, "a missing-data posterior offers mean_and_var only");
   if (post->joint()) return ilmm_post_condition(post, xs, Ns, sigma2, ys, out_post, info_latent);
   cudaStream_t st = ctx->stream;

@@ -556,6 +556,7 @@ extern "C" int lmm_post_mean_and_cov(lmm_post* post, const double* xs, int Ns, d
   lmm_ctx* ctx = post->ctx;
   std::lock_guard<std::mutex> lk(ctx->mu);
   CU(cudaSetDevice(ctx->device));
+  if (int rcz = post_fill_zeros(post)) return rcz;  // the factor is read below
   cudaStream_t st = ctx->stream;
   const int m = post->m, p = post->p, dim = p * Ns;
   if ((int64_t)p * Ns > 46000) return ctx->fail(LMM_E_UNSUPPORTED, "dense covariance output too large");

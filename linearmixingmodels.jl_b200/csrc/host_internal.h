@@ -78,6 +78,7 @@ struct lmm_ctx {
   size_t chain_cnt_bytes = 0;
   // one large factor (general ILMM, batch 1) partitioned row-cyclically over the ranks of the communicator
   int partition_ilmm = 0;
+  int kmat_skip = 1;  // OILMM / IndependentMOGP evals: build only the kernel-matrix tiles that are not provably exact zeros (kmat.cu)
   int condition_update = 1;  // sequential conditioning of per-latent posteriors: 1 = block-Cholesky update of the factor, 0 = re-factorise the union
   int partition_now = 0;  // set by the callers whose factorisation is replicated on every rank (ILMM joint factor)
   int dist_error = 0;  // NCCL failure inside the partitioned schedule (reported by the caller)
@@ -209,6 +210,8 @@ struct lmm_post {
   double* d_noise_vec = nullptr;  // [nloc][Npad] per-point training noise (sequentially conditioned posteriors), else null
   int* d_obs = nullptr;           // POST_MASKED: observed entries j*N + i (big_n of them)
   double* d_Ept = nullptr;        // POST_ILMM: [N][m*m] per-point projected noise blocks ΣT (extended by sequential conditioning)
+  int* d_env = nullptr;           // [nloc][nt] tile envelope of the factors (OILMM / IndependentMOGP built inside it), else null
+  bool zeros_pending = false;     // the tiles (I, k < env) of d_L were never written: post_fill_zeros writes them before a read
   size_t bytes = 0;
   int big_n = 0, big_nt = 0;  // ILMM joint dimension mN and its tile count
 
@@ -311,6 +314,8 @@ void fill_params(std::vector<LatentParams>& hp, const lmm_gp_desc* d, const doub
 int latents_run(lmm_ctx* ctx, int kind, const lmm_gp_desc* latents, int m, const double* x, int N, int D, int p, double sigma2, const double* y, const Projection& pr, const double* Hhost, const double* Uhost, const double* Shost, RunOut out, const double* noise_vec = nullptr);
 int oilmm_projection(lmm_ctx* ctx, const double* U, const double* S, int p, int m, double sigma2, int N, Projection& pr, std::vector<double>& H);
 int check_common(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const void* x, int N, int D, int p, int out_dim);
+// Every entry point that reads a posterior's factor calls this first: it writes the exact zeros the kernel-matrix build left out.
+int post_fill_zeros(lmm_post* post);
 int post_latent_marginals(lmm_post* post, const double* d_xspad, int Ns, int nts, double* d_ML, double* d_VL, int first = 0, int count = -1);
 int upload_params(lmm_ctx* ctx, DevBuf& buf, const lmm_gp_desc* descs, const double* noise_all, int lo, int hi, int D);
 int stage_latent_vectors(lmm_ctx* ctx, DevBuf& buf, const double* z, int N, size_t npad, int lo, int hi);
@@ -336,6 +341,9 @@ int ilmm_post_condition(lmm_post* post, const double* xs, int Ns, double sigma2,
 // env_d / env_h (both or neither; jstart = 0): the tile envelope of the batch (launch_kmat_sym) on the device and a host copy of it.
 // The batched left-looking schedule then skips every tile product, TRSM and slice that has an all-zero operand -- the factor is
 // bit-identical to the dense schedule's -- and sizes its grids from the host copy.  The other schedules ignore it.
+// Whether chol_factor (jstart = 0) factors `batch` matrices of nt tile rows on the batched left-looking schedule, the one that
+// takes the envelope.  The others read every tile: chol_factor writes the zeros outside the envelope before it runs them.
+bool chol_takes_envelope(const lmm_ctx* ctx, int nt, int batch);
 cudaError_t chol_factor(lmm_ctx* ctx, TiledSym L, double* W, size_t wstride, int batch, double* logdet, int* info, int jstart = 0,
                         const int* env_d = nullptr, const int* env_h = nullptr);
 cudaError_t chol_factor_rowcyclic_dist(lmm_ctx* ctx, TiledSym Lown, int nrows, int nc, double* W, size_t wstride, double* logdet, int* info,

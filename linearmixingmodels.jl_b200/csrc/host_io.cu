@@ -64,6 +64,7 @@ extern "C" int lmm_post_save(lmm_post* post, const char* path) {
   lmm_ctx* ctx = post->ctx;
   std::lock_guard<std::mutex> lk(ctx->mu);
   CU(cudaSetDevice(ctx->device));
+  if (int rcz = post_fill_zeros(post)) return rcz;  // the factor is read below
   FILE* f = fopen(path, "wb");
   if (!f) return ctx->fail(LMM_E_ARG, std::string("cannot open ") + path + " for writing");
   PostFileHeader h{};

@@ -84,7 +84,7 @@ int latents_run(lmm_ctx* ctx, int kind, const lmm_gp_desc* latents, int m, const
   const size_t per_lat = factor_bytes_per_latent(nt);
   int chunk = mloc;
   if (!keep && mloc > 0) CU(mem_fit(ctx, per_lat + 6 * npad * sizeof(double), mloc, &chunk));
-  DevBuf b_L, b_W, b_alpha, b_r, b_z, b_logdet, b_quad, b_info, b_nv, b_env;
+  DevBuf b_L, b_W, b_alpha, b_r, b_z, b_logdet, b_quad, b_info, b_nv, b_env, b_fb, b_rowoff;
   if (noise_vec) {
     const int nl = mloc > 0 ? mloc : 1;
     CU(b_nv.alloc(ctx, (size_t)nl * npad * sizeof(double)));
@@ -99,10 +99,16 @@ int latents_run(lmm_ctx* ctx, int kind, const lmm_gp_desc* latents, int m, const
   std::vector<int> hinfo(mloc > 0 ? mloc : 1, 0);
   // tile envelope of each chunk's kernel matrices: far-apart points give exact zeros that the factorisation and the solves skip
   std::vector<int> henv;
+  // the kernel-matrix build skips the tiles that are provably exact zeros (launch_kmat_bound) where the factorisation takes the envelope
+  std::vector<int> hrowoff;
+  bool skipped = false;
   float ms_kmat = 0, ms_chol = 0, ms_solve = 0;
   if (mloc > 0) {
     henv.resize((size_t)chunk * nt);
+    hrowoff.resize(henv.size() + 1);
     CU(b_env.alloc(ctx, henv.size() * sizeof(int)));
+    CU(b_fb.alloc(ctx, henv.size() * sizeof(int)));
+    CU(b_rowoff.alloc(ctx, hrowoff.size() * sizeof(int)));
     CU(b_L.alloc(ctx, (size_t)chunk * sym_tiles(nt) * TT * sizeof(double)));
     CU(b_W.alloc(ctx, (size_t)chunk * nt * TT * sizeof(double)));
     CU(b_r.alloc(ctx, (size_t)chunk * npad * sizeof(double)));
@@ -122,8 +128,22 @@ int latents_run(lmm_ctx* ctx, int kind, const lmm_gp_desc* latents, int m, const
       double* delta = b_ty.as<double>() + (size_t)c0 * npad;
       CU(cudaEventRecord(ctx->ev[2], st));
       const int* env = b_env.as<int>();
+      const bool skip = ctx->kmat_skip && chol_takes_envelope(ctx, nt, nb);
+      if (skip) {
+        // fb (one small launch) -> host: the build's grid is the tiles (I, fb[b][I] .. I) of all nb latents
+        CU(launch_kmat_bound(st, nb, b_x.as<double>(), N, D, nt, dp, b_fb.as<int>()));
+        ++ctx->launches;
+        CU(copy_out(ctx, henv.data(), b_fb.p, (size_t)nb * nt * sizeof(int)));
+        CU(cudaStreamSynchronize(st));
+        hrowoff[0] = 0;
+        for (int r = 0; r < nb * nt; ++r) hrowoff[r + 1] = hrowoff[r] + (r % nt) + 1 - henv[r];
+        ctx->h2d += (int64_t)((size_t)(nb * nt + 1) * sizeof(int));
+        CU(cudaMemcpyAsync(b_rowoff.p, hrowoff.data(), (size_t)(nb * nt + 1) * sizeof(int), cudaMemcpyHostToDevice, st));
+        skipped = true;
+      }
       CU(launch_kmat_sym(st, L, nb, b_x.as<double>(), N, D, dp, ctx->distance_form,
-                         noise_vec ? b_nv.as<double>() + (size_t)c0 * npad : nullptr, npad, 0, b_env.as<int>()));
+                         noise_vec ? b_nv.as<double>() + (size_t)c0 * npad : nullptr, npad, 0, b_env.as<int>(),
+                         skip ? b_rowoff.as<int>() : nullptr, hrowoff[nb * nt]));
       ++ctx->launches;
       CU(cudaEventRecord(ctx->ev[3], st));
       CU(copy_out(ctx, henv.data(), env, (size_t)nb * nt * sizeof(int)));  // sizes the factorisation's grids
@@ -202,6 +222,10 @@ int latents_run(lmm_ctx* ctx, int kind, const lmm_gp_desc* latents, int m, const
     P->d_params = (LatentParams*)b_params.detach();
     P->d_H = (double*)b_H.detach();
     if (noise_vec) P->d_noise_vec = (double*)b_nv.detach();
+    if (skipped) {  // a kept posterior holds every latent in one chunk: b_env is the envelope of all of them
+      P->d_env = (int*)b_env.detach();
+      P->zeros_pending = true;
+    }
     *out.post = P;
   }
   return LMM_OK;
@@ -320,7 +344,7 @@ extern "C" int lmm_post_free(lmm_post* post) {
   std::lock_guard<std::mutex> lk(ctx->mu);
   cudaSetDevice(ctx->device);
   void* ptrs[] = {post->d_xpad, post->d_L, post->d_W, post->d_alpha, post->d_delta, post->d_params, post->d_H, post->d_noise_vec,
-                  post->d_Ept, post->d_obs};
+                  post->d_Ept, post->d_obs, post->d_env};
   for (void* q : ptrs)
     if (q) cudaFreeAsync(q, ctx->stream);
   cudaStreamSynchronize(ctx->stream);
@@ -344,6 +368,7 @@ extern "C" int lmm_post_export(lmm_post* post, int i, double* Lout, double* alph
   lmm_ctx* ctx = post->ctx;
   std::lock_guard<std::mutex> lk(ctx->mu);
   CU(cudaSetDevice(ctx->device));
+  if (int rcz = post_fill_zeros(post)) return rcz;  // the factor is read below
   int b, n;
   if (post->joint()) {
     if (i != 0) return ctx->fail(LMM_E_ARG, "a joint posterior has one factor (i = 0)");
@@ -371,6 +396,15 @@ extern "C" int lmm_post_export(lmm_post* post, int i, double* Lout, double* alph
 }
 
 namespace lmm_host {
+
+int post_fill_zeros(lmm_post* post) {
+  if (!post->zeros_pending) return LMM_OK;
+  lmm_ctx* ctx = post->ctx;
+  CU(launch_kmat_zero(ctx->stream, post->Lsym(), post->nloc(), post->d_env));
+  ++ctx->launches;
+  post->zeros_pending = false;
+  return LMM_OK;
+}
 
 // Latent posterior marginals at xs for the resident latents: ML/VL [nloc][nspad] on the device.
 // mean*_i = m_i + K(x*,x) α_i ; var*_i = k(x*,x*) - colsumsq(L_i^{-1} K(x,x*))   (AbstractGPs)
@@ -412,6 +446,7 @@ extern "C" int lmm_post_mean_and_var(lmm_post* post, const double* xs, int Ns, d
   lmm_ctx* ctx = post->ctx;
   std::lock_guard<std::mutex> lk(ctx->mu);
   CU(cudaSetDevice(ctx->device));
+  if (int rcz = post_fill_zeros(post)) return rcz;  // the factor is read below
   if (post->kind == POST_MASKED) return masked_post_mean_and_var(post, xs, Ns, sigma2, mean, var);
   if (post->joint()) return ilmm_post_mean_and_var(post, xs, Ns, sigma2, mean, var);
   cudaStream_t st = ctx->stream;
@@ -472,6 +507,7 @@ extern "C" int lmm_post_latent_mean_and_var(lmm_post* post, int i, const double*
   lmm_ctx* ctx = post->ctx;
   std::lock_guard<std::mutex> lk(ctx->mu);
   CU(cudaSetDevice(ctx->device));
+  if (int rcz = post_fill_zeros(post)) return rcz;  // the factor is read below
   if (post->joint()) return ctx->fail(LMM_E_UNSUPPORTED, "a joint posterior has no independent latent posteriors");
   if (i < post->lo || i >= post->hi) return ctx->fail(LMM_E_ARG, "latent not resident on this rank");
   cudaStream_t st = ctx->stream;

@@ -60,6 +60,7 @@ extern "C" int lmm_post_logpdf_grad_full(lmm_post* post, const double* xs, int N
   lmm_ctx* ctx = post->ctx;
   std::lock_guard<std::mutex> lk(ctx->mu);
   CU(cudaSetDevice(ctx->device));
+  if (int rcz = post_fill_zeros(post)) return rcz;  // the factor is read below
   if (post->joint())
     return ctx->fail(LMM_E_UNSUPPORTED, "the posterior-predictive gradient through the conditioning is built for per-latent posteriors "
                                         "(OILMM, IndependentMOGP); joint posteriors (general ILMM, dense Σy, missing data): σ² and y* only");

@@ -289,6 +289,7 @@ extern "C" int lmm_post_rand(lmm_post* post, const double* xs, int Ns, double si
   lmm_ctx* ctx = post->ctx;
   std::lock_guard<std::mutex> lk(ctx->mu);
   CU(cudaSetDevice(ctx->device));
+  if (int rcz = post_fill_zeros(post)) return rcz;  // the factor is read below
   if (post->kind != POST_IMOGP && post->kind != POST_JOINT && post->kind != POST_MASKED && !z_noise) return ctx->fail(LMM_E_ARG, "null pointer");
   if (post->kind == POST_MASKED) return masked_post_rand(post, xs, Ns, sigma2, z_latent, out, info_latent);  // z_latent: p*Ns normals
   if (post->joint()) return ilmm_post_rand(post, xs, Ns, sigma2, z_latent, z_noise, out, info_latent);
@@ -324,6 +325,7 @@ int post_logpdf_impl(lmm_post* post, const double* xs, int Ns, double sigma2, co
                      double* grad_y, int* info_latent, PredictiveKeep* keep) {
   lmm_ctx* ctx = post->ctx;
   CU(cudaSetDevice(ctx->device));
+  if (int rcz = post_fill_zeros(post)) return rcz;  // the factor is read below
   if (post->kind == POST_MASKED) return ctx->fail(LMM_E_UNSUPPORTED, "a missing-data posterior offers mean_and_var only");
   if (post->joint()) return ilmm_post_logpdf(post, xs, Ns, sigma2, ys, out_logpdf, grad_sigma2, grad_y, info_latent);
   const bool want_grad = grad_sigma2 || grad_y;

@@ -10,9 +10,18 @@ namespace lmm {
 // row0: only the tile rows I >= row0 are built (the rows above belong to a factor that is being extended)
 // env (nullable, [batch][nt] ints, row0 = 0): the tile envelope -- env[b][I] = first tile column of tile row I with an entry != 0.
 // The Cholesky factor keeps it (L(I,k) = 0 for k < env[b][I]), so the factorisation and the solves may skip those tiles.
+// rowoff (nullable, row0 = 0, [batch * nt + 1] ints): build only the tiles (I, k >= fb[b][I]) of launch_kmat_bound's envelope;
+// rowoff[b * nt + I] = number of such tiles in the rows before (b, I), ntiles = rowoff[batch * nt].  The tiles left out are NOT
+// written: only code that takes env may read the matrix (launch_kmat_zero writes the zeros).
 cudaError_t launch_kmat_sym(cudaStream_t st, TiledSym out, int batch, const double* xpad, int N, int D,
                             const LatentParams* params, int form, const double* noise_vec = nullptr, size_t noise_stride = 0, int row0 = 0,
-                            int* env = nullptr);
+                            int* env = nullptr, const int* rowoff = nullptr, long long ntiles = 0);
+// fb[b][I] (<= I): a tile column below which every tile (I, k) of launch_kmat_sym's matrix is provably exactly 0 -- from per-tile
+// bounding boxes of the scaled points, a lower bound of the squared distance the build computes, and kappa_zero_d2.  0 (nothing
+// provable) for composite, periodic and rational-quadratic latents and for a non-finite variance.  fb <= env holds for every row.
+cudaError_t launch_kmat_bound(cudaStream_t st, int batch, const double* xpad, int N, int D, int nt, const LatentParams* params, int* fb);
+// Writes the exact zeros of the tiles (I, k < env[b][I]) that a launch_kmat_sym with rowoff may have left out.
+cudaError_t launch_kmat_zero(cudaStream_t st, TiledSym L, int batch, const int* env);
 cudaError_t launch_kmat_cross(cudaStream_t st, TiledRect out, int batch, const double* xa_pad, int Na, const double* xb_pad,
                               int Nb, int D, const LatentParams* params, int form);
 
@@ -70,13 +79,15 @@ cudaError_t launch_potrf_tile(cudaStream_t st, TiledSym L, double* W, size_t w_b
 // Fused panel chain of one tile column (small batches): TRSM of column J, update of the columns (J, c_end) by the k-tiles
 // [k0, J], and (do_potrf) the factorisation of diagonal tile J+1 in ONE launch (potrf.cu: chain_column_kernel).
 // counters: batch * chain_counter_ints(nt) ints, zeroed once per factorisation.
+// env (nullable, [batch][nt]): tile envelope of the factor; the tiles (I, k < env[b][I]) are neither read nor solved.
 size_t chain_counter_ints(int nt);
 cudaError_t launch_chain_column(cudaStream_t st, TiledSym L, double* W, size_t w_batch_stride, int J, int k0, int c_end, int do_potrf,
-                                int batch, double* logdet, int* info, int* counters);
+                                int batch, double* logdet, int* info, int* counters, const int* env = nullptr);
 
 // ---- solve.cu
 // forward: z = L^{-1} r; backward: a = L^{-T} r.  rvec[batch][nt*128] is consumed (destroyed).
-// env (nullable, [batch][nt]): tile envelope of the factor (launch_kmat_sym); the persistent sweeps skip the tiles outside it.
+// env (nullable, [batch][nt]): tile envelope of the factor (launch_kmat_sym); both solve_impl variants skip the tiles outside it
+// (they need not be stored).
 cudaError_t launch_fwd_solve(cudaStream_t st, TiledSym L, const double* W, size_t w_batch_stride, double* rvec, double* zvec,
                              size_t vec_stride, int batch, int64_t* launches, const int* env = nullptr);
 cudaError_t launch_bwd_solve(cudaStream_t st, TiledSym L, const double* W, size_t w_batch_stride, double* rvec, double* avec,

@@ -3,7 +3,8 @@
 // `+ Diagonal(ΣT_i)`).  One pass: scaled inputs -> pairwise squared distance -> κ -> variance
 // scale -> (+ noise on the diagonal) written straight into the tiled factorisation workspace.
 // The two 128-point input tiles are staged into shared memory with one TMA bulk copy each
-// (cp.async.bulk + mbarrier).  HBM-write bound: 8 bytes per stored element, lower tiles only.
+// (cp.async.bulk + mbarrier).  HBM-write bound: 8 bytes per stored element, lower tiles only -- and on the OILMM / IndependentMOGP
+// eval path only the tiles that kmat_bound_kernel cannot prove to be exact zeros.
 #include "common.cuh"
 #include "kernels.h"
 
@@ -181,7 +182,8 @@ template <int DS>
 // (256, 4): 4 CTAs per SM as without the envelope test, which would otherwise take the single-kernel body from 64 to 76 registers
 __global__ void __launch_bounds__(256, 4) kmat_sym_kernel(TiledSym out, const double* __restrict__ xpad, int N, int D,
                                                        const LatentParams* __restrict__ params, int form,
-                                                       const double* __restrict__ noise_vec, size_t noise_stride, int tile0, int* env) {
+                                                       const double* __restrict__ noise_vec, size_t noise_stride, int tile0, int* env,
+                                                       const int* __restrict__ rowoff, int batch) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double* xa = reinterpret_cast<double*>(smem_raw);
   double* xb = xa + TILE * D;
@@ -189,14 +191,32 @@ __global__ void __launch_bounds__(256, 4) kmat_sym_kernel(TiledSym out, const do
   double* sb = sa + TILE;
   __shared__ __align__(8) uint64_t bar;
 
-  const int b = blockIdx.y;
-  // linear lower-tile index -> (I, J); tile0 = first tile of the first row built (rows below a prefix that is already
-  // factored: sequential conditioning extends a factor instead of rebuilding it)
-  const int t = blockIdx.x + tile0;
-  int I = (int)((sqrt(8.0 * (double)t + 1.0) - 1.0) * 0.5);
-  while ((size_t)(I + 1) * (I + 2) / 2 <= (size_t)t) ++I;
-  while ((size_t)I * (I + 1) / 2 > (size_t)t) --I;
-  const int J = t - (int)((size_t)I * (I + 1) / 2);
+  int b, I, J;
+  if (rowoff) {
+    // grid (tiles inside the bound envelopes of the whole batch): the run of (latent, tile row) r that holds tile t,
+    // rowoff[r] <= t < rowoff[r + 1], by a 256-way search -- two rounds for 8192 runs
+    const int t = blockIdx.x;
+    int r0 = 0, r1 = batch * out.nt;
+    while (r1 - r0 > 1) {
+      const int s = (r1 - r0 + (int)blockDim.x - 1) / (int)blockDim.x;
+      const int i = r0 + (int)threadIdx.x * s;
+      const int c = __syncthreads_count(i < r1 && rowoff[i] <= t);  // >= 1: rowoff[r0] <= t
+      r0 += (c - 1) * s;
+      r1 = min(r0 + s, r1);
+    }
+    b = r0 / out.nt;
+    I = r0 - b * out.nt;
+    J = I + 1 - (rowoff[r0 + 1] - rowoff[r0]) + (t - rowoff[r0]);  // the run is the tiles (I, fb .. I)
+  } else {
+    b = blockIdx.y;
+    // linear lower-tile index -> (I, J); tile0 = first tile of the first row built (rows below a prefix that is already
+    // factored: sequential conditioning extends a factor instead of rebuilding it)
+    const int t = blockIdx.x + tile0;
+    I = (int)((sqrt(8.0 * (double)t + 1.0) - 1.0) * 0.5);
+    while ((size_t)(I + 1) * (I + 2) / 2 <= (size_t)t) ++I;
+    while ((size_t)I * (I + 1) / 2 > (size_t)t) --I;
+    J = t - (int)((size_t)I * (I + 1) / 2);
+  }
   const LatentParams lp = params[b];
 
   stage_points(xa, xb, sa, sb, xpad + (size_t)I * TILE * D, xpad + (size_t)J * TILE * D, D, params + b, &bar);
@@ -225,10 +245,90 @@ __global__ void __launch_bounds__(256) kmat_cross_kernel(TiledRect out, const do
   kmat_tile_body<false, DS>(out.tile(b, R, J), xa, xb, sa, sb, D, R * TILE, J * TILE, Na, Nb, lp, form, nullptr, params + b);
 }
 
+// grid (batch), 256 threads, dynamic shared memory nt * (2D + 1) doubles: lo / hi [nt][D] and q [nt].
+// The bound: for tile boxes A, B of the scaled points (the same products x * input_scale that stage_points forms), every pair
+// (a, b) has |a - b|² >= g² = Σ_k gap_k², and the build's computed d² -- |a|²+|b|² - 2 a·b in either rounding order, or Σ (a_k -
+// b_k)² -- differs from |a - b|² by less than (2D + 4) u (|a|² + |b|²) + u d² (u = 2^-53).  With q_T >= max |a|² over box T,
+// lb = g² (1 - r) - r (q_A + q_B), r = 8 (D + 4) u, is below every computed d² of the tile; lb > kappa_zero_d2 proves it all-zero.
+// Padding points are left out of the boxes: the build writes 0 for them off the diagonal.  A non-finite coordinate makes its box
+// unbounded and its q infinite, so nothing involving that tile is skipped.
+__global__ void __launch_bounds__(256) kmat_bound_kernel(const double* __restrict__ xpad, int N, int D, int nt,
+                                                         const LatentParams* __restrict__ params, int* __restrict__ fb) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  double* lo = reinterpret_cast<double*>(smem_raw);
+  double* hi = lo + (size_t)nt * D;
+  double* q = hi + (size_t)nt * D;
+  const int b = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const LatentParams* gp = params + b;
+  int* fbb = fb + (size_t)b * nt;
+  const double thr = kappa_zero_d2(gp->kind);
+  if (needs_raw_points(gp) || !(thr < __builtin_huge_val()) || !isfinite(gp->variance)) {  // ∞·0 = NaN counts as nonzero
+    for (int I = threadIdx.x; I < nt; I += blockDim.x) fbb[I] = 0;
+    return;
+  }
+  // one warp per (tile, dimension)
+  for (int i = warp; i < nt * D; i += (int)blockDim.x / 32) {
+    const int T = i / D, k = i - T * D;
+    const double s = input_scale(gp, k);
+    double l = __builtin_huge_val(), h = -__builtin_huge_val();
+    bool bad = false;
+    for (int r = T * TILE + lane; r < (T + 1) * TILE && r < N; r += 32) {
+      const double v = xpad[(size_t)r * D + k] * s;
+      bad |= !isfinite(v);
+      l = fmin(l, v);
+      h = fmax(h, v);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      l = fmin(l, __shfl_xor_sync(0xffffffffu, l, o));
+      h = fmax(h, __shfl_xor_sync(0xffffffffu, h, o));
+    }
+    if (__any_sync(0xffffffffu, bad)) {
+      l = -__builtin_huge_val();
+      h = __builtin_huge_val();
+    }
+    if (lane == 0) {
+      lo[i] = l;
+      hi[i] = h;
+    }
+  }
+  __syncthreads();
+  for (int T = threadIdx.x; T < nt; T += blockDim.x) {
+    double s = 0.0;
+    for (int k = 0; k < D; ++k) s += fmax(lo[T * D + k] * lo[T * D + k], hi[T * D + k] * hi[T * D + k]);
+    q[T] = s;
+  }
+  __syncthreads();
+  const double rel = (double)(D + 4) * 0x1p-50;
+  for (int I = threadIdx.x; I < nt; I += blockDim.x) {
+    int f = 0;
+    for (; f < I; ++f) {
+      double g2 = 0.0;
+      for (int k = 0; k < D; ++k) {
+        const double g = fmax(0.0, fmax(lo[I * D + k] - hi[f * D + k], lo[f * D + k] - hi[I * D + k]));
+        g2 = fma(g, g, g2);
+      }
+      const double lb = g2 * (1.0 - rel) - rel * (q[I] + q[f]);
+      if (!(lb > thr)) break;
+    }
+    fbb[I] = f;
+  }
+}
+
+// grid (nt, batch, KZ_SPLIT): the KZ_SPLIT CTAs of a tile row share the row's contiguous run of tiles (I, 0 .. env - 1).
+constexpr int KZ_SPLIT = 8;
+__global__ void __launch_bounds__(256) kmat_zero_kernel(TiledSym L, const int* __restrict__ env) {
+  const int I = blockIdx.x, b = blockIdx.y;
+  double2* p = reinterpret_cast<double2*>(L.tile(b, I, 0));
+  const size_t n = (size_t)env[(size_t)b * L.nt + I] * (TT / 2);
+  for (size_t i = (size_t)blockIdx.z * blockDim.x + threadIdx.x; i < n; i += (size_t)KZ_SPLIT * blockDim.x) p[i] = make_double2(0.0, 0.0);
+}
+
 static size_t kmat_smem(int D) { return (size_t)(2 * TILE * D + 2 * TILE) * sizeof(double); }
 
 cudaError_t launch_kmat_sym(cudaStream_t st, TiledSym out, int batch, const double* xpad, int N, int D,
-                            const LatentParams* params, int form, const double* noise_vec, size_t noise_stride, int row0, int* env) {
+                            const LatentParams* params, int form, const double* noise_vec, size_t noise_stride, int row0, int* env,
+                            const int* rowoff, long long ntiles) {
   size_t sm = kmat_smem(D);
   if (sm + 1024 > 48 * 1024) {  // static shared memory counts against the default limit too
     cudaError_t e = cudaFuncSetAttribute(kmat_sym_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
@@ -236,15 +336,36 @@ cudaError_t launch_kmat_sym(cudaStream_t st, TiledSym out, int batch, const doub
   }
   const int tile0 = (int)sym_tiles(row0);  // row-panel-major order: the tiles of rows >= row0 are the tail of the list
   if (row0 >= out.nt) return cudaSuccess;
+  if (rowoff && row0 != 0) return cudaErrorInvalidValue;
   if (env) {
     cudaError_t e = cudaMemsetAsync(env, 0x7f, (size_t)batch * out.nt * sizeof(int), st);
     if (e != cudaSuccess) return e;
   }
-  dim3 grid((unsigned)(sym_tiles(out.nt) - tile0), (unsigned)batch);
+  if (rowoff && ntiles <= 0) return cudaSuccess;
+  dim3 grid(rowoff ? (unsigned)ntiles : (unsigned)(sym_tiles(out.nt) - tile0), rowoff ? 1u : (unsigned)batch);
   if (D == 1)
-    kmat_sym_kernel<1><<<grid, 256, sm, st>>>(out, xpad, N, D, params, form, noise_vec, noise_stride, tile0, env);
+    kmat_sym_kernel<1><<<grid, 256, sm, st>>>(out, xpad, N, D, params, form, noise_vec, noise_stride, tile0, env, rowoff, batch);
   else
-    kmat_sym_kernel<0><<<grid, 256, sm, st>>>(out, xpad, N, D, params, form, noise_vec, noise_stride, tile0, env);
+    kmat_sym_kernel<0><<<grid, 256, sm, st>>>(out, xpad, N, D, params, form, noise_vec, noise_stride, tile0, env, rowoff, batch);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_kmat_bound(cudaStream_t st, int batch, const double* xpad, int N, int D, int nt, const LatentParams* params, int* fb) {
+  if (batch <= 0) return cudaSuccess;
+  const size_t sm = (size_t)nt * (2 * D + 1) * sizeof(double);
+  if (sm > 200 * 1024)  // boxes too large for shared memory: no bound, every tile is built
+    return cudaMemsetAsync(fb, 0, (size_t)batch * nt * sizeof(int), st);
+  if (sm > 48 * 1024) {
+    cudaError_t e = cudaFuncSetAttribute(kmat_bound_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+    if (e != cudaSuccess) return e;
+  }
+  kmat_bound_kernel<<<batch, 256, sm, st>>>(xpad, N, D, nt, params, fb);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_kmat_zero(cudaStream_t st, TiledSym L, int batch, const int* env) {
+  if (batch <= 0) return cudaSuccess;
+  kmat_zero_kernel<<<dim3((unsigned)L.nt, (unsigned)batch, KZ_SPLIT), 256, 0, st>>>(L, env);
   return cudaGetLastError();
 }
 

@@ -489,6 +489,7 @@ struct ChainArgs {
   int* info;
   int* cnt;           // [batch][nt * nt + nt + 1]
   int J, k0, c_end, do_potrf;
+  const int* env;     // nullable: tile envelope [batch][nt] (tiles (I, k < env[I]) are exact zeros that may not be stored)
 };
 
 // grid (batch, 8 * (nT + nU) + (do_potrf ? 1 : 0)), 256 threads, POTRF_SMEM bytes of dynamic shared memory.
@@ -527,8 +528,13 @@ __global__ void __launch_bounds__(256, 1) chain_column_kernel(ChainArgs a) {
     }
   }
   pdl_wait();  // column J (and the trailing updates ordered before this launch) are complete and visible
+  const int* eb = a.env ? a.env + (size_t)b * nt : nullptr;
   if (role == 0) {
     // ---- role T: TRSM of one slice of tile (I, J)
+    if (eb && eb[I] > J) {  // a zero tile stays zero (and is not read: it may not be stored)
+      signal_count(cnt + (size_t)J * nt + I);
+      return;
+    }
     double* Ctile = a.L.tile(b, I, J);
     int nb0, nb1, lim0, nsteps;
     direct_blocks<GEMM_TRSM>(warp, 1, nb0, nb1, lim0, nsteps);
@@ -542,14 +548,20 @@ __global__ void __launch_bounds__(256, 1) chain_column_kernel(ChainArgs a) {
   }
   if (role == 1) {
     // ---- role U: update of one slice of tile (I, c) by the k-tiles [k0, J]
+    // below max(env[I], env[c]) one operand is an exact zero (gemm_first_k): the sum starts there, bit for bit the full one
+    const int kb = eb ? max(a.k0, max(eb[I], eb[c])) : a.k0;
+    if (kb > J) {  // nothing to subtract: C(I,c) stays as it is
+      if (I == J + 1 && c == J + 1) signal_count(cnt + (size_t)nt * nt + J + 1);
+      return;
+    }
     double* Ctile = a.L.tile(b, I, c);
     int nb0 = warp * 2, nb1 = warp * 2 + 1, lim0, nsteps;
     double acc[DIRECT_RB][2][2] = {};
     double2 cv[DIRECT_RB][2];
     direct_load_c(Ctile, slice, nb0, nb1, cv);
-    if (a.k0 < J) {  // the columns of this block before J: final before this launch
-      direct_blocks<GEMM_UPDATE>(warp, J - a.k0, nb0, nb1, lim0, nsteps);
-      direct_accumulate<GEMM_UPDATE>(a.L.tile(b, I, a.k0), a.L.tile(b, c, a.k0), slice, nb0, nb1, lim0, nsteps, acc);
+    if (kb < J) {  // the columns of this block before J: final before this launch
+      direct_blocks<GEMM_UPDATE>(warp, J - kb, nb0, nb1, lim0, nsteps);
+      direct_accumulate<GEMM_UPDATE>(a.L.tile(b, I, kb), a.L.tile(b, c, kb), slice, nb0, nb1, lim0, nsteps, acc);
     }
     // k = J: produced by role T of this launch -- all 8 slices of the B operand's tile (c, J) and of the A operand's tile (I, J)
     wait_count(cnt + (size_t)J * nt + c, DIRECT_SPLIT);
@@ -572,7 +584,7 @@ size_t chain_counter_ints(int nt) { return (size_t)nt * nt + nt + 1; }
 // the factorisation of diagonal tile J+1.  c_end <= J + 1: no update (then do_potrf must be 0: the diagonal tile would not
 // be up to date).
 cudaError_t launch_chain_column(cudaStream_t st, TiledSym L, double* W, size_t w_batch_stride, int J, int k0, int c_end, int do_potrf,
-                                int batch, double* logdet, int* info, int* counters) {
+                                int batch, double* logdet, int* info, int* counters, const int* env) {
   static bool configured_dev[64] = {false};
   int dev = 0;
   cudaGetDevice(&dev);
@@ -591,7 +603,7 @@ cudaError_t launch_chain_column(cudaStream_t st, TiledSym L, double* W, size_t w
   }
   long long nU = 0;
   for (int c = J + 1; c < c_end; ++c) nU += nt - c;
-  ChainArgs a{L, W, w_batch_stride, logdet, info, counters, J, k0, c_end, do_potrf};
+  ChainArgs a{L, W, w_batch_stride, logdet, info, counters, J, k0, c_end, do_potrf, env};
   dim3 grid((unsigned)batch, (unsigned)((nT + nU) * DIRECT_SPLIT + (do_potrf ? 1 : 0)));
   return launch_pdl(pdl_enabled(), chain_column_kernel, grid, dim3(256), POTRF_SMEM, st, a);
 }

@@ -60,10 +60,13 @@ __device__ __forceinline__ void tile_gemv_t(const double* __restrict__ tile, con
 }
 
 // grid (nt - J, batch).  rvec: running right-hand side (destroyed), zvec: solution.
+// env (nullable): tiles (I, J) with env[b][I] > J are exact zeros that are skipped (they need not be stored).
 __global__ void __launch_bounds__(256) fwd_step_kernel(TiledSym L, const double* __restrict__ W, size_t w_batch_stride,
-                                                       double* __restrict__ rvec, double* __restrict__ zvec, size_t vec_stride, int J) {
+                                                       double* __restrict__ rvec, double* __restrict__ zvec, size_t vec_stride, int J,
+                                                       const int* __restrict__ env) {
   __shared__ double xs[TILE], zs[TILE], ys[TILE];
   const int b = blockIdx.y, i = blockIdx.x, t = threadIdx.x;
+  if (i > 0 && env && env[(size_t)b * L.nt + J + i] > J) return;  // r_I -= 0
   double* r = rvec + (size_t)b * vec_stride;
   if (t < TILE) xs[t] = r[J * TILE + t];
   __syncthreads();
@@ -83,12 +86,14 @@ __global__ void __launch_bounds__(256) fwd_step_kernel(TiledSym L, const double*
   if (t < TILE) r[I * TILE + t] -= ys[t];
 }
 
-// grid (J + 1, batch).  rvec: running rhs (destroyed), avec: solution of L^T a = r.
+// grid (J + 1, batch).  rvec: running rhs (destroyed), avec: solution of L^T a = r.  env: as fwd_step_kernel.
 __global__ void __launch_bounds__(256) bwd_step_kernel(TiledSym L, const double* __restrict__ W, size_t w_batch_stride,
-                                                       double* __restrict__ rvec, double* __restrict__ avec, size_t vec_stride, int J) {
+                                                       double* __restrict__ rvec, double* __restrict__ avec, size_t vec_stride, int J,
+                                                       const int* __restrict__ env) {
   __shared__ double xs[TILE], as[TILE], ys[TILE];
   __shared__ double part[8 * TILE];
   const int b = blockIdx.y, k = blockIdx.x, t = threadIdx.x;
+  if (k < J && env && env[(size_t)b * L.nt + J] > k) return;  // r_k -= 0
   double* r = rvec + (size_t)b * vec_stride;
   if (t < TILE) xs[t] = r[J * TILE + t];
   __syncthreads();
@@ -337,7 +342,7 @@ cudaError_t launch_fwd_solve(cudaStream_t st, TiledSym L, const double* W, size_
   }
   for (int J = 0; J < L.nt; ++J) {
     dim3 grid((unsigned)(L.nt - J), (unsigned)batch);
-    fwd_step_kernel<<<grid, 256, 0, st>>>(L, W, w_batch_stride, rvec, zvec, vec_stride, J);
+    fwd_step_kernel<<<grid, 256, 0, st>>>(L, W, w_batch_stride, rvec, zvec, vec_stride, J, env);
     if (launches) ++*launches;
   }
   return cudaGetLastError();
@@ -357,7 +362,7 @@ cudaError_t launch_bwd_solve(cudaStream_t st, TiledSym L, const double* W, size_
   }
   for (int J = L.nt - 1; J >= 0; --J) {
     dim3 grid((unsigned)(J + 1), (unsigned)batch);
-    bwd_step_kernel<<<grid, 256, 0, st>>>(L, W, w_batch_stride, rvec, avec, vec_stride, J);
+    bwd_step_kernel<<<grid, 256, 0, st>>>(L, W, w_batch_stride, rvec, avec, vec_stride, J, env);
     if (launches) ++*launches;
   }
   return cudaGetLastError();
