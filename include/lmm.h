@@ -253,6 +253,26 @@ int lmm_imogp_logpdf_grad_terms(lmm_ctx* ctx, const lmm_gp_desc* fs, int m, cons
                                 double* grad_latents, double* grad_ard, double* grad_sigma2, double* grad_y,
                                 double* grad_terms, int* info_latent);
 
+/* Leave-one-input-out cross-validation (Rasmussen & Williams §5.4.2): out_loo = Σ_i log p(y_i | y_{-i}) where y_i is all p
+ * outputs at input x_i -- the closed form of N refits, at the cost of a factorisation plus one N³/3 TRSM per latent for
+ * the value, about twice the logpdf gradient's cost with a gradient.  For an OILMM it is Σ_l (GP LOO of latent l on the
+ * projected data, noise σ²/S_l) + the regulariser logpdf adds.  loo_mean / loo_var (p*N by outputs) are the LOO predictive
+ * marginals: what mean_and_var(posterior(f(x_{-i}, σ²), y_{-i})(x_i, σ²)) returns at each x_i.  The gradient outputs use the
+ * layouts of lmm_oilmm_logpdf_grad_terms (grad_latents m x 3: term 0's variance and inv_lengthscale, mean_const; grad_ard
+ * m x D; grad_terms m x LMM_MAX_TERMS x LMM_GRAD_TERM_STRIDE; grad_U / grad_S the Euclidean gradient) for every latent the
+ * value path accepts.  Every output is nullable; with every gradient pointer NULL only the value path runs.  A NaN in y,
+ * m > p and a non-positive σ² return LMM_E_ARG; a failed factorisation reports its pivot and info_latent as the logpdf
+ * gradient does. */
+int lmm_oilmm_loo(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D,
+                  const double* U, const double* S, int p, double sigma2, const double* y, int out_dim,
+                  double* out_loo, double* loo_mean, double* loo_var, double* grad_latents, double* grad_ard,
+                  double* grad_sigma2, double* grad_y, double* grad_U, double* grad_S, double* grad_terms,
+                  int* info_latent);
+int lmm_imogp_loo(lmm_ctx* ctx, const lmm_gp_desc* fs, int m, const double* x, int N, int D, double sigma2,
+                  const double* y, int out_dim, double* out_loo, double* loo_mean, double* loo_var,
+                  double* grad_latents, double* grad_ard, double* grad_sigma2, double* grad_y, double* grad_terms,
+                  int* info_latent);
+
 /* ---- posterior handle: the OILMM/ILMM/IndependentMOGP whose latents are PosteriorGPs -------- */
 /* mean_and_var(post(x*, σ²))  src/oilmm.jl:57-76 on PosteriorGP latents (AbstractGPs posterior
  * mean/var); for an IndependentMOGP posterior: src/independent_mogp.jl:50-57; ILMM: src/ilmm.jl:122-129. */

@@ -22,6 +22,9 @@ from .api import (  # noqa: F401
     posterior_missing,
     logpdf_missing,
     logpdf_missing_and_gradient,
+    loo_logpdf,
+    loo_mean_and_var,
+    loo_logpdf_and_gradient,
 )
 from . import _lib, api, dist  # noqa: F401
 

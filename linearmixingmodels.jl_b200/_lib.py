@@ -86,6 +86,9 @@ SIGNATURES = {
     # per-term gradients of composite / periodic / rational-quadratic latents: grad_terms (m x 4 x 11) before the info pointer
     "lmm_oilmm_logpdf_grad_terms": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _dp, _vp, _vp, _vp, _vp, _ip]),
     "lmm_imogp_logpdf_grad_terms": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _dp, _vp, _vp, _ip]),
+    # leave-one-input-out: value, LOO mean, LOO var, latents, ard, σ², y, U, S, terms, info
+    "lmm_oilmm_loo": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _vp, _vp, _dp, _vp, _vp, _vp, _vp, _ip]),
+    "lmm_imogp_loo": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _vp, _vp, _dp, _vp, _vp, _ip]),
     "lmm_post_mean_and_var": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp]),
     "lmm_post_latent_mean_and_var": (C.c_int, [_vp, C.c_int, _vp, C.c_int, C.c_double, _vp, _vp]),
     "lmm_post_mean_and_cov": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp]),

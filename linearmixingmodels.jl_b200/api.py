@@ -1185,6 +1185,86 @@ def predictive_logpdf_and_gradient(fx_post: FiniteGP, y, y_train, with_grad_y: b
     return out.value, grads
 
 
+def _loo_call(fx: FiniteGP, y, value: bool, marginals: bool, grads: bool, with_grad_y: bool = False):
+    """One lmm_oilmm_loo / lmm_imogp_loo call; outputs that are not asked for are passed as NULL."""
+    if isinstance(fx.f, ILMM) and not isinstance(fx.f.H, Orthogonal):
+        raise TypeError("leave-one-out is built for OILMM and IndependentMOGP priors (not a general ILMM)")
+    if not (isinstance(fx.f, (ILMM, IndependentMOGP))):
+        raise TypeError("leave-one-out is built for OILMM and IndependentMOGP priors")
+    if fx.noise is not None:
+        raise TypeError("leave-one-out needs scalar observation noise")
+    _require_by_outputs(fx)
+    if _post_owner(fx) is not None:
+        raise TypeError("leave-one-out is built for prior FiniteGPs, not posteriors")
+    f = fx.f
+    lat = f.f if isinstance(f, ILMM) else f
+    if not isinstance(lat, IndependentMOGP):
+        raise TypeError("ILMM latents must be an IndependentMOGP")
+    if isinstance(f, ILMM) and f.H.shape[0] != fx.x.out_dim:
+        raise RuntimeError("out dim of x != out dim of f.")
+    ctx = _ctx_of(fx)
+    pts = _points(fx.x.x)
+    N, D = int(pts.shape[0]), int(pts.shape[1])
+    p = fx.x.out_dim
+    m = len(lat.fs)
+    yv = _yvec(y, N * p)
+    if not _is_device_tensor(yv) and np.isnan(yv).any():
+        raise ValueError("y has a NaN entry: leave-one-out needs fully observed data")
+    out, gs2, il = C.c_double(), C.c_double(), C.c_int(-1)
+    M = np.zeros(p * N) if marginals else None
+    V = np.zeros(p * N) if marginals else None
+    gl = np.zeros((m, 3)) if grads else None
+    ga = np.zeros((m, D)) if grads else None
+    gt = np.zeros(m * _lib.LMM_MAX_TERMS * _lib.LMM_GRAD_TERM_STRIDE) if grads else None
+    gy = np.zeros(p * N) if grads and with_grad_y else None
+    gs2p = C.byref(gs2) if grads else None
+    outp = C.byref(out) if value else None
+    orth = isinstance(f, ILMM)
+    gU = np.zeros(f.H.shape, order="F") if orth and grads else None
+    gS = np.zeros(m) if orth and grads else None
+    if orth:
+        H = f.H
+        rc = ctx.lib.lmm_oilmm_loo(ctx.handle, _descs(lat.fs), m, ptr(pts), N, D, ptr(H.U), ptr(H.S), H.shape[0], fx.sigma2, ptr(yv), p,
+                                   outp, ptr(M), ptr(V), ptr(gl), ptr(ga), gs2p, ptr(gy), ptr(gU), ptr(gS), ptr(gt), C.byref(il))
+    else:
+        rc = ctx.lib.lmm_imogp_loo(ctx.handle, _descs(lat.fs), m, ptr(pts), N, D, fx.sigma2, ptr(yv), p, outp, ptr(M), ptr(V), ptr(gl),
+                                   ptr(ga), gs2p, ptr(gy), ptr(gt), C.byref(il))
+    ctx.check(rc, il.value)
+    g = None
+    if grads:
+        g = {"terms": _terms_grads(lat.fs, gt, D), "variance": gl[:, 0].copy(), "inv_lengthscale": gl[:, 1].copy(), "ard": ga,
+             "mean_const": gl[:, 2].copy(), "sigma2": gs2.value}
+        if with_grad_y:
+            g["y"] = gy
+        if orth:
+            g["U"], g["S"] = np.ascontiguousarray(gU), gS
+    return out.value, M, V, g
+
+
+def loo_logpdf(fx: FiniteGP, y) -> float:
+    """Leave-one-input-out log predictive density Σ_i log p(y_i | y_{-i}) of an OILMM or IndependentMOGP prior `fx`, where
+    y_i is all outputs at input x_i (Rasmussen & Williams §5.4.2): a cross-validation score in closed form, for comparing
+    models and as a training objective.  Costs one factorisation and one triangular inverse per latent."""
+    return _loo_call(fx, y, True, False, False)[0]
+
+
+def loo_mean_and_var(fx: FiniteGP, y) -> Tuple[np.ndarray, np.ndarray]:
+    """LOO predictive marginals (p*N each, by outputs like `mean_and_var`): at each input x_i, what
+    `mean_and_var(posterior(f(x_{-i}, σ²), y_{-i})(x_i, σ²))` returns -- noise included."""
+    _, M, V, _ = _loo_call(fx, y, False, True, False)
+    return M, V
+
+
+def loo_logpdf_and_gradient(fx: FiniteGP, y, with_grad_y: bool = False):
+    """Value and gradient of `loo_logpdf(fx, y)`.  grads has the keys of `logpdf_and_gradient(fx, y, kernel_terms=True)`:
+    "terms" (per latent, per term in `Kernel.all_terms()` order: {"variance", "inv_lengthscale", "param", "ard"}),
+    "variance" / "inv_lengthscale" / "ard" (term 0's), "mean_const", "sigma2"[, "y" (p*N,)], and for an OILMM "U" (p, m)
+    and "S" (m,), the Euclidean gradient.  General ILMMs, posteriors, by-features inputs and non-scalar noise raise
+    TypeError; a NaN in y raises ValueError."""
+    v, _, _, g = _loo_call(fx, y, True, False, True, with_grad_y)
+    return v, g
+
+
 def logpdf_sweep(fx: FiniteGP, y, inv_lengthscale_scales) -> np.ndarray:
     """BASELINE config 5: OILMM logpdf for a batch of lengthscale settings in one call."""
     lat, H, s2, _ = unpack(fx)

@@ -149,19 +149,6 @@ extern "C" int lmm_post_condition(lmm_post* post, const double* xs, int Ns, doub
 // ------------------------------------------------------------------------------------------------
 namespace lmm_host {
 
-struct GradOut {
-  double* logpdf;
-  double* grad_latents;  // m x 3: d/d variance, d/d inv_lengthscale, d/d mean_const
-  double* grad_sigma2;
-  double* grad_y;        // p*N by outputs (nullable)
-  int* info_latent;
-  double* grad_U = nullptr;  // p x m column-major (OILMM only, nullable)
-  double* grad_S = nullptr;  // m (OILMM only, nullable)
-  const double* Yhost_or_dev = nullptr;
-  double* grad_ard = nullptr;  // m x D row-major: d/d ARD multiplier (zeros for latents without an ARDTransform; nullable)
-  double* grad_terms = nullptr;  // m x LMM_MAX_TERMS x LMM_GRAD_TERM_STRIDE: per-term gradients (nullable)
-};
-
 // Launch bounds of the per-term contraction for latents [lo, hi): the most terms, and whether any term has an ARDTransform.
 void terms_shape(const lmm_gp_desc* latents, int lo, int hi, int& max_terms, bool& any_ard) {
   max_terms = 1;
@@ -190,153 +177,100 @@ void scatter_terms(const lmm_gp_desc* latents, int m, int D, const std::vector<d
   }
 }
 
-int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m, const double* x, int N, int D, int p, double sigma2,
-                     const double* y, const Projection& pr, const double* Shost, GradOut out) {
+int grad_run_setup(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m, const double* x, int N, int D, int p, const double* y,
+                   const Projection& pr, const GradOut& out, GradRun& s) {
   CU(cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   for (double& t : ctx->timings) t = 0.0;
-  int lo, hi;
-  shard_range(ctx, m, lo, hi);
-  const int mloc = hi - lo, nt = ntiles(N);
-  const size_t npad = (size_t)nt * TILE;
-  const bool multi = ctx->comm && ctx->nranks > 1;
+  shard_range(ctx, m, s.lo, s.hi);
+  const int lo = s.lo, hi = s.hi;
+  s.mloc = hi - lo;
+  s.nt = ntiles(N);
+  s.npad = (size_t)s.nt * TILE;
+  s.multi = ctx->comm && ctx->nranks > 1;
+  const int mloc = s.mloc;
+  const size_t npad = s.npad;
   CU(cudaEventRecord(ctx->ev[0], st));
-  DevBuf b_x, b_y, b_T, b_P, b_Q, b_means, b_ty, b_part, b_resid, b_R, b_params, b_vec;
-  int rc = stage_xpad(ctx, b_x, x, N, D);
+  int rc = stage_xpad(ctx, s.b_x, x, N, D);
   if (rc) return rc;
-  const double* d_y = y;
+  s.d_y = y;
   if (!is_device_ptr(y)) {
-    CU(b_y.alloc(ctx, (size_t)p * N * sizeof(double)));
-    CU(copy_in(ctx, b_y.as<double>(), y, (size_t)p * N));
-    d_y = b_y.as<double>();
+    CU(s.b_y.alloc(ctx, (size_t)p * N * sizeof(double)));
+    CU(copy_in(ctx, s.b_y.as<double>(), y, (size_t)p * N));
+    s.d_y = s.b_y.as<double>();
   }
-  CU(b_T.alloc(ctx, pr.T.size() * sizeof(double)));
-  CU(copy_in(ctx, b_T.as<double>(), pr.T.data(), pr.T.size()));
+  CU(s.b_T.alloc(ctx, pr.T.size() * sizeof(double)));
+  CU(copy_in(ctx, s.b_T.as<double>(), pr.T.data(), pr.T.size()));
   if (pr.has_reg) {
-    CU(b_P.alloc(ctx, pr.P.size() * sizeof(double)));
-    CU(copy_in(ctx, b_P.as<double>(), pr.P.data(), pr.P.size()));
-    CU(b_Q.alloc(ctx, pr.Q.size() * sizeof(double)));
-    CU(copy_in(ctx, b_Q.as<double>(), pr.Q.data(), pr.Q.size()));
+    CU(s.b_P.alloc(ctx, pr.P.size() * sizeof(double)));
+    CU(copy_in(ctx, s.b_P.as<double>(), pr.P.data(), pr.P.size()));
+    CU(s.b_Q.alloc(ctx, pr.Q.size() * sizeof(double)));
+    CU(copy_in(ctx, s.b_Q.as<double>(), pr.Q.data(), pr.Q.size()));
   }
-  const int nl = mloc > 0 ? mloc : 1;
+  s.nl = mloc > 0 ? mloc : 1;
+  const int nl = s.nl;
   std::vector<double> hmeans(nl, 0.0);
   for (int i = lo; i < hi; ++i) hmeans[i - lo] = latents[i].mean_const;
-  CU(b_means.alloc(ctx, (size_t)nl * sizeof(double)));
-  CU(copy_in(ctx, b_means.as<double>(), hmeans.data(), (size_t)nl));
-  if ((rc = upload_params(ctx, b_params, latents, pr.noise.data(), lo, hi, D))) return rc;
-  CU(b_ty.alloc(ctx, (size_t)nl * npad * sizeof(double)));
-  CU(cudaMemsetAsync(b_ty.p, 0, (size_t)nl * npad * sizeof(double), st));
+  CU(s.b_means.alloc(ctx, (size_t)nl * sizeof(double)));
+  CU(copy_in(ctx, s.b_means.as<double>(), hmeans.data(), (size_t)nl));
+  if ((rc = upload_params(ctx, s.b_params, latents, pr.noise.data(), lo, hi, D))) return rc;
+  CU(s.b_ty.alloc(ctx, (size_t)nl * npad * sizeof(double)));
+  CU(cudaMemsetAsync(s.b_ty.p, 0, (size_t)nl * npad * sizeof(double), st));
   const int nblk = project_max_partials(N);
-  CU(b_part.alloc(ctx, (size_t)nblk * sizeof(double)));
-  CU(cudaMemsetAsync(b_part.p, 0, (size_t)nblk * sizeof(double), st));
-  CU(b_resid.alloc(ctx, sizeof(double)));
-  CU(cudaMemsetAsync(b_resid.p, 0, sizeof(double), st));
-  const bool do_reg = pr.has_reg && ctx->rank == 0;
-  const bool want_U = orth && out.grad_U;
-  const bool want_R = do_reg && (out.grad_y || want_U);
-  const bool want_Z = do_reg && want_U;
-  DevBuf b_Z;
-  if (want_R) CU(b_R.alloc(ctx, (size_t)p * N * sizeof(double)));
-  if (want_Z) CU(b_Z.alloc(ctx, (size_t)m * N * sizeof(double)));
-  CU(launch_project(st, d_y, N, p, b_T.as<double>(), m, lo, mloc, b_means.as<double>(), b_ty.as<double>(), npad,
-                    do_reg ? b_P.as<double>() : nullptr, do_reg ? b_Q.as<double>() : nullptr, b_part.as<double>(), nullptr,
-                    want_R ? b_R.as<double>() : nullptr, want_Z ? b_Z.as<double>() : nullptr));
+  CU(s.b_part.alloc(ctx, (size_t)nblk * sizeof(double)));
+  CU(cudaMemsetAsync(s.b_part.p, 0, (size_t)nblk * sizeof(double), st));
+  CU(s.b_resid.alloc(ctx, sizeof(double)));
+  CU(cudaMemsetAsync(s.b_resid.p, 0, sizeof(double), st));
+  s.do_reg = pr.has_reg && ctx->rank == 0;
+  s.want_U = orth && out.grad_U;
+  s.want_R = s.do_reg && (out.grad_y || s.want_U);
+  s.want_Z = s.do_reg && s.want_U;
+  if (s.want_R) CU(s.b_R.alloc(ctx, (size_t)p * N * sizeof(double)));
+  if (s.want_Z) CU(s.b_Z.alloc(ctx, (size_t)m * N * sizeof(double)));
+  CU(launch_project(st, s.d_y, N, p, s.b_T.as<double>(), m, lo, mloc, s.b_means.as<double>(), s.b_ty.as<double>(), npad,
+                    s.do_reg ? s.b_P.as<double>() : nullptr, s.do_reg ? s.b_Q.as<double>() : nullptr, s.b_part.as<double>(), nullptr,
+                    s.want_R ? s.b_R.as<double>() : nullptr, s.want_Z ? s.b_Z.as<double>() : nullptr));
   ++ctx->launches;
-  if (do_reg) {
-    CU(launch_sum_partials(st, b_part.as<double>(), nblk, b_resid.as<double>()));
+  if (s.do_reg) {
+    CU(launch_sum_partials(st, s.b_part.as<double>(), nblk, s.b_resid.as<double>()));
     ++ctx->launches;
   }
   // reduction vector: [lml (m) | gv (m) | gs (m) | gmean (m) | gnoise (m) | resid (1) | quad (m)]
-  const size_t nvec = (size_t)6 * m + 1;
-  CU(b_vec.alloc(ctx, nvec * sizeof(double)));
-  CU(cudaMemsetAsync(b_vec.p, 0, nvec * sizeof(double), st));
-  double* d_vec = b_vec.as<double>();
-  if (do_reg) CU(cudaMemcpyAsync(d_vec + 5 * m, b_resid.p, sizeof(double), cudaMemcpyDeviceToDevice, st));
-
-  DevBuf b_L, b_W, b_X, b_alpha, b_r, b_z, b_logdet, b_quad, b_info, b_gpart, b_g4, b_gy, b_apart, b_gard;
-  bool want_ard = false;
+  s.nvec = (size_t)6 * m + 1;
+  CU(s.b_vec.alloc(ctx, s.nvec * sizeof(double)));
+  CU(cudaMemsetAsync(s.b_vec.p, 0, s.nvec * sizeof(double), st));
+  double* d_vec = s.b_vec.as<double>();
+  if (s.do_reg) CU(cudaMemcpyAsync(d_vec + 5 * m, s.b_resid.p, sizeof(double), cudaMemcpyDeviceToDevice, st));
+  s.want_ard = false;
   if (out.grad_ard) {
-    for (int i = 0; i < m; ++i) want_ard |= latents[i].ard != nullptr;
+    for (int i = 0; i < m; ++i) s.want_ard |= latents[i].ard != nullptr;
     for (size_t i = 0; i < (size_t)m * D; ++i) out.grad_ard[i] = 0.0;
   }
-  if (want_ard) {
-    CU(b_gard.alloc(ctx, (size_t)m * MAX_ARD * sizeof(double)));
-    CU(cudaMemsetAsync(b_gard.p, 0, (size_t)m * MAX_ARD * sizeof(double), st));
+  if (s.want_ard) {
+    CU(s.b_gard.alloc(ctx, (size_t)m * MAX_ARD * sizeof(double)));
+    CU(cudaMemsetAsync(s.b_gard.p, 0, (size_t)m * MAX_ARD * sizeof(double), st));
   }
-  DevBuf b_tpart, b_gterms;
-  int max_terms = 1;
-  bool terms_ard = false;
+  s.max_terms = 1;
+  s.terms_ard = false;
   if (out.grad_terms) {
-    terms_shape(latents, lo, hi, max_terms, terms_ard);
-    CU(b_gterms.alloc(ctx, (size_t)m * TERM_SLOTS * sizeof(double)));
-    CU(cudaMemsetAsync(b_gterms.p, 0, (size_t)m * TERM_SLOTS * sizeof(double), st));
+    terms_shape(latents, lo, hi, s.max_terms, s.terms_ard);
+    CU(s.b_gterms.alloc(ctx, (size_t)m * TERM_SLOTS * sizeof(double)));
+    CU(cudaMemsetAsync(s.b_gterms.p, 0, (size_t)m * TERM_SLOTS * sizeof(double), st));
   }
-  std::vector<int> hinfo(nl, 0);
-  std::vector<double> hg4((size_t)nl * 4, 0.0);
+  return LMM_OK;
+}
+
+int grad_run_finish(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m, int N, int D, int p, double sigma2, const Projection& pr,
+                    const double* Shost, GradOut out, GradRun& s, const double* d_a, const std::vector<int>& hinfo,
+                    const std::vector<double>& hg4, const std::vector<double>& hquad) {
+  cudaStream_t st = ctx->stream;
+  const int lo = s.lo, mloc = s.mloc;
+  const size_t npad = s.npad, nvec = s.nvec;
+  const bool multi = s.multi, want_ard = s.want_ard, want_U = s.want_U, want_R = s.want_R, want_Z = s.want_Z;
+  double* d_vec = s.b_vec.as<double>();
+  int rc;
+  DevBuf b_gy;
   if (mloc > 0) {
-    const size_t per_lat = factor_bytes_per_latent(nt) + (size_t)nt * nt * TT * sizeof(double) + 6 * npad * sizeof(double);
-    int chunk = 0;
-    CU(mem_fit(ctx, per_lat, mloc, &chunk));
-    const int ntl = (int)sym_tiles(nt);
-    CU(b_L.alloc(ctx, (size_t)chunk * sym_tiles(nt) * TT * sizeof(double)));
-    CU(b_W.alloc(ctx, (size_t)chunk * nt * TT * sizeof(double)));
-    CU(b_X.alloc(ctx, (size_t)chunk * nt * nt * TT * sizeof(double)));
-    CU(b_alpha.alloc(ctx, (size_t)mloc * npad * sizeof(double)));
-    CU(b_r.alloc(ctx, (size_t)chunk * npad * sizeof(double)));
-    CU(b_z.alloc(ctx, (size_t)chunk * npad * sizeof(double)));
-    CU(b_logdet.alloc(ctx, (size_t)mloc * sizeof(double)));
-    CU(b_quad.alloc(ctx, (size_t)mloc * sizeof(double)));
-    CU(b_info.alloc(ctx, (size_t)mloc * sizeof(int)));
-    CU(b_gpart.alloc(ctx, (size_t)chunk * ntl * 3 * sizeof(double)));
-    CU(b_g4.alloc(ctx, (size_t)mloc * 4 * sizeof(double)));
-    if (want_ard) CU(b_apart.alloc(ctx, (size_t)chunk * ntl * MAX_ARD * sizeof(double)));
-    if (out.grad_terms) CU(b_tpart.alloc(ctx, (size_t)chunk * ntl * TERM_SLOTS * sizeof(double)));
-    CU(cudaMemsetAsync(b_logdet.p, 0, (size_t)mloc * sizeof(double), st));
-    CU(cudaMemsetAsync(b_info.p, 0, (size_t)mloc * sizeof(int), st));
-    for (int c0 = 0; c0 < mloc; c0 += chunk) {
-      const int nb = (c0 + chunk <= mloc) ? chunk : mloc - c0;
-      TiledSym L{b_L.as<double>(), nt, sym_tiles(nt) * TT};
-      TiledRect X{b_X.as<double>(), nt, nt, (size_t)nt * nt * TT};
-      double* W = b_W.as<double>();
-      const size_t wstride = (size_t)nt * TT;
-      const LatentParams* dp = b_params.as<LatentParams>() + c0;
-      double* delta = b_ty.as<double>() + (size_t)c0 * npad;
-      double* alpha = b_alpha.as<double>() + (size_t)c0 * npad;
-      CU(launch_kmat_sym(st, L, nb, b_x.as<double>(), N, D, dp, ctx->distance_form));
-      CU(chol_factor(ctx, L, W, wstride, nb, b_logdet.as<double>() + c0, b_info.as<int>() + c0));
-      CU(cudaMemcpyAsync(b_r.p, delta, (size_t)nb * npad * sizeof(double), cudaMemcpyDeviceToDevice, st));
-      CU(launch_fwd_solve(st, L, W, wstride, b_r.as<double>(), b_z.as<double>(), npad, nb, &ctx->launches));
-      CU(launch_sumsq(st, b_z.as<double>(), npad, (int)npad, nb, b_quad.as<double>() + c0));
-      CU(cudaMemcpyAsync(b_r.p, b_z.p, (size_t)nb * npad * sizeof(double), cudaMemcpyDeviceToDevice, st));
-      CU(launch_bwd_solve(st, L, W, wstride, b_r.as<double>(), alpha, npad, nb, &ctx->launches));
-      CU(launch_lml_terms(st, d_vec, lo + c0, nb, b_logdet.as<double>() + c0, b_quad.as<double>() + c0, N, LOG2PI));
-      // potri: X = L^{-T}, then -C^{-1} = -X X' into the (no longer needed) factor tiles
-      CU(launch_rect_identity(st, X, nb));
-      CU(trsm_right_lt_upper(ctx, st, X, L, W, wstride, nb));
-      CU(cudaMemsetAsync(b_L.p, 0, (size_t)nb * sym_tiles(nt) * TT * sizeof(double), st));
-      GemmArgs g{};
-      g.A = operand(X); g.B = operand(X); g.C = operand(L);
-      g.i0 = 0; g.j0 = 0; g.k0 = 0; g.k1 = nt; g.sym = 1; g.k_from_row = 1;
-      CU(launch_gemm(st, GEMM_UPDATE, g, nt, nt, nb));
-      CU(launch_kgrad(st, L, nb, b_x.as<double>(), N, D, dp, alpha, npad, ctx->distance_form, b_gpart.as<double>()));
-      CU(launch_kgrad_finish(st, b_gpart.as<double>(), ntl, nb, alpha, npad, N, b_g4.as<double>() + (size_t)c0 * 4));
-      ctx->launches += 8;
-      if (want_ard) {
-        CU(launch_kgrad_ard(st, L.base, L.batch_stride, 0, b_x.as<double>(), N, D, dp, nb, alpha, npad, ctx->distance_form,
-                            b_apart.as<double>(), b_gard.as<double>() + (size_t)(lo + c0) * MAX_ARD));
-        ctx->launches += 2;
-      }
-      if (out.grad_terms) {
-        CU(launch_kgrad_terms(st, L.base, L.batch_stride, 0, b_x.as<double>(), N, D, dp, nb, max_terms, terms_ard, alpha, npad,
-                              ctx->distance_form, b_tpart.as<double>(), b_gterms.as<double>() + (size_t)(lo + c0) * TERM_SLOTS));
-        ctx->launches += 2;
-      }
-    }
-    std::vector<double> hquad(mloc, 0.0);
-    CU(copy_out(ctx, hinfo.data(), b_info.p, (size_t)mloc * sizeof(int)));
-    CU(copy_out(ctx, hg4.data(), b_g4.p, (size_t)mloc * 4 * sizeof(double)));
-    CU(copy_out(ctx, hquad.data(), b_quad.p, (size_t)mloc * sizeof(double)));
-    CU(cudaStreamSynchronize(st));
     // scatter the local gradients into the reduction vector
     std::vector<double> hv(nvec, 0.0);
     for (int i = 0; i < mloc; ++i) hv[(size_t)5 * m + 1 + lo + i] = hquad[i];
@@ -355,11 +289,11 @@ int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m,
   std::vector<double> hgard;
   if (want_ard) {
     if (multi) {
-      int r = nccl_api().AllReduce(b_gard.p, b_gard.p, (size_t)m * MAX_ARD, NCCL_DOUBLE, NCCL_SUM, ctx->comm, st);
+      int r = nccl_api().AllReduce(s.b_gard.p, s.b_gard.p, (size_t)m * MAX_ARD, NCCL_DOUBLE, NCCL_SUM, ctx->comm, st);
       if (r != 0) return ctx->fail(LMM_E_NCCL, "ncclAllReduce failed");
     }
     hgard.resize((size_t)m * MAX_ARD);
-    CU(copy_out(ctx, hgard.data(), b_gard.p, hgard.size() * sizeof(double)));
+    CU(copy_out(ctx, hgard.data(), s.b_gard.p, hgard.size() * sizeof(double)));
     CU(cudaStreamSynchronize(st));
     for (int i = 0; i < m; ++i)
       for (int k = 0; k < D && k < MAX_ARD; ++k) out.grad_ard[(size_t)i * D + k] = latents[i].ard ? hgard[(size_t)i * MAX_ARD + k] : 0.0;
@@ -367,14 +301,14 @@ int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m,
   std::vector<double> hterms;
   if (out.grad_terms) {
     if (multi) {
-      int r = nccl_api().AllReduce(b_gterms.p, b_gterms.p, (size_t)m * TERM_SLOTS, NCCL_DOUBLE, NCCL_SUM, ctx->comm, st);
+      int r = nccl_api().AllReduce(s.b_gterms.p, s.b_gterms.p, (size_t)m * TERM_SLOTS, NCCL_DOUBLE, NCCL_SUM, ctx->comm, st);
       if (r != 0) return ctx->fail(LMM_E_NCCL, "ncclAllReduce failed");
     }
     hterms.resize((size_t)m * TERM_SLOTS);
-    CU(copy_out(ctx, hterms.data(), b_gterms.p, hterms.size() * sizeof(double)));
+    CU(copy_out(ctx, hterms.data(), s.b_gterms.p, hterms.size() * sizeof(double)));
     CU(cudaStreamSynchronize(st));
   }
-  // d/dy: -sum_i T[i,:]' α_i  (- R/σ² from the regulariser on rank 0)
+  // d/dy: -sum_i T[i,:]' a_i  (- R/σ² from the regulariser on rank 0)
   if (out.grad_y) {
     const size_t ny = (size_t)p * N;
     CU(b_gy.alloc(ctx, 2 * ny * sizeof(double)));
@@ -387,13 +321,13 @@ int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m,
       DevBuf b_Hn;
       CU(b_Hn.alloc(ctx, Hneg.size() * sizeof(double)));
       CU(copy_in(ctx, b_Hn.as<double>(), Hneg.data(), Hneg.size()));
-      CU(launch_backproject(st, b_Hn.as<double>(), p, m, lo, mloc, b_alpha.as<double>(), b_alpha.as<double>(), npad, N, 0.0, 0.0, 0,
+      CU(launch_backproject(st, b_Hn.as<double>(), p, m, lo, mloc, d_a, d_a, npad, N, 0.0, 0.0, 0,
                             b_gy.as<double>(), b_gy.as<double>() + ny));
       ++ctx->launches;
       CU(cudaStreamSynchronize(st));
     }
     if (want_R) {
-      CU(launch_axpy(st, b_gy.as<double>(), b_R.as<double>(), ny, -1.0 / sigma2));
+      CU(launch_axpy(st, b_gy.as<double>(), s.b_R.as<double>(), ny, -1.0 / sigma2));
       ++ctx->launches;
     }
     if (multi) {
@@ -402,7 +336,7 @@ int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m,
     }
     CU(copy_out(ctx, out.grad_y, b_gy.p, ny * sizeof(double)));
   }
-  // d/dU: -(Y α_i)/sqrt(S_i) per column (latent) + R Z'/σ² from the regulariser (rank 0)
+  // d/dU: -(Y a_i)/sqrt(S_i) per column (latent) + R Z'/σ² from the regulariser (rank 0)
   std::vector<double> hGU;
   if (want_U) {
     DevBuf b_GU;
@@ -410,11 +344,11 @@ int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m,
     CU(b_GU.alloc(ctx, 2 * npm * sizeof(double)));
     CU(cudaMemsetAsync(b_GU.p, 0, 2 * npm * sizeof(double), st));
     if (mloc > 0) {
-      CU(launch_abt(st, d_y, (size_t)N, p, b_alpha.as<double>(), npad, mloc, N, 1.0, b_GU.as<double>() + (size_t)lo * p));
+      CU(launch_abt(st, s.d_y, (size_t)N, p, d_a, npad, mloc, N, 1.0, b_GU.as<double>() + (size_t)lo * p));
       ++ctx->launches;
     }
     if (want_Z) {
-      CU(launch_abt(st, b_R.as<double>(), (size_t)N, p, b_Z.as<double>(), (size_t)N, m, N, 1.0, b_GU.as<double>() + npm));
+      CU(launch_abt(st, s.b_R.as<double>(), (size_t)N, p, s.b_Z.as<double>(), (size_t)N, m, N, 1.0, b_GU.as<double>() + npm));
       ++ctx->launches;
     }
     if (multi) {
@@ -448,9 +382,9 @@ int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m,
     dreg = -((double)N * (double)(p - m) / sigma2 - resid / (sigma2 * sigma2)) / 2.0;
   }
   if (out.logpdf) {
-    double s = 0.0;
-    for (int i = 0; i < m; ++i) s += hv[i];
-    *out.logpdf = s + reg;
+    double sum = 0.0;
+    for (int i = 0; i < m; ++i) sum += hv[i];
+    *out.logpdf = sum + reg;
   }
   if (out.grad_latents)
     for (int i = 0; i < m; ++i) {
@@ -460,9 +394,9 @@ int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m,
     }
   if (out.grad_terms) scatter_terms(latents, m, D, hterms, out.grad_terms, out.grad_latents, out.grad_ard);
   if (out.grad_sigma2) {
-    double s = dreg;
-    for (int i = 0; i < m; ++i) s += hv[(size_t)4 * m + i] * (orth ? 1.0 / Shost[i] : 1.0);  // ν_i = σ²/S_i (OILMM) or σ²
-    *out.grad_sigma2 = s;
+    double sum = dreg;
+    for (int i = 0; i < m; ++i) sum += hv[(size_t)4 * m + i] * (orth ? 1.0 / Shost[i] : 1.0);  // ν_i = σ²/S_i (OILMM) or σ²
+    *out.grad_sigma2 = sum;
   }
   if (orth && out.grad_S)
     for (int i = 0; i < m; ++i) {
@@ -477,6 +411,86 @@ int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m,
         out.grad_U[(size_t)i * p + j] = -hGU[(size_t)i * p + j] / std::sqrt(Shost[i]) + hGU[npm + (size_t)i * p + j] / sigma2;
   }
   return LMM_OK;
+}
+
+int latents_grad_run(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m, const double* x, int N, int D, int p, double sigma2,
+                     const double* y, const Projection& pr, const double* Shost, GradOut out) {
+  GradRun s;
+  int rc = grad_run_setup(ctx, orth, latents, m, x, N, D, p, y, pr, out, s);
+  if (rc) return rc;
+  cudaStream_t st = ctx->stream;
+  const int lo = s.lo, mloc = s.mloc, nt = s.nt, nl = s.nl, max_terms = s.max_terms;
+  const bool want_ard = s.want_ard, terms_ard = s.terms_ard;
+  const size_t npad = s.npad;
+  double* d_vec = s.b_vec.as<double>();
+  DevBuf b_L, b_W, b_X, b_alpha, b_r, b_z, b_logdet, b_quad, b_info, b_gpart, b_g4, b_apart, b_tpart;
+  std::vector<int> hinfo(nl, 0);
+  std::vector<double> hg4((size_t)nl * 4, 0.0), hquad(nl, 0.0);
+  if (mloc > 0) {
+    const size_t per_lat = factor_bytes_per_latent(nt) + (size_t)nt * nt * TT * sizeof(double) + 6 * npad * sizeof(double);
+    int chunk = 0;
+    CU(mem_fit(ctx, per_lat, mloc, &chunk));
+    const int ntl = (int)sym_tiles(nt);
+    CU(b_L.alloc(ctx, (size_t)chunk * sym_tiles(nt) * TT * sizeof(double)));
+    CU(b_W.alloc(ctx, (size_t)chunk * nt * TT * sizeof(double)));
+    CU(b_X.alloc(ctx, (size_t)chunk * nt * nt * TT * sizeof(double)));
+    CU(b_alpha.alloc(ctx, (size_t)mloc * npad * sizeof(double)));
+    CU(b_r.alloc(ctx, (size_t)chunk * npad * sizeof(double)));
+    CU(b_z.alloc(ctx, (size_t)chunk * npad * sizeof(double)));
+    CU(b_logdet.alloc(ctx, (size_t)mloc * sizeof(double)));
+    CU(b_quad.alloc(ctx, (size_t)mloc * sizeof(double)));
+    CU(b_info.alloc(ctx, (size_t)mloc * sizeof(int)));
+    CU(b_gpart.alloc(ctx, (size_t)chunk * ntl * 3 * sizeof(double)));
+    CU(b_g4.alloc(ctx, (size_t)mloc * 4 * sizeof(double)));
+    if (want_ard) CU(b_apart.alloc(ctx, (size_t)chunk * ntl * MAX_ARD * sizeof(double)));
+    if (out.grad_terms) CU(b_tpart.alloc(ctx, (size_t)chunk * ntl * TERM_SLOTS * sizeof(double)));
+    CU(cudaMemsetAsync(b_logdet.p, 0, (size_t)mloc * sizeof(double), st));
+    CU(cudaMemsetAsync(b_info.p, 0, (size_t)mloc * sizeof(int), st));
+    for (int c0 = 0; c0 < mloc; c0 += chunk) {
+      const int nb = (c0 + chunk <= mloc) ? chunk : mloc - c0;
+      TiledSym L{b_L.as<double>(), nt, sym_tiles(nt) * TT};
+      TiledRect X{b_X.as<double>(), nt, nt, (size_t)nt * nt * TT};
+      double* W = b_W.as<double>();
+      const size_t wstride = (size_t)nt * TT;
+      const LatentParams* dp = s.b_params.as<LatentParams>() + c0;
+      double* delta = s.b_ty.as<double>() + (size_t)c0 * npad;
+      double* alpha = b_alpha.as<double>() + (size_t)c0 * npad;
+      CU(launch_kmat_sym(st, L, nb, s.b_x.as<double>(), N, D, dp, ctx->distance_form));
+      CU(chol_factor(ctx, L, W, wstride, nb, b_logdet.as<double>() + c0, b_info.as<int>() + c0));
+      CU(cudaMemcpyAsync(b_r.p, delta, (size_t)nb * npad * sizeof(double), cudaMemcpyDeviceToDevice, st));
+      CU(launch_fwd_solve(st, L, W, wstride, b_r.as<double>(), b_z.as<double>(), npad, nb, &ctx->launches));
+      CU(launch_sumsq(st, b_z.as<double>(), npad, (int)npad, nb, b_quad.as<double>() + c0));
+      CU(cudaMemcpyAsync(b_r.p, b_z.p, (size_t)nb * npad * sizeof(double), cudaMemcpyDeviceToDevice, st));
+      CU(launch_bwd_solve(st, L, W, wstride, b_r.as<double>(), alpha, npad, nb, &ctx->launches));
+      CU(launch_lml_terms(st, d_vec, lo + c0, nb, b_logdet.as<double>() + c0, b_quad.as<double>() + c0, N, LOG2PI));
+      // potri: X = L^{-T}, then -C^{-1} = -X X' into the (no longer needed) factor tiles
+      CU(launch_rect_identity(st, X, nb));
+      CU(trsm_right_lt_upper(ctx, st, X, L, W, wstride, nb));
+      CU(cudaMemsetAsync(b_L.p, 0, (size_t)nb * sym_tiles(nt) * TT * sizeof(double), st));
+      GemmArgs g{};
+      g.A = operand(X); g.B = operand(X); g.C = operand(L);
+      g.i0 = 0; g.j0 = 0; g.k0 = 0; g.k1 = nt; g.sym = 1; g.k_from_row = 1;
+      CU(launch_gemm(st, GEMM_UPDATE, g, nt, nt, nb));
+      CU(launch_kgrad(st, L, nb, s.b_x.as<double>(), N, D, dp, alpha, npad, ctx->distance_form, b_gpart.as<double>()));
+      CU(launch_kgrad_finish(st, b_gpart.as<double>(), ntl, nb, alpha, npad, N, b_g4.as<double>() + (size_t)c0 * 4));
+      ctx->launches += 8;
+      if (want_ard) {
+        CU(launch_kgrad_ard(st, L.base, L.batch_stride, 0, s.b_x.as<double>(), N, D, dp, nb, alpha, npad, ctx->distance_form,
+                            b_apart.as<double>(), s.b_gard.as<double>() + (size_t)(lo + c0) * MAX_ARD));
+        ctx->launches += 2;
+      }
+      if (out.grad_terms) {
+        CU(launch_kgrad_terms(st, L.base, L.batch_stride, 0, s.b_x.as<double>(), N, D, dp, nb, max_terms, terms_ard, alpha, npad,
+                              ctx->distance_form, b_tpart.as<double>(), s.b_gterms.as<double>() + (size_t)(lo + c0) * TERM_SLOTS));
+        ctx->launches += 2;
+      }
+    }
+    CU(copy_out(ctx, hinfo.data(), b_info.p, (size_t)mloc * sizeof(int)));
+    CU(copy_out(ctx, hg4.data(), b_g4.p, (size_t)mloc * 4 * sizeof(double)));
+    CU(copy_out(ctx, hquad.data(), b_quad.p, (size_t)mloc * sizeof(double)));
+    CU(cudaStreamSynchronize(st));
+  }
+  return grad_run_finish(ctx, orth, latents, m, N, D, p, sigma2, pr, Shost, out, s, b_alpha.as<double>(), hinfo, hg4, hquad);
 }
 
 }  // namespace lmm_host

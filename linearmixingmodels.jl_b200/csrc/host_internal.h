@@ -358,6 +358,39 @@ bool per_input_mask(const double* y, int p, int N, std::vector<int>& keep);
 
 constexpr int TERM_SLOTS = LMM_MAX_TERMS * LMM_GRAD_TERM_STRIDE;  // grad_terms doubles per latent
 void terms_shape(const lmm_gp_desc* latents, int lo, int hi, int& max_terms, bool& any_ard);
+
+struct GradOut {
+  double* logpdf;
+  double* grad_latents;  // m x 3: d/d variance, d/d inv_lengthscale, d/d mean_const
+  double* grad_sigma2;
+  double* grad_y;        // p*N by outputs (nullable)
+  int* info_latent;
+  double* grad_U = nullptr;  // p x m column-major (OILMM only, nullable)
+  double* grad_S = nullptr;  // m (OILMM only, nullable)
+  const double* Yhost_or_dev = nullptr;
+  double* grad_ard = nullptr;  // m x D row-major: d/d ARD multiplier (zeros for latents without an ARDTransform; nullable)
+  double* grad_terms = nullptr;  // m x LMM_MAX_TERMS x LMM_GRAD_TERM_STRIDE: per-term gradients (nullable)
+};
+
+// The OILMM / IndependentMOGP logpdf gradient (host_grad.cu) and the LOO driver (host_loo.cu) share everything but the
+// per-latent loop.  grad_run_setup stages the inputs, projects the data (δ = T y - m in b_ty, regulariser pieces) and
+// allocates the reduction buffers; the loop leaves per latent a [mloc][npad] vector a (α for the logpdf, w for LOO) with
+// dvalue/dδ = -a, hg4[i*4 + {0,1,2,3}] = {d/d variance, d/d inv_lengthscale, d/d noise, Σ a}, hdot[i] = a·δ, the value
+// terms in b_vec[lo + i] and (when asked) b_gard / b_gterms; grad_run_finish runs the chain to U, S, σ², y and the means.
+struct GradRun {
+  int lo = 0, hi = 0, mloc = 0, nt = 0, nl = 1;
+  size_t npad = 0, nvec = 0;
+  bool multi = false, do_reg = false, want_U = false, want_R = false, want_Z = false, want_ard = false;
+  int max_terms = 1;
+  bool terms_ard = false;
+  const double* d_y = nullptr;
+  DevBuf b_x, b_y, b_T, b_P, b_Q, b_means, b_ty, b_part, b_resid, b_R, b_Z, b_params, b_vec, b_gard, b_gterms;
+};
+int grad_run_setup(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m, const double* x, int N, int D, int p, const double* y,
+                   const Projection& pr, const GradOut& out, GradRun& s);
+int grad_run_finish(lmm_ctx* ctx, bool orth, const lmm_gp_desc* latents, int m, int N, int D, int p, double sigma2, const Projection& pr,
+                    const double* Shost, GradOut out, GradRun& s, const double* d_a, const std::vector<int>& hinfo,
+                    const std::vector<double>& hg4, const std::vector<double>& hdot);
 // What post_logpdf_impl leaves behind for the gradient through the conditioning (host_post_grad.cu): the predictive factors
 // and inputs (P), β_i = Σ*_i⁻¹(ỹ*_i - μ_i) of the resident latents [nloc][P.nspad], and the rank-summed gradient pieces
 // hg = [β_i'β_i (m) | tr(Σ*_i⁻¹) (m) | |R*|² (1)].

@@ -98,7 +98,7 @@ cudaError_t launch_sumsq(cudaStream_t st, const double* v, size_t stride, int n,
 // y[b][R*128 + r] = add[b] + sum_J T(R,J) x[b][J*128 + :]   over a rectangular tiled matrix
 cudaError_t launch_rect_gemv(cudaStream_t st, TiledRect A, const double* x, size_t x_stride, double* y, size_t y_stride,
                              const LatentParams* params, int add_mean, int batch);
-// y[b][R*128 + r] = base[b] - sum_J sum_c T(R,J)(r,c)^2     (posterior variance)
+// y[b][R*128 + r] = base[b] - sum_J sum_c T(R,J)(r,c)^2     (posterior variance; params == null: base = 0, sign +)
 cudaError_t launch_rect_rowsumsq(cudaStream_t st, TiledRect A, double* y, size_t y_stride, const LatentParams* params, int batch);
 // y = L * z for a packed-lower factor (rand): y[b][I] = sum_{J<=I} L(I,J) z[b][J]
 cudaError_t launch_lower_gemv(cudaStream_t st, TiledSym L, const double* z, size_t z_stride, double* y, size_t y_stride, int batch);
@@ -228,6 +228,20 @@ cudaError_t launch_kgrad_masked(cudaStream_t st, TiledSym negCinv, const int* ob
                                 int m, int p, const double* Hm, const double* alpha, int max_terms, bool any_ard, int form, const int* seg,
                                 double* tpart, double* rowpart, double* colpart, double* v, double* out_terms, double* out_H, double* out_diag);
 cudaError_t launch_scale_sub(cudaStream_t st, double* v, const double* a, double sa, const double* b, size_t n);
+}  // namespace lmm
+
+namespace lmm {
+// ---- loo.cu : leave-one-input-out cross-validation of a batch of latent GPs (C = K + νI, A = C⁻¹, α = Aδ)
+// d_i = A_ii from the diagonal of negA = -A (negA.base != null) or from dvec; per latent b, i < stride (each output nullable):
+// q = α/d, sc = sqrt((1 + α q)/d), v = q/sc, lmean = δ + mean - q, lvar = 1/d - ν (all 0 for i >= N); loo[b] = LOO value.
+cudaError_t launch_loo_terms(cudaStream_t st, TiledSym negA, const double* dvec, const double* alpha, const double* delta, size_t stride,
+                             int N, const LatentParams* params, int batch, double log2pi, double* q, double* sc, double* v, double* lmean,
+                             double* lvar, double* loo);
+// B = A diag(sc) (full square tiles) from the packed-lower negA = -A
+cudaError_t launch_sym_expand_scale(cudaStream_t st, TiledSym negA, const double* sc, size_t sc_stride, TiledRect B, int batch);
+// u = α + w; out[b*4 + 2] = tr G = ½ Σ (u_i² + M_ii), out[b*4 + 3] = Σ w_i, dot[b] = w·δ  (i < N; M = -αα' - ww' - 2ARA)
+cudaError_t launch_loo_grad_vectors(cudaStream_t st, TiledSym M, const double* alpha, const double* w, const double* delta, size_t stride,
+                                    int N, int batch, double* u, double* out, double* dot);
 }  // namespace lmm
 
 namespace lmm {

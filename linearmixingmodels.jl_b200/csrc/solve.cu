@@ -411,7 +411,7 @@ cudaError_t launch_rect_gemv(cudaStream_t st, TiledRect A, const double* x, size
   return cudaGetLastError();
 }
 
-// grid (ntr, batch): y[b][R*128 + r] = variance_b - sum_J sum_c T(R,J)(r,c)^2
+// grid (ntr, batch): y[b][R*128 + r] = variance_b - sum_J sum_c T(R,J)(r,c)^2   (params == null: the row sums of squares)
 __global__ void __launch_bounds__(256) rect_rowsumsq_kernel(TiledRect A, double* __restrict__ y, size_t y_stride,
                                                             const LatentParams* __restrict__ params) {
   __shared__ double ys[TILE];
@@ -428,7 +428,7 @@ __global__ void __launch_bounds__(256) rect_rowsumsq_kernel(TiledRect A, double*
   }
   tile_gemv_n_finish(a0, a1, ys);
   __syncthreads();
-  if (t < TILE) y[(size_t)b * y_stride + R * TILE + t] = params[b].kdiag - ys[t];
+  if (t < TILE) y[(size_t)b * y_stride + R * TILE + t] = params ? params[b].kdiag - ys[t] : ys[t];
 }
 cudaError_t launch_rect_rowsumsq(cudaStream_t st, TiledRect A, double* y, size_t y_stride, const LatentParams* params, int batch) {
   dim3 grid((unsigned)A.ntr, (unsigned)batch);

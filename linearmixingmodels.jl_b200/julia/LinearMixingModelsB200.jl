@@ -359,6 +359,68 @@ function ChainRulesCore.rrule(::typeof(AbstractGPs.logpdf), fx::FiniteGP{<:ILMM{
     return out[], logpdf_pullback
 end
 
+# --- leave-one-input-out cross-validation (lmm_oilmm_loo / lmm_imogp_loo) --------------------------------------------
+# loo_logpdf(fx, y) = Σ_i log p(y_i | y_{-i}) with y_i all outputs at input x_i (closed form, no refits);
+# loo_mean_and_var(fx, y) = the LOO predictive marginals, by outputs.  Outputs left at C_NULL are not computed; without a
+# gradient output only the value path runs.
+const LOOFiniteGP = Union{FiniteGP{<:OILMM{<:IndependentMOGP{<:Vector{<:GP}}}},
+                          FiniteGP{<:IndependentMOGP{<:Vector{<:GP}},<:MOInputIsotopicByOutputs,<:Diagonal{<:Real,<:Fill}}}
+
+function _loo(fx::LOOFiniteGP, y::AbstractVector{<:Real}; out=C_NULL, M=C_NULL, V=C_NULL, gl=C_NULL, gs2=C_NULL, gy=C_NULL,
+              gU=C_NULL, gS=C_NULL, gt=C_NULL)
+    il = Ref{Cint}(-1)
+    if fx.f isa OILMM
+        fs, H, σ², x = unpack(fx)
+        X, D = points(x)
+        descs, keep = gpdescs(fs.fs)
+        check(GC.@preserve keep ccall((:lmm_oilmm_loo, liblmm), Cint,
+            (Ptr{Cvoid}, Ptr{GpDesc}, Cint, Ptr{Float64}, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Cint, Float64, Ptr{Float64}, Cint,
+             Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Float64}, Ptr{Cint}),
+            ctx(), descs, length(descs), X, length(x), D, Matrix{Float64}(H.U), Vector{Float64}(diag(H.S)), size(H, 1), Float64(σ²),
+            Vector{Float64}(y), fx.x.out_dim, out, M, V, gl, C_NULL, gs2, gy, gU, gS, gt, il))
+    else
+        X, D = points(fx.x.x)
+        descs, keep = gpdescs(fx.f.fs)
+        check(GC.@preserve keep ccall((:lmm_imogp_loo, liblmm), Cint,
+            (Ptr{Cvoid}, Ptr{GpDesc}, Cint, Ptr{Float64}, Cint, Cint, Float64, Ptr{Float64}, Cint,
+             Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Cint}),
+            ctx(), descs, length(descs), X, length(fx.x.x), D, Float64(fx.Σy[1]), Vector{Float64}(y), fx.x.out_dim,
+            out, M, V, gl, C_NULL, gs2, gy, gt, il))
+    end
+    return nothing
+end
+
+function loo_logpdf(fx::LOOFiniteGP, y::AbstractVector{<:Real})
+    out = Ref{Float64}(0.0)
+    _loo(fx, y; out = out)
+    return out[]
+end
+
+function loo_mean_and_var(fx::LOOFiniteGP, y::AbstractVector{<:Real})
+    M = Vector{Float64}(undef, length(y)); V = Vector{Float64}(undef, length(y))
+    _loo(fx, y; M = M, V = V)
+    return M, V
+end
+
+# The pullback gives the σ² and y tangents; the per-term kernel tangents (gt), the means (gl row 3) and, for an OILMM, U / S
+# are computed as in the logpdf rrule and, as there, not mapped onto the kernel structs.
+function ChainRulesCore.rrule(::typeof(loo_logpdf), fx::LOOFiniteGP, y::AbstractVector{<:Real})
+    orth = fx.f isa OILMM
+    m = length((orth ? fx.f.f : fx.f).fs)
+    out = Ref{Float64}(0.0); gs2 = Ref{Float64}(0.0)
+    gl = Matrix{Float64}(undef, 3, m); gy = Vector{Float64}(undef, length(y))
+    gt = Matrix{Float64}(undef, GRAD_TERM_DOUBLES, m)
+    gU = orth ? Matrix{Float64}(undef, size(fx.f.H, 1), m) : C_NULL
+    gS = orth ? Vector{Float64}(undef, m) : C_NULL
+    _loo(fx, y; out = out, gl = gl, gs2 = gs2, gy = gy, gU = gU, gS = gS, gt = gt)
+    function loo_pullback(Δ)
+        Σy_tangent = Tangent{typeof(fx.Σy)}(; diag = Tangent{typeof(fx.Σy.diag)}(; value = Δ * gs2[]))
+        return NoTangent(), Tangent{typeof(fx)}(; Σy = Σy_tangent), Δ .* gy
+    end
+    return out[], loo_pullback
+end
+
 # --- rrule for logpdf(post(x*, σ²), y*) (test/oilmm.jl:32 `gradient(logpdf, po, y_test)`) -----------------------------
 # Through the conditioning (lmm_post_logpdf_grad_full): besides the Σy and y* tangents, the posterior's latents get a tangent
 # on their `prior` (per-term hyper-parameters gt as in the prior rrule, mapping onto the kernel structs omitted as there; the
