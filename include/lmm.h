@@ -148,7 +148,11 @@ const char* lmm_version(void);
  *                     instead of 36 MMAs per tile product; exact int32 sums for K * P < 131072 columns, i.e. N <= 18724 at 7 planes --
  *                     beyond that the update of a block column falls back to DMMA).  LMM_OZAKI_BITS sets the initial value.
  *   "ozaki_min_k"     wide updates over fewer k-tiles than this stay on DMMA (default 4: the int8 epilogue costs per output tile); with
- *                     "ozaki" on, "outer_block" defaults to 2 tile columns (the in-block updates stay on DMMA)
+ *                     "ozaki" on, "outer_block" defaults to 2 tile columns (the in-block updates stay on DMMA), and to 1 for the
+ *                     banded factors of the OILMM / IndependentMOGP eval from 64 tile rows (N >= 8192) on (every update of a column by
+ *                     earlier ones takes the int8 path)
+ *   "trsm_slice"      with "ozaki" on: 1 (default) = the panel TRSMs write the int8 digit planes of the tiles they finish; 0 = a separate
+ *                     slice pass per block column (the same bytes: results are bit-identical)
  *   "ozaki_single_nt" with "ozaki" on, batches <= 2 keep the right-looking DMMA schedule unless the factor has at least this many tile
  *                     rows (two thirds of it for a batch of 2), from which on it takes the batched schedule and with it the int8 update
  *                     (default 96, i.e. N >= 12288: N = 16384: 45.9 -> 33 ms, two factors 88.9 -> 44 ms, while a single N = 8192

@@ -261,6 +261,9 @@ extern "C" int lmm_ctx_set_option(lmm_ctx* ctx, const char* key, double value) {
   } else if (k == "ozaki_min_k") {
     if (value < 1 || value > 4096) return ctx->fail(LMM_E_ARG, "ozaki_min_k must be in [1, 4096]");
     ctx->ozaki_min_k = (int)value;
+  } else if (k == "trsm_slice") {
+    if (value != 0.0 && value != 1.0) return ctx->fail(LMM_E_ARG, "trsm_slice must be 0 or 1");
+    ctx->trsm_slice = (int)value;
   } else if (k == "gemm_small") {
     if (value < 0 || value > 4096) return ctx->fail(LMM_E_ARG, "gemm_small must be in [0, 4096]");
     set_gemm_small_threshold((int)value);

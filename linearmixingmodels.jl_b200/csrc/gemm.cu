@@ -21,6 +21,7 @@
 #include "common.cuh"
 #include "kernels.h"
 #include "direct_gemm.cuh"
+#include "ozaki_slice.cuh"
 
 namespace lmm {
 
@@ -69,8 +70,11 @@ __device__ __forceinline__ void bulk_load(void* dst, const void* src, uint32_t b
                : "memory");
 }
 
-template <int MODE, int KC>
-__global__ void __launch_bounds__(256, 1) gemm_tile_kernel_v2(GemmArgs g) {
+// SLICE (TRSM only): after storing the finished tile, the CTA copies it into the freed stage ring (128 of the 192 KB, tile layout)
+// and writes its int8 digit planes from there (oz_slice_tile), for tile rows I >= sl.i0: one read of the tile from HBM and one
+// launch per column fewer than a separate ozaki_slice_kernel pass.
+template <int MODE, int KC, bool SLICE = false>
+__global__ void __launch_bounds__(256, 1) gemm_tile_kernel_v2(GemmArgs g, TrsmSliceArgs sl) {
   constexpr int V2_STAGES = 96 / KC;
   constexpr int SCHUNK = 128 * KC;  // doubles per operand per stage
   extern __shared__ __align__(128) double smem[];
@@ -209,7 +213,16 @@ __global__ void __launch_bounds__(256, 1) gemm_tile_kernel_v2(GemmArgs g) {
         v.x = acct[mb][nb][0];
         v.y = acct[mb][nb][1];
         *reinterpret_cast<double2*>(Ctile + off) = v;
+        if constexpr (SLICE) *reinterpret_cast<double2*>(smem + off) = v;
       }
+    if constexpr (SLICE) {
+      if (I >= sl.i0) {
+        __syncthreads();
+        oz_slice_tile(smem, sl.scale + (size_t)b * sl.scale_stride + (size_t)I * TILE,
+                      sl.slices + (size_t)b * sl.slice_stride + sym_tile_index(I, J) * ((size_t)sl.S * 16384), sl.S, sl.bits,
+                      sl.fp ? sl.fp + (size_t)b * sl.fp_stride + sym_tile_index(I, J) : nullptr);
+      }
+    }
   } else {
 #pragma unroll
     for (int mb = 0; mb < 8; ++mb) {
@@ -228,13 +241,13 @@ __global__ void __launch_bounds__(256, 1) gemm_tile_kernel_v2(GemmArgs g) {
 
 static int g_gemm_small = 74;  // grids of at most this many tiles take the latency-optimised kernel (0 = never)
 void set_gemm_small_threshold(int tiles) { g_gemm_small = tiles; }
+bool gemm_takes_direct(long long tiles) { return tiles <= g_gemm_small; }
 
 static bool g_pdl = true;   // programmatic dependent launch along the panel chain (direct kernels + diagonal-tile kernel)
 void set_pdl(int v) { g_pdl = v != 0; }
 bool pdl_enabled() { return g_pdl; }
 
-cudaError_t launch_gemm(cudaStream_t st, int mode, const GemmArgs& a, int ncols, int nrows, int batch, long long select_tiles) {
-  if (ncols <= 0 || nrows <= 0 || batch <= 0) return cudaSuccess;
+static cudaError_t configure_v2() {
   static bool configured_dev[64] = {false};  // function attributes are per device
   int dev = 0;
   cudaGetDevice(&dev);
@@ -244,18 +257,35 @@ cudaError_t launch_gemm(cudaStream_t st, int mode, const GemmArgs& a, int ncols,
     if (e != cudaSuccess) return e;
     e = cudaFuncSetAttribute(gemm_tile_kernel_v2<GEMM_TRSM, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GEMM_V2_SMEM);
     if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(gemm_tile_kernel_v2<GEMM_TRSM, 32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)GEMM_V2_SMEM);
+    if (e != cudaSuccess) return e;
     configured = true;
   }
-  if ((select_tiles > 0 ? select_tiles : (long long)ncols * nrows * batch) <= g_gemm_small) {
+  return cudaSuccess;
+}
+
+cudaError_t launch_gemm(cudaStream_t st, int mode, const GemmArgs& a, int ncols, int nrows, int batch, long long select_tiles) {
+  if (ncols <= 0 || nrows <= 0 || batch <= 0) return cudaSuccess;
+  cudaError_t e = configure_v2();
+  if (e != cudaSuccess) return e;
+  if (gemm_takes_direct(select_tiles > 0 ? select_tiles : (long long)ncols * nrows * batch)) {
     dim3 gs((unsigned)ncols * DIRECT_SPLIT, (unsigned)nrows, (unsigned)batch);
     if (mode == GEMM_UPDATE) return launch_pdl(g_pdl, gemm_direct2_kernel<GEMM_UPDATE>, gs, dim3(256), 0, st, a);
     return launch_pdl(g_pdl, gemm_direct2_kernel<GEMM_TRSM>, gs, dim3(256), 0, st, a);
   }
   dim3 grid((unsigned)ncols, (unsigned)nrows, (unsigned)batch);
   if (mode == GEMM_UPDATE)
-    gemm_tile_kernel_v2<GEMM_UPDATE, 32><<<grid, 256, GEMM_V2_SMEM, st>>>(a);
+    gemm_tile_kernel_v2<GEMM_UPDATE, 32><<<grid, 256, GEMM_V2_SMEM, st>>>(a, TrsmSliceArgs{});
   else
-    gemm_tile_kernel_v2<GEMM_TRSM, 32><<<grid, 256, GEMM_V2_SMEM, st>>>(a);
+    gemm_tile_kernel_v2<GEMM_TRSM, 32><<<grid, 256, GEMM_V2_SMEM, st>>>(a, TrsmSliceArgs{});
+  return cudaGetLastError();
+}
+
+cudaError_t launch_trsm_slice(cudaStream_t st, const GemmArgs& a, int nrows, int batch, const TrsmSliceArgs& s) {
+  if (nrows <= 0 || batch <= 0) return cudaSuccess;
+  cudaError_t e = configure_v2();
+  if (e != cudaSuccess) return e;
+  gemm_tile_kernel_v2<GEMM_TRSM, 32, true><<<dim3(1u, (unsigned)nrows, (unsigned)batch), 256, GEMM_V2_SMEM, st>>>(a, s);
   return cudaGetLastError();
 }
 

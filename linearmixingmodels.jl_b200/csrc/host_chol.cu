@@ -32,6 +32,9 @@ static cudaError_t chain_counters(lmm_ctx* ctx, cudaStream_t st, int nt, int bat
 // shared-memory-free GEMM roles at one CTA per SM) instead of TMA-pipelined launches per operation.
 constexpr int CHAIN_MAX_TILES = 96;
 
+// Enveloped factors of at least this many tile rows take block width 1 under the int8 update (see chol_factor_stream).
+constexpr int OZ_WIDTH1_MIN_NT = 64;
+
 // Workspace of the optional integer-slice (Ozaki) trailing update for the latents [0, batch) of one chol_factor_stream call.
 struct OzWs {
   uint8_t* slices;
@@ -69,8 +72,15 @@ cudaError_t chol_factor_stream(lmm_ctx* ctx, cudaStream_t st, TiledSym L, double
   if (oz) {
     // narrow blocks: the in-block updates stay on DMMA, so the narrower the block the less of the work is left at the FP64 rate
     // (measured at 16 / 8 latents of N = 16384, final kernel: ob = 4: 286.8 / 147.5 ms, ob = 2 with min_k = 4: 275.5 / 143.1,
-    // ob = 1: 274.8 / 147.1, ob = 3: 281.8 / 144.7; with the first kernel generation: 323 ms at ob = 8, 340 at 12)
-    if (!ctx->outer_block_user) ob = 2;
+    // ob = 1: 274.8 / 147.1, ob = 3: 281.8 / 144.7; with the first kernel generation: 323 ms at ob = 8, 340 at 12).
+    // Large enveloped factors take width 1: every update of column J by k < J then runs in the int8 kernel, whose digit-plane
+    // filter drops most of the banded products, instead of the in-block DMMA update that multiplies all of them (C4, 64 latents:
+    // 97 109 DMMA tile products at width 2, tools/bench_chol_phases.py --model-only; Cholesky stage at 64 latents, width 2 -> 1:
+    // N = 16384 57.0 -> 43.0 ms, 8192 25.2 -> 20.2, 4096 10.2 -> 8.5, 2048 3.75 -> 3.49, profiles/r10_chol_phases_*.json).
+    // Factors below OZ_WIDTH1_MIN_NT tile rows keep width 2, the schedule (and tile-product count) the int8 path has been checked
+    // with at those sizes; the rule is conservative, not a measured crossover.  No fused panel chain (jj + 1 < s1) at width 1:
+    // the last columns' TRSMs take the direct kernels once their grids are small.
+    if (!ctx->outer_block_user) ob = env_h && nt >= OZ_WIDTH1_MIN_NT ? 1 : 2;
     cudaError_t eo = launch_ozaki_scales(st, L, batch, oz->scale, oz->scale_stride);  // reads the diagonal BEFORE it is factored
     if (eo != cudaSuccess) return eo;
     ++ctx->launches;
@@ -88,6 +98,7 @@ cudaError_t chol_factor_stream(lmm_ctx* ctx, cudaStream_t st, TiledSym L, double
   bool factored_ahead = false;  // diagonal tile jj was factored by the previous column's fused chain launch
   for (int s0 = 0; s0 < nt; s0 += ob) {
     const int s1 = (s0 + ob < nt) ? s0 + ob : nt;
+    unsigned long long sliced = 0;  // bit jj - s0: the digit planes of column jj below the block are written
     if (s0 > 0) {
       const int r0 = s0 > jstart ? s0 : jstart;  // first tile row that still has to be computed
       const int nr = rows(r0, s0);  // tile (I, J) has products with two nonzero operands iff env[I] < s0 and env[J] < s0
@@ -157,17 +168,37 @@ cudaError_t chol_factor_stream(lmm_ctx* ctx, cudaStream_t st, TiledSym L, double
         continue;
       }
       const int nr = rows(t0, jj + 1);
-      if (nr <= 0) continue;
+      if (nr <= 0) {
+        sliced |= 1ull << (jj - s0);  // no tile of the column below the block is inside the envelope
+        continue;
+      }
       g.i0 = t0; g.j0 = jj;
-      if ((e = launch_gemm(st, GEMM_TRSM, g, 1, nr, batch, (long long)(nt - t0) * batch)) != cudaSuccess) return e;
+      const long long sel = (long long)(nt - t0) * batch;
+      if (oz && ctx->trsm_slice && !gemm_takes_direct(sel)) {
+        // the TRSM writes the digit planes of the tiles below the block itself (rows in [t0, s1) are updated again in the block)
+        const TrsmSliceArgs sa{oz->scale, oz->scale_stride, oz->slices, oz->slice_stride, oz->fp, oz->fp_stride, oz->S, oz->bits, s1};
+        if ((e = launch_trsm_slice(st, g, nr, batch, sa)) != cudaSuccess) return e;
+        sliced |= 1ull << (jj - s0);
+      } else if ((e = launch_gemm(st, GEMM_TRSM, g, 1, nr, batch, sel)) != cudaSuccess) {
+        return e;
+      }
       ++ctx->launches;
     }
     const int ns = oz && s1 < nt ? rows(s1, s1) : 0;
-    if (ns > 0) {  // the block column is final: digit planes of its tiles below the block, for the later wide updates
-      if ((e = launch_ozaki_slice(st, L, oz->scale, oz->scale_stride, oz->slices, oz->slice_stride, s1, ns, s0, s1 - s0, batch, oz->S, oz->bits,
+    // the block column is final: digit planes of its tiles below the block, for the later wide updates -- for the runs of columns
+    // whose TRSM did not write them (direct kernels, fused chain)
+    for (int c0 = s0; ns > 0 && c0 < s1;) {
+      if (sliced >> (c0 - s0) & 1) {
+        ++c0;
+        continue;
+      }
+      int c1 = c0 + 1;
+      while (c1 < s1 && !(sliced >> (c1 - s0) & 1)) ++c1;
+      if ((e = launch_ozaki_slice(st, L, oz->scale, oz->scale_stride, oz->slices, oz->slice_stride, s1, ns, c0, c1 - c0, batch, oz->S, oz->bits,
                                   env_d, oz->fp, oz->fp_stride)) != cudaSuccess)
         return e;
       ++ctx->launches;
+      c0 = c1;
     }
   }
   return cudaSuccess;

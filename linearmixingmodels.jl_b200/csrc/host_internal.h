@@ -91,6 +91,8 @@ struct lmm_ctx {
   double oz_tile_products = 0.0;
   int ozaki_single_nt = 96;   // batch <= 2: use the batched schedule (and with it the int8 update) from this many tile rows on (0 = never)
   int ozaki_min_k = 4;        // wide updates over fewer k-tiles stay on DMMA (the int8 epilogue is per output tile, not per k)
+  int trsm_slice = 1;         // 1: the panel TRSMs of the int8 Cholesky write the digit planes of the tiles they finish; 0: a
+                              // separate slice launch per block column (the same bytes)
   void* oz_slices = nullptr;  // [latents in flight][sym_tiles][S * 16 KB], grown on demand
   size_t oz_slices_bytes = 0;
   void* oz_x = nullptr;       // prediction sweep: digit planes + row scales of X

@@ -69,6 +69,20 @@ enum { GEMM_UPDATE = 0, GEMM_TRSM = 1 };
 // orders; a grid trimmed to the envelope keeps the kernel, and so the bits, of the full grid)
 cudaError_t launch_gemm(cudaStream_t st, int mode, const GemmArgs& a, int ncols, int nrows, int batch, long long select_tiles = 0);
 void set_gemm_small_threshold(int tiles);  // grids of <= tiles tiles use the latency-optimised direct kernel (default 74; 0 = off)
+bool gemm_takes_direct(long long tiles);  // a grid of that many tiles takes the direct kernel (launch_gemm's choice)
+// Digit planes written by the panel TRSM of the int8 Cholesky: the finished tiles (I, J) with I >= i0 are sliced as launch_ozaki_slice
+// slices them (same digits, first-plane bytes, planes skipped for all-zero tiles)
+struct TrsmSliceArgs {
+  const double* scale;  // [batch][scale_stride]: row scales 2^(E - 6)
+  size_t scale_stride;
+  uint8_t* slices;      // [batch][slice_stride] bytes, packed-lower tile order, S * 16 KB per tile
+  size_t slice_stride;
+  uint8_t* fp;          // nullable: first plane with a nonzero digit per tile [batch][fp_stride]
+  size_t fp_stride;
+  int S, bits, i0;
+};
+// TRSM of column a.j0, tile rows [a.i0, a.i0 + nrows), on the TMA-pipelined kernel whatever the grid size, with the digit planes
+cudaError_t launch_trsm_slice(cudaStream_t st, const GemmArgs& a, int nrows, int batch, const TrsmSliceArgs& s);
 void set_pdl(int v);       // 1: programmatic dependent launch along the batch-1 panel chain (default 1)
 bool pdl_enabled();
 
