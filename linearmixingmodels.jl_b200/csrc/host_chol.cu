@@ -4,6 +4,66 @@
 
 namespace lmm_host {
 
+// ---- device buffers and streams of the schedules ----------------------------------------------------------------------------------
+// Grow-on-demand device buffer (p, bytes) of the context: afterwards it holds at least `need` bytes, or nothing and the error is
+// returned (not cleared: the callers that fall back to the DMMA path clear it).  sync: the old buffer may still be in use by work
+// queued earlier on ctx->stream.  unit > 0: `need` is an upper bound and the buffer takes as many whole units of it as fit with
+// `reserve` bytes left free (room for the caller's later allocations).
+template <class T>
+static cudaError_t grow_buffer(lmm_ctx* ctx, T*& p, size_t& bytes, size_t need, bool sync, size_t unit = 0, size_t reserve = 0) {
+  if (bytes >= need) return cudaSuccess;
+  if (sync) cudaStreamSynchronize(ctx->stream);
+  if (p) cudaFree(p);
+  p = nullptr;
+  bytes = 0;
+  cudaError_t e;
+  if (unit) {
+    size_t free_b = 0, total_b = 0;
+    if ((e = cudaMemGetInfo(&free_b, &total_b)) != cudaSuccess) return e;
+    const size_t fit = free_b > reserve ? (free_b - reserve) / unit * unit : 0;
+    if (fit == 0) return cudaErrorMemoryAllocation;
+    if (fit < need) need = fit;
+  }
+  if ((e = cudaMalloc((void**)&p, need)) == cudaSuccess) bytes = need;
+  return e;
+}
+
+// At least n events in ctx->blk_ev (the per-block events of the two-stream schedules).
+static cudaError_t block_events(lmm_ctx* ctx, int n) {
+  while ((int)ctx->blk_ev.size() < n) {
+    cudaEvent_t ev;
+    const cudaError_t e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+    if (e != cudaSuccess) return e;
+    ctx->blk_ev.push_back(ev);
+  }
+  return cudaSuccess;
+}
+
+// fork: the streams s[0, n) wait for the work queued so far on ctx->stream; join: ctx->stream waits for the work queued on them.
+static cudaError_t fork_streams(lmm_ctx* ctx, const cudaStream_t* s, int n) {
+  cudaError_t e = cudaEventRecord(ctx->ev_fork, ctx->stream);
+  for (int i = 0; e == cudaSuccess && i < n; ++i) e = cudaStreamWaitEvent(s[i], ctx->ev_fork, 0);
+  return e;
+}
+static cudaError_t join_streams(lmm_ctx* ctx, const cudaStream_t* s, int n) {
+  cudaError_t e = cudaSuccess;
+  for (int i = 0; e == cudaSuccess && i < n; ++i)
+    if ((e = cudaEventRecord(ctx->ev_join[i], s[i])) == cudaSuccess) e = cudaStreamWaitEvent(ctx->stream, ctx->ev_join[i], 0);
+  return e;
+}
+
+// run(st, b0, b1) for G latent groups [b0, b1) of the batch, each on its own stream forked from and joined back into ctx->stream;
+// G <= 1: run(ctx->stream, 0, batch).
+template <class F>
+static cudaError_t for_latent_groups(lmm_ctx* ctx, int batch, int G, F run) {
+  if (G <= 1) return run(ctx->stream, 0, batch);
+  cudaError_t e;
+  if ((e = fork_streams(ctx, ctx->gstream, G)) != cudaSuccess) return e;
+  for (int gi = 0; gi < G; ++gi)
+    if ((e = run(ctx->gstream[gi], (int)((int64_t)batch * gi / G), (int)((int64_t)batch * (gi + 1) / G))) != cudaSuccess) return e;
+  return join_streams(ctx, ctx->gstream, G);
+}
+
 // ---- batched blocked Cholesky (left-looking over blocks of `outer_block` tile columns) -------
 // For every block column [s0, s1): one wide trailing update against all previous columns
 // (K = s0 tiles, output written once), then per tile column: narrow update inside the block,
@@ -16,14 +76,8 @@ namespace lmm_host {
 // a context-owned buffer, zeroed on `st` (every column of a factorisation uses its own entries).
 static cudaError_t chain_counters(lmm_ctx* ctx, cudaStream_t st, int nt, int batch, int** out) {
   const size_t need = (size_t)batch * chain_counter_ints(nt) * sizeof(int);
-  if (ctx->chain_cnt_bytes < need) {
-    if (ctx->chain_cnt) cudaFree(ctx->chain_cnt);
-    ctx->chain_cnt = nullptr;
-    ctx->chain_cnt_bytes = 0;
-    cudaError_t e = cudaMalloc(&ctx->chain_cnt, need);
-    if (e != cudaSuccess) return e;
-    ctx->chain_cnt_bytes = need;
-  }
+  const cudaError_t e = grow_buffer(ctx, ctx->chain_cnt, ctx->chain_cnt_bytes, need, false);
+  if (e != cudaSuccess) return e;
   *out = (int*)ctx->chain_cnt;
   return cudaMemsetAsync(ctx->chain_cnt, 0, need, st);
 }
@@ -35,16 +89,11 @@ constexpr int CHAIN_MAX_TILES = 96;
 // Enveloped factors of at least this many tile rows take block width 1 under the int8 update (see chol_factor_stream).
 constexpr int OZ_WIDTH1_MIN_NT = 64;
 
-// Workspace of the optional integer-slice (Ozaki) trailing update for the latents [0, batch) of one chol_factor_stream call.
-struct OzWs {
-  uint8_t* slices;
-  size_t slice_stride;  // bytes per latent
-  double* scale;
-  size_t scale_stride;  // doubles per latent
-  uint8_t* fp;          // first digit plane with a nonzero digit of each sliced tile (S: all zero), written by the slice kernel
-  size_t fp_stride;     // bytes per latent (sym_tiles)
-  int S, min_k, bits;  // digit planes, smallest K (k-tiles) the int8 update takes, bits per digit (7: radix 128, 8: radix 256)
-};
+// A wide update over k k-tiles runs on the int8 tensor cores: it takes at least ozaki_min_k k-tiles, and the int32 accumulation
+// is exact: (pairs per accumulator <= S) * K * (largest digit)^2 < 2^31.
+static bool ozaki_wide(const lmm_ctx* ctx, const DigitPlanes& p, int k) {
+  return k >= ctx->ozaki_min_k && (long long)k * TILE * p.S * (p.bits == 8 ? 16384 : 4096) < (1ll << 31);
+}
 
 // Tile envelope (env_h: host copy, [batch][nt]; L(I,k) = 0 for k < env[b][I]): the last tile row >= r0 that some latent of the
 // batch has inside its envelope for the columns < lim (env[b][I] < lim); r0 - 1 when there is none.  Grids end there; the rows
@@ -60,15 +109,46 @@ static int env_last_row(const int* env_h, int nt, int batch, int r0, int lim) {
   return last;
 }
 
+// The wide int8 update of chol_factor_stream: the columns [s0, s1), tile rows [r0, r0 + nr), by the k-tiles [0, s0).  With
+// "ozaki_time" CUDA events around the launch, and its 128^3 tile products added to oz_tile_products: tiles (I, J), I >= J, times
+// their k-tiles (s0, or from the later envelope on).  Nominal: the kernel skips the k-tiles whose digit products are all zero
+// (first_plane), which no host count sees.
+static cudaError_t ozaki_wide_update(lmm_ctx* ctx, cudaStream_t st, TiledSym L, const DigitPlanes& p, int r0, int nr, int s0, int s1,
+                                     int batch, const int* env_d, const int* env_h) {
+  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+  if (ctx->ozaki_time && cudaEventCreate(&ev0) == cudaSuccess && cudaEventCreate(&ev1) == cudaSuccess) cudaEventRecord(ev0, st);
+  const cudaError_t e = launch_ozaki_update(st, L, p, r0, nr, s0, s1 - s0, s0, batch, env_d);
+  if (!ev0 || !ev1) return e;
+  cudaEventRecord(ev1, st);
+  ctx->oz_events.push_back(ev0);
+  ctx->oz_events.push_back(ev1);
+  double tp = 0.0;
+  for (int J = s0; J < s1; ++J)
+    for (int I = J > r0 ? J : r0; I < r0 + nr; ++I) {
+      if (!env_h) {
+        tp += (double)s0 * batch;
+        continue;
+      }
+      for (int b = 0; b < batch; ++b) {
+        const int* eb = env_h + (size_t)b * L.nt;
+        const int kb = eb[I] > eb[J] ? eb[I] : eb[J];
+        if (kb < s0) tp += (double)(s0 - kb);
+      }
+    }
+  ctx->oz_tile_products += tp;
+  return e;
+}
+
+// oz (nullable): the digit-plane workspace of the latents [0, batch) for the optional integer-slice (Ozaki) trailing update.
 cudaError_t chol_factor_stream(lmm_ctx* ctx, cudaStream_t st, TiledSym L, double* W, size_t wstride, int batch, double* logdet,
-                               int* info, int jstart = 0, int* counters = nullptr, const OzWs* oz = nullptr, const int* env_d = nullptr,
+                               int* info, int jstart = 0, int* counters = nullptr, const DigitPlanes* oz = nullptr, const int* env_d = nullptr,
                                const int* env_h = nullptr) {
   const int nt = L.nt;
   if (jstart != 0 || !env_h) env_d = env_h = nullptr;
   // tile rows of a launch whose first row is r0: all of them, or up to the last one inside some latent's envelope (see above)
   auto rows = [&](int r0, int lim) { return (env_h ? env_last_row(env_h, nt, batch, r0, lim) + 1 : nt) - r0; };
   int ob = ctx->outer_block;
-  if (oz && (jstart != 0 || nt <= ob || nt < oz->min_k + 1)) oz = nullptr;  // no wide update this scheme would take
+  if (oz && (jstart != 0 || nt <= ob || nt < ctx->ozaki_min_k + 1)) oz = nullptr;  // no wide update this scheme would take
   if (oz) {
     // narrow blocks: the in-block updates stay on DMMA, so the narrower the block the less of the work is left at the FP64 rate
     // (measured at 16 / 8 latents of N = 16384, final kernel: ob = 4: 286.8 / 147.5 ms, ob = 2 with min_k = 4: 275.5 / 143.1,
@@ -81,7 +161,8 @@ cudaError_t chol_factor_stream(lmm_ctx* ctx, cudaStream_t st, TiledSym L, double
     // with at those sizes; the rule is conservative, not a measured crossover.  No fused panel chain (jj + 1 < s1) at width 1:
     // the last columns' TRSMs take the direct kernels once their grids are small.
     if (!ctx->outer_block_user) ob = env_h && nt >= OZ_WIDTH1_MIN_NT ? 1 : 2;
-    cudaError_t eo = launch_ozaki_scales(st, L, batch, oz->scale, oz->scale_stride);  // reads the diagonal BEFORE it is factored
+    // reads the diagonal BEFORE it is factored
+    cudaError_t eo = launch_ozaki_scales(st, L, batch, const_cast<double*>(oz->scale), oz->scale_stride);
     if (eo != cudaSuccess) return eo;
     ++ctx->launches;
   }
@@ -104,35 +185,8 @@ cudaError_t chol_factor_stream(lmm_ctx* ctx, cudaStream_t st, TiledSym L, double
       const int nr = rows(r0, s0);  // tile (I, J) has products with two nonzero operands iff env[I] < s0 and env[J] < s0
       g.i0 = r0; g.j0 = s0; g.k0 = 0; g.k1 = s0;
       e = cudaSuccess;
-      // exact int32 accumulation: (pairs per accumulator <= S) * K * (largest digit)^2 < 2^31
-      if (oz && s0 >= oz->min_k && (long long)s0 * TILE * oz->S * (oz->bits == 8 ? 16384 : 4096) < (1ll << 31)) {
-        if (nr > 0) {
-          cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-          if (ctx->ozaki_time && cudaEventCreate(&ev0) == cudaSuccess && cudaEventCreate(&ev1) == cudaSuccess) cudaEventRecord(ev0, st);
-          e = launch_ozaki_update(st, L, oz->slices, oz->slice_stride, oz->scale, oz->scale_stride, r0, nr, s0, s1 - s0, s0, batch, oz->S, oz->bits,
-                                  env_d, oz->fp, oz->fp_stride);
-          if (ev0 && ev1) {
-            cudaEventRecord(ev1, st);
-            ctx->oz_events.push_back(ev0);
-            ctx->oz_events.push_back(ev1);
-            // 128^3 tile products in this launch's envelope: tiles (I, J), I >= J, times their k-tiles (s0, or from the later envelope
-            // on).  Nominal: the kernel skips the k-tiles whose digit products are all zero (first_plane), which no host count sees.
-            double tp = 0.0;
-            for (int J = s0; J < s1; ++J)
-              for (int I = J > r0 ? J : r0; I < r0 + nr; ++I) {
-                if (!env_h) {
-                  tp += (double)s0 * batch;
-                  continue;
-                }
-                for (int b = 0; b < batch; ++b) {
-                  const int* eb = env_h + (size_t)b * nt;
-                  const int kb = eb[I] > eb[J] ? eb[I] : eb[J];
-                  if (kb < s0) tp += (double)(s0 - kb);
-                }
-              }
-            ctx->oz_tile_products += tp;
-          }
-        }
+      if (oz && ozaki_wide(ctx, *oz, s0)) {
+        if (nr > 0) e = ozaki_wide_update(ctx, st, L, *oz, r0, nr, s0, s1, batch, env_d, env_h);
       } else if (nr > 0) {
         e = launch_gemm(st, GEMM_UPDATE, g, s1 - s0, nr, batch, (long long)(s1 - s0) * (nt - r0) * batch);
       }
@@ -176,8 +230,7 @@ cudaError_t chol_factor_stream(lmm_ctx* ctx, cudaStream_t st, TiledSym L, double
       const long long sel = (long long)(nt - t0) * batch;
       if (oz && ctx->trsm_slice && !gemm_takes_direct(sel)) {
         // the TRSM writes the digit planes of the tiles below the block itself (rows in [t0, s1) are updated again in the block)
-        const TrsmSliceArgs sa{oz->scale, oz->scale_stride, oz->slices, oz->slice_stride, oz->fp, oz->fp_stride, oz->S, oz->bits, s1};
-        if ((e = launch_trsm_slice(st, g, nr, batch, sa)) != cudaSuccess) return e;
+        if ((e = launch_trsm_slice(st, g, nr, batch, TrsmSliceArgs{*oz, s1})) != cudaSuccess) return e;
         sliced |= 1ull << (jj - s0);
       } else if ((e = launch_gemm(st, GEMM_TRSM, g, 1, nr, batch, sel)) != cudaSuccess) {
         return e;
@@ -194,9 +247,7 @@ cudaError_t chol_factor_stream(lmm_ctx* ctx, cudaStream_t st, TiledSym L, double
       }
       int c1 = c0 + 1;
       while (c1 < s1 && !(sliced >> (c1 - s0) & 1)) ++c1;
-      if ((e = launch_ozaki_slice(st, L, oz->scale, oz->scale_stride, oz->slices, oz->slice_stride, s1, ns, c0, c1 - c0, batch, oz->S, oz->bits,
-                                  env_d, oz->fp, oz->fp_stride)) != cudaSuccess)
-        return e;
+      if ((e = launch_ozaki_slice(st, L, *oz, s1, ns, c0, c1 - c0, batch, env_d)) != cudaSuccess) return e;
       ++ctx->launches;
       c0 = c1;
     }
@@ -206,52 +257,21 @@ cudaError_t chol_factor_stream(lmm_ctx* ctx, cudaStream_t st, TiledSym L, double
 
 // Grow the context's Ozaki workspace for up to `batch` latents of nt tile rows; returns how many latents fit (0: none -- stay on
 // DMMA).  One cudaMemGetInfo / cudaMalloc when the shape grows, nothing afterwards.
-static int ozaki_workspace(lmm_ctx* ctx, int nt, int batch, OzWs& ws) {
-  const size_t per_slices = sym_tiles(nt) * (size_t)ctx->ozaki * 16384, per_scale = (size_t)nt * TILE;
-  size_t have = per_slices ? ctx->oz_slices_bytes / per_slices : 0;
-  if (have < (size_t)batch) {
-    cudaStreamSynchronize(ctx->stream);  // the old buffer may still be in use by work queued earlier
-    if (ctx->oz_slices) cudaFree(ctx->oz_slices);
-    ctx->oz_slices = nullptr;
-    ctx->oz_slices_bytes = 0;
-    size_t free_b = 0, total_b = 0;
-    if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess) return 0;
-    const size_t reserve = (size_t)6 << 30;  // leave room for the caller's later allocations (solves, predictions)
-    size_t fit = free_b > reserve ? (free_b - reserve) / per_slices : 0;
-    if (fit > (size_t)batch) fit = (size_t)batch;
-    if (fit == 0) return 0;
-    if (cudaMalloc(&ctx->oz_slices, fit * per_slices) != cudaSuccess) {
-      cudaGetLastError();
-      return 0;
-    }
-    ctx->oz_slices_bytes = fit * per_slices;
-    have = fit;
+static int ozaki_workspace(lmm_ctx* ctx, int nt, int batch, DigitPlanes& ws) {
+  const size_t per_slices = sym_tiles(nt) * (size_t)ctx->ozaki * 16384, per_scale = (size_t)nt * TILE, per_fp = sym_tiles(nt);
+  // as many latents as fit with 6 GiB left for the caller's later allocations (solves, predictions)
+  if (grow_buffer(ctx, ctx->oz_slices, ctx->oz_slices_bytes, (size_t)batch * per_slices, true, per_slices, (size_t)6 << 30) != cudaSuccess) {
+    cudaGetLastError();
+    return 0;
   }
+  size_t have = ctx->oz_slices_bytes / per_slices;
   if (have > (size_t)batch) have = (size_t)batch;
-  if (ctx->oz_scale_bytes < have * per_scale * sizeof(double)) {
-    cudaStreamSynchronize(ctx->stream);
-    if (ctx->oz_scale) cudaFree(ctx->oz_scale);
-    ctx->oz_scale = nullptr;
-    ctx->oz_scale_bytes = 0;
-    if (cudaMalloc(&ctx->oz_scale, have * per_scale * sizeof(double)) != cudaSuccess) {
-      cudaGetLastError();
-      return 0;
-    }
-    ctx->oz_scale_bytes = have * per_scale * sizeof(double);
+  if (grow_buffer(ctx, ctx->oz_scale, ctx->oz_scale_bytes, have * per_scale * sizeof(double), true) != cudaSuccess ||
+      grow_buffer(ctx, ctx->oz_fp, ctx->oz_fp_bytes, have * per_fp, true) != cudaSuccess) {
+    cudaGetLastError();
+    return 0;
   }
-  const size_t per_fp = sym_tiles(nt);
-  if (ctx->oz_fp_bytes < have * per_fp) {
-    cudaStreamSynchronize(ctx->stream);
-    if (ctx->oz_fp) cudaFree(ctx->oz_fp);
-    ctx->oz_fp = nullptr;
-    ctx->oz_fp_bytes = 0;
-    if (cudaMalloc(&ctx->oz_fp, have * per_fp) != cudaSuccess) {
-      cudaGetLastError();
-      return 0;
-    }
-    ctx->oz_fp_bytes = have * per_fp;
-  }
-  ws = OzWs{(uint8_t*)ctx->oz_slices, per_slices, ctx->oz_scale, per_scale, ctx->oz_fp, per_fp, ctx->ozaki, ctx->ozaki_min_k, ctx->ozaki_bits};
+  ws = DigitPlanes{ctx->oz_scale, per_scale, (uint8_t*)ctx->oz_slices, per_slices, ctx->oz_fp, per_fp, ctx->ozaki, ctx->ozaki_bits};
   return (int)have;
 }
 
@@ -301,12 +321,9 @@ cudaError_t chol_factor_rightlooking(lmm_ctx* ctx, TiledSym L, double* W, size_t
   const int ob = ctx->outer_block_user ? ctx->outer_block : fused_all ? (nt <= 112 ? 3 : 4) : (nt <= 32 ? 1 : nt <= 48 ? 2 : nt <= 112 ? 3 : 4);
   const int nblk = (nt + ob - 1) / ob;
   cudaError_t e;
-  while ((int)ctx->blk_ev.size() < 2 * nblk + 2) {
-    cudaEvent_t ev;
-    if ((e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming)) != cudaSuccess) return e;
-    ctx->blk_ev.push_back(ev);
-  }
-  cudaStream_t X = ctx->panel_stream, Y = ctx->update_stream;
+  if ((e = block_events(ctx, 2 * nblk + 2)) != cudaSuccess) return e;
+  const cudaStream_t XY[2] = {ctx->panel_stream, ctx->update_stream};
+  const cudaStream_t X = XY[0], Y = XY[1];
   cudaEvent_t* evX = ctx->blk_ev.data();          // panel(b) done on X
   cudaEvent_t* evY = ctx->blk_ev.data() + nblk;   // trailing update from block b done on Y
   GemmArgs g{};
@@ -314,9 +331,7 @@ cudaError_t chol_factor_rightlooking(lmm_ctx* ctx, TiledSym L, double* W, size_t
   g.W = W; g.w_batch_stride = wstride; g.sym = 1;
   int* counters = nullptr;
   if (fused && (e = chain_counters(ctx, ctx->stream, nt, batch, &counters)) != cudaSuccess) return e;
-  if ((e = cudaEventRecord(ctx->ev_fork, ctx->stream)) != cudaSuccess) return e;
-  if ((e = cudaStreamWaitEvent(X, ctx->ev_fork, 0)) != cudaSuccess) return e;
-  if ((e = cudaStreamWaitEvent(Y, ctx->ev_fork, 0)) != cudaSuccess) return e;
+  if ((e = fork_streams(ctx, XY, 2)) != cudaSuccess) return e;
   bool factored_ahead = false;  // the block's first diagonal tile was factored by the previous block's boundary launch
   for (int b = 0; b < nblk; ++b) {
     const int s0 = b * ob, s1 = (s0 + ob < nt) ? s0 + ob : nt;
@@ -363,10 +378,7 @@ cudaError_t chol_factor_rightlooking(lmm_ctx* ctx, TiledSym L, double* W, size_t
     }
     if ((e = cudaEventRecord(evY[b], Y)) != cudaSuccess) return e;
   }
-  if ((e = cudaStreamWaitEvent(ctx->stream, evX[nblk - 1], 0)) != cudaSuccess) return e;
-  if ((e = cudaEventRecord(ctx->ev_join[0], Y)) != cudaSuccess) return e;
-  if ((e = cudaStreamWaitEvent(ctx->stream, ctx->ev_join[0], 0)) != cudaSuccess) return e;
-  return cudaSuccess;
+  return join_streams(ctx, XY, 2);
 }
 
 // Row-cyclic multi-GPU factorisation of ONE large matrix (north star: "ILMM runs on one GPU unless its blocked
@@ -382,24 +394,15 @@ cudaError_t chol_factor_rowcyclic(lmm_ctx* ctx, TiledSym L, double* W, size_t ws
   const int ob = ctx->outer_block_user ? ctx->outer_block : (nt <= 72 ? 2 : nt <= 112 ? 3 : 4);
   const int nblk = (nt + ob - 1) / ob;
   cudaError_t e;
-  while ((int)ctx->blk_ev.size() < 2 * nblk + 2) {
-    cudaEvent_t ev;
-    if ((e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming)) != cudaSuccess) return e;
-    ctx->blk_ev.push_back(ev);
-  }
+  if ((e = block_events(ctx, 2 * nblk + 2)) != cudaSuccess) return e;
   // exchange buffers: [send: slots*ob tiles][recv: G*slots*ob tiles], sized for the first (largest) exchange
   const int max_slots = (nt + G - 1) / G;
   const size_t send_elems = (size_t)max_slots * ob * TT, need = (send_elems * (size_t)(G + 1)) * sizeof(double);
-  if (ctx->xbuf_bytes < need) {
-    if (ctx->xbuf) cudaFree(ctx->xbuf);
-    ctx->xbuf = nullptr;
-    ctx->xbuf_bytes = 0;
-    if ((e = cudaMalloc(&ctx->xbuf, need)) != cudaSuccess) return e;
-    ctx->xbuf_bytes = need;
-  }
+  if ((e = grow_buffer(ctx, ctx->xbuf, ctx->xbuf_bytes, need, false)) != cudaSuccess) return e;
   double* sendb = (double*)ctx->xbuf;
   double* recvb = sendb + send_elems;
-  cudaStream_t X = ctx->panel_stream, Y = ctx->update_stream;
+  const cudaStream_t XY[2] = {ctx->panel_stream, ctx->update_stream};
+  const cudaStream_t X = XY[0], Y = XY[1];
   cudaEvent_t* evX = ctx->blk_ev.data();
   cudaEvent_t* evY = ctx->blk_ev.data() + nblk;
   GemmArgs g{};
@@ -409,9 +412,7 @@ cudaError_t chol_factor_rowcyclic(lmm_ctx* ctx, TiledSym L, double* W, size_t ws
   auto own_count = [&](int s) { const int f = first_own(s); return f >= nt ? 0 : (nt - 1 - f) / G + 1; };
   int* counters = nullptr;
   if (ctx->chain_fused && (e = chain_counters(ctx, ctx->stream, nt, 1, &counters)) != cudaSuccess) return e;
-  if ((e = cudaEventRecord(ctx->ev_fork, ctx->stream)) != cudaSuccess) return e;
-  if ((e = cudaStreamWaitEvent(X, ctx->ev_fork, 0)) != cudaSuccess) return e;
-  if ((e = cudaStreamWaitEvent(Y, ctx->ev_fork, 0)) != cudaSuccess) return e;
+  if ((e = fork_streams(ctx, XY, 2)) != cudaSuccess) return e;
   for (int b = 0; b < nblk; ++b) {
     const int s0 = b * ob, s1 = (s0 + ob < nt) ? s0 + ob : nt;
     if (b >= 1) {
@@ -470,10 +471,7 @@ cudaError_t chol_factor_rowcyclic(lmm_ctx* ctx, TiledSym L, double* W, size_t ws
     }
     if ((e = cudaEventRecord(evY[b], Y)) != cudaSuccess) return e;
   }
-  if ((e = cudaStreamWaitEvent(ctx->stream, evX[nblk - 1], 0)) != cudaSuccess) return e;
-  if ((e = cudaEventRecord(ctx->ev_join[0], Y)) != cudaSuccess) return e;
-  if ((e = cudaStreamWaitEvent(ctx->stream, ctx->ev_join[0], 0)) != cudaSuccess) return e;
-  return cudaSuccess;
+  return join_streams(ctx, XY, 2);
 }
 
 // Row-cyclic factorisation with DISTRIBUTED STORAGE (VERDICT r01 next #8): rank r holds only the tile rows I = r (mod G) of
@@ -502,25 +500,16 @@ cudaError_t chol_factor_rowcyclic_dist(lmm_ctx* ctx, TiledSym Lown, int nrows, i
   const int ob = rowcyclic_dist_block(ctx, nc);
   const int nblk = (nc + ob - 1) / ob;
   cudaError_t e;
-  while ((int)ctx->blk_ev.size() < 2 * nblk + 2) {
-    cudaEvent_t ev;
-    if ((e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming)) != cudaSuccess) return e;
-    ctx->blk_ev.push_back(ev);
-  }
+  if ((e = block_events(ctx, 2 * nblk + 2)) != cudaSuccess) return e;
   const int max_slots = (nrows + G - 1) / G;
   const size_t send_elems = (size_t)max_slots * ob * TT, win_elems = (size_t)nrows * ob * TT;
   const size_t need = rowcyclic_dist_workspace_tiles(nrows, G, ob) * TT * sizeof(double);
-  if (ctx->xbuf_bytes < need) {
-    if (ctx->xbuf) cudaFree(ctx->xbuf);
-    ctx->xbuf = nullptr;
-    ctx->xbuf_bytes = 0;
-    if ((e = cudaMalloc(&ctx->xbuf, need)) != cudaSuccess) return e;
-    ctx->xbuf_bytes = need;
-  }
+  if ((e = grow_buffer(ctx, ctx->xbuf, ctx->xbuf_bytes, need, false)) != cudaSuccess) return e;
   double* sendb = (double*)ctx->xbuf;
   double* recvb = sendb + send_elems;
   double* win[2] = {recvb + send_elems * (size_t)G, recvb + send_elems * (size_t)G + win_elems};
-  cudaStream_t X = ctx->panel_stream, Y = ctx->update_stream;
+  const cudaStream_t XY[2] = {ctx->panel_stream, ctx->update_stream};
+  const cudaStream_t X = XY[0], Y = XY[1];
   cudaEvent_t* evX = ctx->blk_ev.data();
   cudaEvent_t* evY = ctx->blk_ev.data() + nblk;
   auto first_own = [&](int s) { return s + (((me - s % G) % G) + G) % G; };
@@ -532,9 +521,7 @@ cudaError_t chol_factor_rowcyclic_dist(lmm_ctx* ctx, TiledSym Lown, int nrows, i
   };
   int* counters = nullptr;
   if (ctx->chain_fused && (e = chain_counters(ctx, ctx->stream, nrows, 1, &counters)) != cudaSuccess) return e;
-  if ((e = cudaEventRecord(ctx->ev_fork, ctx->stream)) != cudaSuccess) return e;
-  if ((e = cudaStreamWaitEvent(X, ctx->ev_fork, 0)) != cudaSuccess) return e;
-  if ((e = cudaStreamWaitEvent(Y, ctx->ev_fork, 0)) != cudaSuccess) return e;
+  if ((e = fork_streams(ctx, XY, 2)) != cudaSuccess) return e;
   GemmArgs g{};
   g.W = W; g.w_batch_stride = wstride; g.sym = 1;
   for (int b = 0; b < nblk; ++b) {
@@ -611,11 +598,7 @@ cudaError_t chol_factor_rowcyclic_dist(lmm_ctx* ctx, TiledSym Lown, int nrows, i
       ++ctx->launches;
     }
   }
-  if ((e = cudaEventRecord(ctx->ev_join[1], X)) != cudaSuccess) return e;
-  if ((e = cudaStreamWaitEvent(ctx->stream, ctx->ev_join[1], 0)) != cudaSuccess) return e;
-  if ((e = cudaEventRecord(ctx->ev_join[0], Y)) != cudaSuccess) return e;
-  if ((e = cudaStreamWaitEvent(ctx->stream, ctx->ev_join[0], 0)) != cudaSuccess) return e;
-  return cudaSuccess;
+  return join_streams(ctx, XY, 2);
 }
 
 // Fork the batch into latent groups on separate streams (joined back into ctx->stream).  jstart > 0: extend a factor whose
@@ -635,7 +618,6 @@ bool chol_takes_envelope(const lmm_ctx* ctx, int nt, int batch) { return !use_ro
 
 cudaError_t chol_factor(lmm_ctx* ctx, TiledSym L, double* W, size_t wstride, int batch, double* logdet, int* info, int jstart,
                         const int* env_d, const int* env_h) {
-  const int G = ctx->ngroups < batch ? ctx->ngroups : batch;
   if (!env_d || !env_h) env_d = env_h = nullptr;
   auto env_at = [&](const int* e, int b0) { return e ? e + (size_t)b0 * L.nt : nullptr; };
   if (jstart == 0) {  // the look-ahead / partitioned schedules factor from scratch only
@@ -652,8 +634,8 @@ cudaError_t chol_factor(lmm_ctx* ctx, TiledSym L, double* W, size_t wstride, int
   }
   cudaError_t e;
   // optional integer-slice trailing update: workspace for as many latents as fit; a larger batch is factored in chunks
-  OzWs ozws{};
-  const OzWs* oz = nullptr;
+  DigitPlanes ozws{};
+  const DigitPlanes* oz = nullptr;
   if (ctx->ozaki && jstart == 0 && L.nt > ctx->outer_block && L.nt > ctx->ozaki_min_k && L.ntc == 0 && L.cyc_G == 0) {
     const int fit = ozaki_workspace(ctx, L.nt, batch, ozws);
     if (fit > 0) {
@@ -670,45 +652,28 @@ cudaError_t chol_factor(lmm_ctx* ctx, TiledSym L, double* W, size_t wstride, int
       }
     }
   }
-  auto oz_at = [&](int b0, OzWs& tmp) -> const OzWs* {
-    if (!oz) return nullptr;
-    tmp = *oz;
-    tmp.slices += (size_t)b0 * oz->slice_stride;
-    tmp.scale += (size_t)b0 * oz->scale_stride;
-    tmp.fp += (size_t)b0 * oz->fp_stride;
-    return &tmp;
-  };
   // small grids (few latents x few tile rows, e.g. the reference's notebook shape: 20 latents, 5 tile columns): ONE stream,
   // one fused launch per tile column -- stream groups would only multiply the launches
   int* counters = nullptr;
   const bool chain_all = ctx->chain_fused && (long long)(L.nt - 1) * batch <= CHAIN_MAX_TILES && L.nt > 1;
   if (ctx->chain_fused && L.nt > 1 && (e = chain_counters(ctx, ctx->stream, L.nt, batch, &counters)) != cudaSuccess) return e;
-  if (G <= 1 || L.nt <= 1 || chain_all)
-    return chol_factor_stream(ctx, ctx->stream, L, W, wstride, batch, logdet, info, jstart, counters, oz, env_d, env_h);
-  if ((e = cudaEventRecord(ctx->ev_fork, ctx->stream)) != cudaSuccess) return e;
-  for (int gi = 0; gi < G; ++gi) {
-    const int b0 = (int)((int64_t)batch * gi / G), b1 = (int)((int64_t)batch * (gi + 1) / G);
-    cudaStream_t st = ctx->gstream[gi];
-    if ((e = cudaStreamWaitEvent(st, ctx->ev_fork, 0)) != cudaSuccess) return e;
-    TiledSym Lg{L.base + (size_t)b0 * L.batch_stride, L.nt, L.batch_stride};
-    OzWs oztmp{};
-    if ((e = chol_factor_stream(ctx, st, Lg, W + (size_t)b0 * wstride, wstride, b1 - b0, logdet + b0, info + b0, jstart,
-                                counters ? counters + (size_t)b0 * chain_counter_ints(L.nt) : nullptr, oz_at(b0, oztmp), env_at(env_d, b0),
-                                env_at(env_h, b0))) != cudaSuccess)
-      return e;
-    if ((e = cudaEventRecord(ctx->ev_join[gi], st)) != cudaSuccess) return e;
-    if ((e = cudaStreamWaitEvent(ctx->stream, ctx->ev_join[gi], 0)) != cudaSuccess) return e;
-  }
-  return cudaSuccess;
+  const int G = L.nt <= 1 || chain_all ? 1 : ctx->ngroups < batch ? ctx->ngroups : batch;
+  return for_latent_groups(ctx, batch, G, [&](cudaStream_t st, int b0, int b1) {
+    TiledSym Lg = L;
+    Lg.base += (size_t)b0 * L.batch_stride;
+    const DigitPlanes ozg = oz ? oz->at(b0) : DigitPlanes{};
+    return chol_factor_stream(ctx, st, Lg, W + (size_t)b0 * wstride, wstride, b1 - b0, logdet + b0, info + b0, jstart,
+                              counters ? counters + (size_t)b0 * chain_counter_ints(L.nt) : nullptr, oz ? &ozg : nullptr, env_at(env_d, b0),
+                              env_at(env_h, b0));
+  });
 }
 
 // Workspace of the integer-slice path of the prediction sweep for the latents [0, batch) of one trsm_right_lt_stream call: digit planes
 // and row scales of the finished factor (right operand) and of the finished columns of X (left operand).
 struct OzPred {
-  uint8_t* lsl; size_t lsl_stride; double* lsc; size_t lsc_stride;
-  uint8_t* xsl; size_t xsl_stride; double* xsc; size_t xsc_stride;
+  DigitPlanes l, x;
   const LatentParams* params;  // kdiag = k(x*, x*) bounds the squared row norms of X = K(x*,x) L^{-T}
-  int S, bits, min_k;
+  OzPred at(int b0) const { return OzPred{l.at(b0), x.at(b0), params + b0}; }
 };
 
 // X <- X L^{-T} for a rectangular tiled X (rows = e.g. test points): the same update/TRSM sweep
@@ -723,9 +688,9 @@ cudaError_t trsm_right_lt_stream(lmm_ctx* ctx, cudaStream_t st, TiledRect X, Til
   if (oz && nt <= 8) oz = nullptr;
   if (oz) {
     if (!ctx->outer_block_user) ob = 2;
-    if ((e = launch_ozaki_factor_scales(st, L, batch, oz->lsc, oz->lsc_stride)) != cudaSuccess) return e;
-    if ((e = launch_ozaki_slice(st, L, oz->lsc, oz->lsc_stride, oz->lsl, oz->lsl_stride, 1, nt - 1, 0, nt - 1, batch, oz->S, oz->bits)) != cudaSuccess) return e;
-    if ((e = launch_ozaki_const_scales(st, oz->params, X.ntr, batch, oz->xsc, oz->xsc_stride)) != cudaSuccess) return e;
+    if ((e = launch_ozaki_factor_scales(st, L, batch, const_cast<double*>(oz->l.scale), oz->l.scale_stride)) != cudaSuccess) return e;
+    if ((e = launch_ozaki_slice(st, L, oz->l, 1, nt - 1, 0, nt - 1, batch)) != cudaSuccess) return e;
+    if ((e = launch_ozaki_const_scales(st, oz->params, X.ntr, batch, const_cast<double*>(oz->x.scale), oz->x.scale_stride)) != cudaSuccess) return e;
     ctx->launches += 3;
   }
   GemmArgs g{};
@@ -740,9 +705,8 @@ cudaError_t trsm_right_lt_stream(lmm_ctx* ctx, cudaStream_t st, TiledRect X, Til
     const int s1 = (s0 + ob < nt) ? s0 + ob : nt;
     if (s0 > 0) {
       g.j0 = s0; g.k0 = 0; g.k1 = s0;
-      if (oz && s0 >= oz->min_k && (long long)s0 * TILE * oz->S * (oz->bits == 8 ? 16384 : 4096) < (1ll << 31))
-        e = launch_ozaki_update_rect(st, X, oz->xsl, oz->xsl_stride, oz->xsc, oz->xsc_stride, oz->lsl, oz->lsl_stride, oz->lsc, oz->lsc_stride, s0,
-                                     s1 - s0, s0, batch, oz->S, oz->bits);
+      if (oz && ozaki_wide(ctx, oz->l, s0))
+        e = launch_ozaki_update_rect(st, X, oz->x, oz->l, s0, s1 - s0, s0, batch);
       else
         e = launch_gemm(st, GEMM_UPDATE, g, s1 - s0, X.ntr, batch);
       if (e != cudaSuccess) return e;
@@ -759,7 +723,7 @@ cudaError_t trsm_right_lt_stream(lmm_ctx* ctx, cudaStream_t st, TiledRect X, Til
       ++ctx->launches;
     }
     if (oz && s1 < nt) {  // the block column of X is final: its digit planes, for the later wide updates
-      if ((e = launch_ozaki_slice_rect(st, X, oz->xsc, oz->xsc_stride, oz->xsl, oz->xsl_stride, s0, s1 - s0, batch, oz->S, oz->bits)) != cudaSuccess) return e;
+      if ((e = launch_ozaki_slice_rect(st, X, oz->x, s0, s1 - s0, batch)) != cudaSuccess) return e;
       ++ctx->launches;
     }
   }
@@ -769,56 +733,30 @@ cudaError_t trsm_right_lt_stream(lmm_ctx* ctx, cudaStream_t st, TiledRect X, Til
 // `xbound` (device, one LatentParams per latent of the batch; nullable): kdiag bounds the squared row norms of the result -- what the
 // integer-slice path needs to fix the row scales of X in advance.  Without it, or with the option off, every update runs on DMMA.
 cudaError_t trsm_right_lt(lmm_ctx* ctx, TiledRect X, TiledSym L, const double* W, size_t wstride, int batch, const LatentParams* xbound) {
-  const int G = ctx->ngroups < batch ? ctx->ngroups : batch;
   OzPred oz{};
   bool use_oz = false;
-  if (ctx->ozaki && xbound && L.nt > 8 && L.ntc == 0 && L.cyc_G == 0) {
-    OzWs ws{};
-    if (ozaki_workspace(ctx, L.nt, batch, ws) >= batch) {
-      const size_t per_x = (size_t)X.ntr * X.ntc * ctx->ozaki * 16384, per_xs = (size_t)X.ntr * TILE;
-      const size_t need = (size_t)batch * (per_x + per_xs * sizeof(double));
-      if (ctx->oz_x_bytes < need) {
-        cudaStreamSynchronize(ctx->stream);
-        if (ctx->oz_x) cudaFree(ctx->oz_x);
-        ctx->oz_x = nullptr;
-        ctx->oz_x_bytes = 0;
-        size_t free_b = 0, total_b = 0;
-        if (cudaMemGetInfo(&free_b, &total_b) == cudaSuccess && free_b > need + ((size_t)4 << 30) && cudaMalloc(&ctx->oz_x, need) == cudaSuccess)
-          ctx->oz_x_bytes = need;
-        else
-          cudaGetLastError();
-      }
-      if (ctx->oz_x_bytes >= need) {
-        use_oz = true;
-        oz = OzPred{ws.slices, ws.slice_stride, ws.scale, ws.scale_stride, (uint8_t*)ctx->oz_x, per_x,
-                    (double*)((uint8_t*)ctx->oz_x + (size_t)batch * per_x), per_xs, xbound, ws.S, ws.bits, ws.min_k};
-      }
+  DigitPlanes ws{};
+  if (ctx->ozaki && xbound && L.nt > 8 && L.ntc == 0 && L.cyc_G == 0 && ozaki_workspace(ctx, L.nt, batch, ws) >= batch) {
+    const size_t per_x = (size_t)X.ntr * X.ntc * ctx->ozaki * 16384, per_xs = (size_t)X.ntr * TILE;
+    const size_t need = (size_t)batch * (per_x + per_xs * sizeof(double));
+    if (grow_buffer(ctx, ctx->oz_x, ctx->oz_x_bytes, need, true, need, (size_t)4 << 30) != cudaSuccess) cudaGetLastError();
+    if (ctx->oz_x_bytes >= need) {
+      use_oz = true;
+      oz.l = ws;
+      oz.l.fp = nullptr;  // the factor is sliced whole: every tile's planes are written
+      oz.l.fp_stride = 0;
+      oz.x = DigitPlanes{(double*)((uint8_t*)ctx->oz_x + (size_t)batch * per_x), per_xs, (uint8_t*)ctx->oz_x, per_x, nullptr, 0, ws.S, ws.bits};
+      oz.params = xbound;
     }
   }
-  auto oz_at = [&](int b0, OzPred& tmp) -> const OzPred* {
-    if (!use_oz) return nullptr;
-    tmp = oz;
-    tmp.lsl += (size_t)b0 * oz.lsl_stride; tmp.lsc += (size_t)b0 * oz.lsc_stride;
-    tmp.xsl += (size_t)b0 * oz.xsl_stride; tmp.xsc += (size_t)b0 * oz.xsc_stride;
-    tmp.params += b0;
-    return &tmp;
-  };
-  OzPred t0{};
-  if (G <= 1) return trsm_right_lt_stream(ctx, ctx->stream, X, L, W, wstride, batch, oz_at(0, t0));
-  cudaError_t e;
-  if ((e = cudaEventRecord(ctx->ev_fork, ctx->stream)) != cudaSuccess) return e;
-  for (int gi = 0; gi < G; ++gi) {
-    const int b0 = (int)((int64_t)batch * gi / G), b1 = (int)((int64_t)batch * (gi + 1) / G);
-    cudaStream_t st = ctx->gstream[gi];
-    if ((e = cudaStreamWaitEvent(st, ctx->ev_fork, 0)) != cudaSuccess) return e;
-    TiledRect Xg{X.base + (size_t)b0 * X.batch_stride, X.ntr, X.ntc, X.batch_stride};
-    TiledSym Lg{L.base + (size_t)b0 * L.batch_stride, L.nt, L.batch_stride};
-    OzPred tg{};
-    if ((e = trsm_right_lt_stream(ctx, st, Xg, Lg, W + (size_t)b0 * wstride, wstride, b1 - b0, oz_at(b0, tg))) != cudaSuccess) return e;
-    if ((e = cudaEventRecord(ctx->ev_join[gi], st)) != cudaSuccess) return e;
-    if ((e = cudaStreamWaitEvent(ctx->stream, ctx->ev_join[gi], 0)) != cudaSuccess) return e;
-  }
-  return cudaSuccess;
+  const int G = ctx->ngroups < batch ? ctx->ngroups : batch;
+  return for_latent_groups(ctx, batch, G, [&](cudaStream_t st, int b0, int b1) {
+    const TiledRect Xg{X.base + (size_t)b0 * X.batch_stride, X.ntr, X.ntc, X.batch_stride};
+    TiledSym Lg = L;
+    Lg.base += (size_t)b0 * L.batch_stride;
+    const OzPred ozg = use_oz ? oz.at(b0) : OzPred{};
+    return trsm_right_lt_stream(ctx, st, Xg, Lg, W + (size_t)b0 * wstride, wstride, b1 - b0, use_oz ? &ozg : nullptr);
+  });
 }
 
 // X <- X L^{-T} for an upper-triangular X given as full rectangular tiles (zero tiles skipped).

@@ -70,16 +70,30 @@ enum { GEMM_UPDATE = 0, GEMM_TRSM = 1 };
 cudaError_t launch_gemm(cudaStream_t st, int mode, const GemmArgs& a, int ncols, int nrows, int batch, long long select_tiles = 0);
 void set_gemm_small_threshold(int tiles);  // grids of <= tiles tiles use the latency-optimised direct kernel (default 74; 0 = off)
 bool gemm_takes_direct(long long tiles);  // a grid of that many tiles takes the direct kernel (launch_gemm's choice)
-// Digit planes written by the panel TRSM of the int8 Cholesky: the finished tiles (I, J) with I >= i0 are sliced as launch_ozaki_slice
-// slices them (same digits, first-plane bytes, planes skipped for all-zero tiles)
-struct TrsmSliceArgs {
+// Int8 digit-plane workspace of a batch of tiled matrices (ozaki.cu): S planes of `bits`-bit digits per tile and the row scales they
+// are taken against.  scale is const as the kernels read it; launch_ozaki_*scales fill it.
+struct DigitPlanes {
   const double* scale;  // [batch][scale_stride]: row scales 2^(E - 6)
   size_t scale_stride;
-  uint8_t* slices;      // [batch][slice_stride] bytes, packed-lower tile order, S * 16 KB per tile
+  uint8_t* slices;      // [batch][slice_stride] bytes, S * 16 KB per tile (packed-lower tile order for a factor)
   size_t slice_stride;
-  uint8_t* fp;          // nullable: first plane with a nonzero digit per tile [batch][fp_stride]
+  uint8_t* fp;          // nullable: first plane with a nonzero digit per tile [batch][fp_stride] (packed-lower factor only)
   size_t fp_stride;
-  int S, bits, i0;
+  int S, bits;          // digit planes, bits per digit (7: radix 128, 8: radix 256)
+  // the workspace of the latents [b0, ...)
+  DigitPlanes at(int b0) const {
+    DigitPlanes p = *this;
+    p.scale += (size_t)b0 * scale_stride;
+    p.slices += (size_t)b0 * slice_stride;
+    if (fp) p.fp += (size_t)b0 * fp_stride;
+    return p;
+  }
+};
+// Digit planes written by the panel TRSM of the int8 Cholesky: the finished tiles (I, J) with I >= i0 are sliced as launch_ozaki_slice
+// slices them (same digits, first-plane bytes, planes skipped for all-zero tiles).  A by-value kernel parameter: the layout is the
+// DigitPlanes fields followed by i0.
+struct TrsmSliceArgs : DigitPlanes {
+  int i0;
 };
 // TRSM of column a.j0, tile rows [a.i0, a.i0 + nrows), on the TMA-pipelined kernel whatever the grid size, with the digit planes
 cudaError_t launch_trsm_slice(cudaStream_t st, const GemmArgs& a, int nrows, int batch, const TrsmSliceArgs& s);
@@ -134,28 +148,24 @@ cudaError_t launch_rhs_row_extract(cudaStream_t st, TiledSym L, int I, int s0, i
 // ---- ozaki.cu : integer-slice (Ozaki) FP64 trailing update on the int8 tensor cores (tcgen05 / TMEM); optional
 // scale[b][row] = 2^(E_row - 6) from the diagonal of the matrix about to be factored (2^E > sqrt(A_ii))
 cudaError_t launch_ozaki_scales(cudaStream_t st, TiledSym L, int batch, double* scale, size_t scale_batch_stride);
-// slice the finished tiles (I, k), I in [i0, i0 + nrows), k in [k0, k0 + ncols), into S int8 digit planes (S * 16 KB per tile)
+// slice the finished tiles (I, k), I in [i0, i0 + nrows), k in [k0, k0 + ncols), into the digit planes p
 // env (nullable, [batch][L.nt]): tiles with k < env[b][I] are zero, are never read, and are not sliced
-// first_plane (nullable, [batch][fp_stride], packed-lower tile order): per sliced tile the first plane with a nonzero digit, S when
-// every digit is zero (such a tile's planes are then not written)
-cudaError_t launch_ozaki_slice(cudaStream_t st, TiledSym L, const double* scale, size_t scale_batch_stride, uint8_t* slices,
-                               size_t slice_batch_stride, int i0, int nrows, int k0, int ncols, int batch, int S, int bits,
-                               const int* env = nullptr, uint8_t* first_plane = nullptr, size_t fp_stride = 0);
-// C(I,J) -= sum_{k < k1} L(I,k) L(J,k)' for I in [i0, i0 + nrows), J in [j0, j0 + ncols), I >= J, from the sliced factor;
+// p.fp (nullable): per sliced tile the first plane with a nonzero digit, S when every digit is zero (such a tile's planes are then
+// not written)
+cudaError_t launch_ozaki_slice(cudaStream_t st, TiledSym L, const DigitPlanes& p, int i0, int nrows, int k0, int ncols, int batch,
+                               const int* env = nullptr);
+// C(I,J) -= sum_{k < k1} L(I,k) L(J,k)' for I in [i0, i0 + nrows), J in [j0, j0 + ncols), I >= J, from the sliced factor p;
 // env (nullable, [batch][L.nt]): the k range of tile (I, J) starts at max(env[b][I], env[b][J]);
-// first_plane (nullable, as written by launch_ozaki_slice): k-tiles whose digit products are all exactly zero are skipped
-cudaError_t launch_ozaki_update(cudaStream_t st, TiledSym L, const uint8_t* slices, size_t slice_batch_stride, const double* scale,
-                                size_t scale_batch_stride, int i0, int nrows, int j0, int ncols, int k1, int batch, int S, int bits,
-                                const int* env = nullptr, const uint8_t* first_plane = nullptr, size_t fp_stride = 0);
+// p.fp (nullable, as written by launch_ozaki_slice): k-tiles whose digit products are all exactly zero are skipped
+cudaError_t launch_ozaki_update(cudaStream_t st, TiledSym L, const DigitPlanes& p, int i0, int nrows, int j0, int ncols, int k1, int batch,
+                                const int* env = nullptr);
 // the prediction sweep X <- X L^{-T} on the same path: row scales of a FINISHED factor (row 2-norms) and of X (prior variance bound),
 // digit planes of rectangular tiles, wide update with the left operand from the sliced X
 cudaError_t launch_ozaki_factor_scales(cudaStream_t st, TiledSym L, int batch, double* scale, size_t scale_batch_stride);
 cudaError_t launch_ozaki_const_scales(cudaStream_t st, const LatentParams* params, int ntr, int batch, double* scale, size_t scale_batch_stride);
-cudaError_t launch_ozaki_slice_rect(cudaStream_t st, TiledRect X, const double* scale, size_t scale_batch_stride, uint8_t* slices,
-                                    size_t slice_batch_stride, int k0, int ncols, int batch, int S, int bits);
-cudaError_t launch_ozaki_update_rect(cudaStream_t st, TiledRect X, const uint8_t* xslices, size_t xslice_batch_stride, const double* xscale,
-                                     size_t xscale_stride, const uint8_t* lslices, size_t lslice_batch_stride, const double* lscale,
-                                     size_t lscale_stride, int j0, int ncols, int k1, int batch, int S, int bits);
+cudaError_t launch_ozaki_slice_rect(cudaStream_t st, TiledRect X, const DigitPlanes& xp, int k0, int ncols, int batch);
+cudaError_t launch_ozaki_update_rect(cudaStream_t st, TiledRect X, const DigitPlanes& xp, const DigitPlanes& lp, int j0, int ncols, int k1,
+                                     int batch);
 
 // ---- proj.cu
 // Ty[i][n] = sum_j T[i + lat0][j] Y[j][n] - mean_i  (i < mloc), written to ty[i*ty_stride + n], zero padding to ty_stride

@@ -464,20 +464,18 @@ cudaError_t launch_ozaki_scales(cudaStream_t st, TiledSym L, int batch, double* 
   ozaki_scale_kernel<<<dim3((unsigned)L.nt, (unsigned)batch), 128, 0, st>>>(L, scale, scale_batch_stride);
   return cudaGetLastError();
 }
-cudaError_t launch_ozaki_slice(cudaStream_t st, TiledSym L, const double* scale, size_t scale_batch_stride, uint8_t* slices,
-                               size_t slice_batch_stride, int i0, int nrows, int k0, int ncols, int batch, int S, int bits, const int* env,
-                               uint8_t* first_plane, size_t fp_stride) {
+cudaError_t launch_ozaki_slice(cudaStream_t st, TiledSym L, const DigitPlanes& p, int i0, int nrows, int k0, int ncols, int batch,
+                               const int* env) {
   if (nrows <= 0 || ncols <= 0 || batch <= 0) return cudaSuccess;
-  ozaki_slice_kernel<<<dim3((unsigned)ncols, (unsigned)nrows, (unsigned)batch), 256, 0, st>>>(operand(L), scale, scale_batch_stride, slices,
-                                                                                            slice_batch_stride, i0, k0, S, bits, 0, env, L.nt,
-                                                                                            first_plane, fp_stride);
+  ozaki_slice_kernel<<<dim3((unsigned)ncols, (unsigned)nrows, (unsigned)batch), 256, 0, st>>>(operand(L), p.scale, p.scale_stride, p.slices,
+                                                                                            p.slice_stride, i0, k0, p.S, p.bits, 0, env, L.nt,
+                                                                                            p.fp, p.fp_stride);
   return cudaGetLastError();
 }
-cudaError_t launch_ozaki_slice_rect(cudaStream_t st, TiledRect X, const double* scale, size_t scale_batch_stride, uint8_t* slices,
-                                    size_t slice_batch_stride, int k0, int ncols, int batch, int S, int bits) {
+cudaError_t launch_ozaki_slice_rect(cudaStream_t st, TiledRect X, const DigitPlanes& xp, int k0, int ncols, int batch) {
   if (X.ntr <= 0 || ncols <= 0 || batch <= 0) return cudaSuccess;
-  ozaki_slice_kernel<<<dim3((unsigned)ncols, (unsigned)X.ntr, (unsigned)batch), 256, 0, st>>>(operand(X), scale, scale_batch_stride, slices,
-                                                                                             slice_batch_stride, 0, k0, S, bits, X.ntc, nullptr, 0,
+  ozaki_slice_kernel<<<dim3((unsigned)ncols, (unsigned)X.ntr, (unsigned)batch), 256, 0, st>>>(operand(X), xp.scale, xp.scale_stride, xp.slices,
+                                                                                             xp.slice_stride, 0, k0, xp.S, xp.bits, X.ntc, nullptr, 0,
                                                                                              nullptr, 0);
   return cudaGetLastError();
 }
@@ -531,26 +529,24 @@ static cudaError_t oz_launch(cudaStream_t st, dim3 grid, const OzakiArgs& a) {
 }
 cudaError_t oz_dispatch(cudaStream_t st, dim3 grid, const OzakiArgs& a, int S, int bits);
 
-cudaError_t launch_ozaki_update(cudaStream_t st, TiledSym L, const uint8_t* slices, size_t slice_batch_stride, const double* scale,
-                                size_t scale_batch_stride, int i0, int nrows, int j0, int ncols, int k1, int batch, int S, int bits,
-                                const int* env, const uint8_t* first_plane, size_t fp_stride) {
+cudaError_t launch_ozaki_update(cudaStream_t st, TiledSym L, const DigitPlanes& p, int i0, int nrows, int j0, int ncols, int k1, int batch,
+                                const int* env) {
   if (nrows <= 0 || ncols <= 0 || batch <= 0 || k1 <= 0) return cudaSuccess;
-  if (k1 > 32 * OZ_KMASK_WORDS) first_plane = nullptr;  // the member masks cover at most this many k-tiles
-  OzakiArgs a{slices, slice_batch_stride, scale, scale_batch_stride, operand(L), i0, j0, k1, S, nullptr, 0, 0, nullptr, 0, env, L.nt,
-              first_plane, fp_stride};
+  const uint8_t* first_plane = k1 > 32 * OZ_KMASK_WORDS ? nullptr : p.fp;  // the member masks cover at most this many k-tiles
+  OzakiArgs a{p.slices, p.slice_stride, p.scale, p.scale_stride, operand(L), i0, j0, k1, p.S, nullptr, 0, 0, nullptr, 0, env, L.nt,
+              first_plane, p.fp_stride};
   const dim3 grid((unsigned)ncols, (unsigned)nrows, (unsigned)batch);
-  return oz_dispatch(st, grid, a, S, bits);
+  return oz_dispatch(st, grid, a, p.S, p.bits);
 }
 // X(R, J) -= sum_{k < k1} X(R,k) L(J,k)' for all tile rows R of the rectangular X and J in [j0, j0 + ncols): the wide update of the
-// prediction sweep X <- X L^{-T}, left operand from the sliced finished columns of X, right operand from the sliced factor.
-cudaError_t launch_ozaki_update_rect(cudaStream_t st, TiledRect X, const uint8_t* xslices, size_t xslice_batch_stride, const double* xscale,
-                                     size_t xscale_stride, const uint8_t* lslices, size_t lslice_batch_stride, const double* lscale,
-                                     size_t lscale_stride, int j0, int ncols, int k1, int batch, int S, int bits) {
+// prediction sweep X <- X L^{-T}, left operand from the sliced finished columns of X (xp), right operand from the sliced factor (lp).
+cudaError_t launch_ozaki_update_rect(cudaStream_t st, TiledRect X, const DigitPlanes& xp, const DigitPlanes& lp, int j0, int ncols, int k1,
+                                     int batch) {
   if (X.ntr <= 0 || ncols <= 0 || batch <= 0 || k1 <= 0) return cudaSuccess;
-  OzakiArgs a{lslices, lslice_batch_stride, lscale, lscale_stride, operand(X), 0, j0, k1, S, xslices, xslice_batch_stride, X.ntc, xscale, xscale_stride,
-              nullptr, 0, nullptr, 0};
+  OzakiArgs a{lp.slices, lp.slice_stride, lp.scale, lp.scale_stride, operand(X), 0, j0, k1, lp.S, xp.slices, xp.slice_stride, X.ntc, xp.scale,
+              xp.scale_stride, nullptr, 0, nullptr, 0};
   const dim3 grid((unsigned)ncols, (unsigned)X.ntr, (unsigned)batch);
-  return oz_dispatch(st, grid, a, S, bits);
+  return oz_dispatch(st, grid, a, lp.S, lp.bits);
 }
 cudaError_t oz_dispatch(cudaStream_t st, dim3 grid, const OzakiArgs& a, int S, int bits) {
   if (bits == 8) {

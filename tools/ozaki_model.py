@@ -66,7 +66,7 @@ def product(pa, sa, pb, sb, bits):
 
 
 def int32_bound_ok(K, S, bits):
-    """the host's check (chol_factor_stream): pairs per accumulator <= S, each product <= (largest digit)^2."""
+    """the host's check (host_chol.cu: ozaki_wide): pairs per accumulator <= S, each product <= (largest digit)^2."""
     return K * S * (16384 if bits == 8 else 4096) < 2 ** 31
 
 
