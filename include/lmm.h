@@ -109,6 +109,9 @@ const char* lmm_version(void);
  *   "kmat_skip"       OILMM / IndependentMOGP logpdf and posterior: 1 = build only the kernel-matrix tiles that are not provably
  *                     exact zeros (far-apart point tiles of the SE / Matern kernels) [default]; a kept posterior writes those
  *                     zeros on its first read.  0 = build every tile.  The results are the same bits either way.
+ *   "vfe_chunk"       VFE bound and posterior (lmm_*_vfe*): tile rows (128 training points each) of K(x, z) formed per chunk;
+ *                     0 = as many as fit in device memory [default].  The chunks' Gram sums are added in chunk order, so a
+ *                     different chunking changes the result in the last bits only.
  *   "chain_fused"     1 = where the grids are small (batches <= 2, or few latents x few tile rows) the panel chain of a tile
  *                     column -- TRSM of the column, update of the next column(s), factorisation of the next diagonal tile --
  *                     is ONE launch whose CTAs hand tiles to each other through ready counters in global memory, the
@@ -276,6 +279,38 @@ int lmm_imogp_loo(lmm_ctx* ctx, const lmm_gp_desc* fs, int m, const double* x, i
                   const double* y, int out_dim, double* out_loo, double* loo_mean, double* loo_var,
                   double* grad_latents, double* grad_ard, double* grad_sigma2, double* grad_y, double* grad_terms,
                   int* info_latent);
+
+/* Sparse variational inference (Titsias' collapsed VFE bound; AbstractGPs `elbo(VFE(f(z)), fx, y)` / `posterior(VFE(f(z)), fx, y)`)
+ * with M inducing inputs z (D x M column-major, like x) shared by every latent, u_l = f_l(z), and Kz = K_l(z, z) + jitter I.
+ * out_elbo = Σ_l ELBO_l(ỹ_l = (T y)_l; ν_l = σ²/S_l) + the regulariser lmm_oilmm_logpdf adds (IndependentMOGP: ν = σ², none), where
+ *   ELBO_l = log N(ỹ_l; μ_l, Q_l + ν_l I) - tr(K_l - Q_l) / (2 ν_l),   Q_l = K_l(x, z) Kz⁻¹ K_l(z, x)
+ * is a lower bound of the exact logpdf, equal to it for z = x with jitter 0.  Cost per latent about 2 M² N flop and O(M² + M N_c)
+ * memory: the training points are streamed in chunks of N_c (option "vfe_chunk"); nothing N x N is formed.  Limits: M >= 1,
+ * scalar σ² > 0, jitter >= 0, inputs by outputs, fully observed y (a NaN returns LMM_E_ARG), m <= p.  A failed factorisation of Kz
+ * (e.g. duplicate inducing inputs with jitter 0) or of I + Ψ/ν returns its pivot with info_latent, as lmm_oilmm_logpdf does.
+ * The gradient outputs (z and the jitter held fixed) use the layouts of lmm_oilmm_loo / lmm_oilmm_logpdf_grad_terms: grad_latents
+ * m x 3 (term 0's variance and inv_lengthscale, mean_const), grad_ard m x D, grad_terms m x LMM_MAX_TERMS x LMM_GRAD_TERM_STRIDE,
+ * grad_sigma2, grad_y (p*N by outputs), grad_U (p x m column-major) / grad_S (m) the Euclidean gradient.  With every gradient
+ * pointer NULL only the value path runs; the gradient re-forms B' chunk by chunk in a second pass (about twice the value's cost).
+ * Every output is nullable. */
+int lmm_oilmm_vfe(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D, const double* z, int M,
+                  double jitter, const double* U, const double* S, int p, double sigma2, const double* y, int out_dim,
+                  double* out_elbo, double* grad_latents, double* grad_ard, double* grad_sigma2, double* grad_y,
+                  double* grad_U, double* grad_S, double* grad_terms, int* info_latent);
+int lmm_imogp_vfe(lmm_ctx* ctx, const lmm_gp_desc* fs, int m, const double* x, int N, int D, const double* z, int M,
+                  double jitter, double sigma2, const double* y, int out_dim, double* out_elbo, double* grad_latents,
+                  double* grad_ard, double* grad_sigma2, double* grad_y, double* grad_terms, int* info_latent);
+/* The bound's optimal approximate posterior q(f_l) (Titsias 2009), as a handle: at x*, with V = K(x*, z) Lz^{-T} and
+ * Σ_l = I + Lz⁻¹ K(z, x) K(x, z) Lz^{-T} / ν_l, latent mean μ_l + V Σ_l⁻¹ Lz⁻¹ K(z, x) δ_l / ν_l and variance
+ * k(x*, x*) - |V|²_rows + |V Σ_l^{-1/2}|²_rows, mixed and noised like the exact posterior's.  The handle answers
+ * lmm_post_mean_and_var, lmm_post_latent_mean_and_var, lmm_post_info (its N is M) and lmm_post_free; every other lmm_post_*
+ * call returns LMM_E_UNSUPPORTED and leaves it usable.  out_post required, out_elbo / info_latent nullable. */
+int lmm_oilmm_vfe_posterior(lmm_ctx* ctx, const lmm_gp_desc* latents, int m, const double* x, int N, int D, const double* z,
+                            int M, double jitter, const double* U, const double* S, int p, double sigma2, const double* y,
+                            int out_dim, lmm_post** out_post, double* out_elbo, int* info_latent);
+int lmm_imogp_vfe_posterior(lmm_ctx* ctx, const lmm_gp_desc* fs, int m, const double* x, int N, int D, const double* z, int M,
+                            double jitter, double sigma2, const double* y, int out_dim, lmm_post** out_post,
+                            double* out_elbo, int* info_latent);
 
 /* ---- posterior handle: the OILMM/ILMM/IndependentMOGP whose latents are PosteriorGPs -------- */
 /* mean_and_var(post(x*, σ²))  src/oilmm.jl:57-76 on PosteriorGP latents (AbstractGPs posterior

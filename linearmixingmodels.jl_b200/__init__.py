@@ -25,6 +25,9 @@ from .api import (  # noqa: F401
     loo_logpdf,
     loo_mean_and_var,
     loo_logpdf_and_gradient,
+    VFE,
+    elbo,
+    elbo_and_gradient,
 )
 from . import _lib, api, dist  # noqa: F401
 

@@ -89,6 +89,12 @@ SIGNATURES = {
     # leave-one-input-out: value, LOO mean, LOO var, latents, ard, σ², y, U, S, terms, info
     "lmm_oilmm_loo": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, _vp, C.c_int, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _vp, _vp, _dp, _vp, _vp, _vp, _vp, _ip]),
     "lmm_imogp_loo": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _vp, _vp, _dp, _vp, _vp, _ip]),
+    # sparse variational bound: inducing inputs z, M, jitter before the model arguments; (posterior handle,) value, info
+    # value, latents, ard, σ², y, (U, S,) terms, info
+    "lmm_oilmm_vfe": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, C.c_int, C.c_double, _vp, _vp, C.c_int, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _dp, _vp, _vp, _vp, _vp, _ip]),
+    "lmm_imogp_vfe": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, C.c_int, C.c_double, C.c_double, _vp, C.c_int, _dp, _vp, _vp, _dp, _vp, _vp, _ip]),
+    "lmm_oilmm_vfe_posterior": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, C.c_int, C.c_double, _vp, _vp, C.c_int, C.c_double, _vp, C.c_int, C.POINTER(_vp), _dp, _ip]),
+    "lmm_imogp_vfe_posterior": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_int, C.c_int, _vp, C.c_int, C.c_double, C.c_double, _vp, C.c_int, C.POINTER(_vp), _dp, _ip]),
     "lmm_post_mean_and_var": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp]),
     "lmm_post_latent_mean_and_var": (C.c_int, [_vp, C.c_int, _vp, C.c_int, C.c_double, _vp, _vp]),
     "lmm_post_mean_and_cov": (C.c_int, [_vp, _vp, C.c_int, C.c_double, _vp, _vp]),

@@ -726,7 +726,10 @@ def set_ilmm_form(form: int) -> None:
 
 def posterior(fx: FiniteGP, y, with_logpdf: bool = False):
     """`posterior(fx, y)`: src/oilmm.jl:116-134, src/ilmm.jl:184-198, src/independent_mogp.jl:119-126.
-    `with_logpdf=True` additionally returns logpdf(fx, y) from the same factorisation."""
+    `with_logpdf=True` additionally returns logpdf(fx, y) from the same factorisation.
+    `posterior(VFE(z), fx, y)` is the sparse variational posterior (see `VFE`)."""
+    if isinstance(fx, VFE):
+        return _vfe_call(fx, y, with_logpdf, want_post=True)[1]
     f = fx.f
     ctx = _ctx_of(fx)
     lib = ctx.lib
@@ -1263,6 +1266,110 @@ def loo_logpdf_and_gradient(fx: FiniteGP, y, with_grad_y: bool = False):
     TypeError; a NaN in y raises ValueError."""
     v, _, _, g = _loo_call(fx, y, True, False, True, with_grad_y)
     return v, g
+
+
+class VFE:
+    """AbstractGPs `VFE(f(z))`: Titsias' sparse variational approximation with the inducing inputs z (a vector, ColVecs or
+    RowVecs, like x) shared by every latent, u_l = f_l(z), and `jitter` added to K(z, z) (the default noise of `f(z)`).
+    `elbo(VFE(z), fx, y)` is the collapsed bound -- a lower bound of `logpdf(fx, y)`, equal to it for z = x and jitter 0 --
+    and `posterior(VFE(z), fx, y)` its optimal approximate posterior, whose `mean_and_var` / `marginals` / `mean` / `var`
+    work (cov, rand, conditioning, saving and export raise).  Built for OILMM and IndependentMOGP priors under scalar noise
+    with by-outputs inputs and fully observed y; the cost per latent is about 2 M² N flop, and no N x N matrix is formed."""
+
+    def __init__(self, z, jitter: float = 1e-18):
+        self.z, self.jitter = z, float(jitter)
+
+
+def _vfe_call(approx: VFE, fx: FiniteGP, y, want_post: bool, grads: bool = False, with_grad_y: bool = False):
+    """One lmm_*_vfe / lmm_*_vfe_posterior call: (elbo, posterior or gradient dict or None)."""
+    if not isinstance(fx, FiniteGP):
+        raise TypeError("VFE needs a FiniteGP fx = f(x, σ²)")
+    if isinstance(fx.f, ILMM) and not isinstance(fx.f.H, Orthogonal):
+        raise TypeError("VFE is built for OILMM and IndependentMOGP priors (not a general ILMM)")
+    if not isinstance(fx.f, (ILMM, IndependentMOGP)):
+        raise TypeError("VFE is built for OILMM and IndependentMOGP priors")
+    if fx.noise is not None:
+        raise TypeError("VFE needs scalar observation noise")
+    _require_by_outputs(fx)
+    if _post_owner(fx) is not None:
+        raise TypeError("VFE is built for prior FiniteGPs, not posteriors")
+    f = fx.f
+    lat = f.f if isinstance(f, ILMM) else f
+    if not isinstance(lat, IndependentMOGP):
+        raise TypeError("ILMM latents must be an IndependentMOGP")
+    if isinstance(f, ILMM) and f.H.shape[0] != fx.x.out_dim:
+        raise RuntimeError("out dim of x != out dim of f.")
+    ctx = _ctx_of(fx)
+    pts = _points(fx.x.x)
+    zp = _points(approx.z)
+    N, D = int(pts.shape[0]), int(pts.shape[1])
+    M = int(zp.shape[0])
+    if int(zp.shape[1]) != D:
+        raise ValueError("the inducing inputs z and the inputs x have different dimensions")
+    p = fx.x.out_dim
+    m = len(lat.fs)
+    yv = _yvec(y, N * p)
+    if not _is_device_tensor(yv) and np.isnan(yv).any():
+        raise ValueError("y has a NaN entry: the VFE bound needs fully observed data")
+    out, gs2, il, h = C.c_double(), C.c_double(), C.c_int(-1), C.c_void_p()
+    lib = ctx.lib
+    orth = isinstance(f, ILMM)
+    gl = np.zeros((m, 3)) if grads else None
+    ga = np.zeros((m, D)) if grads else None
+    gt = np.zeros(m * _lib.LMM_MAX_TERMS * _lib.LMM_GRAD_TERM_STRIDE) if grads else None
+    gy = np.zeros(p * N) if grads and with_grad_y else None
+    gs2p = C.byref(gs2) if grads else None
+    gU = np.zeros(f.H.shape, order="F") if orth and grads else None
+    gS = np.zeros(m) if orth and grads else None
+    if orth:
+        H = f.H
+        if want_post:
+            rc = lib.lmm_oilmm_vfe_posterior(ctx.handle, _descs(lat.fs), m, ptr(pts), N, D, ptr(zp), M, approx.jitter, ptr(H.U), ptr(H.S),
+                                             H.shape[0], fx.sigma2, ptr(yv), p, C.byref(h), C.byref(out), C.byref(il))
+        else:
+            rc = lib.lmm_oilmm_vfe(ctx.handle, _descs(lat.fs), m, ptr(pts), N, D, ptr(zp), M, approx.jitter, ptr(H.U), ptr(H.S), H.shape[0],
+                                   fx.sigma2, ptr(yv), p, C.byref(out), ptr(gl), ptr(ga), gs2p, ptr(gy), ptr(gU), ptr(gS), ptr(gt),
+                                   C.byref(il))
+    else:
+        if want_post:
+            rc = lib.lmm_imogp_vfe_posterior(ctx.handle, _descs(lat.fs), m, ptr(pts), N, D, ptr(zp), M, approx.jitter, fx.sigma2, ptr(yv), p,
+                                             C.byref(h), C.byref(out), C.byref(il))
+        else:
+            rc = lib.lmm_imogp_vfe(ctx.handle, _descs(lat.fs), m, ptr(pts), N, D, ptr(zp), M, approx.jitter, fx.sigma2, ptr(yv), p,
+                                   C.byref(out), ptr(gl), ptr(ga), gs2p, ptr(gy), ptr(gt), C.byref(il))
+    ctx.check(rc, il.value)
+    if grads:
+        g = {"terms": _terms_grads(lat.fs, gt, D), "variance": gl[:, 0].copy(), "inv_lengthscale": gl[:, 1].copy(), "ard": ga,
+             "mean_const": gl[:, 2].copy(), "sigma2": gs2.value}
+        if with_grad_y:
+            g["y"] = gy
+        if orth:
+            g["U"], g["S"] = np.ascontiguousarray(gU), gS
+        return out.value, g
+    if not want_post:
+        return out.value, None
+    owner = _PostHandle(ctx, h, M)
+    newlat = IndependentMOGP([PosteriorGP(owner, i, g) for i, g in enumerate(lat.fs)])
+    return out.value, (ILMM(newlat, f.H) if isinstance(f, ILMM) else newlat)
+
+
+def elbo(approx: VFE, fx: FiniteGP, y) -> float:
+    """AbstractGPs `elbo(VFE(f(z)), fx, y)`: Titsias' collapsed variational lower bound of `logpdf(fx, y)` for an OILMM or
+    IndependentMOGP prior (see `VFE`).  General ILMMs, posteriors, by-features inputs and non-scalar noise raise TypeError;
+    a NaN in y raises ValueError."""
+    if not isinstance(approx, VFE):
+        raise TypeError("elbo(VFE(z), fx, y)")
+    return _vfe_call(approx, fx, y, want_post=False)[0]
+
+
+def elbo_and_gradient(approx: VFE, fx: FiniteGP, y, with_grad_y: bool = False):
+    """Value and gradient of `elbo(VFE(z), fx, y)` with z and the jitter held fixed.  grads has the keys of
+    `loo_logpdf_and_gradient`: "terms" (per latent, per term: {"variance", "inv_lengthscale", "param", "ard"}), "variance" /
+    "inv_lengthscale" / "ard" (term 0's), "mean_const", "sigma2"[, "y" (p*N,)], and for an OILMM "U" (p, m) and "S" (m,), the
+    Euclidean gradient.  Refusals as `elbo`."""
+    if not isinstance(approx, VFE):
+        raise TypeError("elbo_and_gradient(VFE(z), fx, y)")
+    return _vfe_call(approx, fx, y, want_post=False, grads=True, with_grad_y=with_grad_y)
 
 
 def logpdf_sweep(fx: FiniteGP, y, inv_lengthscale_scales) -> np.ndarray:

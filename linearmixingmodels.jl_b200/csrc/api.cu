@@ -235,6 +235,9 @@ extern "C" int lmm_ctx_set_option(lmm_ctx* ctx, const char* key, double value) {
   } else if (k == "kmat_skip") {
     if (value != 0.0 && value != 1.0) return ctx->fail(LMM_E_ARG, "kmat_skip must be 0 (build every kernel-matrix tile) or 1");
     ctx->kmat_skip = (int)value;
+  } else if (k == "vfe_chunk") {
+    if (value < 0 || value > 1e6 || value != (double)(int)value) return ctx->fail(LMM_E_ARG, "vfe_chunk must be a whole number of tile rows >= 0 (0 = by memory)");
+    ctx->vfe_chunk = (int)value;
   } else if (k == "chain_fused") {
     if (value != 0.0 && value != 1.0 && value != 2.0) return ctx->fail(LMM_E_ARG, "chain_fused must be 0, 1 (where it pays off) or 2 (everywhere)");
     ctx->chain_fused = (int)value;

@@ -244,6 +244,18 @@ __device__ __forceinline__ double kernel_value_raw(const LatentParams* gp, const
 // true if the latent needs the raw-point path (composite, or a kernel whose metric is not (Sq)Euclidean)
 __device__ __forceinline__ bool needs_raw_points(const LatentParams* gp) { return gp->nterms > 1 || gp->kind == 5; }
 
+// Fixed-order sum over the 256 threads of a CTA (the result is valid in thread 0).
+__device__ __forceinline__ double cta_sum256(double v, double* red) {
+  const int t = threadIdx.x;
+  red[t] = v;
+  __syncthreads();
+  for (int w = 128; w > 0; w >>= 1) {
+    if (t < w) red[t] += red[t + w];
+    __syncthreads();
+  }
+  return red[0];
+}
+
 // Programmatic dependent launch (the panel chain of a batch-1 factorisation is three dependent small kernels per tile
 // column): a kernel launched with launch_pdl() may be scheduled as soon as its predecessor in the stream executes
 // pdl_trigger(); it must execute pdl_wait() before touching anything the predecessor wrote (pdl_wait returns when the

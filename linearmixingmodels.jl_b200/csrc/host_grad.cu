@@ -18,6 +18,7 @@ extern "C" int lmm_post_condition(lmm_post* post, const double* xs, int Ns, doub
   *out_post = nullptr;
   lmm_ctx* ctx = post->ctx;
   std::lock_guard<std::mutex> lk(ctx->mu);
+  if (post->kind == POST_VFE) return ctx->fail(LMM_E_UNSUPPORTED, VFE_POST_ONLY);
   CU(cudaSetDevice(ctx->device));
   if (int rcz = post_fill_zeros(post)) return rcz;  // the factor is read below
   if (post->kind == POST_MASKED) return ctx->fail(LMM_E_UNSUPPORTED, "a missing-data posterior offers mean_and_var only");

@@ -7,6 +7,7 @@
 //   host_ilmm.cu     general-ILMM joint factor: logpdf, posterior, marginals, covariances, conditioning, dense-noise IMOGP
 //   host_grad.cu     rrule of logpdf (OILMM, IndependentMOGP, general ILMM), sequential conditioning, cross-covariance
 //   host_io.cu       serialisable posteriors, generic MVN logpdf / rand
+//   host_vfe.cu      sparse variational (VFE) bound and posterior of an OILMM / IndependentMOGP
 // There is no CPU fallback anywhere on the host side: every compute entry point needs a CUDA device.
 #pragma once
 #include <cmath>
@@ -78,6 +79,7 @@ struct lmm_ctx {
   size_t chain_cnt_bytes = 0;
   // one large factor (general ILMM, batch 1) partitioned row-cyclically over the ranks of the communicator
   int partition_ilmm = 0;
+  int vfe_chunk = 0;  // VFE bound: tile rows of training points per chunk of K(x, z) (0 = as many as fit in memory)
   int kmat_skip = 1;  // OILMM / IndependentMOGP evals: build only the kernel-matrix tiles that are not provably exact zeros (kmat.cu)
   int condition_update = 1;  // sequential conditioning of per-latent posteriors: 1 = block-Cholesky update of the factor, 0 = re-factorise the union
   int partition_now = 0;  // set by the callers whose factorisation is replicated on every rank (ILMM joint factor)
@@ -188,7 +190,11 @@ struct PartitionScope {
 // POST_JOINT: IndependentMOGP conditioned under a dense Σy (AbstractGPs generic path): one joint (mN) factor like
 // POST_ILMM, identity mixing, no projection.
 // POST_MASKED: heterotopic / missing-data dense model -- one factor over the observed entries (d_obs), any mixing matrix.
-enum { POST_OILMM = 0, POST_IMOGP = 1, POST_ILMM = 2, POST_JOINT = 3, POST_MASKED = 4 };
+// POST_VFE: sparse variational (VFE) posterior of an OILMM / IndependentMOGP (host_vfe.cu) -- per latent the inducing inputs z
+// (d_xpad, N = M points), Lz = chol(K(z, z) + jitter I) (d_L / d_W), L_Σ = chol(I + Ψ/ν) (d_L2 / d_W2) and the weights
+// Lz^{-T} Σ^{-1} B δ / ν (d_alpha); vfe_oilmm selects the back-projection.  It answers mean_and_var only.
+enum { POST_OILMM = 0, POST_IMOGP = 1, POST_ILMM = 2, POST_JOINT = 3, POST_MASKED = 4, POST_VFE = 5 };
+constexpr const char* VFE_POST_ONLY = "a VFE posterior offers mean_and_var and the latent marginals only";
 
 struct lmm_post {
   lmm_ctx* ctx = nullptr;
@@ -212,6 +218,9 @@ struct lmm_post {
   double* d_noise_vec = nullptr;  // [nloc][Npad] per-point training noise (sequentially conditioned posteriors), else null
   int* d_obs = nullptr;           // POST_MASKED: observed entries j*N + i (big_n of them)
   double* d_Ept = nullptr;        // POST_ILMM: [N][m*m] per-point projected noise blocks ΣT (extended by sequential conditioning)
+  double* d_L2 = nullptr;         // POST_VFE: L_Σ per latent (TiledSym like d_L)
+  double* d_W2 = nullptr;         // POST_VFE: its inverse diagonal tiles
+  bool vfe_oilmm = false;         // POST_VFE: OILMM (back-projection by H) or IndependentMOGP
   int* d_env = nullptr;           // [nloc][nt] tile envelope of the factors (OILMM / IndependentMOGP built inside it), else null
   bool zeros_pending = false;     // the tiles (I, k < env) of d_L were never written: post_fill_zeros writes them before a read
   size_t bytes = 0;

@@ -63,6 +63,7 @@ extern "C" int lmm_post_save(lmm_post* post, const char* path) {
   if (!post || !path) return LMM_E_ARG;
   lmm_ctx* ctx = post->ctx;
   std::lock_guard<std::mutex> lk(ctx->mu);
+  if (post->kind == POST_VFE) return ctx->fail(LMM_E_UNSUPPORTED, VFE_POST_ONLY);
   CU(cudaSetDevice(ctx->device));
   if (int rcz = post_fill_zeros(post)) return rcz;  // the factor is read below
   FILE* f = fopen(path, "wb");

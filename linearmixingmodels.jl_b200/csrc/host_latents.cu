@@ -344,7 +344,7 @@ extern "C" int lmm_post_free(lmm_post* post) {
   std::lock_guard<std::mutex> lk(ctx->mu);
   cudaSetDevice(ctx->device);
   void* ptrs[] = {post->d_xpad, post->d_L, post->d_W, post->d_alpha, post->d_delta, post->d_params, post->d_H, post->d_noise_vec,
-                  post->d_Ept, post->d_obs, post->d_env};
+                  post->d_Ept, post->d_obs, post->d_env, post->d_L2, post->d_W2};
   for (void* q : ptrs)
     if (q) cudaFreeAsync(q, ctx->stream);
   cudaStreamSynchronize(ctx->stream);
@@ -368,6 +368,7 @@ extern "C" int lmm_post_export(lmm_post* post, int i, double* Lout, double* alph
   lmm_ctx* ctx = post->ctx;
   std::lock_guard<std::mutex> lk(ctx->mu);
   CU(cudaSetDevice(ctx->device));
+  if (post->kind == POST_VFE) return ctx->fail(LMM_E_UNSUPPORTED, VFE_POST_ONLY);
   if (int rcz = post_fill_zeros(post)) return rcz;  // the factor is read below
   int b, n;
   if (post->joint()) {
@@ -418,8 +419,10 @@ int post_latent_marginals(lmm_post* post, const double* d_xspad, int Ns, int nts
   const size_t per_lat = (size_t)nts * nt * TT * sizeof(double);
   int chunk = 0;
   CU(mem_fit(ctx, per_lat, nloc, &chunk));
-  DevBuf b_V;
+  const bool vfe = post->kind == POST_VFE;
+  DevBuf b_V, b_q;
   CU(b_V.alloc(ctx, (size_t)chunk * per_lat));
+  if (vfe) CU(b_q.alloc(ctx, (size_t)chunk * nspad * sizeof(double)));
   const TiledSym L = post->Lsym();
   for (int c0 = 0; c0 < nloc; c0 += chunk) {
     const int nb = (c0 + chunk <= nloc) ? chunk : nloc - c0;
@@ -434,6 +437,13 @@ int post_latent_marginals(lmm_post* post, const double* d_xspad, int Ns, int nts
     CU(trsm_right_lt(ctx, V, Lc, Wc, post->wstride(), nb, dp));  // dp: k(x*,x*) bounds the row norms (int8 path, if the option is on)
     CU(launch_rect_rowsumsq(st, V, d_VL + (size_t)c0 * nspad, nspad, dp, nb));
     ++ctx->launches;
+    if (vfe) {  // VFE: var += |V L_Σ^{-T}|²_rows, V = K(x*, z) Lz^{-T} (its rows stay bounded by k(x*, x*))
+      const TiledSym Ls{post->d_L2 + (size_t)g0 * L.batch_stride, nt, L.batch_stride};
+      CU(trsm_right_lt(ctx, V, Ls, post->d_W2 + (size_t)g0 * post->wstride(), post->wstride(), nb, dp));
+      CU(launch_rect_rowsumsq(st, V, b_q.as<double>(), nspad, nullptr, nb));
+      CU(launch_axpy(st, d_VL + (size_t)c0 * nspad, b_q.as<double>(), (size_t)nb * nspad, 1.0));
+      ctx->launches += 2;
+    }
   }
   return LMM_OK;
 }
@@ -468,7 +478,7 @@ extern "C" int lmm_post_mean_and_var(lmm_post* post, const double* xs, int Ns, d
   double* d_mean = b_mean.as<double>();
   double* d_var = d_mean + nout;
   const bool multi = ctx->comm && ctx->nranks > 1;
-  if (post->kind == POST_OILMM) {
+  if (post->kind == POST_OILMM || (post->kind == POST_VFE && post->vfe_oilmm)) {
     // M = H M_lat ; V = (H∘H)(V_lat + 1e-18) + σ²     src/oilmm.jl:61-75 (1e-18: default FiniteGP noise)
     CU(cudaMemsetAsync(d_mean, 0, 2 * nout * sizeof(double), st));
     CU(launch_backproject(st, post->d_H, p, m, post->lo, nloc, b_ML.as<double>(), b_VL.as<double>(), nspad, Ns, 1e-18, sigma2,

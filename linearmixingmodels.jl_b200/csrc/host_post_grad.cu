@@ -59,6 +59,7 @@ extern "C" int lmm_post_logpdf_grad_full(lmm_post* post, const double* xs, int N
   if (!post || !xs || Ns <= 0 || !ys) return LMM_E_ARG;
   lmm_ctx* ctx = post->ctx;
   std::lock_guard<std::mutex> lk(ctx->mu);
+  if (post->kind == POST_VFE) return ctx->fail(LMM_E_UNSUPPORTED, VFE_POST_ONLY);
   CU(cudaSetDevice(ctx->device));
   if (int rcz = post_fill_zeros(post)) return rcz;  // the factor is read below
   if (post->joint())

@@ -288,6 +288,7 @@ extern "C" int lmm_post_rand(lmm_post* post, const double* xs, int Ns, double si
   if (!post || !xs || Ns <= 0 || !z_latent || !out) return LMM_E_ARG;
   lmm_ctx* ctx = post->ctx;
   std::lock_guard<std::mutex> lk(ctx->mu);
+  if (post->kind == POST_VFE) return ctx->fail(LMM_E_UNSUPPORTED, VFE_POST_ONLY);
   CU(cudaSetDevice(ctx->device));
   if (int rcz = post_fill_zeros(post)) return rcz;  // the factor is read below
   if (post->kind != POST_IMOGP && post->kind != POST_JOINT && post->kind != POST_MASKED && !z_noise) return ctx->fail(LMM_E_ARG, "null pointer");
@@ -499,6 +500,7 @@ extern "C" int lmm_post_logpdf(lmm_post* post, const double* xs, int Ns, double 
                                int* info_latent) {
   if (!post || !xs || Ns <= 0 || !ys || !out_logpdf) return LMM_E_ARG;
   std::lock_guard<std::mutex> lk(post->ctx->mu);
+  if (post->kind == POST_VFE) return post->ctx->fail(LMM_E_UNSUPPORTED, VFE_POST_ONLY);
   return post_logpdf_impl(post, xs, Ns, sigma2, ys, out_logpdf, nullptr, nullptr, info_latent);
 }
 
@@ -506,6 +508,7 @@ extern "C" int lmm_post_logpdf_grad(lmm_post* post, const double* xs, int Ns, do
                                     double* grad_sigma2, double* grad_y, int* info_latent) {
   if (!post || !xs || Ns <= 0 || !ys) return LMM_E_ARG;
   std::lock_guard<std::mutex> lk(post->ctx->mu);
+  if (post->kind == POST_VFE) return post->ctx->fail(LMM_E_UNSUPPORTED, VFE_POST_ONLY);
   return post_logpdf_impl(post, xs, Ns, sigma2, ys, out_logpdf, grad_sigma2, grad_y, info_latent);
 }
 

@@ -269,6 +269,33 @@ cudaError_t launch_loo_grad_vectors(cudaStream_t st, TiledSym M, const double* a
 }  // namespace lmm
 
 namespace lmm {
+// ---- vfe.cu : sparse variational (VFE) bound of a batch of latent GPs with M inducing inputs (Bt = B' = K(x, z) Lz^{-T}, N x M)
+// Splits of the Gram's row range for a batch of `batch` latents with mt tile columns over chunks of ntr row tiles (sizes the scratch).
+int vfe_gram_splits(int mt, int batch, int ntr);
+// psi (+)= Bt' Bt (packed lower, mt = Bt.ntc tiles), bvec (+)= Bt' δ ([batch][mt*128]), dd (+)= δ'δ over the Bt.ntr row tiles of the
+// chunk (δ of the chunk's first row at delta + b * delta_stride); accumulate = 0 overwrites.  Every sum has a fixed order.
+// Scratch: part splits*batch*sym_tiles(mt)*TT, bpart splits*batch*mt*128, ddpart splits*batch doubles (splits = vfe_gram_splits).
+// splits (>= 1): the split of the row range, the same for every chunk of a call (the scratch is sized for it; splits beyond Bt.ntr
+// add empty ranges)
+cudaError_t launch_vfe_gram(cudaStream_t st, TiledRect Bt, const double* delta, size_t delta_stride, int batch, TiledSym psi, double* bvec,
+                            double* dd, int accumulate, int splits, double* part, double* bpart, double* ddpart);
+// sig = I + psi / ν_b (ν_b = params[b].noise), every stored tile
+cudaError_t launch_vfe_sigma(cudaStream_t st, TiledSym psi, TiledSym sig, const LatentParams* params, int batch);
+// elbo[b] = -½ [N log 2π + N log ν + logdet[b] + dd[b]/ν - |c_b|²/ν² + (N kdiag - tr psi_b)/ν];  cnu (nullable) = c / ν
+// gradient: A = ((I - Σ⁻¹) - qq')/ν and P = I - Σ⁻¹ - Ψ/ν - qq' as full mt x mt tiles from the packed negSinv = -Σ⁻¹ and psi
+// (q = Σ⁻¹b/ν), and v = w/ν
+cudaError_t launch_vfe_brackets(cudaStream_t st, TiledSym negSinv, TiledSym psi, const double* q, const double* w, const LatentParams* params,
+                                TiledRect A, TiledRect P, double* v, int batch);
+// gradient, per latent: y (= B'q on entry) <- a = (δ - B'q)/ν; out4[b*4 + {2, 3}] = {dELBO/dν, Σa}, dot[b] = a·δ;
+// gterms = gz + gx + the k(x, x) part of every term's variance slot (LMM_MAX_TERMS * LMM_GRAD_TERM_STRIDE slots per latent)
+cudaError_t launch_vfe_grad(cudaStream_t st, TiledSym negSinv, TiledSym psi, const double* q, const double* c, const double* dd,
+                            const double* delta, size_t npad, int N, const LatentParams* params, int batch, double* y, double* out4,
+                            double* dot, const double* gz, const double* gx, double* gterms);
+cudaError_t launch_vfe_terms(cudaStream_t st, TiledSym psi, const double* logdet, const double* c, const double* dd, int N,
+                             const LatentParams* params, int batch, double log2pi, double* cnu, double* elbo);
+}  // namespace lmm
+
+namespace lmm {
 cudaError_t launch_untile_rect_blockdiag(cudaStream_t st, TiledRect A, int batch, int Na, int Nb, double* dense, size_t ld);
 }  // namespace lmm
 

@@ -8,18 +8,6 @@
 
 namespace lmm {
 
-// Fixed-order sum over the 256 threads of a CTA (the result is valid in thread 0).
-__device__ __forceinline__ double cta_sum256(double v, double* red) {
-  const int t = threadIdx.x;
-  red[t] = v;
-  __syncthreads();
-  for (int w = 128; w > 0; w >>= 1) {
-    if (t < w) red[t] += red[t + w];
-    __syncthreads();
-  }
-  return red[0];
-}
-
 // grid (batch), one CTA per latent.  d_i = -negA(i,i) (negA.base != null) or dvec[b][i].  Outputs per latent b, i < npad
 // (each nullable): q, sc = sqrt(2 r) and v = q / sc (0 on padding: B = A diag(sc) gives -B B' = -2 A R A and w = B v = A q),
 // lmean = ỹ_i - q_i = δ_i + mean - q_i and lvar = 1/d_i - ν (0 on padding); loo[b] = LOO of the latent.

@@ -421,6 +421,61 @@ function ChainRulesCore.rrule(::typeof(loo_logpdf), fx::LOOFiniteGP, y::Abstract
     return out[], loo_pullback
 end
 
+# --- sparse variational bound (lmm_oilmm_vfe / lmm_imogp_vfe) ------------------------------------------------------------
+# vfe_elbo(fx, z, y; jitter) = AbstractGPs `elbo(VFE(f(z, jitter)), fx, y)` for every latent f of an OILMM / IndependentMOGP,
+# with the inducing inputs z shared by the latents (a Vector or ColVecs, like x).  Outputs left at C_NULL are not computed.
+function _vfe(fx::LOOFiniteGP, z, y::AbstractVector{<:Real}, jitter::Real; out=C_NULL, gl=C_NULL, gs2=C_NULL, gy=C_NULL, gU=C_NULL,
+              gS=C_NULL, gt=C_NULL)
+    il = Ref{Cint}(-1)
+    Z, Dz = points(z)
+    if fx.f isa OILMM
+        fs, H, σ², x = unpack(fx)
+        X, D = points(x)
+        Dz == D || throw(DimensionMismatch("z and x have different dimensions"))
+        descs, keep = gpdescs(fs.fs)
+        check(GC.@preserve keep ccall((:lmm_oilmm_vfe, liblmm), Cint,
+            (Ptr{Cvoid}, Ptr{GpDesc}, Cint, Ptr{Float64}, Cint, Cint, Ptr{Float64}, Cint, Float64, Ptr{Float64}, Ptr{Float64}, Cint,
+             Float64, Ptr{Float64}, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64},
+             Ptr{Float64}, Ptr{Float64}, Ptr{Cint}),
+            ctx(), descs, length(descs), X, length(x), D, Z, length(z), Float64(jitter), Matrix{Float64}(H.U),
+            Vector{Float64}(diag(H.S)), size(H, 1), Float64(σ²), Vector{Float64}(y), fx.x.out_dim, out, gl, C_NULL, gs2, gy, gU, gS,
+            gt, il))
+    else
+        X, D = points(fx.x.x)
+        Dz == D || throw(DimensionMismatch("z and x have different dimensions"))
+        descs, keep = gpdescs(fx.f.fs)
+        check(GC.@preserve keep ccall((:lmm_imogp_vfe, liblmm), Cint,
+            (Ptr{Cvoid}, Ptr{GpDesc}, Cint, Ptr{Float64}, Cint, Cint, Ptr{Float64}, Cint, Float64, Float64, Ptr{Float64}, Cint,
+             Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Cint}),
+            ctx(), descs, length(descs), X, length(fx.x.x), D, Z, length(z), Float64(jitter), Float64(fx.Σy[1]), Vector{Float64}(y),
+            fx.x.out_dim, out, gl, C_NULL, gs2, gy, gt, il))
+    end
+    return nothing
+end
+
+function vfe_elbo(fx::LOOFiniteGP, z, y::AbstractVector{<:Real}; jitter::Real=1e-18)
+    out = Ref{Float64}(0.0)
+    _vfe(fx, z, y, jitter; out = out)
+    return out[]
+end
+
+# The pullback gives the σ² and y tangents, as the rrule of loo_logpdf does (z and the jitter are held fixed).
+function ChainRulesCore.rrule(::typeof(vfe_elbo), fx::LOOFiniteGP, z, y::AbstractVector{<:Real}; jitter::Real=1e-18)
+    orth = fx.f isa OILMM
+    m = length((orth ? fx.f.f : fx.f).fs)
+    out = Ref{Float64}(0.0); gs2 = Ref{Float64}(0.0)
+    gl = Matrix{Float64}(undef, 3, m); gy = Vector{Float64}(undef, length(y))
+    gt = Matrix{Float64}(undef, GRAD_TERM_DOUBLES, m)
+    gU = orth ? Matrix{Float64}(undef, size(fx.f.H, 1), m) : C_NULL
+    gS = orth ? Vector{Float64}(undef, m) : C_NULL
+    _vfe(fx, z, y, jitter; out = out, gl = gl, gs2 = gs2, gy = gy, gU = gU, gS = gS, gt = gt)
+    function vfe_pullback(Δ)
+        Σy_tangent = Tangent{typeof(fx.Σy)}(; diag = Tangent{typeof(fx.Σy.diag)}(; value = Δ * gs2[]))
+        return NoTangent(), Tangent{typeof(fx)}(; Σy = Σy_tangent), NoTangent(), Δ .* gy
+    end
+    return out[], vfe_pullback
+end
+
 # --- rrule for logpdf(post(x*, σ²), y*) (test/oilmm.jl:32 `gradient(logpdf, po, y_test)`) -----------------------------
 # Through the conditioning (lmm_post_logpdf_grad_full): besides the Σy and y* tangents, the posterior's latents get a tangent
 # on their `prior` (per-term hyper-parameters gt as in the prior rrule, mapping onto the kernel structs omitted as there; the
